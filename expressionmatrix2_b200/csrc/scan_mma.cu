@@ -7,6 +7,8 @@
 // (scan_popc.cu, topk.cuh); Hamming distances are bit-exact because every partial sum is an integer
 // far below 2^31.
 //
+// The symmetric scan (scanMmaSymKernel, below) runs the same contraction on FP4 operands (kind::mxf4, f32 accumulators).
+//
 // Replaces (reference): countMismatches src/BitSet.hpp:277-288 + the findSimilarPairs4 pair loop
 // src/ExpressionMatrixLsh.cpp:218-269.  Nothing here is derived from src/Lsh.cl.
 //
@@ -614,15 +616,37 @@ scanMmaSsKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
 // Operand traffic: per tile the one-directional kernel re-reads the row block's A chunks from L2 (48 KB per
 // K-chunk and SM, ~19 TB/s at full tensor rate -- sustainable only because all CTAs stream the SAME B tile).
 // Here the B tiles of concurrently running CTAs differ (a sliding window of ~74 super blocks), so A is kept
-// RESIDENT IN SHARED MEMORY for the whole item (K x 128 B <= 128 KB) and only B streams: 32 KB per K-chunk.
+// RESIDENT IN SHARED MEMORY for the whole item and only B streams.
+//
+// Operand format: FP4.  +-1 is exact in e2m1 (+1.0 = nibble 0x2, -1.0 = 0xA), so tcgen05.mma.kind::mxf4 with every
+// UE8M0 scale factor 1.0 computes the same dot products as int8 at twice the elements per byte and per instruction
+// (K = 64); the f32 accumulator holds them exactly (|dot| <= 1024 < 2^24).  K is padded to a multiple of 256 bits (one
+// 128-byte swizzle atom), pad bits -1 in every row.  A is K/2 x 128 B <= 64 KB; a K chunk of B is 32 KB per 256 columns.
+// A tile is run as its two 128-column halves (N = 128 instructions): half h of tile t accumulates into TMEM slot
+// (2t + h) mod 3 of a three-slot ring (3 x 128 columns; the scale factors, all 0x7F, sit in the columns above), and
+// epilogue sub-stream h drains exactly the halves h.  A ring of three slots gives every sub-stream about one tile period
+// to drain its half, the slack two full-width accumulators gave -- whose 512 columns would leave none for the scales.
 // ---------------------------------------------------------------------------------------------------------
-constexpr int kSymMaxStages = 6;
+constexpr int kSymMaxStages = 20;
 constexpr uint32_t kLogChunk = 64;
-constexpr uint32_t kPaceWindow = 256;      // tiles a CTA may run ahead of the slowest one (64 MB of distinct B tiles)
-constexpr uint32_t kSymSmallBytes = 192 + 2 * kSsTileN * 2 + 2 * (kSsTileN / 8) * 2 + kEpiThreads * 2;
+constexpr uint32_t kPaceWindow = 256;      // tiles a CTA may run ahead of the slowest one (32 MB of distinct B tiles)
+constexpr uint32_t kSymBarBytes = 512;
+constexpr uint32_t kSymSmallBytes = kSymBarBytes + 2 * kSsTileN * 4 + 2 * (kSsTileN / 8) * 4 + kEpiThreads * 2;
 constexpr int kMaxInboxSources = 8;        // GPUs whose column-direction candidates a cell's merge reads
 constexpr int kSymThreads = kThreads + 32;  // + one warp that stages the column thresholds
-constexpr uint32_t kInstrDescSsPair = (kInstrDescSs & ~(0x1Fu << 24)) | (uint32_t(kPairRows >> 4) << 24);   // M = 256 over two CTAs, N = 256
+constexpr uint32_t kSymKBits = 256;         // FP4 K granularity: bits per 128-byte chunk
+constexpr uint32_t kSymHalfN = kSsTileN / 2;                   // N of one instruction: a tile's column half
+constexpr uint32_t kSymAccSlots = 3;
+constexpr uint32_t kSymTmemSf = kSymAccSlots * kSymHalfN;      // first TMEM column of the scale factors (all 1.0)
+constexpr uint32_t kSymHalfBytes = kSymHalfN * kChunkBytes;    // one K chunk of a column half: 16 KB
+constexpr uint32_t kInstrDescSym = instrDescMxf4(kRowsPerItem, kSymHalfN);
+constexpr uint32_t kInstrDescSymPair = instrDescMxf4(kPairRows, kSymHalfN);   // M = 256 over two CTAs
+static_assert(kSymTmemSf + 128 <= 512, "accumulator ring + scale factors fit in tensor memory");
+
+// The epilogue compares the f32 accumulators by their bit patterns as signed integers (the integer max chain of the
+// int8 form): for a threshold T >= 0, v > T  <=>  bits(v) >= bits(T) + 1.  A negative T (a bound above K/2 mismatches)
+// lets every value through this test; the exact float compare behind it decides.
+__device__ __forceinline__ int32_t thrKey(int32_t t) { return t >= 0 ? __float_as_int(float(t)) + 1 : INT32_MIN; }
 
 struct SymParams {
     uint64_t cellCount;            // N: scan positions of the WHOLE job (all ranks); rows == columns
@@ -668,35 +692,35 @@ static __device__ __noinline__ ulonglong2* nextLogChunk(uint32_t* chunkFill, uin
     return pool + uint64_t(c) * kLogChunk;
 }
 
-// PAIR: the two CTAs of a cluster (the two SMs of a TPC) take the two row blocks of ONE super block and run every tile
+// PAIR: the two CTAs of a cluster (the two SMs of a TPC) take the two row blocks of ONE super block and run every half tile
 // as one M = 256 instruction (tcgen05.mma.cta_group::2): each CTA keeps its own 128 rows of A and of the accumulators and
-// streams HALF of every B tile (its 128 columns; 16 KB per K chunk), the leader (cluster rank 0) issues.  Per 128 x 256 x 32
-// MMA an SM then reads 8 KB of shared memory instead of 12 KB -- the operand traffic of the TMEM-operand form, whose
-// issue rate is 4223 TOP/s against the 3414 of the single-CTA shared-memory form -- and the L2 -> SM traffic halves.
+// streams HALF of every B half tile (64 columns; 8 KB per K chunk), the leader (cluster rank 0) issues.  Per 128 x 128 x 64
+// instruction an SM then reads 6 KB of shared memory instead of 8 KB, and the L2 -> SM traffic halves.
 // Barriers: full[] / accEmpty[] / aFull live in the leader (both CTAs' TMA bytes and epilogue warps arrive there),
 // empty[] / accFull[] / aEmpty are per CTA and receive the leader's multicast commits.
 template <bool PAIR>
 __global__ void __launch_bounds__(kSymThreads, 1)
 scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const SymParams p)
 {
-    constexpr uint32_t kBStageBytes = PAIR ? kSsBBytes / 2 : kSsBBytes;      // PAIR: this CTA's 128 columns of a K chunk
+    constexpr uint32_t kBStageBytes = PAIR ? kSymHalfBytes / 2 : kSymHalfBytes;      // one K chunk of this CTA's columns of a half
     extern __shared__ uint8_t smemRaw[];
     uint8_t* smA = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smemRaw) + 1023) & ~uintptr_t(1023));
     uint8_t* ring = smA + size_t(p.panels) * kSsABytes;
     uint8_t* small = ring + size_t(p.stages) * kBStageBytes;
     uint64_t* bars = reinterpret_cast<uint64_t*>(small);
-    uint64_t* accFull = bars + 0;    // [2]
-    uint64_t* accEmpty = bars + 2;   // [2]
-    uint64_t* aFull = bars + 4;      // the item's A operand has landed
-    uint64_t* aEmpty = bars + 5;     // every MMA of the item has read it
-    uint64_t* full = bars + 6;       // [stages]
+    uint64_t* accFull = bars + 0;    // [kSymAccSlots]
+    uint64_t* accEmpty = bars + 3;   // [kSymAccSlots]
+    uint64_t* aFull = bars + 6;      // the item's A operand has landed
+    uint64_t* aEmpty = bars + 7;     // every MMA of the item has read it
+    uint64_t* full = bars + 8;       // [stages]
     uint64_t* empty = full + kSymMaxStages;
     uint64_t* thrFull = empty + kSymMaxStages;      // [2] the producer warp has staged the tile's column thresholds
     uint64_t* thrEmpty = thrFull + 2;               // [2] every epilogue warp is done with them
     uint32_t* tmemSlot = reinterpret_cast<uint32_t*>(thrEmpty + 2);
-    int16_t* colThr = reinterpret_cast<int16_t*>(small + 192);          // [2][256] dot thresholds of the tile's columns
-    int16_t* grpThr = colThr + 2 * kSsTileN;                             // [2][32]  loosest threshold of each 8 columns
-    uint16_t* tauShare = reinterpret_cast<uint16_t*>(grpThr + 2 * (kSsTileN / 8));   // [kSubStreams][kRowsPerItem]
+    static_assert((8 + 2 * kSymMaxStages + 4) * 8 + 4 <= kSymBarBytes, "barrier block");
+    float* colThr = reinterpret_cast<float*>(small + kSymBarBytes);      // [2][256] dot thresholds of the tile's columns
+    int32_t* grpKey = reinterpret_cast<int32_t*>(colThr + 2 * kSsTileN);  // [2][32]  thrKey of the loosest threshold of each 8 columns
+    uint16_t* tauShare = reinterpret_cast<uint16_t*>(grpKey + 2 * (kSsTileN / 8));   // [kSubStreams][kRowsPerItem]
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
@@ -704,9 +728,12 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     const uint32_t worker = PAIR ? (blockIdx.x >> 1) : blockIdx.x;
     const uint32_t workers = PAIR ? (gridDim.x >> 1) : gridDim.x;
     if (threadIdx.x == 0) {
-        for (int i = 0; i < 2; i++) {
+        for (int i = 0; i < int(kSymAccSlots); i++) {
             mbarInit(accFull + i, 1);
-            mbarInit(accEmpty + i, PAIR ? 2 * kEpiWarps : kEpiWarps * 32);      // PAIR: one arrival per epilogue warp of either CTA
+            // a slot is drained by ONE sub-stream: its 4 warps (PAIR: one arrival per warp, of either CTA)
+            mbarInit(accEmpty + i, PAIR ? 2 * (kEpiWarps / kSubStreams) : kRowsPerItem);
+        }
+        for (int i = 0; i < 2; i++) {
             mbarInit(thrFull + i, 1);
             mbarInit(thrEmpty + i, kEpiWarps);
         }
@@ -727,6 +754,23 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     else __syncthreads();
     fenceAfter();
     const uint32_t tmemBase = *tmemSlot;
+    // scale factors: columns [kSymTmemSf, 512) of every lane hold UE8M0 1.0 (0x7F) -- whatever part of them the
+    // instruction reads for A and for B; written before the first MMA (PAIR: in both CTAs, the leader's MMAs read both)
+    if (warp < kEpiWarps) {
+        uint32_t ones[32];
+#pragma unroll
+        for (int j = 0; j < 32; j++) ones[j] = 0x7F7F7F7Fu;
+        const uint32_t col = kSymTmemSf + uint32_t(warp / 4) * 64;
+        const uint32_t lanes = uint32_t((warp & 3) * 32) << 16;
+        tmemStore32(tmemBase + lanes + col, ones);
+        tmemStore32(tmemBase + lanes + col + 32, ones);
+        tmemStoreWait();
+    }
+    fenceBefore();
+    if (PAIR) clusterSync();
+    else __syncthreads();
+    fenceAfter();
+    const uint32_t sfA = tmemBase + kSymTmemSf, sfB = tmemBase + kSymTmemSf + 64;
     const uint32_t items = p.items;
     const uint64_t virtualCols = uint64_t(p.offsetsHere) * kSsTileN;
     const uint32_t N = uint32_t(p.cellCount);
@@ -784,19 +828,22 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
                 }
                 const uint32_t colSuper = colSuperOf(super, d);
                 if (lane == 0) {
-                    const int32_t col0 = int32_t(colSuper * kSsTileN + (PAIR ? rank * (kSsTileN / 2) : 0));
-                    for (uint32_t kc = 0; kc < p.panels; kc++) {
-                        mbarWait(empty + stage, phase ^ 1);
-                        if (PAIR) {      // this CTA's 128 columns (mapA's box is 128 rows); the leader's barrier collects both halves
-                            if (rank == 0) mbarExpectTx(full + stage, 2 * kBStageBytes);
-                            tmaLoad2dPair(ring + size_t(stage) * kBStageBytes, &mapA, full + stage, int32_t(kc * kChunkBytes), col0);
-                        } else {
-                            mbarExpectTx(full + stage, kSsBBytes);
-                            tmaLoad2d(ring + size_t(stage) * kSsBBytes, &mapB, full + stage, int32_t(kc * kChunkBytes), col0);
-                        }
-                        if (++stage == p.stages) {
-                            stage = 0;
-                            phase ^= 1;
+                    // in the MMA warp's order: the K chunks of column half 0, then those of half 1
+                    for (uint32_t h = 0; h < 2; h++) {
+                        const int32_t col0 = int32_t(colSuper * kSsTileN + h * kSymHalfN + (PAIR ? rank * (kSymHalfN / 2) : 0));
+                        for (uint32_t kc = 0; kc < p.panels; kc++) {
+                            mbarWait(empty + stage, phase ^ 1);
+                            if (PAIR) {      // this CTA's 64 columns of the half (mapB's box); the leader's barrier collects both
+                                if (rank == 0) mbarExpectTx(full + stage, 2 * kBStageBytes);
+                                tmaLoad2dPair(ring + size_t(stage) * kBStageBytes, &mapB, full + stage, int32_t(kc * kChunkBytes), col0);
+                            } else {
+                                mbarExpectTx(full + stage, kBStageBytes);
+                                tmaLoad2d(ring + size_t(stage) * kBStageBytes, &mapB, full + stage, int32_t(kc * kChunkBytes), col0);
+                            }
+                            if (++stage == p.stages) {
+                                stage = 0;
+                                phase ^= 1;
+                            }
                         }
                     }
                 }
@@ -823,21 +870,18 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
                     uint32_t lim[8];
 #pragma unroll
                     for (int j = 0; j < 8; j++) lim[j] = pos0 + j < N ? __ldcg(p.limEx + pos0 + j) : 0u;      // padding columns: nothing passes
-                    int32_t t[8];
-                    int32_t loosest = 0x7fff;
+                    float t[8];
+                    int32_t loosest = 0x7fffffff;
 #pragma unroll
                     for (int j = 0; j < 8; j++) {
-                        t[j] = int32_t(p.K) - 2 * int32_t(lim[j]);
-                        loosest = min(loosest, t[j]);
+                        const int32_t tj = int32_t(p.K) - 2 * int32_t(lim[j]);
+                        t[j] = float(tj);
+                        loosest = min(loosest, tj);
                     }
-                    uint4 packed;
-                    packed.x = uint32_t(uint16_t(t[0])) | (uint32_t(uint16_t(t[1])) << 16);
-                    packed.y = uint32_t(uint16_t(t[2])) | (uint32_t(uint16_t(t[3])) << 16);
-                    packed.z = uint32_t(uint16_t(t[4])) | (uint32_t(uint16_t(t[5])) << 16);
-                    packed.w = uint32_t(uint16_t(t[6])) | (uint32_t(uint16_t(t[7])) << 16);
                     mbarWait(thrEmpty + slot, ((tileIter >> 1) & 1) ^ 1);      // every epilogue warp is done with the slot's last tile
-                    *reinterpret_cast<uint4*>(colThr + slot * kSsTileN + lane * 8) = packed;
-                    grpThr[slot * (kSsTileN / 8) + lane] = int16_t(loosest);
+                    *reinterpret_cast<float4*>(colThr + slot * kSsTileN + lane * 8) = make_float4(t[0], t[1], t[2], t[3]);
+                    *reinterpret_cast<float4*>(colThr + slot * kSsTileN + lane * 8 + 4) = make_float4(t[4], t[5], t[6], t[7]);
+                    grpKey[slot * (kSsTileN / 8) + lane] = thrKey(loosest);
                     __syncwarp();
                     if (lane == 0) mbarArrive(thrFull + slot);
                 }
@@ -854,42 +898,42 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
             mbarWait(aFull, itemIter & 1);
             fenceAfter();
             for (uint32_t t = 0; t < tiles; t++, tileIter++) {
-                const uint32_t buf = tileIter & 1;
-                mbarWait(accEmpty + buf, ((tileIter >> 1) & 1) ^ 1);
-                fenceAfter();
-                const uint32_t tmemD = tmemBase + buf * kSsTileN;
-                for (uint32_t kc = 0; kc < p.panels; kc++) {
-                    mbarWait(full + stage, phase);
+                for (uint32_t h = 0; h < 2; h++) {
+                    const uint32_t half = 2 * tileIter + h;          // -> accumulator slot half % 3, its (half / 3)-th use
+                    const uint32_t slot = half % kSymAccSlots;
+                    mbarWait(accEmpty + slot, ((half / kSymAccSlots) & 1) ^ 1);
                     fenceAfter();
-                    const uint64_t descA = makeSmemDesc(aBase + kc * kSsABytes);
-                    const uint64_t descB = makeSmemDesc(ringBase + stage * kBStageBytes);
-                    if (electOne()) {
+                    const uint32_t tmemD = tmemBase + slot * kSymHalfN;
+                    for (uint32_t kc = 0; kc < p.panels; kc++) {
+                        mbarWait(full + stage, phase);
+                        fenceAfter();
+                        const uint64_t descA = makeSmemDesc(aBase + kc * kSsABytes);
+                        const uint64_t descB = makeSmemDesc(ringBase + stage * kBStageBytes);
+                        if (electOne()) {
 #pragma unroll
-                        for (int ks = 0; ks < kChunkBytes / kUmmaK; ks++) {      // + 32 bytes along K = + 2 in the descriptor's address field
-                            const uint32_t accumulate = (kc | uint32_t(ks)) != 0 ? 1u : 0u;
-                            if (PAIR) mmaI8SsPair(tmemD, descA + uint64_t(ks * (kUmmaK >> 4)), descB + uint64_t(ks * (kUmmaK >> 4)), kInstrDescSsPair, accumulate);
-                            else mmaI8Ss(tmemD, descA + uint64_t(ks * (kUmmaK >> 4)), descB + uint64_t(ks * (kUmmaK >> 4)), kInstrDescSs, accumulate);
-                        }
-                        // the same lane commits everything it issued: the ring stage, the tile's accumulator, and after the
-                        // item's last tile the A operand (the producer may then overwrite it); PAIR: in both CTAs
-                        if (PAIR) {
-                            commitPair(empty + stage);
-                            if (kc + 1 == p.panels) {
-                                commitPair(accFull + buf);
-                                if (t + 1 == tiles) commitPair(aEmpty);
+                            for (int ks = 0; ks < kChunkBytes / 32; ks++) {      // K = 64 FP4 = 32 bytes = + 2 in the descriptor's address field
+                                const uint32_t accumulate = (kc | uint32_t(ks)) != 0 ? 1u : 0u;
+                                if (PAIR) mmaMxf4SsPair(tmemD, descA + uint64_t(2 * ks), descB + uint64_t(2 * ks), kInstrDescSymPair, sfA, sfB, accumulate);
+                                else mmaMxf4Ss(tmemD, descA + uint64_t(2 * ks), descB + uint64_t(2 * ks), kInstrDescSym, sfA, sfB, accumulate);
                             }
-                        } else {
-                            commit(empty + stage);
-                            if (kc + 1 == p.panels) {
-                                commit(accFull + buf);
-                                if (t + 1 == tiles) commit(aEmpty);
+                            // the same lane commits everything it issued: the ring stage, the half's accumulator, and after the
+                            // item's last half the A operand (the producer may then overwrite it); PAIR: in both CTAs
+                            const bool lastK = kc + 1 == p.panels, lastOfItem = lastK && h == 1 && t + 1 == tiles;
+                            if (PAIR) {
+                                commitPair(empty + stage);
+                                if (lastK) commitPair(accFull + slot);
+                                if (lastOfItem) commitPair(aEmpty);
+                            } else {
+                                commit(empty + stage);
+                                if (lastK) commit(accFull + slot);
+                                if (lastOfItem) commit(aEmpty);
                             }
                         }
-                    }
-                    __syncwarp();
-                    if (++stage == p.stages) {
-                        stage = 0;
-                        phase ^= 1;
+                        __syncwarp();
+                        if (++stage == p.stages) {
+                            stage = 0;
+                            phase ^= 1;
+                        }
                     }
                 }
             }
@@ -931,23 +975,27 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
             tauShare[sub * kRowsPerItem + rowInItem] = 0xffffu;      // harmless for any row (see scanMmaKernel)
             asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");
             int32_t dotThr = int32_t(dotK) - 2 * int32_t(st.lim);      // mismatch < lim  <=>  dot > K - 2 lim
+            int32_t dotKey = thrKey(dotThr);
 
             for (int32_t d = d0; d < d1; d++, tileIter++) {
                 const uint32_t buf = tileIter & 1;
+                const uint32_t half = 2 * tileIter + sub;      // this sub-stream's half of the tile: see the MMA warp
+                const uint32_t slot = half % kSymAccSlots;
                 const uint32_t colSuper = colSuperOf(super, d);
                 const bool colDir = !p.rowOnly && d != 0 && uint32_t(d) != p.halfOffset;          // CTA-uniform
-                const int16_t* thr = colThr + buf * kSsTileN + sub * kSubCols;
-                const int16_t* grp = grpThr + buf * (kSsTileN / 8) + sub * (kSubCols / 8);
+                const float* thr = colThr + buf * kSsTileN + sub * kSubCols;
+                const int32_t* grp = grpKey + buf * (kSsTileN / 8) + sub * (kSubCols / 8);
                 if (!p.rowOnly) mbarWait(thrFull + buf, (tileIter >> 1) & 1);
-                mbarWait(accFull + buf, (tileIter >> 1) & 1);
+                mbarWait(accFull + slot, (half / kSymAccSlots) & 1);
                 fenceAfter();
                 const uint32_t posBase = colSuper * kSsTileN + sub * kSubCols;
-                const uint32_t taddr = tmemBase + buf * kSsTileN + sub * kSubCols + laneField;
+                const uint32_t taddr = tmemBase + slot * kSymHalfN + laneField;
                 {
                     const uint32_t other = tauShare[(sub ^ 1) * kRowsPerItem + rowInItem];
                     if (other < st.lim && !(p.flags & 1)) {
                         st.lim = other;
                         dotThr = int32_t(dotK) - 2 * int32_t(st.lim);
+                        dotKey = thrKey(dotThr);
                     }
                 }
 #pragma unroll 1
@@ -959,9 +1007,9 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
                         fenceBefore();
                         if (PAIR) {
                             __syncwarp();
-                            if (lane == 0) mbarArriveLeader(accEmpty + buf);
+                            if (lane == 0) mbarArriveLeader(accEmpty + slot);
                         } else {
-                            mbarArrive(accEmpty + buf);
+                            mbarArrive(accEmpty + slot);
                         }
                     }
                     int32_t m[4];
@@ -972,17 +1020,17 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
                         for (int j = 1; j < 8; j++) m[g] = max(m[g], int32_t(v[8 * g + j]));
                     }
                     const int32_t mx = max(max(m[0], m[1]), max(m[2], m[3]));
-                    // ---- row direction
-                    if (mx > dotThr) {
+                    // ---- row direction (m[] are maxima of bit patterns: see thrKey)
+                    if (mx >= dotKey) {
 #pragma unroll
                         for (int g = 0; g < 4; g++) {
-                            if (m[g] > dotThr) {
+                            if (m[g] >= dotKey) {
 #pragma unroll
                                 for (int j = 0; j < 8; j++) {
-                                    const int32_t dv = int32_t(v[8 * g + j]);
+                                    const float dv = __int_as_float(v[8 * g + j]);
                                     const uint32_t pos = posBase + c + 8 * g + j;
-                                    if (dv > dotThr && pos < N && pos != st.rowId) {
-                                        const uint32_t ham = uint32_t(int32_t(dotK) - dv) >> 1;
+                                    if (dv > float(dotThr) && pos < N && pos != st.rowId) {
+                                        const uint32_t ham = uint32_t(int32_t(dotK) - __float2int_rn(dv)) >> 1;
                                         st.buf[st.count++] = (uint64_t(ham) << 32) | pos;
                                         st.appended++;
                                     }
@@ -992,17 +1040,17 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
                     }
                     // ---- column direction
                     if (colDir && valid) {
-                        const short4 gt = *reinterpret_cast<const short4*>(grp + (c >> 3));
+                        const int4 gt = *reinterpret_cast<const int4*>(grp + (c >> 3));
                         const int32_t gtv[4] = {gt.x, gt.y, gt.z, gt.w};
-                        if (m[0] > gtv[0] || m[1] > gtv[1] || m[2] > gtv[2] || m[3] > gtv[3]) {
+                        if (m[0] >= gtv[0] || m[1] >= gtv[1] || m[2] >= gtv[2] || m[3] >= gtv[3]) {
 #pragma unroll
                             for (int g = 0; g < 4; g++) {
-                                if (m[g] > gtv[g]) {
+                                if (m[g] >= gtv[g]) {
 #pragma unroll
                                     for (int j = 0; j < 8; j++) {
-                                        const int32_t dv = int32_t(v[8 * g + j]);
-                                        if (dv > int32_t(thr[c + 8 * g + j])) {
-                                            const uint32_t ham = uint32_t(int32_t(dotK) - dv) >> 1;
+                                        const float dv = __int_as_float(v[8 * g + j]);
+                                        if (dv > thr[c + 8 * g + j]) {
+                                            const uint32_t ham = uint32_t(int32_t(dotK) - __float2int_rn(dv)) >> 1;
                                             if (logFill == kLogChunk) logNext = nextLogChunk(p.chunkFill, p.chunkNext, p.chunkCap, p.colLog, logNext, logFill);
                                             *logNext++ = make_ulonglong2((uint64_t(ham) << 32) | rowCell, posBase + c + 8 * g + j);
                                             logFill++;
@@ -1012,9 +1060,10 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
                             }
                         }
                     }
-                    if (__any_sync(0xffffffffu, mx > dotThr)) {
+                    if (__any_sync(0xffffffffu, mx >= dotKey)) {
                         warpPruneIfNeededAnyOrder(st, p.k, p.cap, limPtr, p.perm);
                         dotThr = int32_t(dotK) - 2 * int32_t(st.lim);
+                        dotKey = thrKey(dotThr);
                     }
                 }
                 if (valid) tauShare[sub * kRowsPerItem + rowInItem] = uint16_t(min(st.tau, 0xffffu));
@@ -1480,6 +1529,45 @@ __global__ void encodeKernel(const uint64_t* __restrict__ sig, uint32_t W, uint6
     *reinterpret_cast<uint4*>(enc + row * K + size_t(g) * 16) = make_uint4(out[0], out[1], out[2], out[3]);
 }
 
+// FP4 (e2m1) expansion for the symmetric scan: element p of row n is +1.0 (nibble 0x2) if bit p is set, else -1.0
+// (0xA); elements 2i and 2i + 1 are the low and high nibble of byte i.  K (a multiple of 256) elements = K / 2 bytes per
+// row; bits at and beyond lshCount encode as -1 in every row, as in encodeKernel.
+__global__ void encodeFp4Kernel(const uint64_t* __restrict__ sig, uint32_t W, uint64_t cellCount, uint32_t K,
+                                uint8_t* __restrict__ enc, const uint32_t* __restrict__ index)
+{
+    const uint32_t groupsPerRow = K / 32;      // 32 bits -> 16 bytes per thread
+    const uint64_t idx = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x;
+    if (idx >= cellCount * groupsPerRow) return;
+    const uint64_t row = idx / groupsPerRow;
+    const uint32_t g = uint32_t(idx - row * groupsPerRow);
+    const uint32_t w = g >> 1;
+    uint32_t bits = 0;
+    const uint64_t srcRow = index ? uint64_t(index[row]) : row;
+    if (w < W) bits = uint32_t(sig[srcRow * W + w] >> (32 - 32 * (g & 1)));      // MSB-first
+    uint32_t out[4];
+#pragma unroll
+    for (int q = 0; q < 4; q++) {
+        uint32_t word = 0;
+#pragma unroll
+        for (int e = 0; e < 8; e++) {
+            const uint32_t bit = (bits >> (31 - (8 * q + e))) & 1u;
+            word |= (0xAu ^ (bit << 3)) << (4 * e);
+        }
+        out[q] = word;
+    }
+    *reinterpret_cast<uint4*>(enc + row * (K / 2) + size_t(g) * 16) = make_uint4(out[0], out[1], out[2], out[3]);
+}
+
+int encodeFp4(em2_context* ctx, const uint64_t* sig, uint32_t W, uint64_t rows, uint32_t K, uint8_t* enc, const uint32_t* index,
+              cudaStream_t s)
+{
+    const uint64_t threads = rows * (K / 32);
+    if (threads) encodeFp4Kernel<<<unsigned((threads + 255) / 256), 256, 0, s>>>(sig, W, rows, K, enc, index);
+    EM2_CUDA(ctx, cudaGetLastError());
+    ctx->stats.kernel_launches++;
+    return EM2_OK;
+}
+
 __global__ void fillU32Kernel(uint32_t* __restrict__ dst, uint64_t n, uint32_t value)
 {
     const uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x;
@@ -1487,7 +1575,8 @@ __global__ void fillU32Kernel(uint32_t* __restrict__ dst, uint64_t n, uint32_t v
 }
 
 // Symmetric scan: every unordered pair of cells is evaluated once -- on one GPU or across the GPUs of a job.
-//   encP    encoded signatures of ALL N cells in scan-position order (rows and columns)
+//   encP    FP4 encoding (encodeFp4Kernel) of ALL N cells in scan-position order (rows and columns), K bits (a multiple
+//           of 256) = K / 2 bytes per cell
 //   perm    position -> cell id (nullptr: identity)
 //   this GPU owns the positions [posBegin, posBegin + ownRows) (posBegin = rank * shard, a multiple of 256; its cells
 //   are the SAME id range, permuted); pairs / usedCount hold its rows, indexed by cell id - posBegin.
@@ -1510,7 +1599,7 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
 {
     const uint64_t N = cellCount;
     const int P = ctx->world;
-    const uint32_t panels = K / kChunkBytes;
+    const uint32_t panels = K / kSymKBits;
     const uint32_t S = uint32_t((N + kSsTileN - 1) / kSsTileN);
     *overflowed = 0;
     // Half width of the near window, in super blocks.  Default: N/32 columns in total (what a sample must hold for the
@@ -1675,7 +1764,7 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
     p.K = K;
     p.panels = panels;
     const size_t budget = 227 * 1024 - 1024 - kSymSmallBytes - size_t(panels) * kSsABytes;
-    const size_t bStageBytes = pair ? kSsBBytes / 2 : kSsBBytes;
+    const size_t bStageBytes = pair ? kSymHalfBytes / 2 : kSymHalfBytes;
     p.stages = uint32_t(std::min<size_t>(kSymMaxStages, budget / bStageBytes));
     p.superBlocks = S;
     p.halfOffset = S % 2 == 0 ? S / 2 : 0;
@@ -1695,8 +1784,8 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
     p.perm = perm;
     p.flags = uint32_t(ctx->debugFlags);
     CUtensorMap mapA, mapB;
-    EM2_TRY(makeTensorMapU8(ctx, &mapA, encP, N, K, K, kRowsPerItem));
-    EM2_TRY(makeTensorMapU8(ctx, &mapB, encP, N, K, K, kSsTileN));
+    EM2_TRY(makeTensorMapU8(ctx, &mapA, encP, N, K / 2, K / 2, kRowsPerItem));
+    EM2_TRY(makeTensorMapU8(ctx, &mapB, encP, N, K / 2, K / 2, pair ? kSymHalfN / 2 : kSymHalfN));
     const size_t smem = 1024 + size_t(panels) * kSsABytes + size_t(p.stages) * bStageBytes + kSymSmallBytes;
     EM2_CUDA(ctx, cudaFuncSetAttribute(scanMmaSymKernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     EM2_CUDA(ctx, cudaFuncSetAttribute(scanMmaSymKernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
@@ -1934,39 +2023,20 @@ int runMma(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uin
     const bool streamed = K > kMaxPanels * kChunkBytes || ctx->mmaKernel == 2 || (ctx->mmaKernel == 0 && K >= 512);
     if (cellCount > 0x7fffff00ull) return fail(ctx, EM2_ERR_INVALID, "cellCount too large for the MMA variant");
 
-    // 1. encode
-    void* enc = nullptr;
-    EM2_TRY(reserve(ctx, em2_context::S_ENC, cellCount * K, &enc));
-    {
-        const uint64_t threads = cellCount * (K / 16);
-        encodeKernel<<<unsigned((threads + 255) / 256), 256, 0, s>>>(signatures, W, cellCount, K, static_cast<uint8_t*>(enc), nullptr);
-        ctx->stats.kernel_launches++;
-        EM2_CUDA(ctx, cudaGetLastError());
-    }
-
-    // 1b. the scanned rows in grouped order (see "Row grouping") and their encoded signatures by scan position
+    // 1. the scanned rows in grouped order (see "Row grouping")
     const uint32_t tau0 = mismatchMax < 0 ? 0u : uint32_t(std::min<int64_t>(mismatchMax, int64_t(lshCount)) + 1);
     const bool grouped = !dump && (ctx->rowGrouping == 2 || (ctx->rowGrouping == 0 && rows >= 8192));
-    const uint8_t* encRows = static_cast<const uint8_t*>(enc) + rowBegin * uint64_t(K);
-    const uint32_t* rowPerm = nullptr;
+    uint32_t* rowPerm = nullptr;
     uint32_t* groupStats = nullptr;
     if (grouped) {
         void* permBuf = nullptr;
         EM2_TRY(reserve(ctx, em2_context::S_PERM, rows * sizeof(uint32_t), &permBuf));
-        uint32_t* perm = static_cast<uint32_t*>(permBuf);
-        EM2_TRY(groupRows(ctx, signatures, W, lshCount, tau0, rowBegin, rows, perm, s, &groupStats));
-        void* er = nullptr;
-        EM2_TRY(reserve(ctx, em2_context::S_ENCROWS, rows * uint64_t(K), &er));
-        const uint64_t threads = rows * (K / 16);
-        encodeKernel<<<unsigned((threads + 255) / 256), 256, 0, s>>>(signatures, W, rows, K, static_cast<uint8_t*>(er), perm);
-        EM2_CUDA(ctx, cudaGetLastError());
-        ctx->stats.kernel_launches++;
-        encRows = static_cast<const uint8_t*>(er);
-        rowPerm = perm;
+        rowPerm = static_cast<uint32_t*>(permBuf);
+        EM2_TRY(groupRows(ctx, signatures, W, lshCount, tau0, rowBegin, rows, rowPerm, s, &groupStats));
     }
 
-    // 1c. whole-matrix jobs, on request: every unordered pair once (scanMmaSymKernel); falls through to the
-    //     one-directional kernels if a capacity ran out (nothing of the symmetric attempt is kept)
+    // 2. whole-matrix jobs, on request: every unordered pair once (scanMmaSymKernel, FP4 operands of the cells in scan
+    //    order); falls through to the one-directional kernels if a capacity ran out (nothing of the symmetric attempt is kept)
     ctx->stats.scan_symmetric = 0;
     {
         const uint32_t capSym = scanCandidateCapacity(uint32_t(k), uint32_t(ctx->candCapExtra));
@@ -1987,14 +2057,39 @@ int runMma(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uin
             automatic = want <= have + freeBytes / 10 * 9;
         }
         if (eligible && ctx->world == 1 && (ctx->scanSymmetric == 2 || automatic)) {
+            const uint32_t Ksym = uint32_t(roundUp(lshCount, kSymKBits));
+            void* encSym = nullptr;
+            EM2_TRY(reserve(ctx, em2_context::S_ENCROWS, cellCount * uint64_t(Ksym / 2), &encSym));
+            EM2_TRY(encodeFp4(ctx, signatures, W, cellCount, Ksym, static_cast<uint8_t*>(encSym), rowPerm, s));
             int overflowed = 0;
-            EM2_TRY(runSymmetric(ctx, encRows, rowPerm, groupStats, grouped, cellCount, 0, cellCount, cellCount, K, k, tau0, lut, pairs, usedCount, s, &overflowed));
+            EM2_TRY(runSymmetric(ctx, static_cast<const uint8_t*>(encSym), rowPerm, groupStats, grouped, cellCount, 0, cellCount, cellCount,
+                                 Ksym, k, tau0, lut, pairs, usedCount, s, &overflowed));
             ctx->stats.scan_symmetric = overflowed ? 2 + 16 * overflowed : 1;      // 2 + 16 * (which capacity ran out)
             if (!overflowed) return EM2_OK;
         }
     }
 
-    // 2. plan + scratch
+    // 3. int8 encode: all cells in id order (the columns) and the scanned rows by scan position
+    void* enc = nullptr;
+    EM2_TRY(reserve(ctx, em2_context::S_ENC, cellCount * K, &enc));
+    {
+        const uint64_t threads = cellCount * (K / 16);
+        encodeKernel<<<unsigned((threads + 255) / 256), 256, 0, s>>>(signatures, W, cellCount, K, static_cast<uint8_t*>(enc), nullptr);
+        ctx->stats.kernel_launches++;
+        EM2_CUDA(ctx, cudaGetLastError());
+    }
+    const uint8_t* encRows = static_cast<const uint8_t*>(enc) + rowBegin * uint64_t(K);
+    if (grouped) {
+        void* er = nullptr;
+        EM2_TRY(reserve(ctx, em2_context::S_ENCROWS, rows * uint64_t(K), &er));
+        const uint64_t threads = rows * (K / 16);
+        encodeKernel<<<unsigned((threads + 255) / 256), 256, 0, s>>>(signatures, W, rows, K, static_cast<uint8_t*>(er), rowPerm);
+        EM2_CUDA(ctx, cudaGetLastError());
+        ctx->stats.kernel_launches++;
+        encRows = static_cast<const uint8_t*>(er);
+    }
+
+    // 4. plan + scratch
     MmaParams p{};
     const uint32_t panels = K / kChunkBytes;
     p.stages = kStages;
@@ -2147,12 +2242,12 @@ int launchScanSymDist(em2_context* ctx, const uint64_t* allSig, uint64_t cellCou
     const DistPartition part = distPartition(cellCount, ctx->world, ctx->rank);
     const uint64_t rows = part.rowEnd - part.rowBegin;
     const uint32_t W = uint32_t(wordCount(lshCount));
-    const uint32_t K = uint32_t(roundUp(lshCount, kChunkBytes));
+    const uint32_t K = uint32_t(roundUp(lshCount, kSymKBits));
     const uint32_t tau0 = uint32_t(std::min<int64_t>(mismatchMax, int64_t(lshCount)) + 1);
     ctx->stats.variant_used = EM2_VARIANT_MMA_I8;
     void *permBuf = nullptr, *enc = nullptr;
     int rc = reserve(ctx, em2_context::S_PERM, uint64_t(ctx->world) * part.shard * sizeof(uint32_t), &permBuf);
-    if (rc == EM2_OK) rc = reserve(ctx, em2_context::S_ENC, cellCount * K, &enc);
+    if (rc == EM2_OK) rc = reserve(ctx, em2_context::S_ENC, cellCount * uint64_t(K / 2), &enc);
     uint32_t* perm = static_cast<uint32_t*>(permBuf);
     uint32_t* groupStats = nullptr;
     // scan order: every GPU groups ITS cells (similar rows into the same warps, similar columns into the same tiles);
@@ -2170,12 +2265,7 @@ int launchScanSymDist(em2_context* ctx, const uint64_t* allSig, uint64_t cellCou
     // allocation may wait for OTHER devices (peer mappings), whose NCCL kernels wait for this rank's.
     EM2_TRY(distAgree(ctx, rc));
     EM2_TRY(distAllGather(ctx, perm, part.shard, sizeof(uint32_t), s));
-    {
-        const uint64_t threads = cellCount * (K / 16);
-        encodeKernel<<<unsigned((threads + 255) / 256), 256, 0, s>>>(allSig, W, cellCount, K, static_cast<uint8_t*>(enc), perm);
-        EM2_CUDA(ctx, cudaGetLastError());
-        ctx->stats.kernel_launches++;
-    }
+    EM2_TRY(encodeFp4(ctx, allSig, W, cellCount, K, static_cast<uint8_t*>(enc), perm, s));
     int overflowed = 0;
     EM2_TRY(runSymmetric(ctx, static_cast<const uint8_t*>(enc), perm, groupStats, ctx->rowGrouping != 1, cellCount, part.rowBegin, rows,
                          part.shard, K, k, tau0, lut, pairs, usedCount, s, &overflowed));

@@ -1,5 +1,5 @@
 // Thin PTX wrappers for the Blackwell (sm_100a) tensor-core path: mbarriers, TMA tile loads,
-// tcgen05.mma (kind::i8) with operands from shared memory or tensor memory, TMEM allocation and
+// tcgen05.mma (kind::i8, kind::mxf4) with operands from shared memory or tensor memory, TMEM allocation and
 // tcgen05.ld/st.  Shared by the Hamming scan (scan_mma.cu), the signature filter (sig_filter.cu) and the
 // exact-similarity path (exact.cu).  Nothing here comes from the reference (it has no tensor-core code).
 #pragma once
@@ -213,6 +213,32 @@ __device__ __forceinline__ void mmaI8SsPair(uint32_t tmemD, uint64_t descA, uint
         "l"(descA), "l"(descB), "r"(idesc), "r"(accumulate), "r"(z)
         : "memory");
 }
+// kind::mxf4 (e2m1 operands packed two per byte, K = 64 per instruction, f32 accumulator), both operands in shared
+// memory; sfA / sfB: tensor-memory addresses of the UE8M0 scale factors (one per 32 elements along K)
+__device__ __forceinline__ void mmaMxf4Ss(uint32_t tmemD, uint64_t descA, uint64_t descB, uint32_t idesc, uint32_t sfA, uint32_t sfB,
+                                          uint32_t accumulate)
+{
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %6, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::mxf4.block_scale.scale_vec::2X [%0], %1, %2, %3, [%4], [%5], p;\n\t"
+        "}\n" ::"r"(tmemD),
+        "l"(descA), "l"(descB), "r"(idesc), "r"(sfA), "r"(sfB), "r"(accumulate)
+        : "memory");
+}
+__device__ __forceinline__ void mmaMxf4SsPair(uint32_t tmemD, uint64_t descA, uint64_t descB, uint32_t idesc, uint32_t sfA, uint32_t sfB,
+                                              uint32_t accumulate)
+{
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %6, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::mxf4.block_scale.scale_vec::2X [%0], %1, %2, %3, [%4], [%5], p;\n\t"
+        "}\n" ::"r"(tmemD),
+        "l"(descA), "l"(descB), "r"(idesc), "r"(sfA), "r"(sfB), "r"(accumulate)
+        : "memory");
+}
 __device__ __forceinline__ void tmemAllocPair(uint32_t* slot, uint32_t cols)
 {
     asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smemAddr(slot)), "r"(cols) : "memory");
@@ -244,6 +270,16 @@ __host__ __device__ constexpr uint32_t instrDescI8(bool aSigned, bool bSigned, u
            | (uint32_t(aSigned ? 1 : 0) << 7) // a_format: 0 = unsigned 8-bit, 1 = signed 8-bit
            | (uint32_t(bSigned ? 1 : 0) << 10)
            | ((n >> 3) << 17)                 // n_dim
+           | ((m >> 4) << 24);                // m_dim
+}
+
+// Instruction descriptor of kind::mxf4 (block-scaled): D = f32, A/B e2m1 K-major, UE8M0 scale factors, dense K = 64.
+__host__ __device__ constexpr uint32_t instrDescMxf4(uint32_t m, uint32_t n)
+{
+    return (1u << 7)                          // a_format: e2m1
+           | (1u << 10)                       // b_format: e2m1
+           | ((n >> 3) << 17)                 // n_dim
+           | (1u << 23)                       // scale_format: UE8M0
            | ((m >> 4) << 24);                // m_dim
 }
 
