@@ -77,6 +77,7 @@ def lib():
     L.em2_compute_signatures.argtypes = [vp, u64, u64, vp, vp, vp, u64, vp, vp, vp]
     L.em2_find_similar_pairs.argtypes = [vp, vp, u64, u64, u64, u64, u64, dbl, i32, vp, vp]
     L.em2_lsh_similar_pairs.argtypes = [vp, u64, u64, vp, vp, vp, u64, u64, dbl, i32, vp, vp, vp]
+    L.em2_extend_similar_pairs.argtypes = [vp, vp, u64, u64, u64, u64, dbl, i32, vp, vp, vp, vp]
     L.em2_exact_similar_pairs.argtypes = [vp, u64, u64, vp, vp, u64, dbl, vp, vp]
     L.em2_cell_graph_edges.argtypes = [vp, u64, u64, vp, vp, vp, dbl, u64, vp, u64, vp]
     L.em2_signature_graph.argtypes = [vp, vp, u64, u64, u64, vp, vp, u64, vp, vp, u64, vp]
@@ -262,6 +263,30 @@ class Engine:
         self._check(self._L.em2_find_similar_pairs(self._h, _ptr(sig), n, lsh_count, row_begin, row_end, k,
                                                    similarity_threshold, variant, _ptr(out), _ptr(used)),
                     "em2_find_similar_pairs")
+        return np.ascontiguousarray(out["cell"]), np.ascontiguousarray(out["similarity"]), used
+
+    def extend_similar_pairs(self, signatures, old_cell_count: int, old_ids, old_sims, old_used, lsh_count: int, k: int,
+                             similarity_threshold: float, variant: int = VARIANT_AUTO):
+        """Lists of find_similar_pairs over signatures[:old_cell_count] (old_ids / old_sims [old, k], old_used [old]),
+        extended to the cells after them (em2_extend_similar_pairs).  Returns (ids, sims, used) for all rows, equal to
+        find_similar_pairs over all signatures.  Raises Em2Error if the old lists do not belong to these signatures, k,
+        lsh_count and threshold.  Lists made with a HIGHER threshold than this call's cannot be detected (their rows lack
+        the cells between the two thresholds) and give wrong lists; lists made with a lower threshold are rejected or
+        are already exact."""
+        sig = np.ascontiguousarray(signatures, np.uint64)
+        n = sig.shape[0]
+        old = np.zeros((old_cell_count, k), SIMPAIR_DTYPE)
+        if old_cell_count:
+            old["cell"] = np.asarray(old_ids, np.uint32).reshape(old_cell_count, k)
+            old["similarity"] = np.asarray(old_sims, np.float32).reshape(old_cell_count, k)
+        old_used = np.ascontiguousarray(old_used, np.uint32)
+        if old_used.shape != (old_cell_count,):
+            raise ValueError("old_used must hold one count per old cell")
+        out = np.zeros((n, k), SIMPAIR_DTYPE)
+        used = np.zeros(n, np.uint32)
+        self._check(self._L.em2_extend_similar_pairs(self._h, _ptr(sig), old_cell_count, n, lsh_count, k, similarity_threshold,
+                                                     variant, _ptr(old), _ptr(old_used), _ptr(out), _ptr(used)),
+                    "em2_extend_similar_pairs")
         return np.ascontiguousarray(out["cell"]), np.ascontiguousarray(out["similarity"]), used
 
     def lsh_similar_pairs(self, toc, counts, lsh_vectors, k: int, similarity_threshold: float, gene_ids=None,

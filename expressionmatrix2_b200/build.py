@@ -14,7 +14,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libem2b200.so")
-SOURCES = ["capi.cu", "signatures.cu", "sig_filter.cu", "scan_popc.cu", "scan_mma.cu", "exact.cu", "subset.cu", "cellgraph.cu", "siggraph.cu", "bucketed.cu", "multi.cu", "hostgen.cpp"]
+SOURCES = ["capi.cu", "signatures.cu", "sig_filter.cu", "scan_popc.cu", "scan_mma.cu", "extend.cu", "exact.cu", "subset.cu", "cellgraph.cu", "siggraph.cu", "bucketed.cu", "multi.cu", "hostgen.cpp"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -64,6 +64,7 @@ struct em2_context {
         S_COLLOGFILL,    // symmetric scan: entries per log chunk + the chunk allocator
         S_DIST0, S_DIST1, S_DIST2, S_DIST3,   // multi-GPU exchange buffers (multi.cu)
         S_PERM,          // scan position -> cell id
+        S_EXTEND,        // em2_extend_similar_pairs: old lists, their keys, lengths and column bounds, the validation flags
         S_COUNT
     };
     int signatureMode = 0;   // 0 auto, 1 FP64 kernel only, 2 force the tensor-core filter path
@@ -306,5 +307,11 @@ int launchScanMma(em2_context* ctx, const uint64_t* signatures, uint64_t cellCou
                   em2_pair* pairs, uint32_t* usedCount, cudaStream_t s);
 int launchMismatchBlockMma(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uint64_t lshCount,
                            uint64_t rowBegin, uint64_t rowEnd, uint16_t* out, cudaStream_t s);
+// Extension of the lists of cells [0, oldN) to the cells appended after them (scan_mma.cu; extend.cu has the entry point).
+bool extendRectEligible(const em2_context* ctx, uint64_t oldCellCount, uint64_t cellCount, uint64_t lshCount, uint64_t k,
+                        int64_t mismatchMax, int variant);
+int launchExtendRect(em2_context* ctx, const uint64_t* sig, uint64_t oldN, uint64_t N, uint64_t lshCount, uint64_t k, uint32_t tau0,
+                     const float* lut, const uint64_t* oldKeys, const uint32_t* oldUsed, const uint32_t* oldBound, em2_pair* pairs,
+                     uint32_t* usedCount, cudaStream_t s, int* overflowed);
 
 }  // namespace em2

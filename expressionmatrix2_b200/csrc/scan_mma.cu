@@ -667,6 +667,7 @@ struct SymParams {
     uint32_t* candCount;
     unsigned long long* appendedTotal;   // both directions
     uint32_t* limEx;               // per position (all N): accept iff mismatch count < limEx
+    uint32_t colDirEnd;            // the column direction only serves column positions below this (N: all of them)
     ulonglong2* colLog;            // column-direction survivors {mismatch << 32 | row cell id, column position}: a pool of
     uint32_t* chunkFill;           //   64-entry chunks; a thread takes a chunk at a time (one atomic per 64 survivors);
     uint32_t* chunkNext;           //   chunkFill[c] = valid entries of chunk c; scattered to the inboxes afterwards
@@ -869,7 +870,7 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
                     const uint32_t pos0 = colSuperOf(super, d) * kSsTileN + uint32_t(lane) * 8;
                     uint32_t lim[8];
 #pragma unroll
-                    for (int j = 0; j < 8; j++) lim[j] = pos0 + j < N ? __ldcg(p.limEx + pos0 + j) : 0u;      // padding columns: nothing passes
+                    for (int j = 0; j < 8; j++) lim[j] = pos0 + j < p.colDirEnd ? __ldcg(p.limEx + pos0 + j) : 0u;      // padding / gated columns: nothing passes
                     float t[8];
                     int32_t loosest = 0x7fffffff;
 #pragma unroll
@@ -1102,12 +1103,13 @@ scanMmaSymKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
 
 // Files the column-direction log into per-cell inboxes of exactly the needed length (count -> exclusive scan -> fill,
 // one warp per log chunk): FILL = false counts the entries per column cell, FILL = true writes them at
-// inOffset[cell] + (a running cursor per cell).
+// inOffset[cell] + (a running cursor per cell).  Entries whose row cell id is below dropBelow are left out (an extension
+// drops the pairs of two old cells, which the old lists already account for).
 template <bool FILL>
 __global__ void __launch_bounds__(256)
 scatterLogKernel(const uint32_t* __restrict__ chunkNext, uint32_t chunkCap, const ulonglong2* __restrict__ log,
                  const uint32_t* __restrict__ chunkFill, uint32_t* __restrict__ inCount, const uint32_t* __restrict__ inOffset,
-                 uint64_t* __restrict__ inbox, unsigned long long* __restrict__ appendedTotal)
+                 uint64_t* __restrict__ inbox, unsigned long long* __restrict__ appendedTotal, uint32_t dropBelow)
 {
     const uint32_t chunks = min(*chunkNext, chunkCap);
     const uint32_t lane = threadIdx.x & 31;
@@ -1116,6 +1118,7 @@ scatterLogKernel(const uint32_t* __restrict__ chunkNext, uint32_t chunkCap, cons
         if (!FILL && lane == 0 && n) atomicAdd(appendedTotal, (unsigned long long)n);      // statistics
         for (uint32_t i = lane; i < n; i += 32) {
             const ulonglong2 e = log[uint64_t(w) * kLogChunk + i];
+            if (uint32_t(e.x) < dropBelow) continue;
             const uint32_t pos = uint32_t(e.y);
             const uint32_t slot = atomicAdd(inCount + pos, 1u);
             if (FILL) inbox[uint64_t(inOffset[pos]) + slot] = e.x;
@@ -1574,6 +1577,112 @@ __global__ void fillU32Kernel(uint32_t* __restrict__ dst, uint64_t n, uint32_t v
     if (i < n) dst[i] = value;
 }
 
+// ---- pieces shared by the whole-matrix symmetric scan (runSymmetric) and the extension rectangle (runExtendRect)
+
+// Column-direction log pool, in entries: 24 k per row at least, up to 64 k when memory allows (a third of what is free;
+// log 16 B + outbox 8 B per entry).  Measured needs: 0.8 k per cell on the 1 M-cell bench workload, 25 k per cell on
+// config 3 (64 loose clusters of 20k cells spread over 8 GPUs: a rank's near window only sees its own eighth of a
+// cluster) -- which overflowed a 24 k pool and fell back to the one-directional kernels (296 instead of 116 ms).
+// Buffers only grow.
+static uint64_t symLogPoolEntries(em2_context* ctx, uint64_t rowsAlloc, uint64_t k)
+{
+    uint64_t perRow = 24;
+    const uint64_t slack = 2 * uint64_t(ctx->smCount) * kEpiThreads * kLogChunk + kLogChunk;
+    const uint64_t haveEntries = std::min<uint64_t>(ctx->scratch[em2_context::S_COLLOG].bytes / sizeof(ulonglong2),
+                                                    ctx->scratch[em2_context::S_INBOX].bytes / sizeof(uint64_t));
+    if (haveEntries >= 24 * rowsAlloc * k + slack) {
+        // buffers of an earlier call are large enough: use what they hold (cudaMemGetInfo costs milliseconds)
+        perRow = std::min<uint64_t>(64, (haveEntries - slack) / (rowsAlloc * k));
+    } else {
+        size_t freeBytes = 0, totalBytes = 0;
+        if (cudaMemGetInfo(&freeBytes, &totalBytes) != cudaSuccess) {
+            cudaGetLastError();
+            freeBytes = 0;
+        }
+        const size_t have = ctx->scratch[em2_context::S_COLLOG].bytes + ctx->scratch[em2_context::S_INBOX].bytes;
+        const uint64_t affordable = (uint64_t(freeBytes) / 3 + have) / 24 / std::max<uint64_t>(1, rowsAlloc * k);
+        perRow = std::min<uint64_t>(64, std::max<uint64_t>(24, affordable));
+    }
+    return perRow * rowsAlloc * k;
+}
+
+// Ring depth and dynamic shared memory of scanMmaSymKernel for K = 256 * panels; sets the limit of both forms.
+static int symKernelSmem(em2_context* ctx, uint32_t panels, bool pair, uint32_t* stages, size_t* smem)
+{
+    const size_t budget = 227 * 1024 - 1024 - kSymSmallBytes - size_t(panels) * kSsABytes;
+    const size_t bStageBytes = pair ? kSymHalfBytes / 2 : kSymHalfBytes;
+    *stages = uint32_t(std::min<size_t>(kSymMaxStages, budget / bStageBytes));
+    *smem = 1024 + size_t(panels) * kSsABytes + size_t(*stages) * bStageBytes + kSymSmallBytes;
+    EM2_CUDA(ctx, cudaFuncSetAttribute(scanMmaSymKernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(*smem)));
+    EM2_CUDA(ctx, cudaFuncSetAttribute(scanMmaSymKernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(*smem)));
+    return EM2_OK;
+}
+
+// One launch of scanMmaSymKernel over the p.items items: CTA pairs (clusters of two, one TPC) or single CTAs.
+static int launchSymKernel(em2_context* ctx, bool pair, uint32_t slots, size_t smem, const CUtensorMap& mapA, const CUtensorMap& mapB,
+                           const SymParams& p, cudaStream_t s)
+{
+    if (pair) {
+        cudaLaunchConfig_t cfg = {};
+        cfg.blockDim = dim3(kSymThreads);
+        cfg.dynamicSmemBytes = smem;
+        cfg.stream = s;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeClusterDimension;      // the two CTAs of a pair: one TPC
+        attr[0].val.clusterDim.x = 2;
+        attr[0].val.clusterDim.y = 1;
+        attr[0].val.clusterDim.z = 1;
+        cfg.attrs = attr;
+        cfg.numAttrs = 1;
+        cfg.gridDim = dim3(2 * std::min<uint32_t>(p.items, slots));
+        EM2_CUDA(ctx, cudaLaunchKernelEx(&cfg, scanMmaSymKernel<true>, mapA, mapB, p));
+    } else {
+        scanMmaSymKernel<false><<<unsigned(std::min<uint32_t>(p.items, slots)), kSymThreads, smem, s>>>(mapA, mapB, p);
+    }
+    EM2_CUDA(ctx, cudaGetLastError());
+    ctx->stats.kernel_launches++;
+    return EM2_OK;
+}
+
+// The log -> per-cell inboxes in position order: count per column cell, exclusive scan, fill.  inCount holds N + 1
+// zeros on entry; inOffset[N] is the total afterwards.
+static int fileColumnLog(em2_context* ctx, const SymParams& p, uint64_t N, uint32_t* inCount, uint32_t* inOffset, uint64_t* outbox,
+                         void* cubTemp, size_t cubBytes, uint32_t dropBelow, cudaStream_t s)
+{
+    scatterLogKernel<false><<<unsigned(ctx->smCount) * 8, 256, 0, s>>>(p.chunkNext, p.chunkCap, p.colLog, p.chunkFill, inCount, nullptr,
+                                                                      nullptr, p.appendedTotal, dropBelow);
+    EM2_CUDA(ctx, cudaGetLastError());
+    // inCount[N] is 0: inOffset[N] = total
+    EM2_CUDA(ctx, cub::DeviceScan::ExclusiveSum(cubTemp, cubBytes, inCount, inOffset, int(N + 1), s));
+    EM2_CUDA(ctx, cudaMemsetAsync(inCount, 0, N * sizeof(uint32_t), s));
+    scatterLogKernel<true><<<unsigned(ctx->smCount) * 8, 256, 0, s>>>(p.chunkNext, p.chunkCap, p.colLog, p.chunkFill, inCount, inOffset,
+                                                                     outbox, p.appendedTotal, dropBelow);
+    EM2_CUDA(ctx, cudaGetLastError());
+    ctx->stats.kernel_launches += 2;      // + the scan's own kernels (library code, not counted)
+    return EM2_OK;
+}
+
+// finalizeSymKernel over `rows` cells.  Staging: 16-bit mismatch counts of everything below the bound (cells with longer
+// lists bisect in place), then the k best keys plus the ties at the k-th place.
+static int launchFinalizeSym(em2_context* ctx, uint64_t rows, uint64_t posBegin, uint32_t streams, uint32_t cap, uint64_t k,
+                             const uint64_t* cand, const uint32_t* candCount, const InboxSources& src, const uint32_t* limEx,
+                             const float* lut, em2_pair* pairs, uint32_t* usedCount, const uint32_t* perm, uint32_t* overflow,
+                             cudaStream_t s)
+{
+    if (!rows) return EM2_OK;
+    const uint32_t hamsPerWarp = uint32_t(roundUp(uint64_t(streams) * cap + 40 * k + 256, 64));
+    const uint32_t keysPerWarp = uint32_t(roundUp(2 * k + 256, 64));
+    const size_t smemF = size_t(kSymFinalWarps) * (size_t(keysPerWarp) * sizeof(uint64_t) + size_t(hamsPerWarp) * sizeof(uint16_t));
+    if (smemF > 200 * 1024) return fail(ctx, EM2_ERR_INVALID, "k too large for the symmetric finalize kernel");
+    EM2_CUDA(ctx, cudaFuncSetAttribute(finalizeSymKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemF)));
+    finalizeSymKernel<<<unsigned((rows + kSymFinalWarps - 1) / kSymFinalWarps), kSymFinalWarps * 32, smemF, s>>>(
+        uint32_t(rows), uint32_t(posBegin), streams, cap, uint32_t(k), cand, candCount, src, limEx, lut, pairs, usedCount, perm,
+        overflow, hamsPerWarp, keysPerWarp);
+    EM2_CUDA(ctx, cudaGetLastError());
+    ctx->stats.kernel_launches++;
+    return EM2_OK;
+}
+
 // Symmetric scan: every unordered pair of cells is evaluated once -- on one GPU or across the GPUs of a job.
 //   encP    FP4 encoding (encodeFp4Kernel) of ALL N cells in scan-position order (rows and columns), K bits (a multiple
 //           of 256) = K / 2 bytes per cell
@@ -1663,32 +1772,8 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
     void *cand = nullptr, *candCount = nullptr, *counters = nullptr, *sym = nullptr, *outbox = nullptr, *colLog = nullptr,
          *chunkFill = nullptr, *cubTemp = nullptr, *dist0 = nullptr, *dist2 = nullptr;
     const uint64_t rowsAlloc = std::max<uint64_t>(ownRows, 1);
-    // column-direction log pool: 24 k entries per row on average (measured: 1.5-12 k per cell on clustered data); the
-    // outbox is cut from a buffer of the same number of keys (count -> scan -> fill)
-    // 24 k entries per row at least, up to 64 k when memory allows (a third of what is free; log 16 B + outbox 8 B per
-    // entry).  Measured needs: 0.8 k per cell on the 1 M-cell bench workload, 25 k per cell on config 3 (64 loose clusters
-    // of 20k cells spread over 8 GPUs: a rank's near window only sees its own eighth of a cluster) -- which overflowed a
-    // 24 k pool and fell back to the one-directional kernels (296 instead of 116 ms).  Buffers only grow.
-    uint64_t perRow = 24;
-    {
-        const uint64_t slack = 2 * uint64_t(ctx->smCount) * kEpiThreads * kLogChunk + kLogChunk;
-        const uint64_t haveEntries = std::min<uint64_t>(ctx->scratch[em2_context::S_COLLOG].bytes / sizeof(ulonglong2),
-                                                        ctx->scratch[em2_context::S_INBOX].bytes / sizeof(uint64_t));
-        if (haveEntries >= 24 * rowsAlloc * k + slack) {
-            // buffers of an earlier call are large enough: use what they hold (cudaMemGetInfo costs milliseconds)
-            perRow = std::min<uint64_t>(64, (haveEntries - slack) / (rowsAlloc * k));
-        } else {
-            size_t freeBytes = 0, totalBytes = 0;
-            if (cudaMemGetInfo(&freeBytes, &totalBytes) != cudaSuccess) {
-                cudaGetLastError();
-                freeBytes = 0;
-            }
-            const size_t have = ctx->scratch[em2_context::S_COLLOG].bytes + ctx->scratch[em2_context::S_INBOX].bytes;
-            const uint64_t affordable = (uint64_t(freeBytes) / 3 + have) / 24 / std::max<uint64_t>(1, rowsAlloc * k);
-            perRow = std::min<uint64_t>(64, std::max<uint64_t>(24, affordable));
-        }
-    }
-    const uint64_t poolEntries = std::min<uint64_t>(0xf0000000ull * uint64_t(kLogChunk) / 64, perRow * rowsAlloc * k + 2 * uint64_t(ctx->smCount) * kEpiThreads * kLogChunk);
+    // column-direction log pool (symLogPoolEntries); the outbox is cut from a buffer of the same number of keys
+    const uint64_t poolEntries = std::min<uint64_t>(0xf0000000ull * uint64_t(kLogChunk) / 64, symLogPoolEntries(ctx, rowsAlloc, k) + 2 * uint64_t(ctx->smCount) * kEpiThreads * kLogChunk);
     const uint32_t chunkCap = uint32_t(std::min<uint64_t>(0xfffffff0ull, poolEntries / kLogChunk));
     size_t cubBytes = 0, cubBytes2 = 0;
     cub::DeviceScan::ExclusiveSum(nullptr, cubBytes, static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), int(N + 1), s);
@@ -1763,9 +1848,8 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
     p.cellCount = N;
     p.K = K;
     p.panels = panels;
-    const size_t budget = 227 * 1024 - 1024 - kSymSmallBytes - size_t(panels) * kSsABytes;
-    const size_t bStageBytes = pair ? kSymHalfBytes / 2 : kSymHalfBytes;
-    p.stages = uint32_t(std::min<size_t>(kSymMaxStages, budget / bStageBytes));
+    size_t smem = 0;
+    EM2_TRY(symKernelSmem(ctx, panels, pair, &p.stages, &smem));
     p.superBlocks = S;
     p.halfOffset = S % 2 == 0 ? S / 2 : 0;
     p.posBegin = uint32_t(posBegin);
@@ -1776,6 +1860,7 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
     p.candCount = static_cast<uint32_t*>(candCount);
     p.appendedTotal = appended;
     p.limEx = limEx;
+    p.colDirEnd = uint32_t(N);
     p.colLog = static_cast<ulonglong2*>(colLog);
     p.chunkFill = static_cast<uint32_t*>(chunkFill);
     p.chunkNext = chunkNext;
@@ -1786,9 +1871,6 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
     CUtensorMap mapA, mapB;
     EM2_TRY(makeTensorMapU8(ctx, &mapA, encP, N, K / 2, K / 2, kRowsPerItem));
     EM2_TRY(makeTensorMapU8(ctx, &mapB, encP, N, K / 2, K / 2, pair ? kSymHalfN / 2 : kSymHalfN));
-    const size_t smem = 1024 + size_t(panels) * kSsABytes + size_t(p.stages) * bStageBytes + kSymSmallBytes;
-    EM2_CUDA(ctx, cudaFuncSetAttribute(scanMmaSymKernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    EM2_CUDA(ctx, cudaFuncSetAttribute(scanMmaSymKernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     auto sweep = [&](const ScanPlan& pl, int32_t dBegin, uint32_t count, uint32_t resume, uint32_t rowOnly) -> int {
         if (!ownRows || !count) return EM2_OK;
         p.segBase = resume ? nearPlan.segments - 1 : 0;
@@ -1804,26 +1886,7 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
         // (390 tiles per item) the sweep was 1.5x SLOWER, at 1 M cells (1953 tiles) 1.2x faster
         p.progress = (count >= 768 && !(ctx->debugFlags & 16)) ? progress : nullptr;
         if (p.progress) EM2_CUDA(ctx, cudaMemsetAsync(progress, 0, 1024 * sizeof(uint32_t), s));
-        if (pair) {
-            cudaLaunchConfig_t cfg = {};
-            cfg.blockDim = dim3(kSymThreads);
-            cfg.dynamicSmemBytes = smem;
-            cfg.stream = s;
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeClusterDimension;      // the two CTAs of a pair: one TPC
-            attr[0].val.clusterDim.x = 2;
-            attr[0].val.clusterDim.y = 1;
-            attr[0].val.clusterDim.z = 1;
-            cfg.attrs = attr;
-            cfg.numAttrs = 1;
-            cfg.gridDim = dim3(2 * std::min<uint32_t>(pl.items, slots));
-            EM2_CUDA(ctx, cudaLaunchKernelEx(&cfg, scanMmaSymKernel<true>, mapA, mapB, p));
-        } else {
-            scanMmaSymKernel<false><<<unsigned(std::min<uint32_t>(pl.items, slots)), kSymThreads, smem, s>>>(mapA, mapB, p);
-        }
-        EM2_CUDA(ctx, cudaGetLastError());
-        ctx->stats.kernel_launches++;
-        return EM2_OK;
+        return launchSymKernel(ctx, pair, slots, smem, mapA, mapB, p, s);
     };
     phase("set-up");
     // ---- 1. near window
@@ -1836,16 +1899,7 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
     EM2_TRY(sweep(farPlan, int32_t(farBegin), farCount, 1, 0));
     report("far sweep");
     // ---- 4. log -> outbox in position order: count per column cell, exclusive scan, fill
-    scatterLogKernel<false><<<unsigned(ctx->smCount) * 8, 256, 0, s>>>(chunkNext, chunkCap, p.colLog, p.chunkFill, inCount, nullptr,
-                                                                      nullptr, appended);
-    EM2_CUDA(ctx, cudaGetLastError());
-    // inCount[N] is 0: inOffset[N] = total
-    EM2_CUDA(ctx, cub::DeviceScan::ExclusiveSum(cubTemp, cubBytes, inCount, inOffset, int(N + 1), s));
-    EM2_CUDA(ctx, cudaMemsetAsync(inCount, 0, N * sizeof(uint32_t), s));
-    scatterLogKernel<true><<<unsigned(ctx->smCount) * 8, 256, 0, s>>>(chunkNext, chunkCap, p.colLog, p.chunkFill, inCount, inOffset,
-                                                                     static_cast<uint64_t*>(outbox), appended);
-    EM2_CUDA(ctx, cudaGetLastError());
-    ctx->stats.kernel_launches += 2;      // + the scan's own kernels (library code, not counted)
+    EM2_TRY(fileColumnLog(ctx, p, N, inCount, inOffset, static_cast<uint64_t*>(outbox), cubTemp, cubBytes, 0, s));
     phase("log filing");
 
     InboxSources src{};
@@ -1911,20 +1965,9 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
         src.count = uint32_t(P);
         phase("candidate exchange");
     }
-    // ---- 5. merge.  Staging: 16-bit mismatch counts of everything below the bound (cells with longer lists bisect in
-    // place), then the k best keys plus the ties at the k-th place
-    if (ownRows) {
-        const uint32_t hamsPerWarp = uint32_t(roundUp(uint64_t(streams) * cap + 40 * k + 256, 64));
-        const uint32_t keysPerWarp = uint32_t(roundUp(2 * k + 256, 64));
-        const size_t smemF = size_t(kSymFinalWarps) * (size_t(keysPerWarp) * sizeof(uint64_t) + size_t(hamsPerWarp) * sizeof(uint16_t));
-        if (smemF > 200 * 1024) return fail(ctx, EM2_ERR_INVALID, "k too large for the symmetric finalize kernel");
-        EM2_CUDA(ctx, cudaFuncSetAttribute(finalizeSymKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemF)));
-        finalizeSymKernel<<<unsigned((ownRows + kSymFinalWarps - 1) / kSymFinalWarps), kSymFinalWarps * 32, smemF, s>>>(
-            uint32_t(ownRows), uint32_t(posBegin), streams, cap, uint32_t(k), p.cand, p.candCount, src, limEx, lut, pairs, usedCount, perm,
-            overflow, hamsPerWarp, keysPerWarp);
-        EM2_CUDA(ctx, cudaGetLastError());
-        ctx->stats.kernel_launches++;
-    }
+    // ---- 5. merge
+    EM2_TRY(launchFinalizeSym(ctx, ownRows, posBegin, streams, cap, k, p.cand, p.candCount, src, limEx, lut, pairs, usedCount, perm,
+                              overflow, s));
     // the overflow flag decides whether the result stands (P > 1: the log pools were checked job-wide above; what is
     // left is this rank's own merge guard)
     EM2_CUDA(ctx, cudaMemcpyAsync(matrixHost, overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
@@ -2285,6 +2328,158 @@ int launchMismatchBlockMma(em2_context* ctx, const uint64_t* signatures, uint64_
 {
     return runMma(ctx, signatures, cellCount, lshCount, rowBegin, rowEnd, 1, int64_t(lshCount), nullptr, nullptr,
                   nullptr, out, s);
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Extension of a finished job (em2_extend_similar_pairs): the lists of the cells [0, oldN) are final, cells [oldN, N) were
+// appended.  Every new id is larger than every old id, so the full-rerun list of an old cell c is the k best of its old
+// list and the new cells that beat its k-th entry; a new cell needs an ordinary row scan over all N columns.
+//
+// One launch of scanMmaSymKernel on a RECTANGLE: the own rows are the positions [N0, N), N0 = oldN rounded down to 256
+// (the new cells and the at most 255 old cells of the boundary super block, whose lists the row direction recomputes in
+// full), and every row block visits every column super block once (dBegin = 0, S offsets).  Positions are cell ids.
+//   row direction     complete lists of the own rows, as in a whole-matrix scan;
+//   column direction  gated to the columns below N0 (colDirEnd), which carry the FINAL bounds of the validated old lists:
+//                     the k-th entry's mismatch count when the list is full, else tau0.  "Beats the k-th entry" is then
+//                     exactly mismatch < bound, the kernel's exclusive test.  Survivors are filed into inboxes; the
+//                     boundary cells' entries (old-old pairs, already in the old lists) are dropped while filing.
+// Merge: own rows as in runSymmetric (their inboxes are empty); rows below N0 run the same merge kernel with the old keys
+// as their one stream (bound tau0: every key qualifies).  Each pair of a new cell and a cell below N0 is evaluated once;
+// pairs of two own rows once from each side (both rows need them in their row direction).
+bool extendRectEligible(const em2_context* ctx, uint64_t oldCellCount, uint64_t cellCount, uint64_t lshCount, uint64_t k,
+                        int64_t mismatchMax, int variant)
+{
+    if (ctx->world != 1 || variant == EM2_VARIANT_POPC || mismatchMax < 0 || lshCount > kMaxPanels * kChunkBytes) return false;
+    if (oldCellCount == 0 || oldCellCount >= cellCount || cellCount > 0x7fffff00ull) return false;
+    if (scanCandidateCapacity(uint32_t(k), uint32_t(ctx->candCapExtra)) > 32 * kPruneRegsPerLane) return false;
+    if (ctx->scanSymmetric == 1) return false;
+    // AUTO: whenever the appended cells are at most as many as the old ones (beyond that the rectangle's own rows are most
+    // of a whole-matrix job, which the symmetric scan does in half the pair evaluations)
+    return ctx->scanSymmetric == 2 || cellCount - oldCellCount <= oldCellCount;
+}
+
+// sig: all N cells (device).  oldKeys [oldN][k]: the validated old lists as {mismatch << 32 | id}, oldUsed their lengths,
+// oldBound the column bounds described above.  pairs / usedCount: all N rows (device).  *overflowed != 0: a capacity ran
+// out and nothing written may be used.
+int launchExtendRect(em2_context* ctx, const uint64_t* sig, uint64_t oldN, uint64_t N, uint64_t lshCount, uint64_t k, uint32_t tau0,
+                     const float* lut, const uint64_t* oldKeys, const uint32_t* oldUsed, const uint32_t* oldBound, em2_pair* pairs,
+                     uint32_t* usedCount, cudaStream_t s, int* overflowed)
+{
+    *overflowed = 0;
+    const uint32_t W = uint32_t(wordCount(lshCount));
+    const uint32_t K = uint32_t(roundUp(lshCount, kSymKBits));
+    const uint32_t panels = K / kSymKBits;
+    const uint64_t N0 = oldN / kSsTileN * kSsTileN;
+    const uint64_t ownRows = N - N0;
+    const uint32_t S = uint32_t((N + kSsTileN - 1) / kSsTileN);
+    const bool pair = ctx->symCtaPair != 1 && ctx->smCount >= 2;
+    const uint32_t rowsPerItem = pair ? kPairRows : kRowsPerItem;
+    const uint32_t slots = pair ? uint32_t(ctx->smCount / 2) : uint32_t(ctx->smCount);
+    ScanPlan plan = makeScanPlan(ctx, ownRows, uint64_t(S) * kSsTileN, k, kSsTileN, rowsPerItem, 1, kSubStreams, slots);
+    plan.cap = candidateCapacity(uint32_t(k)) + uint32_t(k) * uint32_t(ctx->candCapExtra);
+    const uint32_t streams = plan.segments * kSubStreams;
+
+    // column-direction traffic goes onto the N0 old cells: at most N0 entries per own row, sized like the whole-matrix
+    // scan's pool per own row plus k per old cell
+    const uint64_t slack = 2 * uint64_t(ctx->smCount) * kEpiThreads * kLogChunk;
+    const uint64_t want = std::min<uint64_t>(N0 * ownRows, symLogPoolEntries(ctx, ownRows, k) + N0 * k);
+    const uint64_t poolEntries = std::min<uint64_t>(0xf0000000ull * uint64_t(kLogChunk) / 64, want + slack);
+    // debug_flags bit 6: a pool of one chunk, so that the overflow fallback can be exercised
+    const uint32_t chunkCap = (ctx->debugFlags & 64) ? 1u : uint32_t(std::min<uint64_t>(0xfffffff0ull, (poolEntries + kLogChunk - 1) / kLogChunk));
+    size_t cubBytes = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, cubBytes, static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), int(N + 1), s);
+    void *enc = nullptr, *cand = nullptr, *candCount = nullptr, *counters = nullptr, *sym = nullptr, *outbox = nullptr,
+         *colLog = nullptr, *chunkFill = nullptr, *cubTemp = nullptr, *pin = nullptr;
+    EM2_TRY(reserve(ctx, em2_context::S_ENCROWS, N * uint64_t(K / 2), &enc));
+    EM2_TRY(reserve(ctx, em2_context::S_CAND, size_t(streams) * ownRows * plan.cap * sizeof(uint64_t), &cand));
+    EM2_TRY(reserve(ctx, em2_context::S_CANDCOUNT, size_t(streams) * ownRows * sizeof(uint32_t), &candCount));
+    EM2_TRY(reserve(ctx, em2_context::S_COUNTERS, 64, &counters));
+    // [limEx N][inCount N + 1][inOffset N + 1][overflow 8][progress 1024]
+    EM2_TRY(reserve(ctx, em2_context::S_SYM, (3 * N + 2 + 8 + 1024) * sizeof(uint32_t), &sym));
+    EM2_TRY(reserve(ctx, em2_context::S_INBOX, size_t(chunkCap) * kLogChunk * sizeof(uint64_t), &outbox));
+    EM2_TRY(reserve(ctx, em2_context::S_COLLOG, (size_t(chunkCap) + 1) * kLogChunk * sizeof(ulonglong2), &colLog));   // + spill chunk
+    EM2_TRY(reserve(ctx, em2_context::S_COLLOGFILL, (size_t(chunkCap) + 4) * sizeof(uint32_t), &chunkFill));
+    EM2_TRY(reserve(ctx, em2_context::S_MISC, cubBytes, &cubTemp));
+    EM2_TRY(reservePinned(ctx, 2, 64, &pin));
+    uint32_t* limEx = static_cast<uint32_t*>(sym);
+    uint32_t* inCount = limEx + N;
+    uint32_t* inOffset = inCount + N + 1;
+    uint32_t* overflow = inOffset + N + 1;
+    uint32_t* progress = overflow + 8;
+
+    EM2_TRY(encodeFp4(ctx, sig, W, N, K, static_cast<uint8_t*>(enc), nullptr, s));
+    EM2_CUDA(ctx, cudaMemsetAsync(chunkFill, 0, (size_t(chunkCap) + 4) * sizeof(uint32_t), s));
+    EM2_CUDA(ctx, cudaMemsetAsync(inCount, 0, (N + 1) * sizeof(uint32_t), s));
+    EM2_CUDA(ctx, cudaMemsetAsync(overflow, 0, 8 * sizeof(uint32_t), s));
+    EM2_CUDA(ctx, cudaMemsetAsync(candCount, 0, size_t(streams) * ownRows * sizeof(uint32_t), s));
+    if (N0) EM2_CUDA(ctx, cudaMemcpyAsync(limEx, oldBound, N0 * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
+    fillU32Kernel<<<unsigned((ownRows + 255) / 256), 256, 0, s>>>(limEx + N0, ownRows, tau0);
+    EM2_CUDA(ctx, cudaGetLastError());
+    ctx->stats.kernel_launches++;
+
+    SymParams p{};
+    p.cellCount = N;
+    p.K = K;
+    p.panels = panels;
+    size_t smem = 0;
+    EM2_TRY(symKernelSmem(ctx, panels, pair, &p.stages, &smem));
+    p.mainBlocks = plan.mainBlocks;
+    p.segments = plan.segments;
+    p.items = plan.items;
+    p.segmentCols = plan.segmentCols;
+    p.superBlocks = S;
+    p.halfOffset = 0;          // every column super block is visited by this row block only: no offset is seen twice
+    p.dBegin = 0;
+    p.offsetsHere = S;
+    p.resume = 0;
+    p.segBase = 0;
+    p.rowOnly = 0;
+    p.posBegin = uint32_t(N0);
+    p.ownRows = uint32_t(ownRows);
+    p.k = uint32_t(k);
+    p.cap = plan.cap;
+    p.cand = static_cast<uint64_t*>(cand);
+    p.candCount = static_cast<uint32_t*>(candCount);
+    p.appendedTotal = static_cast<unsigned long long*>(counters) + 1;
+    p.limEx = limEx;
+    p.colDirEnd = uint32_t(N0);
+    p.colLog = static_cast<ulonglong2*>(colLog);
+    p.chunkFill = static_cast<uint32_t*>(chunkFill);
+    p.chunkNext = static_cast<uint32_t*>(chunkFill) + chunkCap;
+    p.chunkCap = chunkCap;
+    p.overflow = overflow;
+    p.perm = nullptr;
+    p.flags = uint32_t(ctx->debugFlags);
+    // pacing as in the whole-matrix scan's far sweep: only for rows long enough for the CTAs to drift apart
+    p.progress = (S >= 768 && !(ctx->debugFlags & 16)) ? progress : nullptr;
+    if (p.progress) EM2_CUDA(ctx, cudaMemsetAsync(progress, 0, 1024 * sizeof(uint32_t), s));
+    CUtensorMap mapA, mapB;
+    EM2_TRY(makeTensorMapU8(ctx, &mapA, enc, N, K / 2, K / 2, kRowsPerItem));
+    EM2_TRY(makeTensorMapU8(ctx, &mapB, enc, N, K / 2, K / 2, pair ? kSymHalfN / 2 : kSymHalfN));
+    EM2_TRY(launchSymKernel(ctx, pair, slots, smem, mapA, mapB, p, s));
+    EM2_TRY(fileColumnLog(ctx, p, N, inCount, inOffset, static_cast<uint64_t*>(outbox), cubTemp, cubBytes, uint32_t(oldN), s));
+
+    InboxSources src{};
+    src.count = 1;
+    src.keys[0] = static_cast<const uint64_t*>(outbox);
+    src.offsets[0] = inOffset + N0;      // own rows: indexed by position - N0 (their inboxes are empty)
+    EM2_TRY(launchFinalizeSym(ctx, ownRows, N0, streams, plan.cap, k, p.cand, p.candCount, src, limEx, lut, pairs + N0 * k,
+                              usedCount + N0, nullptr, overflow, s));
+    if (N0) {
+        // old rows: the old keys are the one stream, the inbox holds the new cells that beat the k-th entry; every key is
+        // below tau0, which becomes the merge bound
+        fillU32Kernel<<<unsigned((N0 + 255) / 256), 256, 0, s>>>(limEx, N0, tau0);
+        EM2_CUDA(ctx, cudaGetLastError());
+        ctx->stats.kernel_launches++;
+        src.offsets[0] = inOffset;
+        EM2_TRY(launchFinalizeSym(ctx, N0, 0, 1, uint32_t(k), k, oldKeys, oldUsed, src, limEx, lut, pairs, usedCount, nullptr,
+                                  overflow, s));
+    }
+    uint32_t* host = static_cast<uint32_t*>(pin);
+    EM2_CUDA(ctx, cudaMemcpyAsync(host, overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    EM2_CUDA(ctx, cudaStreamSynchronize(s));
+    *overflowed = int(*host);
+    return EM2_OK;
 }
 
 }  // namespace em2

@@ -220,6 +220,47 @@ void ExpressionMatrix::findSimilarPairs4(const std::string& geneSetName, const s
     findSimilarPairs4(std::cout, geneSetName, cellSetName, similarPairsName, k, similarityThreshold, lshCount, seed);
 }
 
+void ExpressionMatrix::extendSimilarPairs4(const std::string& oldName, const std::string& newName, double similarityThreshold,
+                                           size_t lshCount, unsigned int seed)
+{
+    if (newName == oldName)
+        throw std::runtime_error("extendSimilarPairs4: the new SimilarPairs object needs a name other than " + oldName + ".");
+    if (lshCount == 0 || lshCount > 65535) throw std::runtime_error("extendSimilarPairs4: lshCount must be in [1, 65535] on the GPU path.");
+    // the old object, opened for a cell set that may have grown by appending (gene set unchanged, old ids a prefix)
+    const SimilarPairs oldPairs(directoryName, oldName, SimilarPairs::AppendedCells{});
+    const std::string geneSetName = oldPairs.geneSetName(), cellSetName = oldPairs.cellSetName();
+    const GeneSet& geneSet = findGeneSet(geneSetName);
+    const CellSet& cellSet = findCellSet(cellSetName);
+    const size_t k = oldPairs.k();
+    const CellId oldCount = oldPairs.storedCellCount(), n = CellId(cellSet.size());
+    Gpu& gpu = Gpu::instance();            // throws without a device: before anything is written to the data directory
+
+    // signatures of the current cell set, as computeLshSignatures makes them, in a temporary Lsh object
+    ExpressionMatrixSubset subset(directoryName + "/tmp-ExpressionMatrixSubset-" + newName, geneSet, cellSet, cellExpressionCounts);
+    Lsh lsh(directoryName + "/tmp-Lsh-" + newName, subset, lshCount, seed);
+    lastSignatureMs = gpu.stats().signatures_ms;
+    std::vector<uint32_t> oldUsed(oldCount), used(n);
+    for (CellId c = 0; c < oldCount; c++) oldUsed[c] = uint32_t(oldPairs.size(c));
+    try {
+        SimilarPairs similarPairs(directoryName, newName, geneSetName, cellSetName, k);
+        try {
+            gpu.check(em2_extend_similar_pairs(gpu.context(), lsh.getSignature(0).begin, oldCount, n, lshCount, k, similarityThreshold,
+                                               scanVariant, reinterpret_cast<const em2_pair*>(oldPairs.begin(0)), oldUsed.data(),
+                                               reinterpret_cast<em2_pair*>(similarPairs.begin(0)), used.data()),
+                      "em2_extend_similar_pairs");
+        } catch (...) {
+            similarPairs.remove();      // no valid-looking SimilarPairs-<new> set stays behind a failed call
+            throw;
+        }
+        similarPairs.setUsedCounts(used);
+    } catch (...) {
+        lsh.remove();
+        throw;
+    }
+    lsh.remove();
+    lastScanMs = gpu.stats().scan_ms;
+}
+
 void ExpressionMatrix::computeLshSignatures(const std::string& geneSetName, const std::string& cellSetName,
                                             const std::string& lshName, size_t lshCount, unsigned int seed)
 {

@@ -50,6 +50,13 @@ public:
     void findSimilarPairs4(std::ostream&, const std::string& geneSetName, const std::string& cellSetName,
                            const std::string& similarPairsName, size_t k, double similarityThreshold, size_t lshCount,
                            unsigned int seed);
+    // The lists of SimilarPairs-<similarPairsName>, made by findSimilarPairs4 before cells were appended to its cell
+    // set, extended to the appended cells: SimilarPairs-<newSimilarPairsName> on the current cell set holds what
+    // findSimilarPairs4 would store for it.  similarityThreshold, lshCount and seed must be those of the old call (the
+    // old object does not record them): other signatures or a higher threshold are detected and throw, a LOWER
+    // threshold than the old call's is not and gives wrong lists.  The old object is not modified.
+    void extendSimilarPairs4(const std::string& similarPairsName, const std::string& newSimilarPairsName,
+                             double similarityThreshold, size_t lshCount, unsigned int seed);
     // Persistent signatures (reference src/ExpressionMatrixLsh.cpp:1150-1192): files Lsh-<lshName>-*.
     void computeLshSignatures(const std::string& geneSetName, const std::string& cellSetName,
                               const std::string& lshName, size_t lshCount, unsigned int seed);

@@ -96,6 +96,11 @@ PYBIND11_MODULE(ExpressionMatrix2, module)
              "(candidate order and lists of the reference's findSimilarPairs7).",
              arg("geneSetName") = "AllGenes", arg("cellSetName") = "AllCells", arg("lshName"), arg("similarPairsName"),
              arg("k") = 100, arg("similarityThreshold") = 0.2, arg("lshSliceLengths"), arg("maxCheck"), arg("log2BucketCount"))
+        .def("extendSimilarPairs4", &ExpressionMatrix::extendSimilarPairs4,
+             "Extends the lists of an existing findSimilarPairs4 object to the cells appended to its cell set since; "
+             "the result is what findSimilarPairs4 would store on the grown cell set.  The old object is not modified.",
+             arg("similarPairsName"), arg("newSimilarPairsName"), arg("similarityThreshold") = 0.2, arg("lshCount") = 1024,
+             arg("seed") = 231)
         .def("computeLshSignatures", &ExpressionMatrix::computeLshSignatures, arg("geneSetName") = "AllGenes",
              arg("cellSetName") = "AllCells", arg("lshName"), arg("lshCount") = 1024, arg("seed") = 231)
         .def_readwrite("scanVariant", &ExpressionMatrix::scanVariant)

@@ -35,6 +35,16 @@ SimilarPairs::SimilarPairs(const std::string& dir, const std::string& name, cons
 
 SimilarPairs::SimilarPairs(const std::string& dir, const std::string& name, bool /*allowReadOnly*/)
 {
+    accessExisting(dir, name, false);
+}
+
+SimilarPairs::SimilarPairs(const std::string& dir, const std::string& name, AppendedCells)
+{
+    accessExisting(dir, name, true);
+}
+
+void SimilarPairs::accessExisting(const std::string& dir, const std::string& name, bool cellSetMayHaveGrown)
+{
     const std::string base = pathBase(dir, name);
     info.accessExistingReadOnly(base + "-Info");
     accessSets(dir, info->geneSetName, info->cellSetName);
@@ -43,12 +53,19 @@ SimilarPairs::SimilarPairs(const std::string& dir, const std::string& name, bool
     if (geneSet.genes().hash() != info->geneSetHash)
         throw std::runtime_error("Hash for gene set " + std::string(info->geneSetName) +
                                  " is not consistent with the value at the time SimilarPairs object " + name + " was created.");
-    if (cellSet.hash() != info->cellSetHash)
+    // the stored rows are those of the first cellInfo.size() cells of the set; a set that only grew by appending still
+    // starts with exactly those ids
+    const size_t rows = cellSetMayHaveGrown ? cellInfo.size() : cellSet.size();
+    if (cellSetMayHaveGrown && (cellSet.size() < rows ||
+                                murmurHash64A(cellSet.begin(), rows * sizeof(CellId), 231) != info->cellSetHash))
+        throw std::runtime_error("Cell set " + std::string(info->cellSetName) + " does not start with the cells SimilarPairs object " +
+                                 name + " was created for: it changed other than by appending cells.");
+    if (!cellSetMayHaveGrown && cellSet.hash() != info->cellSetHash)
         throw std::runtime_error("Hash for cell set " + std::string(info->cellSetName) +
                                  " is not consistent with the value at the time SimilarPairs object " + name + " was created.");
-    if (similarPairs.size() != info->k * size_t(cellSet.size()))
+    if (similarPairs.size() != info->k * rows)
         throw std::runtime_error("SimilarPairs object " + name + " has similarPairs vector of inconsistent length.");
-    if (cellInfo.size() != cellSet.size())
+    if (cellInfo.size() != rows)
         throw std::runtime_error("SimilarPairs object " + name + " has cellInfo vector of inconsistent length.");
 }
 

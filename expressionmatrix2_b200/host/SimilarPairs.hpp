@@ -25,8 +25,16 @@ public:
                  const std::string& cellSetName, size_t k);
     // Access an existing object; throws if the gene set or cell set changed since it was created.
     SimilarPairs(const std::string& directoryName, const std::string& similarPairsName, bool allowReadOnly);
+    // Access an existing object whose cell set may have grown by appending since it was created: the gene set must be
+    // unchanged and the first storedCellCount() ids of the cell set must hash to the stored value; the rows are those of
+    // the first storedCellCount() cells (extendSimilarPairs4).
+    struct AppendedCells {};
+    SimilarPairs(const std::string& directoryName, const std::string& similarPairsName, AppendedCells);
 
     size_t k() const { return info->k; }
+    CellId storedCellCount() const { return CellId(cellInfo.size()); }
+    std::string geneSetName() const { return std::string(info->geneSetName); }
+    std::string cellSetName() const { return std::string(info->cellSetName); }
     CellId cellCount() const { return CellId(cellSet.size()); }
     size_t size(CellId cellId) const { return cellInfo[cellId].usedCount; }
     Pair* begin(CellId cellId) { return similarPairs.begin() + size_t(cellId) * k(); }
@@ -84,6 +92,7 @@ private:
     GeneSet geneSet;
     CellSet cellSet;
     void accessSets(const std::string& directoryName, const std::string& geneSetName, const std::string& cellSetName);
+    void accessExisting(const std::string& directoryName, const std::string& similarPairsName, bool cellSetMayHaveGrown);
     void addOne(CellId cellId, Pair pair);
     static std::string pathBase(const std::string& directoryName, const std::string& similarPairsName)
     {

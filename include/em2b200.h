@@ -141,7 +141,9 @@ int em2_get_stats(const em2_context* ctx, em2_stats* stats);
  *   "stage_threads"    host threads that copy a pageable buffer into / out of the pinned bounce buffers (0 = 4)
  *   "no_bounce"        1 = pageable host buffers go straight to cudaMemcpyAsync instead of through the pinned bounce buffers
  *   "debug_flags"      bit 0: no bound sharing between the MMA scan's sub-streams; bit 3: candidate counters of the
- *                      symmetric scan's phases; bit 5: wall-clock time of its phases (both print to stderr and synchronise) */
+ *                      symmetric scan's phases; bit 5: wall-clock time of its phases (both print to stderr and synchronise);
+ *                      bit 6: em2_extend_similar_pairs gets a column-direction log of one 64-entry chunk (its overflow
+ *                      fallback, for tests) */
 int em2_set_option(em2_context* ctx, const char* name, int64_t value);
 
 /* ------------------------------------------------------------------------------------------------
@@ -176,6 +178,28 @@ int em2_compute_signatures(em2_context* ctx, uint64_t cellCount, uint64_t geneCo
 int em2_find_similar_pairs(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uint64_t lshCount,
                            uint64_t rowBegin, uint64_t rowEnd, uint64_t k, double similarityThreshold,
                            int variant, em2_pair* pairs, uint32_t* usedCount);
+
+/* Lists of a findSimilarPairs4 job over cells [0, oldCellCount), extended to the cells appended after them
+ * (ExpressionMatrix::addCells appends, so the new cells get the ids oldCellCount..cellCount-1).
+ * signatures: uint64[cellCount*W] of ALL cells, old cells first, bit-identical to those the old lists were made from.
+ * oldPairs/oldUsedCount: rows [0, oldCellCount) as em2_find_similar_pairs wrote them with the same lshCount, k and
+ * similarityThreshold.  pairs/usedCount: all cellCount rows; must not overlap the old buffers.
+ * Result: bit for bit what em2_find_similar_pairs(signatures, cellCount, ...) returns.
+ * Every stored old entry is checked on the device before any output is written: its id is below oldCellCount and not
+ * the row's own, usedCount <= k, its similarity is float(table[m]) for the mismatch count m of the two signatures,
+ * table[m] > similarityThreshold, and each row strictly increases in (m, id); a failure returns EM2_ERR_INVALID (other
+ * signatures -- a different seed or lshCount -- are caught this way).  Old lists made with a HIGHER threshold than this
+ * call's cannot be detected: every stored entry also passes the lower threshold, but rows that are not full lack the
+ * cells between the two thresholds, and the result is wrong.  Old lists made with a LOWER threshold are either rejected
+ * (a stored entry fails this call's threshold) or already exact.  The caller passes the old job's threshold.
+ * The new cells' rows are scanned against all cells and the old cells are judged by the k-th entry of their validated
+ * lists, about M*(N+M) pair evaluations instead of (N+M)^2/2 (M = cellCount - oldCellCount).  Stats: scan_symmetric 1 =
+ * that sweep ran; 0 = full rescan (shape not eligible: L > 1024, k > 112, no threshold passes, POPC variant, option
+ * "scan_symmetric" = 1, or, with the option at 0, more cells appended than there were); 2 + 16 f = a capacity ran out
+ * and the call rescanned all rows. */
+int em2_extend_similar_pairs(em2_context* ctx, const uint64_t* signatures, uint64_t oldCellCount, uint64_t cellCount,
+                             uint64_t lshCount, uint64_t k, double similarityThreshold, int variant,
+                             const em2_pair* oldPairs, const uint32_t* oldUsedCount, em2_pair* pairs, uint32_t* usedCount);
 
 /* Whole job, counts -> similar pairs, signatures never leave the device (optionally also returned). */
 int em2_lsh_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
