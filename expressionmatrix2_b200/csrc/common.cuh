@@ -2,6 +2,7 @@
 #pragma once
 
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <cstdint>
 #include <cstdio>
 #include <string>
@@ -57,8 +58,7 @@ struct em2_context {
         S_FLAGS,         // per-cell eligibility flags / fallback list / uncertain list
         S_SRCTOC, S_SRCCOUNTS, S_GENEMAP,   // subset construction: gathered global rows, gene id map
         S_MISC,
-        S_SAMPLE,        // symmetric scan: encoded signatures of the pre-pass sample
-        S_SYM,           // symmetric scan: per-cell bounds, inbox counts, sample index, overflow flag
+        S_SYM,           // symmetric scan: per-cell bounds, inbox counts and offsets, overflow flags, pacing counters
         S_INBOX,         // symmetric scan: column-direction candidates, uint64[N][inCap]
         S_COLLOG,        // symmetric scan: chunked log of column-direction survivors
         S_COLLOGFILL,    // symmetric scan: entries per log chunk + the chunk allocator
@@ -166,6 +166,14 @@ int scanToHost(em2_context* ctx, StageTimer& T, const uint64_t* dSig, uint64_t c
 
 inline uint64_t wordCount(uint64_t lshCount) { return (lshCount - 1) / 64 + 1; }
 inline uint64_t roundUp(uint64_t x, uint64_t m) { return (x + m - 1) / m * m; }
+// A scan's initial exclusive bound in mismatching bits: a pair is kept iff mismatch < tau0 (0: no threshold passes).
+inline uint32_t scanTau0(int64_t mismatchMax, uint64_t lshCount)
+{
+    return mismatchMax < 0 ? 0u : uint32_t(std::min<int64_t>(mismatchMax, int64_t(lshCount)) + 1);
+}
+// em2_stats.scan_symmetric after a symmetric-kernel attempt: 1 if its result stands; otherwise 2, plus 16 times the
+// overflow flag (which capacity ran out), and the caller rescans one-directionally.
+inline int symScanStatus(int overflowed) { return overflowed ? 2 + 16 * overflowed : 1; }
 
 // ---- stage launchers (each returns an em2_status and adds to ctx->stats.kernel_launches) ----------
 // sums of cells [cellBegin, cellBegin + cellCount); toc/sum1/sum2 are indexed by absolute cell id

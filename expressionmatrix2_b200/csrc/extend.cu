@@ -155,7 +155,7 @@ int em2_extend_similar_pairs(em2_context* ctx, const uint64_t* signatures, uint6
     float* dLut = nullptr;
     EM2_TRY(uploadLut(ctx, lshCount, &dLut));
     const int64_t mismatchMax = em2_mismatch_max(lshCount, similarityThreshold);
-    const uint32_t tau0 = mismatchMax < 0 ? 0u : uint32_t(std::min<int64_t>(mismatchMax, int64_t(lshCount)) + 1);
+    const uint32_t tau0 = scanTau0(mismatchMax, lshCount);
 
     // 1. the old lists against the signatures; nothing is written to the caller's buffers unless all of them hold
     const int e2 = T.mark();
@@ -186,7 +186,7 @@ int em2_extend_similar_pairs(em2_context* ctx, const uint64_t* signatures, uint6
             EM2_TRY(launchExtendRect(ctx, static_cast<const uint64_t*>(dSig), oldN, N, lshCount, k, tau0, dLut, dKeys, dOldUsed, dBound,
                                      outPairs, outUsed, s, &overflowed));
             ctx->stats.variant_used = EM2_VARIANT_MMA_I8;
-            scanSymmetric = overflowed ? 2 + 16 * overflowed : 1;
+            scanSymmetric = symScanStatus(overflowed);
             rescan = overflowed != 0;
         }
         if (rescan) {

@@ -607,11 +607,11 @@ scanMmaSsKernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
 //                     per-cell inboxes of exactly the needed length (count -> scan -> fill).
 //                     For the same reason candidate keys carry scan positions, not cell ids; ids are looked up where
 //                     they decide something (ties at a prune, the finalize kernel).
-// limEx starts from a sampling pre-pass (the k-th best of every cell against N/32 sample cells, a valid upper
-// bound of its final k-th best) and tightens as the cell's own row streams progress; a stale bound is only
-// looser.  The finalize kernel merges a cell's row streams and its inbox.  If the log pool runs dry a flag is
-// raised and the caller reruns the job with the one-directional kernels: exactness never depends on the bounds
-// being tight.
+// limEx starts at the threshold bound and tightens as the cell's own row streams progress -- first in the near window
+// (the row direction against the super blocks around the cell's own, see runSymmetric), so that the column direction
+// of the far sweep meets bounds close to the final ones; a stale bound is only looser.  The finalize kernel merges a
+// cell's row streams and its inbox.  If the log pool runs dry a flag is raised and the caller reruns the job with the
+// one-directional kernels: exactness never depends on the bounds being tight.
 //
 // Operand traffic: per tile the one-directional kernel re-reads the row block's A chunks from L2 (48 KB per
 // K-chunk and SM, ~19 TB/s at full tensor rate -- sustainable only because all CTAs stream the SAME B tile).
@@ -1577,7 +1577,7 @@ __global__ void fillU32Kernel(uint32_t* __restrict__ dst, uint64_t n, uint32_t v
     if (i < n) dst[i] = value;
 }
 
-// ---- pieces shared by the whole-matrix symmetric scan (runSymmetric) and the extension rectangle (runExtendRect)
+// ---- pieces shared by the whole-matrix symmetric scan (runSymmetric) and the extension rectangle (launchExtendRect)
 
 // Column-direction log pool, in entries: 24 k per row at least, up to 64 k when memory allows (a third of what is free;
 // log 16 B + outbox 8 B per entry).  Measured needs: 0.8 k per cell on the 1 M-cell bench workload, 25 k per cell on
@@ -1618,49 +1618,180 @@ static int symKernelSmem(em2_context* ctx, uint32_t panels, bool pair, uint32_t*
     return EM2_OK;
 }
 
-// One launch of scanMmaSymKernel over the p.items items: CTA pairs (clusters of two, one TPC) or single CTAs.
-static int launchSymKernel(em2_context* ctx, bool pair, uint32_t slots, size_t smem, const CUtensorMap& mapA, const CUtensorMap& mapB,
-                           const SymParams& p, cudaStream_t s)
-{
-    if (pair) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.blockDim = dim3(kSymThreads);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = s;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;      // the two CTAs of a pair: one TPC
-        attr[0].val.clusterDim.x = 2;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        cfg.gridDim = dim3(2 * std::min<uint32_t>(p.items, slots));
-        EM2_CUDA(ctx, cudaLaunchKernelEx(&cfg, scanMmaSymKernel<true>, mapA, mapB, p));
-    } else {
-        scanMmaSymKernel<false><<<unsigned(std::min<uint32_t>(p.items, slots)), kSymThreads, smem, s>>>(mapA, mapB, p);
-    }
-    EM2_CUDA(ctx, cudaGetLastError());
-    ctx->stats.kernel_launches++;
-    return EM2_OK;
-}
+// One job of scanMmaSymKernel over N scan positions: its scratch, its kernel parameters and its sweeps.
+//   reserve     lays out the scratch; returns the status instead of leaving early, so that a multi-GPU caller can fold
+//               its own reservations into the one agreement before its first collective
+//   initialise  clears the log, the inbox counts, the flags and the candidate counts, sets the own rows' bounds to tau0,
+//               fills the parameters that do not depend on the sweep and builds the tensor maps
+//   launch      one sweep of the own row blocks
+// then fileLog (log -> inboxes) and readOverflow (whether the result stands).
+struct SymJob {
+    bool pair;                 // CTA pairs (cta_group::2; an item = one super block of 256 rows) unless option "sym_cta_pair" = 1
+    uint32_t rowsPerItem, slots;
+    SymParams p{};
+    CUtensorMap mapA, mapB;
+    size_t smem = 0;
+    uint64_t positions = 0;    // entries of limEx (inCount and inOffset have one more)
+    size_t candCountBytes = 0;
+    uint32_t *inCount = nullptr, *inOffset = nullptr, *progress = nullptr;
+    uint64_t* outbox = nullptr;        // the filed log: every column cell's inbox, in position order
+    void* cubTemp = nullptr;
+    size_t cubBytes = 0, cubBytesShard = 0;   // exclusive scans of N + 1 and of shard + 1 counts
+    void* pinned = nullptr;    // the overflow flag's read-back; the multi-GPU size matrix (world x (world + 1) entries)
 
-// The log -> per-cell inboxes in position order: count per column cell, exclusive scan, fill.  inCount holds N + 1
-// zeros on entry; inOffset[N] is the total afterwards.
-static int fileColumnLog(em2_context* ctx, const SymParams& p, uint64_t N, uint32_t* inCount, uint32_t* inOffset, uint64_t* outbox,
-                         void* cubTemp, size_t cubBytes, uint32_t dropBelow, cudaStream_t s)
-{
-    scatterLogKernel<false><<<unsigned(ctx->smCount) * 8, 256, 0, s>>>(p.chunkNext, p.chunkCap, p.colLog, p.chunkFill, inCount, nullptr,
-                                                                      nullptr, p.appendedTotal, dropBelow);
-    EM2_CUDA(ctx, cudaGetLastError());
-    // inCount[N] is 0: inOffset[N] = total
-    EM2_CUDA(ctx, cub::DeviceScan::ExclusiveSum(cubTemp, cubBytes, inCount, inOffset, int(N + 1), s));
-    EM2_CUDA(ctx, cudaMemsetAsync(inCount, 0, N * sizeof(uint32_t), s));
-    scatterLogKernel<true><<<unsigned(ctx->smCount) * 8, 256, 0, s>>>(p.chunkNext, p.chunkCap, p.colLog, p.chunkFill, inCount, inOffset,
-                                                                     outbox, p.appendedTotal, dropBelow);
-    EM2_CUDA(ctx, cudaGetLastError());
-    ctx->stats.kernel_launches += 2;      // + the scan's own kernels (library code, not counted)
-    return EM2_OK;
-}
+    SymJob(const em2_context* ctx, uint64_t k)
+        : pair(ctx->symCtaPair != 1 && ctx->smCount >= 2), rowsPerItem(pair ? kPairRows : kRowsPerItem),
+          slots(pair ? uint32_t(ctx->smCount / 2) : uint32_t(ctx->smCount))
+    {
+        p.k = uint32_t(k);
+        // small regions here: a cell's bound is published when its region is pruned, and the column direction of other
+        // CTAs lives on fresh bounds (with the one-directional kernels' 4k + 32 keys: 90 M instead of 70 M survivors at config 2)
+        p.cap = candidateCapacity(uint32_t(k)) + uint32_t(k) * uint32_t(ctx->candCapExtra);
+    }
+
+    // nPositions: entries of each per-position array (N, or `shard` for each GPU of a job); rows: own rows, `streams`
+    // candidate streams each; chunkCap: 64-entry chunks of the column-direction log pool
+    int reserve(em2_context* ctx, uint64_t N, uint64_t nPositions, uint64_t shard, uint64_t rows, uint32_t streams,
+                uint32_t chunkCap, cudaStream_t s)
+    {
+        positions = nPositions;
+        const uint64_t rowsAlloc = std::max<uint64_t>(rows, 1);
+        candCountBytes = size_t(streams) * rowsAlloc * sizeof(uint32_t);
+        cub::DeviceScan::ExclusiveSum(nullptr, cubBytes, static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), int(N + 1), s);
+        cub::DeviceScan::ExclusiveSum(nullptr, cubBytesShard, static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), int(shard + 1), s);
+        void *cand = nullptr, *candCount = nullptr, *counters = nullptr, *sym = nullptr, *box = nullptr, *colLog = nullptr,
+             *chunkFill = nullptr;
+        int rc = EM2_OK;
+        auto res = [&](int which, size_t bytes, void** out) {
+            if (rc == EM2_OK) rc = em2::reserve(ctx, which, bytes, out);
+        };
+        res(em2_context::S_CAND, size_t(streams) * rowsAlloc * p.cap * sizeof(uint64_t), &cand);
+        res(em2_context::S_CANDCOUNT, candCountBytes, &candCount);
+        res(em2_context::S_COUNTERS, 64, &counters);
+        // [limEx positions][inCount positions + 1][inOffset positions + 1][overflow 8][progress 1024]
+        res(em2_context::S_SYM, (3 * positions + 2 + 8 + 1024) * sizeof(uint32_t), &sym);
+        res(em2_context::S_INBOX, size_t(chunkCap) * kLogChunk * sizeof(uint64_t), &box);
+        res(em2_context::S_COLLOG, (size_t(chunkCap) + 1) * kLogChunk * sizeof(ulonglong2), &colLog);   // + spill chunk
+        res(em2_context::S_COLLOGFILL, (size_t(chunkCap) + 4) * sizeof(uint32_t), &chunkFill);
+        res(em2_context::S_MISC, std::max(cubBytes, cubBytesShard), &cubTemp);
+        if (rc == EM2_OK)
+            rc = reservePinned(ctx, 2, std::max<size_t>(64, size_t(ctx->world) * (ctx->world + 1) * sizeof(uint64_t)), &pinned);
+        if (rc != EM2_OK) return rc;
+        p.cellCount = N;
+        p.cand = static_cast<uint64_t*>(cand);
+        p.candCount = static_cast<uint32_t*>(candCount);
+        p.appendedTotal = static_cast<unsigned long long*>(counters) + 1;
+        p.limEx = static_cast<uint32_t*>(sym);
+        inCount = p.limEx + positions;
+        inOffset = inCount + positions + 1;
+        p.overflow = inOffset + positions + 1;
+        progress = p.overflow + 8;
+        outbox = static_cast<uint64_t*>(box);
+        p.colLog = static_cast<ulonglong2*>(colLog);
+        p.chunkFill = static_cast<uint32_t*>(chunkFill);
+        p.chunkNext = p.chunkFill + chunkCap;
+        p.chunkCap = chunkCap;
+        return EM2_OK;
+    }
+
+    // enc: FP4 encoding of the N positions, K bits each; own rows [posBegin, posBegin + rows); the column direction
+    // serves the columns below colDirEnd; perm: position -> cell id (nullptr: identity)
+    int initialise(em2_context* ctx, const uint8_t* enc, uint32_t K, uint64_t posBegin, uint64_t rows, uint32_t tau0,
+                   uint64_t colDirEnd, const uint32_t* perm, cudaStream_t s)
+    {
+        EM2_CUDA(ctx, cudaMemsetAsync(p.chunkFill, 0, (size_t(p.chunkCap) + 4) * sizeof(uint32_t), s));
+        EM2_CUDA(ctx, cudaMemsetAsync(inCount, 0, (positions + 1) * sizeof(uint32_t), s));
+        EM2_CUDA(ctx, cudaMemsetAsync(p.overflow, 0, 8 * sizeof(uint32_t), s));
+        EM2_CUDA(ctx, cudaMemsetAsync(p.candCount, 0, candCountBytes, s));   // untouched streams read as empty
+        if (rows) {
+            fillU32Kernel<<<unsigned((rows + 255) / 256), 256, 0, s>>>(p.limEx + posBegin, rows, tau0);
+            EM2_CUDA(ctx, cudaGetLastError());
+            ctx->stats.kernel_launches++;
+        }
+        const uint64_t N = p.cellCount;
+        p.K = K;
+        p.panels = K / kSymKBits;
+        EM2_TRY(symKernelSmem(ctx, p.panels, pair, &p.stages, &smem));
+        p.superBlocks = uint32_t((N + kSsTileN - 1) / kSsTileN);
+        p.posBegin = uint32_t(posBegin);
+        p.ownRows = uint32_t(rows);
+        p.colDirEnd = uint32_t(colDirEnd);
+        p.perm = perm;
+        p.flags = uint32_t(ctx->debugFlags);
+        EM2_TRY(makeTensorMapU8(ctx, &mapA, enc, N, K / 2, K / 2, kRowsPerItem));
+        EM2_TRY(makeTensorMapU8(ctx, &mapB, enc, N, K / 2, K / 2, pair ? kSymHalfN / 2 : kSymHalfN));
+        return EM2_OK;
+    }
+
+    // One launch over the items of plan `pl` and the offsets [dBegin, dBegin + offsets), on CTA pairs (clusters of two,
+    // one TPC) or single CTAs; resume, segBase, rowOnly, halfOffset: see SymParams.
+    int launch(em2_context* ctx, const ScanPlan& pl, int32_t dBegin, uint32_t offsets, uint32_t resume, uint32_t segBase,
+               uint32_t rowOnly, uint32_t halfOffset, cudaStream_t s)
+    {
+        p.mainBlocks = pl.mainBlocks;
+        p.segments = pl.segments;
+        p.items = pl.items;
+        p.segmentCols = pl.segmentCols;
+        p.dBegin = dBegin;
+        p.offsetsHere = offsets;
+        p.resume = resume;
+        p.segBase = segBase;
+        p.rowOnly = rowOnly;
+        p.halfOffset = halfOffset;
+        // only sweeps long enough for the CTAs to drift apart by more blocks than L2 holds (~490): paced at 200k cells
+        // (390 tiles per item) the sweep was 1.5x SLOWER, at 1 M cells (1953 tiles) 1.2x faster
+        p.progress = (offsets >= 768 && !(ctx->debugFlags & 16)) ? progress : nullptr;
+        if (p.progress) EM2_CUDA(ctx, cudaMemsetAsync(progress, 0, 1024 * sizeof(uint32_t), s));
+        if (pair) {
+            cudaLaunchConfig_t cfg = {};
+            cfg.blockDim = dim3(kSymThreads);
+            cfg.dynamicSmemBytes = smem;
+            cfg.stream = s;
+            cudaLaunchAttribute attr[1];
+            attr[0].id = cudaLaunchAttributeClusterDimension;      // the two CTAs of a pair: one TPC
+            attr[0].val.clusterDim.x = 2;
+            attr[0].val.clusterDim.y = 1;
+            attr[0].val.clusterDim.z = 1;
+            cfg.attrs = attr;
+            cfg.numAttrs = 1;
+            cfg.gridDim = dim3(2 * std::min<uint32_t>(p.items, slots));
+            EM2_CUDA(ctx, cudaLaunchKernelEx(&cfg, scanMmaSymKernel<true>, mapA, mapB, p));
+        } else {
+            scanMmaSymKernel<false><<<unsigned(std::min<uint32_t>(p.items, slots)), kSymThreads, smem, s>>>(mapA, mapB, p);
+        }
+        EM2_CUDA(ctx, cudaGetLastError());
+        ctx->stats.kernel_launches++;
+        return EM2_OK;
+    }
+
+    // The log -> per-cell inboxes in position order: count per column cell, exclusive scan, fill.  Entries of column
+    // positions below dropBelow are dropped.  inOffset[N] is the total afterwards.
+    int fileLog(em2_context* ctx, uint32_t dropBelow, cudaStream_t s)
+    {
+        const uint64_t N = p.cellCount;
+        scatterLogKernel<false><<<unsigned(ctx->smCount) * 8, 256, 0, s>>>(p.chunkNext, p.chunkCap, p.colLog, p.chunkFill, inCount,
+                                                                          nullptr, nullptr, p.appendedTotal, dropBelow);
+        EM2_CUDA(ctx, cudaGetLastError());
+        // inCount[N] is 0: inOffset[N] = total
+        EM2_CUDA(ctx, cub::DeviceScan::ExclusiveSum(cubTemp, cubBytes, inCount, inOffset, int(N + 1), s));
+        EM2_CUDA(ctx, cudaMemsetAsync(inCount, 0, N * sizeof(uint32_t), s));
+        scatterLogKernel<true><<<unsigned(ctx->smCount) * 8, 256, 0, s>>>(p.chunkNext, p.chunkCap, p.colLog, p.chunkFill, inCount,
+                                                                         inOffset, outbox, p.appendedTotal, dropBelow);
+        EM2_CUDA(ctx, cudaGetLastError());
+        ctx->stats.kernel_launches += 2;      // + the scan's own kernels (library code, not counted)
+        return EM2_OK;
+    }
+
+    // After the merge: the overflow flag decides whether the result stands
+    int readOverflow(em2_context* ctx, cudaStream_t s, int* overflowed)
+    {
+        uint32_t* host = static_cast<uint32_t*>(pinned);
+        EM2_CUDA(ctx, cudaMemcpyAsync(host, p.overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        EM2_CUDA(ctx, cudaStreamSynchronize(s));
+        *overflowed = int(*host);
+        return EM2_OK;
+    }
+};
 
 // finalizeSymKernel over `rows` cells.  Staging: 16-bit mismatch counts of everything below the bound (cells with longer
 // lists bisect in place), then the k best keys plus the ties at the k-th place.
@@ -1693,7 +1824,7 @@ static int launchFinalizeSym(em2_context* ctx, uint64_t rows, uint64_t posBegin,
 //   1. near window   own row blocks x the column tiles within +-w super blocks of the row's own, row direction only --
 //                    both owners of such a tile pair visit it.  In grouped order a cell's neighbours sit next to it, so
 //                    this short launch (max(33 tiles, N/32 columns) per row block, ~3 % of the job at 1 M cells) leaves
-//                    every cell with a bound close to its final one; it replaces the sampling pre-pass of round 1.
+//                    every cell with a bound close to its final one.
 //   2. all-gather of the bounds (4 bytes per cell)
 //   3. far sweep     own row blocks x the offsets w+1 .. S/2, both directions; the column direction judges a cell by its
 //                    bound of phase 1 (cells of this GPU keep tightening theirs), survivors go to the log
@@ -1708,7 +1839,6 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
 {
     const uint64_t N = cellCount;
     const int P = ctx->world;
-    const uint32_t panels = K / kSymKBits;
     const uint32_t S = uint32_t((N + kSsTileN - 1) / kSsTileN);
     *overflowed = 0;
     // Half width of the near window, in super blocks.  Default: N/32 columns in total (what a sample must hold for the
@@ -1749,77 +1879,32 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
     const uint32_t farCount = S / 2 >= farBegin ? S / 2 - farBegin + 1 : 0;
     ctx->lastNearHalfWidth = int(w);
 
+    SymJob job(ctx, k);
     ScanPlan nearPlan{}, farPlan{};
-    uint32_t cap = candidateCapacity(uint32_t(k)) + uint32_t(k) * uint32_t(ctx->candCapExtra);
     uint32_t streams = kSubStreams;
-    // CTA pairs (cta_group::2; an item = one super block of 256 rows) unless option "sym_cta_pair" = 1
-    const bool pair = ctx->symCtaPair != 1 && ctx->smCount >= 2;
-    const uint32_t rowsPerItem = pair ? kPairRows : kRowsPerItem;
-    const uint32_t slots = pair ? uint32_t(ctx->smCount / 2) : uint32_t(ctx->smCount);
     if (ownRows) {
-        nearPlan = makeScanPlan(ctx, ownRows, uint64_t(nearCount) * kSsTileN, k, kSsTileN, rowsPerItem, 1, kSubStreams, slots);
-        farPlan = farCount ? makeScanPlan(ctx, ownRows, uint64_t(farCount) * kSsTileN, k, kSsTileN, rowsPerItem, 1, kSubStreams, slots) : nearPlan;
-        // small regions here: a cell's bound is published when its region is pruned, and the column direction of other
-        // CTAs lives on fresh bounds (with the one-directional kernels' 4k + 32 keys: 90 M instead of 70 M survivors at config 2)
-        nearPlan.cap = farPlan.cap = cap;
+        nearPlan = makeScanPlan(ctx, ownRows, uint64_t(nearCount) * kSsTileN, k, kSsTileN, job.rowsPerItem, 1, kSubStreams, job.slots);
+        farPlan = farCount ? makeScanPlan(ctx, ownRows, uint64_t(farCount) * kSsTileN, k, kSsTileN, job.rowsPerItem, 1, kSubStreams, job.slots) : nearPlan;
         // stream pair 0 of a row is shared by the near launch and segment 0 of the far launch (which continues it); the
         // other segments of the two launches own their pairs
         streams = (nearPlan.segments + (farCount ? farPlan.segments - 1 : 0)) * kSubStreams;
     }
-    const uint64_t Npad = uint64_t(P) * shard;      // every rank's slice of the per-position arrays has `shard` entries
 
     // ---- scratch: everything is reserved before the first collective, then the ranks agree to go on
-    void *cand = nullptr, *candCount = nullptr, *counters = nullptr, *sym = nullptr, *outbox = nullptr, *colLog = nullptr,
-         *chunkFill = nullptr, *cubTemp = nullptr, *dist0 = nullptr, *dist2 = nullptr;
-    const uint64_t rowsAlloc = std::max<uint64_t>(ownRows, 1);
     // column-direction log pool (symLogPoolEntries); the outbox is cut from a buffer of the same number of keys
-    const uint64_t poolEntries = std::min<uint64_t>(0xf0000000ull * uint64_t(kLogChunk) / 64, symLogPoolEntries(ctx, rowsAlloc, k) + 2 * uint64_t(ctx->smCount) * kEpiThreads * kLogChunk);
+    const uint64_t poolEntries = std::min<uint64_t>(0xf0000000ull * uint64_t(kLogChunk) / 64, symLogPoolEntries(ctx, std::max<uint64_t>(ownRows, 1), k) + 2 * uint64_t(ctx->smCount) * kEpiThreads * kLogChunk);
     const uint32_t chunkCap = uint32_t(std::min<uint64_t>(0xfffffff0ull, poolEntries / kLogChunk));
-    size_t cubBytes = 0, cubBytes2 = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, cubBytes, static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), int(N + 1), s);
-    cub::DeviceScan::ExclusiveSum(nullptr, cubBytes2, static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), int(shard + 1), s);
-    int rc = EM2_OK;
-    auto res = [&](int which, size_t bytes, void** out) {
-        if (rc == EM2_OK) rc = reserve(ctx, which, bytes, out);
-    };
-    res(em2_context::S_CAND, size_t(streams) * rowsAlloc * cap * sizeof(uint64_t), &cand);
-    res(em2_context::S_CANDCOUNT, size_t(streams) * rowsAlloc * sizeof(uint32_t), &candCount);
-    res(em2_context::S_COUNTERS, 64, &counters);
-    // [limEx Npad][inCount Npad + 1][inOffset Npad + 1][overflow 4][progress 1024]
-    res(em2_context::S_SYM, (3 * Npad + 2 + 8 + 1024) * sizeof(uint32_t), &sym);
-    res(em2_context::S_INBOX, size_t(chunkCap) * kLogChunk * sizeof(uint64_t), &outbox);
-    res(em2_context::S_COLLOG, (size_t(chunkCap) + 1) * kLogChunk * sizeof(ulonglong2), &colLog);   // + spill chunk
-    res(em2_context::S_COLLOGFILL, (size_t(chunkCap) + 4) * sizeof(uint32_t), &chunkFill);
-    res(em2_context::S_MISC, std::max(cubBytes, cubBytes2), &cubTemp);
+    // every rank's slice of the per-position arrays has `shard` entries
+    int rc = job.reserve(ctx, N, uint64_t(P) * shard, shard, ownRows, streams, chunkCap, s);
+    void *dist0 = nullptr, *dist2 = nullptr;
     if (P > 1) {
         // [recvCounts P x (shard + 1)][recvOffsets P x (shard + 1)]
-        res(em2_context::S_DIST0, 2 * size_t(P) * (shard + 1) * sizeof(uint32_t), &dist0);
-        res(em2_context::S_DIST2, size_t(P) * (P + 1) * sizeof(uint64_t), &dist2);
-    }
-    uint32_t* matrixHost = nullptr;
-    {
-        void* pin = nullptr;
-        if (rc == EM2_OK) rc = reservePinned(ctx, 2, std::max<size_t>(64, size_t(P) * (P + 1) * sizeof(uint64_t)), &pin);
-        matrixHost = static_cast<uint32_t*>(pin);
+        if (rc == EM2_OK) rc = reserve(ctx, em2_context::S_DIST0, 2 * size_t(P) * (shard + 1) * sizeof(uint32_t), &dist0);
+        if (rc == EM2_OK) rc = reserve(ctx, em2_context::S_DIST2, size_t(P) * (P + 1) * sizeof(uint64_t), &dist2);
     }
     EM2_TRY(distAgree(ctx, rc));
 
-    uint32_t* limEx = static_cast<uint32_t*>(sym);
-    uint32_t* inCount = limEx + Npad;
-    uint32_t* inOffset = inCount + Npad + 1;
-    uint32_t* overflow = inOffset + Npad + 1;
-    uint32_t* progress = overflow + 8;
-    uint32_t* chunkNext = static_cast<uint32_t*>(chunkFill) + chunkCap;
-    unsigned long long* appended = static_cast<unsigned long long*>(counters) + 1;
-    EM2_CUDA(ctx, cudaMemsetAsync(chunkFill, 0, (size_t(chunkCap) + 4) * sizeof(uint32_t), s));
-    EM2_CUDA(ctx, cudaMemsetAsync(inCount, 0, (Npad + 1) * sizeof(uint32_t), s));
-    EM2_CUDA(ctx, cudaMemsetAsync(overflow, 0, 8 * sizeof(uint32_t), s));
-    EM2_CUDA(ctx, cudaMemsetAsync(candCount, 0, size_t(streams) * rowsAlloc * sizeof(uint32_t), s));   // untouched streams read as empty
-    if (ownRows) {
-        fillU32Kernel<<<unsigned((ownRows + 255) / 256), 256, 0, s>>>(limEx + posBegin, ownRows, tau0);
-        EM2_CUDA(ctx, cudaGetLastError());
-        ctx->stats.kernel_launches++;
-    }
+    const SymParams& p = job.p;
     // debug_flags bit 3: report the candidate counters after every stage (synchronises)
     // debug_flags bit 5: wall-clock time of every phase (synchronises the stream at each mark) -- how a rank's scan
     // divides into sweeps, collectives and waiting for the other ranks
@@ -1838,80 +1923,38 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
         unsigned long long v = 0;
         uint32_t chunksUsed = 0;
         cudaStreamSynchronize(s);
-        cudaMemcpy(&v, appended, sizeof(v), cudaMemcpyDeviceToHost);
-        cudaMemcpy(&chunksUsed, chunkNext, sizeof(chunksUsed), cudaMemcpyDeviceToHost);
+        cudaMemcpy(&v, p.appendedTotal, sizeof(v), cudaMemcpyDeviceToHost);
+        cudaMemcpy(&chunksUsed, p.chunkNext, sizeof(chunksUsed), cudaMemcpyDeviceToHost);
         std::fprintf(stderr, "[em2 sym rank %d] after %s: candidates so far %llu, column-direction log chunks %u of %u (near half width %d of %u super blocks)\n",
                      ctx->rank, what, v, chunksUsed, chunkCap, ctx->lastNearHalfWidth, S);
     };
 
-    SymParams p{};
-    p.cellCount = N;
-    p.K = K;
-    p.panels = panels;
-    size_t smem = 0;
-    EM2_TRY(symKernelSmem(ctx, panels, pair, &p.stages, &smem));
-    p.superBlocks = S;
-    p.halfOffset = S % 2 == 0 ? S / 2 : 0;
-    p.posBegin = uint32_t(posBegin);
-    p.ownRows = uint32_t(ownRows);
-    p.k = uint32_t(k);
-    p.cap = cap;
-    p.cand = static_cast<uint64_t*>(cand);
-    p.candCount = static_cast<uint32_t*>(candCount);
-    p.appendedTotal = appended;
-    p.limEx = limEx;
-    p.colDirEnd = uint32_t(N);
-    p.colLog = static_cast<ulonglong2*>(colLog);
-    p.chunkFill = static_cast<uint32_t*>(chunkFill);
-    p.chunkNext = chunkNext;
-    p.chunkCap = chunkCap;
-    p.overflow = overflow;
-    p.perm = perm;
-    p.flags = uint32_t(ctx->debugFlags);
-    CUtensorMap mapA, mapB;
-    EM2_TRY(makeTensorMapU8(ctx, &mapA, encP, N, K / 2, K / 2, kRowsPerItem));
-    EM2_TRY(makeTensorMapU8(ctx, &mapB, encP, N, K / 2, K / 2, pair ? kSymHalfN / 2 : kSymHalfN));
-    auto sweep = [&](const ScanPlan& pl, int32_t dBegin, uint32_t count, uint32_t resume, uint32_t rowOnly) -> int {
-        if (!ownRows || !count) return EM2_OK;
-        p.segBase = resume ? nearPlan.segments - 1 : 0;
-        p.mainBlocks = pl.mainBlocks;
-        p.segments = pl.segments;
-        p.items = pl.items;
-        p.segmentCols = pl.segmentCols;
-        p.dBegin = dBegin;
-        p.offsetsHere = count;
-        p.resume = resume;
-        p.rowOnly = rowOnly;
-        // only sweeps long enough for the CTAs to drift apart by more blocks than L2 holds (~490): paced at 200k cells
-        // (390 tiles per item) the sweep was 1.5x SLOWER, at 1 M cells (1953 tiles) 1.2x faster
-        p.progress = (count >= 768 && !(ctx->debugFlags & 16)) ? progress : nullptr;
-        if (p.progress) EM2_CUDA(ctx, cudaMemsetAsync(progress, 0, 1024 * sizeof(uint32_t), s));
-        return launchSymKernel(ctx, pair, slots, smem, mapA, mapB, p, s);
-    };
+    EM2_TRY(job.initialise(ctx, encP, K, posBegin, ownRows, tau0, N, perm, s));
+    const uint32_t halfOffset = S % 2 == 0 ? S / 2 : 0;
     phase("set-up");
     // ---- 1. near window
-    EM2_TRY(sweep(nearPlan, -int32_t(w), nearCount, 0, 1));
+    if (ownRows) EM2_TRY(job.launch(ctx, nearPlan, -int32_t(w), nearCount, 0, 0, 1, halfOffset, s));
     report("near window");
     // ---- 2. bounds of all cells
-    if (P > 1) EM2_TRY(distAllGather(ctx, limEx, shard, sizeof(uint32_t), s));
+    if (P > 1) EM2_TRY(distAllGather(ctx, p.limEx, shard, sizeof(uint32_t), s));
     phase("bounds all-gather");
     // ---- 3. far sweep
-    EM2_TRY(sweep(farPlan, int32_t(farBegin), farCount, 1, 0));
+    if (ownRows && farCount) EM2_TRY(job.launch(ctx, farPlan, int32_t(farBegin), farCount, 1, nearPlan.segments - 1, 0, halfOffset, s));
     report("far sweep");
-    // ---- 4. log -> outbox in position order: count per column cell, exclusive scan, fill
-    EM2_TRY(fileColumnLog(ctx, p, N, inCount, inOffset, static_cast<uint64_t*>(outbox), cubTemp, cubBytes, 0, s));
+    // ---- 4. log -> outbox in position order
+    EM2_TRY(job.fileLog(ctx, 0, s));
     phase("log filing");
 
     InboxSources src{};
     if (P == 1) {
         src.count = 1;
-        src.keys[0] = static_cast<const uint64_t*>(outbox);
-        src.offsets[0] = inOffset;
+        src.keys[0] = job.outbox;
+        src.offsets[0] = job.inOffset;
     } else {
         // sizes (and overflow flags) of every rank for every rank
         uint64_t* matrix = static_cast<uint64_t*>(dist2);
-        uint64_t* mh = reinterpret_cast<uint64_t*>(matrixHost);
-        exchangeSizesKernel<<<1, 32, 0, s>>>(inOffset, N, shard, uint32_t(P), uint32_t(ctx->rank), overflow, matrix);
+        uint64_t* mh = static_cast<uint64_t*>(job.pinned);
+        exchangeSizesKernel<<<1, 32, 0, s>>>(job.inOffset, N, shard, uint32_t(P), uint32_t(ctx->rank), p.overflow, matrix);
         EM2_CUDA(ctx, cudaGetLastError());
         ctx->stats.kernel_launches++;
         EM2_TRY(distAllGather(ctx, matrix, size_t(P + 1), sizeof(uint64_t), s));
@@ -1949,15 +1992,15 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
                 ro[d] = uint64_t(d) * (shard + 1) * sizeof(uint32_t);
                 rb[d] = shard * sizeof(uint32_t);
             }
-            EM2_TRY(distAllToAll(ctx, inCount, so, sb, recvCounts, ro, rb, s));
+            EM2_TRY(distAllToAll(ctx, job.inCount, so, sb, recvCounts, ro, rb, s));
         }
-        EM2_TRY(distAllToAll(ctx, outbox, sendOff, sendBytes, recvKeys, recvOff, recvBytes, s));
+        EM2_TRY(distAllToAll(ctx, job.outbox, sendOff, sendBytes, recvKeys, recvOff, recvBytes, s));
         EM2_CUDA(ctx, cudaEventRecord(x1, s));
         ctx->symExchangeTimed = true;
         for (int d = 0; d < P; d++)
             if (d != ctx->rank) ctx->stats.exchange_bytes += sendBytes[d] + shard * sizeof(uint32_t);
         for (int r = 0; r < P; r++) {
-            EM2_CUDA(ctx, cub::DeviceScan::ExclusiveSum(cubTemp, cubBytes2, recvCounts + size_t(r) * (shard + 1),
+            EM2_CUDA(ctx, cub::DeviceScan::ExclusiveSum(job.cubTemp, job.cubBytesShard, recvCounts + size_t(r) * (shard + 1),
                                                         recvOffsets + size_t(r) * (shard + 1), int(shard + 1), s));
             src.keys[r] = static_cast<const uint64_t*>(recvKeys) + recvOff[r] / sizeof(uint64_t);
             src.offsets[r] = recvOffsets + size_t(r) * (shard + 1);
@@ -1966,13 +2009,10 @@ int runSymmetric(em2_context* ctx, const uint8_t* encP, const uint32_t* perm, co
         phase("candidate exchange");
     }
     // ---- 5. merge
-    EM2_TRY(launchFinalizeSym(ctx, ownRows, posBegin, streams, cap, k, p.cand, p.candCount, src, limEx, lut, pairs, usedCount, perm,
-                              overflow, s));
-    // the overflow flag decides whether the result stands (P > 1: the log pools were checked job-wide above; what is
-    // left is this rank's own merge guard)
-    EM2_CUDA(ctx, cudaMemcpyAsync(matrixHost, overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    *overflowed = int(*matrixHost);
+    EM2_TRY(launchFinalizeSym(ctx, ownRows, posBegin, streams, p.cap, k, p.cand, p.candCount, src, p.limEx, lut, pairs, usedCount, perm,
+                              p.overflow, s));
+    // P > 1: the log pools were checked job-wide above; what is left is this rank's own merge guard
+    EM2_TRY(job.readOverflow(ctx, s, overflowed));
     phase("merge");
     if (ctx->symExchangeTimed) {
         ctx->symExchangeTimed = false;
@@ -2052,6 +2092,25 @@ int groupRows(em2_context* ctx, const uint64_t* signatures, uint32_t W, uint64_t
     return EM2_OK;
 }
 
+// Which one-directional tcgen05 kernel for K = lshCount rounded up to 128 bits: above 1024 bits the A operand does not
+// fit in tensor memory, so both operands stream (scanMmaSsKernel, N = 256 instructions).  Measured at 512..1024 bits the
+// streamed kernel is also the faster one (3500 vs 2480 TOP/s on iid signatures at L = 1024: N = 128 instructions with A
+// in TMEM top out at 2971), so it is the default from 512 bits; "mma_kernel" = 1 / 2 forces the TMEM-resident / the
+// streamed form.
+bool mmaStreamed(const em2_context* ctx, uint32_t K)
+{
+    return K > kMaxPanels * kChunkBytes || ctx->mmaKernel == 2 || (ctx->mmaKernel == 0 && K >= 512);
+}
+
+// What every use of scanMmaSymKernel needs (whole matrix on one or several GPUs, extension rectangle): A resident in
+// shared memory (L <= 1024), candidate regions the register prune holds, a passing threshold, positions below 2^31,
+// and option "scan_symmetric" != 1.  Each caller adds its own conditions.
+bool symKernelEligible(const em2_context* ctx, uint64_t cellCount, uint64_t lshCount, uint64_t k, int64_t mismatchMax)
+{
+    return lshCount <= kMaxPanels * kChunkBytes && scanCandidateCapacity(uint32_t(k), uint32_t(ctx->candCapExtra)) <= 32 * kPruneRegsPerLane &&
+           mismatchMax >= 0 && cellCount <= 0x7fffff00ull && ctx->scanSymmetric != 1;
+}
+
 int runMma(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uint64_t lshCount, uint64_t rowBegin,
            uint64_t rowEnd, uint64_t k, int64_t mismatchMax, const float* lut, em2_pair* pairs, uint32_t* usedCount,
            uint16_t* dump, cudaStream_t s)
@@ -2059,15 +2118,11 @@ int runMma(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uin
     const uint64_t rows = rowEnd - rowBegin;
     const uint32_t W = uint32_t(wordCount(lshCount));
     const uint32_t K = uint32_t(roundUp(lshCount, kChunkBytes));
-    // Which tcgen05 kernel: above 1024 bits the A operand does not fit in tensor memory, so both operands stream
-    // (scanMmaSsKernel, N = 256 instructions).  Measured at 512..1024 bits the streamed kernel is also the faster one
-    // (3500 vs 2480 TOP/s on iid signatures at L = 1024: N = 128 instructions with A in TMEM top out at 2971), so it
-    // is the default from 512 bits; "mma_kernel" = 1 / 2 forces the TMEM-resident / the streamed form.
-    const bool streamed = K > kMaxPanels * kChunkBytes || ctx->mmaKernel == 2 || (ctx->mmaKernel == 0 && K >= 512);
+    const bool streamed = mmaStreamed(ctx, K);
     if (cellCount > 0x7fffff00ull) return fail(ctx, EM2_ERR_INVALID, "cellCount too large for the MMA variant");
 
     // 1. the scanned rows in grouped order (see "Row grouping")
-    const uint32_t tau0 = mismatchMax < 0 ? 0u : uint32_t(std::min<int64_t>(mismatchMax, int64_t(lshCount)) + 1);
+    const uint32_t tau0 = scanTau0(mismatchMax, lshCount);
     const bool grouped = !dump && (ctx->rowGrouping == 2 || (ctx->rowGrouping == 0 && rows >= 8192));
     uint32_t* rowPerm = nullptr;
     uint32_t* groupStats = nullptr;
@@ -2082,15 +2137,14 @@ int runMma(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uin
     //    order); falls through to the one-directional kernels if a capacity ran out (nothing of the symmetric attempt is kept)
     ctx->stats.scan_symmetric = 0;
     {
-        const uint32_t capSym = scanCandidateCapacity(uint32_t(k), uint32_t(ctx->candCapExtra));
-        const bool eligible = streamed && !dump && K <= kMaxPanels * kChunkBytes && rowBegin == 0 && rows == cellCount &&
-                              capSym <= 32 * kPruneRegsPerLane && cellCount >= 1024 && tau0 > 0;
+        const bool eligible = symKernelEligible(ctx, cellCount, lshCount, k, mismatchMax) && streamed && !dump && rowBegin == 0 &&
+                              rows == cellCount && cellCount >= 1024;
         // "scan_symmetric" = 2 asks for the symmetric kernel whenever it is eligible.  AUTO takes it from 65,536 cells: with
         // the near window and the leader-clustering scan order it wins from config 2's 100k cells on (8.2 vs 8.7 ms) and by
         // 1.9x at 1 M cells; above 2 M cells per GPU its logs outgrow the memory.
         bool automatic = ctx->scanSymmetric == 0 && cellCount >= 65536 && cellCount <= 2000000;
         if (automatic) {
-            // its scratch (log pool 16 B + inbox 8 B per entry, 24 k entries per cell; candidate regions; sample) must fit
+            // its scratch (log pool 16 B + inbox 8 B per entry, 24 k entries per cell; candidate regions; per-cell arrays) must fit
             // beside what is already allocated -- otherwise stay with the one-directional kernels instead of failing
             const size_t want = size_t(cellCount) * (24 * k * 24 + 8 * (2 * k + 32) * 8 + 64) + (size_t(1) << 30);
             size_t have = ctx->scratch[em2_context::S_COLLOG].bytes + ctx->scratch[em2_context::S_INBOX].bytes +
@@ -2107,7 +2161,7 @@ int runMma(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uin
             int overflowed = 0;
             EM2_TRY(runSymmetric(ctx, static_cast<const uint8_t*>(encSym), rowPerm, groupStats, grouped, cellCount, 0, cellCount, cellCount,
                                  Ksym, k, tau0, lut, pairs, usedCount, s, &overflowed));
-            ctx->stats.scan_symmetric = overflowed ? 2 + 16 * overflowed : 1;      // 2 + 16 * (which capacity ran out)
+            ctx->stats.scan_symmetric = symScanStatus(overflowed);
             if (!overflowed) return EM2_OK;
         }
     }
@@ -2262,12 +2316,9 @@ bool distSymmetricEligible(const em2_context* ctx, uint64_t cellCount, uint64_t 
     if (ctx->world < 1 || ctx->world > kMaxInboxSources) return false;
     if (variant == EM2_VARIANT_POPC) return false;
     if (variant == EM2_VARIANT_AUTO && !(lshCount >= 256 && double(cellCount) * double(cellCount) / ctx->world >= 1e7)) return false;
-    const uint32_t K = uint32_t(roundUp(lshCount, kChunkBytes));
-    const bool streamed = K > kMaxPanels * kChunkBytes || ctx->mmaKernel == 2 || (ctx->mmaKernel == 0 && K >= 512);
-    const uint32_t capSym = scanCandidateCapacity(uint32_t(k), uint32_t(ctx->candCapExtra));
-    const bool eligible = streamed && K <= kMaxPanels * kChunkBytes && capSym <= 32 * kPruneRegsPerLane && cellCount >= 1024 &&
-                          cellCount <= 0x7fffff00ull && mismatchMax >= 0 && k <= 1024;
-    if (!eligible || ctx->scanSymmetric == 1) return false;
+    if (!symKernelEligible(ctx, cellCount, lshCount, k, mismatchMax) || !mmaStreamed(ctx, uint32_t(roundUp(lshCount, kChunkBytes))) ||
+        cellCount < 1024 || k > 1024)
+        return false;
     if (ctx->scanSymmetric == 2) return true;
     return cellCount >= 65536 && cellCount <= 2000000ull * uint64_t(ctx->world);
 }
@@ -2286,7 +2337,7 @@ int launchScanSymDist(em2_context* ctx, const uint64_t* allSig, uint64_t cellCou
     const uint64_t rows = part.rowEnd - part.rowBegin;
     const uint32_t W = uint32_t(wordCount(lshCount));
     const uint32_t K = uint32_t(roundUp(lshCount, kSymKBits));
-    const uint32_t tau0 = uint32_t(std::min<int64_t>(mismatchMax, int64_t(lshCount)) + 1);
+    const uint32_t tau0 = scanTau0(mismatchMax, lshCount);
     ctx->stats.variant_used = EM2_VARIANT_MMA_I8;
     void *permBuf = nullptr, *enc = nullptr;
     int rc = reserve(ctx, em2_context::S_PERM, uint64_t(ctx->world) * part.shard * sizeof(uint32_t), &permBuf);
@@ -2312,14 +2363,12 @@ int launchScanSymDist(em2_context* ctx, const uint64_t* allSig, uint64_t cellCou
     int overflowed = 0;
     EM2_TRY(runSymmetric(ctx, static_cast<const uint8_t*>(enc), perm, groupStats, ctx->rowGrouping != 1, cellCount, part.rowBegin, rows,
                          part.shard, K, k, tau0, lut, pairs, usedCount, s, &overflowed));
-    if (!overflowed) {
-        ctx->stats.scan_symmetric = 1;
-        return EM2_OK;
+    if (overflowed) {
+        // a capacity ran out somewhere in the job: every rank scans its rows one-directionally (no collective involved)
+        EM2_TRY(launchScanTopK(ctx, allSig, cellCount, lshCount, part.rowBegin, part.rowEnd, k, mismatchMax, lut, EM2_VARIANT_MMA_I8,
+                               pairs, usedCount, s));
     }
-    // a capacity ran out somewhere in the job: every rank scans its rows one-directionally (no collective involved)
-    EM2_TRY(launchScanTopK(ctx, allSig, cellCount, lshCount, part.rowBegin, part.rowEnd, k, mismatchMax, lut, EM2_VARIANT_MMA_I8, pairs,
-                           usedCount, s));
-    ctx->stats.scan_symmetric = 2 + 16 * overflowed;
+    ctx->stats.scan_symmetric = symScanStatus(overflowed);
     return EM2_OK;
 }
 
@@ -2349,10 +2398,8 @@ int launchMismatchBlockMma(em2_context* ctx, const uint64_t* signatures, uint64_
 bool extendRectEligible(const em2_context* ctx, uint64_t oldCellCount, uint64_t cellCount, uint64_t lshCount, uint64_t k,
                         int64_t mismatchMax, int variant)
 {
-    if (ctx->world != 1 || variant == EM2_VARIANT_POPC || mismatchMax < 0 || lshCount > kMaxPanels * kChunkBytes) return false;
-    if (oldCellCount == 0 || oldCellCount >= cellCount || cellCount > 0x7fffff00ull) return false;
-    if (scanCandidateCapacity(uint32_t(k), uint32_t(ctx->candCapExtra)) > 32 * kPruneRegsPerLane) return false;
-    if (ctx->scanSymmetric == 1) return false;
+    if (ctx->world != 1 || variant == EM2_VARIANT_POPC || !symKernelEligible(ctx, cellCount, lshCount, k, mismatchMax)) return false;
+    if (oldCellCount == 0 || oldCellCount >= cellCount) return false;
     // AUTO: whenever the appended cells are at most as many as the old ones (beyond that the rectangle's own rows are most
     // of a whole-matrix job, which the symmetric scan does in half the pair evaluations)
     return ctx->scanSymmetric == 2 || cellCount - oldCellCount <= oldCellCount;
@@ -2368,15 +2415,11 @@ int launchExtendRect(em2_context* ctx, const uint64_t* sig, uint64_t oldN, uint6
     *overflowed = 0;
     const uint32_t W = uint32_t(wordCount(lshCount));
     const uint32_t K = uint32_t(roundUp(lshCount, kSymKBits));
-    const uint32_t panels = K / kSymKBits;
     const uint64_t N0 = oldN / kSsTileN * kSsTileN;
     const uint64_t ownRows = N - N0;
     const uint32_t S = uint32_t((N + kSsTileN - 1) / kSsTileN);
-    const bool pair = ctx->symCtaPair != 1 && ctx->smCount >= 2;
-    const uint32_t rowsPerItem = pair ? kPairRows : kRowsPerItem;
-    const uint32_t slots = pair ? uint32_t(ctx->smCount / 2) : uint32_t(ctx->smCount);
-    ScanPlan plan = makeScanPlan(ctx, ownRows, uint64_t(S) * kSsTileN, k, kSsTileN, rowsPerItem, 1, kSubStreams, slots);
-    plan.cap = candidateCapacity(uint32_t(k)) + uint32_t(k) * uint32_t(ctx->candCapExtra);
+    SymJob job(ctx, k);
+    const ScanPlan plan = makeScanPlan(ctx, ownRows, uint64_t(S) * kSsTileN, k, kSsTileN, job.rowsPerItem, 1, kSubStreams, job.slots);
     const uint32_t streams = plan.segments * kSubStreams;
 
     // column-direction traffic goes onto the N0 old cells: at most N0 entries per own row, sized like the whole-matrix
@@ -2386,100 +2429,35 @@ int launchExtendRect(em2_context* ctx, const uint64_t* sig, uint64_t oldN, uint6
     const uint64_t poolEntries = std::min<uint64_t>(0xf0000000ull * uint64_t(kLogChunk) / 64, want + slack);
     // debug_flags bit 6: a pool of one chunk, so that the overflow fallback can be exercised
     const uint32_t chunkCap = (ctx->debugFlags & 64) ? 1u : uint32_t(std::min<uint64_t>(0xfffffff0ull, (poolEntries + kLogChunk - 1) / kLogChunk));
-    size_t cubBytes = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, cubBytes, static_cast<uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), int(N + 1), s);
-    void *enc = nullptr, *cand = nullptr, *candCount = nullptr, *counters = nullptr, *sym = nullptr, *outbox = nullptr,
-         *colLog = nullptr, *chunkFill = nullptr, *cubTemp = nullptr, *pin = nullptr;
+    void* enc = nullptr;
     EM2_TRY(reserve(ctx, em2_context::S_ENCROWS, N * uint64_t(K / 2), &enc));
-    EM2_TRY(reserve(ctx, em2_context::S_CAND, size_t(streams) * ownRows * plan.cap * sizeof(uint64_t), &cand));
-    EM2_TRY(reserve(ctx, em2_context::S_CANDCOUNT, size_t(streams) * ownRows * sizeof(uint32_t), &candCount));
-    EM2_TRY(reserve(ctx, em2_context::S_COUNTERS, 64, &counters));
-    // [limEx N][inCount N + 1][inOffset N + 1][overflow 8][progress 1024]
-    EM2_TRY(reserve(ctx, em2_context::S_SYM, (3 * N + 2 + 8 + 1024) * sizeof(uint32_t), &sym));
-    EM2_TRY(reserve(ctx, em2_context::S_INBOX, size_t(chunkCap) * kLogChunk * sizeof(uint64_t), &outbox));
-    EM2_TRY(reserve(ctx, em2_context::S_COLLOG, (size_t(chunkCap) + 1) * kLogChunk * sizeof(ulonglong2), &colLog));   // + spill chunk
-    EM2_TRY(reserve(ctx, em2_context::S_COLLOGFILL, (size_t(chunkCap) + 4) * sizeof(uint32_t), &chunkFill));
-    EM2_TRY(reserve(ctx, em2_context::S_MISC, cubBytes, &cubTemp));
-    EM2_TRY(reservePinned(ctx, 2, 64, &pin));
-    uint32_t* limEx = static_cast<uint32_t*>(sym);
-    uint32_t* inCount = limEx + N;
-    uint32_t* inOffset = inCount + N + 1;
-    uint32_t* overflow = inOffset + N + 1;
-    uint32_t* progress = overflow + 8;
-
+    EM2_TRY(job.reserve(ctx, N, N, N, ownRows, streams, chunkCap, s));
     EM2_TRY(encodeFp4(ctx, sig, W, N, K, static_cast<uint8_t*>(enc), nullptr, s));
-    EM2_CUDA(ctx, cudaMemsetAsync(chunkFill, 0, (size_t(chunkCap) + 4) * sizeof(uint32_t), s));
-    EM2_CUDA(ctx, cudaMemsetAsync(inCount, 0, (N + 1) * sizeof(uint32_t), s));
-    EM2_CUDA(ctx, cudaMemsetAsync(overflow, 0, 8 * sizeof(uint32_t), s));
-    EM2_CUDA(ctx, cudaMemsetAsync(candCount, 0, size_t(streams) * ownRows * sizeof(uint32_t), s));
+    EM2_TRY(job.initialise(ctx, static_cast<const uint8_t*>(enc), K, N0, ownRows, tau0, N0, nullptr, s));
+    const SymParams& p = job.p;
+    uint32_t* limEx = p.limEx;
     if (N0) EM2_CUDA(ctx, cudaMemcpyAsync(limEx, oldBound, N0 * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
-    fillU32Kernel<<<unsigned((ownRows + 255) / 256), 256, 0, s>>>(limEx + N0, ownRows, tau0);
-    EM2_CUDA(ctx, cudaGetLastError());
-    ctx->stats.kernel_launches++;
-
-    SymParams p{};
-    p.cellCount = N;
-    p.K = K;
-    p.panels = panels;
-    size_t smem = 0;
-    EM2_TRY(symKernelSmem(ctx, panels, pair, &p.stages, &smem));
-    p.mainBlocks = plan.mainBlocks;
-    p.segments = plan.segments;
-    p.items = plan.items;
-    p.segmentCols = plan.segmentCols;
-    p.superBlocks = S;
-    p.halfOffset = 0;          // every column super block is visited by this row block only: no offset is seen twice
-    p.dBegin = 0;
-    p.offsetsHere = S;
-    p.resume = 0;
-    p.segBase = 0;
-    p.rowOnly = 0;
-    p.posBegin = uint32_t(N0);
-    p.ownRows = uint32_t(ownRows);
-    p.k = uint32_t(k);
-    p.cap = plan.cap;
-    p.cand = static_cast<uint64_t*>(cand);
-    p.candCount = static_cast<uint32_t*>(candCount);
-    p.appendedTotal = static_cast<unsigned long long*>(counters) + 1;
-    p.limEx = limEx;
-    p.colDirEnd = uint32_t(N0);
-    p.colLog = static_cast<ulonglong2*>(colLog);
-    p.chunkFill = static_cast<uint32_t*>(chunkFill);
-    p.chunkNext = static_cast<uint32_t*>(chunkFill) + chunkCap;
-    p.chunkCap = chunkCap;
-    p.overflow = overflow;
-    p.perm = nullptr;
-    p.flags = uint32_t(ctx->debugFlags);
-    // pacing as in the whole-matrix scan's far sweep: only for rows long enough for the CTAs to drift apart
-    p.progress = (S >= 768 && !(ctx->debugFlags & 16)) ? progress : nullptr;
-    if (p.progress) EM2_CUDA(ctx, cudaMemsetAsync(progress, 0, 1024 * sizeof(uint32_t), s));
-    CUtensorMap mapA, mapB;
-    EM2_TRY(makeTensorMapU8(ctx, &mapA, enc, N, K / 2, K / 2, kRowsPerItem));
-    EM2_TRY(makeTensorMapU8(ctx, &mapB, enc, N, K / 2, K / 2, pair ? kSymHalfN / 2 : kSymHalfN));
-    EM2_TRY(launchSymKernel(ctx, pair, slots, smem, mapA, mapB, p, s));
-    EM2_TRY(fileColumnLog(ctx, p, N, inCount, inOffset, static_cast<uint64_t*>(outbox), cubTemp, cubBytes, uint32_t(oldN), s));
+    // every column super block once (dBegin 0, S offsets), by this row block only: no offset is seen twice (halfOffset 0)
+    EM2_TRY(job.launch(ctx, plan, 0, S, 0, 0, 0, 0, s));
+    EM2_TRY(job.fileLog(ctx, uint32_t(oldN), s));
 
     InboxSources src{};
     src.count = 1;
-    src.keys[0] = static_cast<const uint64_t*>(outbox);
-    src.offsets[0] = inOffset + N0;      // own rows: indexed by position - N0 (their inboxes are empty)
-    EM2_TRY(launchFinalizeSym(ctx, ownRows, N0, streams, plan.cap, k, p.cand, p.candCount, src, limEx, lut, pairs + N0 * k,
-                              usedCount + N0, nullptr, overflow, s));
+    src.keys[0] = job.outbox;
+    src.offsets[0] = job.inOffset + N0;      // own rows: indexed by position - N0 (their inboxes are empty)
+    EM2_TRY(launchFinalizeSym(ctx, ownRows, N0, streams, p.cap, k, p.cand, p.candCount, src, limEx, lut, pairs + N0 * k,
+                              usedCount + N0, nullptr, p.overflow, s));
     if (N0) {
         // old rows: the old keys are the one stream, the inbox holds the new cells that beat the k-th entry; every key is
         // below tau0, which becomes the merge bound
         fillU32Kernel<<<unsigned((N0 + 255) / 256), 256, 0, s>>>(limEx, N0, tau0);
         EM2_CUDA(ctx, cudaGetLastError());
         ctx->stats.kernel_launches++;
-        src.offsets[0] = inOffset;
+        src.offsets[0] = job.inOffset;
         EM2_TRY(launchFinalizeSym(ctx, N0, 0, 1, uint32_t(k), k, oldKeys, oldUsed, src, limEx, lut, pairs, usedCount, nullptr,
-                                  overflow, s));
+                                  p.overflow, s));
     }
-    uint32_t* host = static_cast<uint32_t*>(pin);
-    EM2_CUDA(ctx, cudaMemcpyAsync(host, overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    *overflowed = int(*host);
-    return EM2_OK;
+    return job.readOverflow(ctx, s, overflowed);
 }
 
 }  // namespace em2

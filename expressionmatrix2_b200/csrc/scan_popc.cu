@@ -557,7 +557,7 @@ int launchScanTopK(em2_context* ctx, const uint64_t* signatures, uint64_t cellCo
     const bool regs = W <= 16;
     const uint32_t tileCols = regs ? kTileCols : 16;
     ScanPlan plan = makeScanPlan(ctx, rows, cellCount, k, tileCols, kScanThreads, 2, 1);
-    const uint32_t tau0 = mismatchMax < 0 ? 0u : uint32_t(std::min<int64_t>(mismatchMax, int64_t(lshCount)) + 1);
+    const uint32_t tau0 = scanTau0(mismatchMax, lshCount);
 
     void* cand = nullptr;
     void* candCount = nullptr;
