@@ -79,6 +79,7 @@ def lib():
     L.em2_lsh_similar_pairs.argtypes = [vp, u64, u64, vp, vp, vp, u64, u64, dbl, i32, vp, vp, vp]
     L.em2_extend_similar_pairs.argtypes = [vp, vp, u64, u64, u64, u64, dbl, i32, vp, vp, vp, vp]
     L.em2_exact_similar_pairs.argtypes = [vp, u64, u64, vp, vp, u64, dbl, vp, vp]
+    L.em2_extend_exact_similar_pairs.argtypes = [vp, u64, u64, u64, vp, vp, u64, dbl, vp, vp, vp, vp]
     L.em2_cell_graph_edges.argtypes = [vp, u64, u64, vp, vp, vp, dbl, u64, vp, u64, vp]
     L.em2_signature_graph.argtypes = [vp, vp, u64, u64, u64, vp, vp, u64, vp, vp, u64, vp]
     L.em2_find_similar_pairs7.argtypes = [vp, vp, u64, u64, u64, dbl, vp, u64, C.c_uint32, u64, vp, vp]
@@ -433,6 +434,31 @@ class Engine:
         self._check(self._L.em2_exact_similar_pairs(self._h, n, gene_count, _ptr(toc), _ptr(pairs), k,
                                                     similarity_threshold, _ptr(out), _ptr(used)),
                     "em2_exact_similar_pairs")
+        return np.ascontiguousarray(out["cell"]), np.ascontiguousarray(out["similarity"]), used
+
+    def extend_exact_similar_pairs(self, toc, counts, gene_count: int, old_cell_count: int, old_ids, old_sims, old_used, k: int,
+                                   similarity_threshold: float, gene_ids=None):
+        """Lists of exact_similar_pairs over the first old_cell_count cells (old_ids / old_sims [old, k], old_used [old]),
+        extended to the cells after them (em2_extend_exact_similar_pairs); toc / counts hold all cells, old cells first.
+        Returns (ids, sims, used) for all rows, equal to exact_similar_pairs over all cells.  Raises Em2Error if the old lists
+        do not belong to these counts, k and threshold.  Lists made with a HIGHER threshold than this call's cannot be
+        detected (their rows lack the cells between the two thresholds) and give wrong lists; lists made with a lower
+        threshold are rejected or are already exact."""
+        toc = np.ascontiguousarray(toc, np.uint64)
+        pairs = _as_pairs(counts, gene_ids)
+        n = len(toc) - 1
+        old = np.zeros((old_cell_count, k), SIMPAIR_DTYPE)
+        if old_cell_count:
+            old["cell"] = np.asarray(old_ids, np.uint32).reshape(old_cell_count, k)
+            old["similarity"] = np.asarray(old_sims, np.float32).reshape(old_cell_count, k)
+        old_used = np.ascontiguousarray(old_used, np.uint32)
+        if old_used.shape != (old_cell_count,):
+            raise ValueError("old_used must hold one count per old cell")
+        out = np.zeros((n, k), SIMPAIR_DTYPE)
+        used = np.zeros(n, np.uint32)
+        self._check(self._L.em2_extend_exact_similar_pairs(self._h, old_cell_count, n, gene_count, _ptr(toc), _ptr(pairs), k,
+                                                           similarity_threshold, _ptr(old), _ptr(old_used), _ptr(out), _ptr(used)),
+                    "em2_extend_exact_similar_pairs")
         return np.ascontiguousarray(out["cell"]), np.ascontiguousarray(out["similarity"]), used
 
     # ---- device-resident calls (torch CUDA tensors or raw device pointers) ------------------------

@@ -247,6 +247,30 @@ int launchMismatchBlock(em2_context* ctx, const uint64_t* signatures, uint64_t c
 int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
                 const em2_count* counts, const double* sum1, const double* sum2, uint64_t k,
                 double similarityThreshold, em2_pair* pairs, uint32_t* usedCount, cudaStream_t s);
+// The exact path's argument checks: k in [1, 1024], the size limits, similarityThreshold <= 1.
+int checkExactArguments(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, uint64_t k, double similarityThreshold);
+// Extension of exact lists of cells [0, oldN) to cells [oldN, N) (exact.cu; extend.cu has the entry point).  Device pointers:
+// oldPairs / oldUsed the old lists, winPairs / winUsed scratch for oldN rows, flags one word.  *badFlags (kExtend*) != 0: the
+// old lists failed validation and nothing was computed.  *scanSymmetric: 1 = the rectangle ran, 0 = the full job or nothing
+// appended.
+int launchExtendExact(em2_context* ctx, uint64_t oldN, uint64_t N, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
+                      const double* sum1, const double* sum2, uint64_t k, double similarityThreshold, const em2_pair* oldPairs,
+                      const uint32_t* oldUsed, em2_pair* winPairs, uint32_t* winUsed, uint32_t* flags, em2_pair* pairs,
+                      uint32_t* usedCount, cudaStream_t s, uint32_t* badFlags, int* scanSymmetric);
+
+// Validation of old lists by the extension calls: what a stored entry got wrong, OR-ed over all entries.
+enum : uint32_t {
+    kExtendBadUsed = 1,        // usedCount > k
+    kExtendBadId = 2,          // an id >= oldCellCount
+    kExtendBadSelf = 4,        // a row lists its own cell
+    kExtendBadThreshold = 8,   // the recomputed similarity does not pass the threshold
+    kExtendBadSimilarity = 16, // the stored similarity is not the recomputed one
+    kExtendBadOrder = 32,      // a row is not strictly increasing in (similarity desc, id asc)
+};
+// Text of those flags; `source` names what the similarities were recomputed from.
+std::string describeFlags(uint32_t flags, const char* source);
+// Whether two byte ranges overlap.
+bool overlaps(const void* a, size_t aBytes, const void* b, size_t bBytes);
 
 // ---- multi-GPU (multi.cu) -------------------------------------------------------------------------------------
 // Rank r owns the cells [r * shard, min(N, (r + 1) * shard)); shard is a multiple of 256 when there is more than one rank.

@@ -25,6 +25,10 @@
 // warp 5 MMA issuer; tile 128 x 128 cells, K = genes in 128-byte chunks, both operands are row blocks of the
 // SAME dense planes (128B-swizzled TMA boxes).  Tiles are visited in 12 x 12 super-tiles so that the ~148
 // CTAs running at any moment share 24 row/column panels through L2 instead of streaming 148 distinct ones.
+//
+// launchExtendExact extends the lists of a job over the first N cells to cells appended after them with the same kernels:
+// the new rows against all columns, the old rows against a column window of the new cells (ExactParams.colBegin), and a
+// merge with the old lists after exactValidateKernel has recomputed every stored entry with the full job's bits.
 #include "common.cuh"
 #include "tc05.cuh"
 
@@ -45,6 +49,18 @@ constexpr uint32_t kXPlaneBytes = kXTile * kXChunk;   // 16 KB: one operand tile
 constexpr int kXThreads = 192;
 constexpr int kXSuper = 12;
 constexpr float kRejected = -2.f;     // marker in the similarity matrix (r >= -1 always)
+
+// The reference's operation sequence for r (src/ExpressionMatrixSubset.cpp:118-126): separate multiplies, subtract, sqrt,
+// divide, each rounded to nearest.  The GEMM epilogue, the general kernel and the validation of old lists
+// (exactValidateKernel) all go through these two functions, so their bits cannot drift apart.
+__device__ __forceinline__ double pearsonNumerator(double n, double scalarProduct, double s1a, double s1b)
+{
+    return __dsub_rn(__dmul_rn(n, scalarProduct), __dmul_rn(s1a, s1b));
+}
+__device__ __forceinline__ double pearsonR(double numerator, double va, double vb)
+{
+    return __ddiv_rn(numerator, __dsqrt_rn(__dmul_rn(va, vb)));
+}
 
 // max count, integrality, max sum2, max nnz: decides the digit count on the host.
 __global__ void exactScanKernel(uint64_t cellCount, uint64_t geneCount, const uint64_t* __restrict__ toc,
@@ -116,7 +132,8 @@ exactDensifyKernel(uint64_t cellCount, uint64_t geneCount, uint64_t gPad, const 
 }
 
 struct ExactParams {
-    uint64_t cellCount;          // N (columns)
+    uint64_t cellCount;          // end of the column window (N for whole-matrix calls)
+    uint64_t colBegin;           // first column of the window: column j of the output is cell colBegin + j
     uint64_t rowBegin, rows;     // rows of this chunk
     uint64_t geneCount;
     uint32_t kChunks;
@@ -212,7 +229,7 @@ exactGemmKernel(const __grid_constant__ CUtensorMap mapLo, const __grid_constant
                 uint32_t rb, ct;
                 if (!itemToTile(p, item, rb, ct)) continue;
                 const int32_t rowA = int32_t(p.rowBegin + uint64_t(rb) * p.rowsPerItem + rank * kXTile);
-                const int32_t rowB = int32_t(ct * kN + (PAIR ? rank * (kN / 2) : 0));
+                const int32_t rowB = int32_t(p.colBegin + ct * kN + (PAIR ? rank * (kN / 2) : 0));
                 for (uint32_t kc = 0; kc < p.kChunks; kc++) {
                     mbarWait(empty + stage, phase ^ 1);
                     uint8_t* dst = ring + size_t(stage) * kStageBytes;
@@ -335,18 +352,17 @@ exactGemmKernel(const __grid_constant__ CUtensorMap mapLo, const __grid_constant
 #pragma unroll
                     for (int jj = 0; jj < 4; jj++) {
                         const int j = j4 + jj;
-                        const uint64_t b = bBase + j;
+                        const uint64_t b = p.colBegin + bBase + j;                           // column cell
                         float res = kRejected;
                         if (b < p.cellCount && b != a) {
                             double sp = double(ll[j]);                                        // u8 x u8 sums are non-negative
                             if (DIGITS == 2) sp = fma(fma(double(hh[j]), 256., double(xx[j])), 256., sp);   // exact
-                            const double num = __dsub_rn(__dmul_rn(n, sp), __dmul_rn(s1a, __ldg(p.sum1 + b)));
+                            const double num = pearsonNumerator(n, sp, s1a, __ldg(p.sum1 + b));
                             // float estimate of r (relative error < 1e-6, |r| <= 1): only candidates within
                             // 1e-4 of the threshold or above it pay for the exact double sqrt and divide
                             const float estimate = float(num) * rinvA * __ldg(p.rinv + b);
                             if (!(estimate < p.thresholdLow)) {
-                                const double den = __dsqrt_rn(__dmul_rn(va, __ldg(p.var + b)));
-                                const double r = __ddiv_rn(num, den);
+                                const double r = pearsonR(num, va, __ldg(p.var + b));
                                 if (r > p.threshold) res = float(r);
                             }
                         }
@@ -356,7 +372,7 @@ exactGemmKernel(const __grid_constant__ CUtensorMap mapLo, const __grid_constant
                         if (bBase + j4 + 3 < p.ldOut)
                             *reinterpret_cast<float4*>(outRow + q * 32 + j4) = make_float4(r4[0], r4[1], r4[2], r4[3]);
                         // r(a,b) == r(b,a): a tile above the diagonal also fills its mirror image.  For a fixed b the
-                        // 32 lanes of a warp write 32 consecutive floats of row b.
+                        // 32 lanes of a warp write 32 consecutive floats of row b.  (Symmetric mode has colBegin == 0.)
                         if (mirror) {
 #pragma unroll
                             for (int jj = 0; jj < 4; jj++) {
@@ -398,7 +414,7 @@ exactGemmKernel(const __grid_constant__ CUtensorMap mapLo, const __grid_constant
 constexpr int kGenWarps = 8;
 
 __global__ void __launch_bounds__(kGenWarps * 32)
-exactGeneralKernel(uint64_t cellCount, uint64_t geneCount, uint64_t gPad, uint64_t rowBegin, uint64_t rows,
+exactGeneralKernel(uint64_t colBegin, uint64_t colEnd, uint64_t geneCount, uint64_t gPad, uint64_t rowBegin, uint64_t rows,
                    const uint64_t* __restrict__ toc, const em2_count* __restrict__ counts, const double* __restrict__ sum1,
                    const double* __restrict__ var, double threshold, uint64_t ldOut, float* __restrict__ out)
 {
@@ -419,7 +435,7 @@ exactGeneralKernel(uint64_t cellCount, uint64_t geneCount, uint64_t gPad, uint64
     const bool has1 = local0 + 1 < rows;
     const double s1a0 = sum1[a0], va0 = var[a0];
     const double s1a1 = has1 ? sum1[a1] : 0., va1 = has1 ? var[a1] : 0.;
-    for (uint64_t b = warp; b < cellCount; b += kGenWarps) {
+    for (uint64_t b = colBegin + warp; b < colEnd; b += kGenWarps) {
         double acc0 = 0., acc1 = 0.;
         const uint64_t end = toc[b + 1];
         for (uint64_t e = toc[b] + lane; e < end; e += 32) {
@@ -437,11 +453,10 @@ exactGeneralKernel(uint64_t cellCount, uint64_t geneCount, uint64_t gPad, uint64
             const uint64_t a = lane == 0 ? a0 : a1;
             float res = kRejected;
             if (b != a) {
-                const double num = __dsub_rn(__dmul_rn(n, sp), __dmul_rn(s1a, sum1[b]));
-                const double r = __ddiv_rn(num, __dsqrt_rn(__dmul_rn(va, var[b])));
+                const double r = pearsonR(pearsonNumerator(n, sp, s1a, sum1[b]), va, var[b]);
                 if (r > threshold) res = float(r);
             }
-            out[(local0 + lane) * ldOut + b] = res;
+            out[(local0 + lane) * ldOut + (b - colBegin)] = res;
         }
     }
 }
@@ -524,18 +539,174 @@ exactSelectKernel(uint64_t rows, uint64_t cellCount, uint64_t ldOut, const float
     if (lane == 0) usedCount[row] = count;
 }
 
+// ---- extension of old lists to appended cells (launchExtendExact) --------------------------------------------------
+// The stored count of `gene` in cell c, 0 when there is none (genes ascend within a cell): the value the general kernel's
+// dense row holds for that gene.
+__device__ __forceinline__ float storedCount(const uint64_t* __restrict__ toc, const em2_count* __restrict__ counts, uint64_t c,
+                                             uint32_t gene)
+{
+    uint64_t lo = toc[c], hi = toc[c + 1];
+    const uint64_t end = hi;
+    while (lo < hi) {
+        const uint64_t mid = (lo + hi) >> 1;
+        if (counts[mid].gene < gene) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo < end && counts[lo].gene == gene ? counts[lo].count : 0.f;
+}
+
+// One warp per old row a.  Every stored entry (a, b) is recomputed with the bits of the full job, the row cell on the dense
+// side as in both full-job kernels:
+//   integer path: the exact integer scalar product, the row's counts read from its digit planes;
+//   general path: the general kernel's lane partition (b's entries strided over the lanes, float products, double sums) and
+//                 its shuffle tree, the row's counts found by search in its CSR.
+// Then r through pearsonNumerator / pearsonR.  Flags as em2_extend_similar_pairs (kExtend*).  outPairs / outUsed: the row as
+// em2_exact_similar_pairs writes it (unused slots zeroed) -- the result when nothing was appended.
+constexpr int kValWarps = 8;
+template <bool GENERAL>
+__global__ void __launch_bounds__(kValWarps * 32)
+exactValidateKernel(uint64_t oldN, uint64_t geneCount, uint64_t gPad, const uint64_t* __restrict__ toc,
+                    const em2_count* __restrict__ counts, const uint8_t* __restrict__ lo, const uint8_t* __restrict__ hi,
+                    const double* __restrict__ sum1, const double* __restrict__ var, double threshold, uint32_t k,
+                    const em2_pair* __restrict__ oldPairs, const uint32_t* __restrict__ oldUsed, em2_pair* __restrict__ outPairs,
+                    uint32_t* __restrict__ outUsed, uint32_t* __restrict__ flags)
+{
+    const uint64_t a = uint64_t(blockIdx.x) * kValWarps + (threadIdx.x >> 5);
+    const uint32_t lane = threadIdx.x & 31;
+    if (a >= oldN) return;
+    const uint32_t used = oldUsed[a];
+    if (used > k) {
+        if (lane == 0) atomicOr(flags, kExtendBadUsed);
+        return;
+    }
+    const double n = double(geneCount), s1a = sum1[a], va = var[a];
+    const em2_pair* row = oldPairs + a * k;
+    uint32_t bad = 0;
+    uint64_t prevKey = 0;
+    for (uint32_t i = 0; i < used; i++) {
+        const em2_pair e = row[i];
+        const uint64_t key = (uint64_t(~orderable(e.similarity)) << 32) | e.cell;
+        if (i && !(prevKey < key)) bad |= kExtendBadOrder;
+        prevKey = key;
+        if (e.cell >= oldN) {
+            bad |= kExtendBadId;
+            continue;
+        }
+        if (e.cell == a) {
+            bad |= kExtendBadSelf;
+            continue;
+        }
+        const uint64_t b = e.cell, end = toc[b + 1];
+        double sp;
+        if (GENERAL) {
+            double acc = 0.;
+            for (uint64_t x = toc[b] + lane; x < end; x += 32) {
+                const em2_count q = counts[x];
+                acc += double(__fmul_rn(storedCount(toc, counts, a, q.gene), q.count));
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+            sp = acc;
+        } else {
+            unsigned long long acc = 0;
+            for (uint64_t x = toc[b] + lane; x < end; x += 32) {
+                const em2_count q = counts[x];
+                uint32_t ca = lo[a * gPad + q.gene];
+                if (hi) ca |= uint32_t(hi[a * gPad + q.gene]) << 8;
+                acc += (unsigned long long)ca * uint32_t(q.count);
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+            sp = double(acc);     // < 2^53: the host's s32 bounds keep the digit sums far below
+        }
+        const double r = pearsonR(pearsonNumerator(n, sp, s1a, sum1[b]), va, var[b]);
+        if (!(r > threshold)) bad |= kExtendBadThreshold;
+        else if (__float_as_uint(float(r)) != __float_as_uint(e.similarity)) bad |= kExtendBadSimilarity;
+    }
+    if (lane == 0 && bad) atomicOr(flags, bad);
+    for (uint32_t i = lane; i < k; i += 32) {
+        em2_pair out;
+        out.cell = 0;
+        out.similarity = 0.f;
+        if (i < used) out = row[i];
+        outPairs[a * k + i] = out;
+    }
+    if (lane == 0) outUsed[a] = used;
+}
+
+// One warp per old row: the k best of its validated old list and its list over the appended columns (window ids, + oldN).
+// Every new id is above every old one, so the keys (similarity desc, id asc) of the two lists are distinct and an entry's
+// place in the merged row is its own index plus the number of entries of the other list with a smaller key.
+__device__ __forceinline__ uint64_t pairKey(em2_pair e, uint32_t idOffset)
+{
+    return (uint64_t(~orderable(e.similarity)) << 32) | (e.cell + idOffset);
+}
+__device__ __forceinline__ uint32_t countBelow(const em2_pair* list, uint32_t used, uint32_t idOffset, uint64_t key)
+{
+    uint32_t lo = 0, hi = used;
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (pairKey(list[mid], idOffset) < key) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+constexpr int kMergeWarps = 8;
+__global__ void __launch_bounds__(kMergeWarps * 32)
+exactMergeKernel(uint64_t oldN, uint32_t k, const em2_pair* __restrict__ oldPairs, const uint32_t* __restrict__ oldUsed,
+                 const em2_pair* __restrict__ winPairs, const uint32_t* __restrict__ winUsed, em2_pair* __restrict__ pairs,
+                 uint32_t* __restrict__ usedCount)
+{
+    const uint64_t a = uint64_t(blockIdx.x) * kMergeWarps + (threadIdx.x >> 5);
+    const uint32_t lane = threadIdx.x & 31;
+    if (a >= oldN) return;
+    const uint32_t newId = uint32_t(oldN);
+    const uint32_t uo = oldUsed[a], uw = winUsed[a];
+    const em2_pair* A = oldPairs + a * k;
+    const em2_pair* B = winPairs + a * k;
+    em2_pair* out = pairs + a * k;
+    for (uint32_t i = lane; i < uo; i += 32) {
+        const uint32_t pos = i + countBelow(B, uw, newId, pairKey(A[i], 0));
+        if (pos < k) out[pos] = A[i];
+    }
+    for (uint32_t i = lane; i < uw; i += 32) {
+        em2_pair e = B[i];
+        const uint32_t pos = i + countBelow(A, uo, 0, pairKey(e, newId));
+        e.cell += newId;
+        if (pos < k) out[pos] = e;
+    }
+    const uint32_t total = min(k, uo + uw);
+    for (uint32_t i = total + lane; i < k; i += 32) {
+        em2_pair z;
+        z.cell = 0;
+        z.similarity = 0.f;
+        out[i] = z;
+    }
+    if (lane == 0) usedCount[a] = total;
+}
+
 }  // namespace
 
-int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
-                const double* sum1, const double* sum2, uint64_t k, double similarityThreshold, em2_pair* pairs,
-                uint32_t* usedCount, cudaStream_t s)
+int checkExactArguments(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, uint64_t k, double similarityThreshold)
 {
     if (k == 0 || k > 1024) return fail(ctx, EM2_ERR_INVALID, "k must be in [1, 1024]");
     if (cellCount > 0x7fffff00ull || geneCount > 0x7fffff00ull) return fail(ctx, EM2_ERR_INVALID, "matrix too large for the exact path");
     if (!(similarityThreshold <= 1.)) return fail(ctx, EM2_ERR_INVALID, "similarityThreshold must be <= 1");   // CZI_ASSERT, FindSimilarPairs.cpp:27
-    const uint64_t gPad = roundUp(geneCount, kXChunk);
+    return EM2_OK;
+}
 
-    // ---- what do the counts look like? ---------------------------------------------------------------
+namespace {
+
+// The arithmetic the exact path uses for a set of cells, decided from all of their counts: the general FP64 kernel, or the
+// integer tensor-core path with one or two digit planes.
+struct ExactArith {
+    bool general;
+    int digits;
+};
+
+int exactArithmetic(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
+                    const double* sum2, cudaStream_t s, ExactArith* arith)
+{
     void* misc = nullptr;
     EM2_TRY(reserve(ctx, em2_context::S_MISC, 64, &misc));
     EM2_CUDA(ctx, cudaMemsetAsync(misc, 0, 64, s));
@@ -552,21 +723,77 @@ int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const 
     const double llBound = digits == 1 ? maxSum2 : std::min(maxSum2, 65025. * double(h[3]));
     // Counts that are not integers in [0, 65535], or sums that would overflow the s32 accumulators, take the general
     // FP64 kernel (exactGeneralKernel); "exact_general" = 1 forces it (tests).
-    const bool general = (h[1] & 1) || llBound >= 2147483648. || maxSum2 / 128. >= 2147483648. || ctx->exactGeneral != 0;
-    if (general) {
-        const uint64_t ldG = roundUp(cellCount, 256);
-        if (2 * gPad * sizeof(float) > 200 * 1024)
+    arith->general = (h[1] & 1) || llBound >= 2147483648. || maxSum2 / 128. >= 2147483648. || ctx->exactGeneral != 0;
+    arith->digits = digits;
+    return EM2_OK;
+}
+
+// Per-cell operands of all cells for the chosen arithmetic.
+struct ExactOperands {
+    ExactArith arith;
+    uint64_t cellCount, geneCount, gPad;
+    const uint64_t* toc;
+    const em2_count* counts;
+    const double* sum1;
+    double* var;                 // n * sum2 - sum1^2
+    float* rinv;                 // integer path: float reciprocal roots of var (the epilogue's pre-filter)
+    uint8_t *lo, *hi;            // integer path: digit planes [cellCount][gPad] (hi: two digits only)
+};
+
+int exactPrepare(em2_context* ctx, const ExactArith& arith, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
+                 const em2_count* counts, const double* sum1, const double* sum2, cudaStream_t s, ExactOperands* o)
+{
+    *o = ExactOperands{};
+    o->arith = arith;
+    o->cellCount = cellCount;
+    o->geneCount = geneCount;
+    o->gPad = roundUp(geneCount, kXChunk);
+    o->toc = toc;
+    o->counts = counts;
+    o->sum1 = sum1;
+    if (arith.general) {
+        if (2 * o->gPad * sizeof(float) > 200 * 1024)
             return fail(ctx, EM2_ERR_INVALID, "em2_exact_similar_pairs: non-integer counts with more than 25,600 genes are not supported");
         void* varG = nullptr;
         EM2_TRY(reserve(ctx, em2_context::S_FLAGS, cellCount * sizeof(double), &varG));
+        o->var = static_cast<double*>(varG);
         // per-cell variance term (the densify kernel's by-product in the tensor-core path)
         exactDensifyKernel<<<unsigned((cellCount + 7) / 8), 256, 0, s>>>(cellCount, geneCount, 0, toc, counts, sum1, sum2, nullptr,
-                                                                        nullptr, static_cast<double*>(varG), nullptr);
+                                                                        nullptr, o->var, nullptr);
         ctx->stats.kernel_launches++;
         EM2_CUDA(ctx, cudaGetLastError());
-        const uint64_t budgetG = ctx->exactMatrixBytes ? ctx->exactMatrixBytes : (48ull << 30);
-        uint64_t chunkG = std::max<uint64_t>(2, budgetG / (ldG * sizeof(float)) / 2 * 2);
-        chunkG = std::min<uint64_t>(chunkG, roundUp(cellCount, 2));
+        return EM2_OK;
+    }
+    // ---- dense digit planes ----------------------------------------------------------------------------
+    void *lo = nullptr, *var = nullptr;
+    EM2_TRY(reserve(ctx, em2_context::S_DENSE, cellCount * o->gPad * arith.digits, &lo));
+    o->lo = static_cast<uint8_t*>(lo);
+    if (arith.digits == 2) o->hi = o->lo + cellCount * o->gPad;
+    EM2_TRY(reserve(ctx, em2_context::S_FLAGS, cellCount * (sizeof(double) + sizeof(float)), &var));
+    o->var = static_cast<double*>(var);
+    o->rinv = reinterpret_cast<float*>(o->var + cellCount);
+    exactDensifyKernel<<<unsigned((cellCount + 7) / 8), 256, 0, s>>>(cellCount, geneCount, o->gPad, toc, counts, sum1, sum2, o->lo,
+                                                                    o->hi, o->var, o->rinv);
+    ctx->stats.kernel_launches++;
+    EM2_CUDA(ctx, cudaGetLastError());
+    return EM2_OK;
+}
+
+// Rows [rowBegin, rowEnd) against the column window [colBegin, colEnd): each row's k best (similarity desc, column asc)
+// among the window's cells other than itself with r > threshold, into pairs / usedCount from the list of row rowBegin on,
+// with ids RELATIVE TO colBegin.  Rows go in chunks under the similarity-matrix budget.  wholeMatrix (all rows against all
+// columns): when the whole N x N matrix fits the budget, only the tiles on or above the diagonal are computed (half the
+// MMAs) and mirrored.
+int exactRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint64_t rowEnd, uint64_t colBegin, uint64_t colEnd,
+              uint64_t k, double similarityThreshold, bool wholeMatrix, em2_pair* pairs, uint32_t* usedCount, cudaStream_t s)
+{
+    const uint64_t rowCount = rowEnd - rowBegin, cols = colEnd - colBegin, gPad = o.gPad;
+    if (rowCount == 0 || cols == 0) return EM2_OK;
+    const uint64_t budget = ctx->exactMatrixBytes ? ctx->exactMatrixBytes : (48ull << 30);
+    if (o.arith.general) {
+        const uint64_t ldG = roundUp(cols, 256);
+        uint64_t chunkG = std::max<uint64_t>(2, budget / (ldG * sizeof(float)) / 2 * 2);
+        chunkG = std::min<uint64_t>(chunkG, roundUp(rowCount, 2));
         void* simG = nullptr;
         EM2_TRY(reserve(ctx, em2_context::S_CAND, chunkG * ldG * sizeof(float), &simG));
         const size_t smemG = 2 * gPad * sizeof(float);
@@ -574,49 +801,35 @@ int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const 
         const uint32_t capG = uint32_t(2 * k + 64);
         const size_t smemSelG = size_t(kSelWarps) * 2 * capG * sizeof(uint64_t);
         EM2_CUDA(ctx, cudaFuncSetAttribute(exactSelectKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemSelG)));
-        for (uint64_t begin = 0; begin < cellCount; begin += chunkG) {
-            const uint64_t rows = std::min(chunkG, cellCount - begin);
+        for (uint64_t begin = 0; begin < rowCount; begin += chunkG) {
+            const uint64_t rows = std::min(chunkG, rowCount - begin);
             exactGeneralKernel<<<unsigned((rows + 1) / 2), kGenWarps * 32, smemG, s>>>(
-                cellCount, geneCount, gPad, begin, rows, toc, counts, sum1, static_cast<const double*>(varG), similarityThreshold,
+                colBegin, colEnd, o.geneCount, gPad, rowBegin + begin, rows, o.toc, o.counts, o.sum1, o.var, similarityThreshold,
                 ldG, static_cast<float*>(simG));
             ctx->stats.kernel_launches++;
             EM2_CUDA(ctx, cudaGetLastError());
             exactSelectKernel<<<unsigned((rows + kSelWarps - 1) / kSelWarps), kSelWarps * 32, smemSelG, s>>>(
-                rows, cellCount, ldG, static_cast<const float*>(simG), uint32_t(k), capG, pairs + begin * k, usedCount + begin);
+                rows, cols, ldG, static_cast<const float*>(simG), uint32_t(k), capG, pairs + begin * k, usedCount + begin);
             ctx->stats.kernel_launches++;
             EM2_CUDA(ctx, cudaGetLastError());
         }
-        ctx->stats.variant_used = EM2_VARIANT_POPC;      // "not the tensor-core path"
         return EM2_OK;
     }
 
-    // ---- dense digit planes ----------------------------------------------------------------------------
-    void *lo = nullptr, *hi = nullptr, *var = nullptr;
-    EM2_TRY(reserve(ctx, em2_context::S_DENSE, cellCount * gPad * digits, &lo));
-    if (digits == 2) hi = static_cast<uint8_t*>(lo) + cellCount * gPad;
-    EM2_TRY(reserve(ctx, em2_context::S_FLAGS, cellCount * (sizeof(double) + sizeof(float)), &var));
-    float* rinv = reinterpret_cast<float*>(static_cast<double*>(var) + cellCount);
-    exactDensifyKernel<<<unsigned((cellCount + 7) / 8), 256, 0, s>>>(cellCount, geneCount, gPad, toc, counts, sum1, sum2,
-                                                                    static_cast<uint8_t*>(lo), static_cast<uint8_t*>(hi),
-                                                                    static_cast<double*>(var), rinv);
-    ctx->stats.kernel_launches++;
-    EM2_CUDA(ctx, cudaGetLastError());
-
     // ---- row chunks: GEMM + epilogue into the similarity matrix, then selection --------------------------
-    const uint64_t ldOut = roundUp(cellCount, 256);
-    // If the whole N x N similarity matrix fits the budget, only the tiles on or above the diagonal are computed
-    // (half the MMAs) and mirrored; otherwise rows go in chunks and every chunk computes all of its tiles.
-    const uint64_t budget = ctx->exactMatrixBytes ? ctx->exactMatrixBytes : (48ull << 30);
+    const int digits = o.arith.digits;
+    const uint64_t cellCount = o.cellCount;
+    const uint64_t ldOut = roundUp(cols, 256);
     uint64_t chunkRows = std::max<uint64_t>(kXTile, budget / (ldOut * sizeof(float)) / kXTile * kXTile);
-    chunkRows = std::min<uint64_t>(chunkRows, roundUp(cellCount, kXTile));
-    const bool symmetric = chunkRows >= cellCount;
+    chunkRows = std::min<uint64_t>(chunkRows, roundUp(rowCount, kXTile));
+    const bool symmetric = wholeMatrix && chunkRows >= cellCount;
     void* simMatrix = nullptr;
     EM2_TRY(reserve(ctx, em2_context::S_CAND, chunkRows * ldOut * sizeof(float), &simMatrix));
 
     CUtensorMap mapLo, mapHi;
-    EM2_TRY(makeTensorMapU8(ctx, &mapLo, lo, cellCount, gPad, gPad, kXTile));
+    EM2_TRY(makeTensorMapU8(ctx, &mapLo, o.lo, cellCount, gPad, gPad, kXTile));
     // one digit: the second map is the same plane with a 256-row box (the B operand of the N = 256 tiles)
-    EM2_TRY(makeTensorMapU8(ctx, &mapHi, digits == 2 ? hi : lo, cellCount, gPad, gPad, digits == 2 ? kXTile : 256));
+    EM2_TRY(makeTensorMapU8(ctx, &mapHi, digits == 2 ? o.hi : o.lo, cellCount, gPad, gPad, digits == 2 ? kXTile : 256));
     const uint32_t colsPerTile = digits == 1 ? 256 : kXTile;
     const int stages = digits == 1 ? 4 : 3;
     const size_t smemGemm = 1024 + size_t(stages) * digits * (kXPlaneBytes + size_t(colsPerTile) * kXChunk) + 256;
@@ -624,13 +837,14 @@ int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const 
     const size_t smemSel = size_t(kSelWarps) * 2 * cap * sizeof(uint64_t);
     EM2_CUDA(ctx, cudaFuncSetAttribute(exactSelectKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemSel)));
 
-    for (uint64_t begin = 0; begin < cellCount; begin += chunkRows) {
-        const uint64_t rows = std::min(chunkRows, cellCount - begin);
+    for (uint64_t begin = 0; begin < rowCount; begin += chunkRows) {
+        const uint64_t rows = std::min(chunkRows, rowCount - begin);
         ExactParams p{};
-        p.cellCount = cellCount;
-        p.rowBegin = begin;
+        p.cellCount = colEnd;
+        p.colBegin = colBegin;
+        p.rowBegin = rowBegin + begin;
         p.rows = rows;
-        p.geneCount = geneCount;
+        p.geneCount = o.geneCount;
         p.kChunks = uint32_t(gPad / kXChunk);
         const bool pair = digits == 1 && ctx->exactCtaPair != 0;
         p.rowsPerItem = pair ? 2 * kXTile : kXTile;
@@ -666,9 +880,9 @@ int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const 
         p.idesc = instrDescI8(false, false, p.rowsPerItem, colsPerTile);
         p.ldOut = ldOut;
         p.threshold = similarityThreshold;
-        p.sum1 = sum1;
-        p.var = static_cast<const double*>(var);
-        p.rinv = rinv;
+        p.sum1 = o.sum1;
+        p.var = o.var;
+        p.rinv = o.rinv;
         p.thresholdLow = float(similarityThreshold) - 1e-4f;
         p.out = static_cast<float*>(simMatrix);
         if (pair) {
@@ -704,11 +918,84 @@ int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const 
         ctx->stats.kernel_launches++;
         EM2_CUDA(ctx, cudaGetLastError());
         exactSelectKernel<<<unsigned((rows + kSelWarps - 1) / kSelWarps), kSelWarps * 32, smemSel, s>>>(
-            rows, cellCount, ldOut, static_cast<const float*>(simMatrix), uint32_t(k), cap, pairs + begin * k, usedCount + begin);
+            rows, cols, ldOut, static_cast<const float*>(simMatrix), uint32_t(k), cap, pairs + begin * k, usedCount + begin);
         ctx->stats.kernel_launches++;
         EM2_CUDA(ctx, cudaGetLastError());
     }
-    ctx->stats.variant_used = EM2_VARIANT_MMA_I8;
+    return EM2_OK;
+}
+
+int exactVariant(const ExactArith& arith) { return arith.general ? EM2_VARIANT_POPC : EM2_VARIANT_MMA_I8; }   // POPC: "not the tensor-core path"
+
+}  // namespace
+
+int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
+                const double* sum1, const double* sum2, uint64_t k, double similarityThreshold, em2_pair* pairs,
+                uint32_t* usedCount, cudaStream_t s)
+{
+    EM2_TRY(checkExactArguments(ctx, cellCount, geneCount, k, similarityThreshold));
+    ExactArith arith;
+    EM2_TRY(exactArithmetic(ctx, cellCount, geneCount, toc, counts, sum2, s, &arith));
+    ExactOperands o;
+    EM2_TRY(exactPrepare(ctx, arith, cellCount, geneCount, toc, counts, sum1, sum2, s, &o));
+    EM2_TRY(exactRect(ctx, o, 0, cellCount, 0, cellCount, k, similarityThreshold, true, pairs, usedCount, s));
+    ctx->stats.variant_used = exactVariant(arith);
+    return EM2_OK;
+}
+
+int launchExtendExact(em2_context* ctx, uint64_t oldN, uint64_t N, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
+                      const double* sum1, const double* sum2, uint64_t k, double similarityThreshold, const em2_pair* oldPairs,
+                      const uint32_t* oldUsed, em2_pair* winPairs, uint32_t* winUsed, uint32_t* flags, em2_pair* pairs,
+                      uint32_t* usedCount, cudaStream_t s, uint32_t* badFlags, int* scanSymmetric)
+{
+    *badFlags = 0;
+    *scanSymmetric = 0;
+    EM2_TRY(checkExactArguments(ctx, N, geneCount, k, similarityThreshold));
+    // The arithmetic of the full job over all cells, and of the job the old lists came from.  If they differ, the old
+    // lists may hold other bits than a full run over all cells: compute the full job (exact by definition).
+    ExactArith arith;
+    EM2_TRY(exactArithmetic(ctx, N, geneCount, toc, counts, sum2, s, &arith));
+    bool full = oldN == 0;
+    if (!full) {
+        ExactArith oldArith;
+        EM2_TRY(exactArithmetic(ctx, oldN, geneCount, toc, counts, sum2, s, &oldArith));
+        full = oldArith.general != arith.general;
+    }
+    ExactOperands o;
+    EM2_TRY(exactPrepare(ctx, arith, N, geneCount, toc, counts, sum1, sum2, s, &o));
+    ctx->stats.variant_used = exactVariant(arith);
+    if (full) return exactRect(ctx, o, 0, N, 0, N, k, similarityThreshold, true, pairs, usedCount, s);
+
+    // 1. the old lists against the counts; the caller's buffers are written only if all of them hold
+    EM2_CUDA(ctx, cudaMemsetAsync(flags, 0, sizeof(uint32_t), s));
+    const unsigned valBlocks = unsigned((oldN + kValWarps - 1) / kValWarps);
+    if (arith.general)
+        exactValidateKernel<true><<<valBlocks, kValWarps * 32, 0, s>>>(oldN, geneCount, o.gPad, toc, counts, nullptr, nullptr, sum1,
+                                                                       o.var, similarityThreshold, uint32_t(k), oldPairs, oldUsed,
+                                                                       pairs, usedCount, flags);
+    else
+        exactValidateKernel<false><<<valBlocks, kValWarps * 32, 0, s>>>(oldN, geneCount, o.gPad, toc, counts, o.lo, o.hi, sum1,
+                                                                        o.var, similarityThreshold, uint32_t(k), oldPairs, oldUsed,
+                                                                        pairs, usedCount, flags);
+    ctx->stats.kernel_launches++;
+    EM2_CUDA(ctx, cudaGetLastError());
+    void* pin = nullptr;
+    EM2_TRY(reservePinned(ctx, 2, 64, &pin));
+    EM2_CUDA(ctx, cudaMemcpyAsync(pin, flags, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    EM2_CUDA(ctx, cudaStreamSynchronize(s));
+    *badFlags = *static_cast<uint32_t*>(pin);
+    if (*badFlags || N == oldN) return EM2_OK;      // nothing appended: the validated old lists are the result
+
+    // 2. the appended rows against all columns: their final lists
+    EM2_TRY(exactRect(ctx, o, oldN, N, 0, N, k, similarityThreshold, false, pairs + oldN * k, usedCount + oldN, s));
+    EM2_CUDA(ctx, cudaStreamSynchronize(s));        // the tile-list staging buffer is reused below
+    // 3. the old rows against the appended columns: each old row's k best new cells, merged with its old list
+    EM2_TRY(exactRect(ctx, o, 0, oldN, oldN, N, k, similarityThreshold, false, winPairs, winUsed, s));
+    exactMergeKernel<<<unsigned((oldN + kMergeWarps - 1) / kMergeWarps), kMergeWarps * 32, 0, s>>>(oldN, uint32_t(k), oldPairs, oldUsed,
+                                                                                                   winPairs, winUsed, pairs, usedCount);
+    ctx->stats.kernel_launches++;
+    EM2_CUDA(ctx, cudaGetLastError());
+    *scanSymmetric = 1;
     return EM2_OK;
 }
 

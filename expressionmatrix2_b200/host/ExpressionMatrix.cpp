@@ -335,3 +335,37 @@ void ExpressionMatrix::findSimilarPairs0(const std::string& geneSetName, const s
 {
     findSimilarPairs0(std::cout, geneSetName, cellSetName, similarPairsName, k, similarityThreshold);
 }
+
+void ExpressionMatrix::extendSimilarPairs0(const std::string& oldName, const std::string& newName, double similarityThreshold)
+{
+    if (newName == oldName)
+        throw std::runtime_error("extendSimilarPairs0: the new SimilarPairs object needs a name other than " + oldName + ".");
+    if (similarityThreshold > 1.) throw std::runtime_error("similarityThreshold must not exceed 1.");
+    // the old object, opened for a cell set that may have grown by appending (gene set unchanged, old ids a prefix)
+    const SimilarPairs oldPairs(directoryName, oldName, SimilarPairs::AppendedCells{});
+    const std::string geneSetName = oldPairs.geneSetName(), cellSetName = oldPairs.cellSetName();
+    const GeneSet& geneSet = findGeneSet(geneSetName);
+    const CellSet& cellSet = findCellSet(cellSetName);
+    const size_t k = oldPairs.k();
+    const CellId oldCount = oldPairs.storedCellCount();
+    Gpu& gpu = Gpu::instance();            // throws without a device: before anything is written to the data directory
+
+    // the grown cell set's counts, as findSimilarPairs0 builds them (a temporary file, removed when `subset` goes away)
+    ExpressionMatrixSubset subset(directoryName + "/tmp-ExpressionMatrixSubset-" + newName, geneSet, cellSet, cellExpressionCounts);
+    const size_t n = subset.cellCount();
+    std::vector<uint32_t> oldUsed(oldCount), used(n);
+    for (CellId c = 0; c < oldCount; c++) oldUsed[c] = uint32_t(oldPairs.size(c));
+    SimilarPairs similarPairs(directoryName, newName, geneSetName, cellSetName, k);
+    try {
+        gpu.check(em2_extend_exact_similar_pairs(gpu.context(), oldCount, n, subset.geneCount(), subset.toc(),
+                                                 reinterpret_cast<const em2_count*>(subset.data()), k, similarityThreshold,
+                                                 reinterpret_cast<const em2_pair*>(oldPairs.begin(0)), oldUsed.data(),
+                                                 reinterpret_cast<em2_pair*>(similarPairs.begin(0)), used.data()),
+                  "em2_extend_exact_similar_pairs");
+    } catch (...) {
+        similarPairs.remove();      // no valid-looking SimilarPairs-<new> set stays behind a failed call
+        throw;
+    }
+    similarPairs.setUsedCounts(used);
+    lastScanMs = gpu.stats().scan_ms;
+}

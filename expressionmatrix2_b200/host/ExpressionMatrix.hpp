@@ -70,6 +70,12 @@ public:
                            const std::string& similarPairsName, size_t k, double similarityThreshold);
     void findSimilarPairs0(std::ostream&, const std::string& geneSetName, const std::string& cellSetName,
                            const std::string& similarPairsName, size_t k, double similarityThreshold);
+    // The lists of SimilarPairs-<similarPairsName>, made by findSimilarPairs0 before cells were appended to its cell set,
+    // extended to the appended cells: SimilarPairs-<newSimilarPairsName> on the current cell set holds what findSimilarPairs0
+    // would store for it.  similarityThreshold must be that of the old call (the old object does not record it): lists
+    // that do not belong to the counts, k or threshold are detected and throw, except lists made with a HIGHER threshold,
+    // which give wrong lists.  The old object is not modified.
+    void extendSimilarPairs0(const std::string& similarPairsName, const std::string& newSimilarPairsName, double similarityThreshold);
 
     // Scan variant for findSimilarPairs4 (em2_variant; 0 = automatic).
     int scanVariant = 0;

@@ -283,6 +283,29 @@ int em2_exact_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneC
                             const em2_count* counts, uint64_t k, double similarityThreshold, em2_pair* pairs,
                             uint32_t* usedCount);
 
+/* Lists of a findSimilarPairs0 job (em2_exact_similar_pairs) over cells [0, oldCellCount), extended to the cells appended
+ * after them (new cells get the ids oldCellCount..cellCount-1).
+ * toc/counts: ALL cellCount cells, old cells first and unchanged.  oldPairs/oldUsedCount: rows [0, oldCellCount) as
+ * em2_exact_similar_pairs wrote them with the same k and similarityThreshold.  pairs/usedCount: all cellCount rows; must not
+ * overlap the old buffers.  Arguments are checked as in em2_exact_similar_pairs.
+ * Result: bit for bit what em2_exact_similar_pairs(cellCount, ...) returns (ids, float bits, usedCount, zeroed unused slots).
+ * The full job picks its arithmetic (integer tensor-core path or general FP64 kernel) from all counts; when that choice
+ * differs between the old cells alone and all cells, the old lists may hold other bits and this call computes the full job.
+ * Otherwise every stored old entry is checked on the device before any output is written: usedCount <= k, its id is below
+ * oldCellCount and not the row's own, r recomputed from the counts with the full job's bits passes r > similarityThreshold
+ * and equals the stored float, and each row strictly follows (similarity desc, id asc); a failure returns EM2_ERR_INVALID
+ * (lists of findSimilarPairs4, or of other counts, are caught this way).  Old lists made with a HIGHER threshold than this
+ * call's cannot be detected: every stored entry also passes the lower threshold, but rows that are not full lack the cells
+ * between the two thresholds, and the result is wrong.  The caller passes the old job's threshold.
+ * Then the new rows are computed against all cells and the old rows against the new cells only, and each old row keeps the
+ * k best of its old list and its new candidates: about M*(2N+M) pair evaluations instead of (N+M)^2/2 or, once the N x N
+ * similarity matrix exceeds option "exact_matrix_bytes", (N+M)^2 (N = oldCellCount, M = cellCount - oldCellCount).
+ * Stats: scan_symmetric 1 = that rectangle ran; 0 = the full job (oldCellCount = 0, or the arithmetic differs) or nothing
+ * was appended; variant_used as em2_exact_similar_pairs sets it. */
+int em2_extend_exact_similar_pairs(em2_context* ctx, uint64_t oldCellCount, uint64_t cellCount, uint64_t geneCount,
+                                   const uint64_t* toc, const em2_count* counts, uint64_t k, double similarityThreshold,
+                                   const em2_pair* oldPairs, const uint32_t* oldUsedCount, em2_pair* pairs, uint32_t* usedCount);
+
 /* ------------------------------------------------------------------------------------------------
  * Device-resident calls: every pointer is a DEVICE pointer on the context's device, work is enqueued
  * on `stream` (a cudaStream_t passed as void*; NULL = legacy default stream) and the call returns
