@@ -80,6 +80,7 @@ def lib():
     L.em2_extend_similar_pairs.argtypes = [vp, vp, u64, u64, u64, u64, dbl, i32, vp, vp, vp, vp]
     L.em2_exact_similar_pairs.argtypes = [vp, u64, u64, vp, vp, u64, dbl, vp, vp]
     L.em2_extend_exact_similar_pairs.argtypes = [vp, u64, u64, u64, vp, vp, u64, dbl, vp, vp, vp, vp]
+    L.em2_rescore_similar_pairs.argtypes = [vp, u64, u64, vp, vp, u64, vp, vp, u64, dbl, vp, vp]
     L.em2_cell_graph_edges.argtypes = [vp, u64, u64, vp, vp, vp, dbl, u64, vp, u64, vp]
     L.em2_signature_graph.argtypes = [vp, vp, u64, u64, u64, vp, vp, u64, vp, vp, u64, vp]
     L.em2_find_similar_pairs7.argtypes = [vp, vp, u64, u64, u64, dbl, vp, u64, C.c_uint32, u64, vp, vp]
@@ -459,6 +460,31 @@ class Engine:
         self._check(self._L.em2_extend_exact_similar_pairs(self._h, old_cell_count, n, gene_count, _ptr(toc), _ptr(pairs), k,
                                                            similarity_threshold, _ptr(old), _ptr(old_used), _ptr(out), _ptr(used)),
                     "em2_extend_exact_similar_pairs")
+        return np.ascontiguousarray(out["cell"]), np.ascontiguousarray(out["similarity"]), used
+
+    def rescore_similar_pairs(self, toc, counts, gene_count: int, cand_ids, cand_used, k: int, similarity_threshold: float,
+                              gene_ids=None):
+        """Exact rescoring of candidate lists (em2_rescore_similar_pairs): cand_ids [N, width] with cand_used [N] entries
+        used per row, e.g. the ids of any *_similar_pairs result; their order within a row is free.  Returns (ids, sims, used)
+        with each row's k best candidates by the similarity exact_similar_pairs stores for the pair (desc, then id asc) among
+        those above similarity_threshold.  Raises Em2Error on an id >= N, a row's own id, an id listed twice in a row, or
+        cand_used above the width."""
+        toc = np.ascontiguousarray(toc, np.uint64)
+        pairs = _as_pairs(counts, gene_ids)
+        n = len(toc) - 1
+        ids = np.asarray(cand_ids, np.uint32)
+        if ids.ndim != 2 or ids.shape[0] != n:
+            raise ValueError("cand_ids must be [N, width]")
+        cand = np.zeros(ids.shape, SIMPAIR_DTYPE)
+        cand["cell"] = ids
+        cand_used = np.ascontiguousarray(cand_used, np.uint32)
+        if cand_used.shape != (n,):
+            raise ValueError("cand_used must hold one count per cell")
+        out = np.zeros((n, k), SIMPAIR_DTYPE)
+        used = np.zeros(n, np.uint32)
+        self._check(self._L.em2_rescore_similar_pairs(self._h, n, gene_count, _ptr(toc), _ptr(pairs), ids.shape[1], _ptr(cand),
+                                                      _ptr(cand_used), k, similarity_threshold, _ptr(out), _ptr(used)),
+                    "em2_rescore_similar_pairs")
         return np.ascontiguousarray(out["cell"]), np.ascontiguousarray(out["similarity"]), used
 
     # ---- device-resident calls (torch CUDA tensors or raw device pointers) ------------------------

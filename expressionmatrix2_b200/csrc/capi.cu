@@ -1047,4 +1047,77 @@ int em2_exact_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneC
     return EM2_OK;
 }
 
+int em2_rescore_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
+                              const em2_count* counts, uint64_t candidateWidth, const em2_pair* candidates,
+                              const uint32_t* candidateCount, uint64_t k, double similarityThreshold, em2_pair* pairs,
+                              uint32_t* usedCount)
+{
+    EM2_TRY(guardDevice(ctx));
+    const uint64_t N = cellCount, width = candidateWidth;
+    if (!toc || !pairs || !usedCount || !candidates || !candidateCount || (!counts && N && toc[N]))
+        return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: null pointer");
+    EM2_TRY(checkExactArguments(ctx, N, geneCount, k, similarityThreshold));
+    if (width == 0 || width > 1024) return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: candidateWidth must be in [1, 1024]");
+    const size_t pairBytes = N * k * sizeof(em2_pair), usedBytes = N * sizeof(uint32_t);
+    const size_t candBytes = N * width * sizeof(em2_pair), candUsedBytes = N * sizeof(uint32_t);
+    if (overlaps(pairs, pairBytes, candidates, candBytes) || overlaps(pairs, pairBytes, candidateCount, candUsedBytes) ||
+        overlaps(usedCount, usedBytes, candidates, candBytes) || overlaps(usedCount, usedBytes, candidateCount, candUsedBytes))
+        return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: the output buffers overlap the candidates");
+    for (uint64_t a = 0; a < N; a++)
+        if (candidateCount[a] > width)
+            return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: candidateCount[" + std::to_string(a) + "] exceeds candidateWidth");
+    resetStats(ctx);
+    const double t0 = nowMs();
+    if (N == 0) return EM2_OK;
+    cudaStream_t s = ctx->stream;
+    StageTimer T(ctx);
+    const uint64_t nnz = toc[N];
+    void *dToc, *dCounts, *dSum1, *dSum2, *dPairs, *dUsed, *dCand;
+    EM2_TRY(reserve(ctx, em2_context::S_TOC, (N + 1) * sizeof(uint64_t), &dToc));
+    EM2_TRY(reserve(ctx, em2_context::S_COUNTS, nnz * sizeof(em2_count), &dCounts));
+    EM2_TRY(reserve(ctx, em2_context::S_SUM1, N * sizeof(double), &dSum1));
+    EM2_TRY(reserve(ctx, em2_context::S_SUM2, N * sizeof(double), &dSum2));
+    EM2_TRY(reserve(ctx, em2_context::S_PAIRS, pairBytes, &dPairs));
+    EM2_TRY(reserve(ctx, em2_context::S_USED, usedBytes, &dUsed));
+    // [candidates N * width][candidateCount N][flags 4]
+    EM2_TRY(reserve(ctx, em2_context::S_RESCORE, candBytes + candUsedBytes + 16, &dCand));
+    auto* dCandUsed = reinterpret_cast<uint32_t*>(static_cast<em2_pair*>(dCand) + N * width);
+    uint32_t* dFlags = dCandUsed + N;
+
+    const int e0 = T.mark();
+    EM2_TRY(stageH2D(ctx, dToc, toc, (N + 1) * sizeof(uint64_t), s));
+    EM2_TRY(stageH2D(ctx, dCounts, counts, nnz * sizeof(em2_count), s));
+    EM2_TRY(stageH2D(ctx, dCand, candidates, candBytes, s));
+    EM2_TRY(stageH2D(ctx, dCandUsed, candidateCount, candUsedBytes, s));
+    ctx->stats.h2d_bytes += (N + 1) * 8 + nnz * 8 + candBytes + candUsedBytes;
+    const int e1 = T.mark();
+    EM2_TRY(launchCellSums(ctx, N, static_cast<uint64_t*>(dToc), static_cast<em2_count*>(dCounts), static_cast<double*>(dSum1),
+                           static_cast<double*>(dSum2), s));
+    const int e2 = T.mark();
+    uint32_t bad = 0;
+    EM2_TRY(launchRescoreExact(ctx, N, geneCount, static_cast<uint64_t*>(dToc), static_cast<em2_count*>(dCounts),
+                               static_cast<double*>(dSum1), static_cast<double*>(dSum2), width, static_cast<em2_pair*>(dCand),
+                               dCandUsed, k, similarityThreshold, dFlags, static_cast<em2_pair*>(dPairs), static_cast<uint32_t*>(dUsed),
+                               s, &bad));
+    if (bad) {
+        std::string what;
+        if (bad & kRescoreBadId) what += "; a candidate id is not below cellCount";
+        if (bad & kRescoreBadSelf) what += "; a row lists its own cell";
+        if (bad & kRescoreBadDuplicate) what += "; a row lists a candidate twice";
+        return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: invalid candidate lists: " + what.substr(2));
+    }
+    const int e3 = T.mark();
+    EM2_TRY(stageD2H(ctx, pairs, dPairs, pairBytes, s));
+    EM2_TRY(stageD2H(ctx, usedCount, dUsed, usedBytes, s));
+    const int e4 = T.mark();
+    EM2_CUDA(ctx, cudaStreamSynchronize(s));
+    ctx->stats.d2h_bytes += pairBytes + usedBytes;
+    ctx->stats.h2d_ms = T.ms(e0, e1);
+    ctx->stats.sums_ms = T.ms(e1, e2);
+    ctx->stats.scan_ms = T.ms(e2, e3);
+    ctx->stats.d2h_ms = T.ms(e3, e4);
+    ctx->stats.total_ms = nowMs() - t0;
+    return EM2_OK;
+}
+
 }  // extern "C"

@@ -65,6 +65,7 @@ struct em2_context {
         S_DIST0, S_DIST1, S_DIST2, S_DIST3,   // multi-GPU exchange buffers (multi.cu)
         S_PERM,          // scan position -> cell id
         S_EXTEND,        // em2_extend_similar_pairs: old lists, their keys, lengths and column bounds, the validation flags
+        S_RESCORE,       // em2_rescore_similar_pairs: candidate lists, their lengths, the check flags
         S_COUNT
     };
     int signatureMode = 0;   // 0 auto, 1 FP64 kernel only, 2 force the tensor-core filter path
@@ -257,6 +258,19 @@ int launchExtendExact(em2_context* ctx, uint64_t oldN, uint64_t N, uint64_t gene
                       const double* sum1, const double* sum2, uint64_t k, double similarityThreshold, const em2_pair* oldPairs,
                       const uint32_t* oldUsed, em2_pair* winPairs, uint32_t* winUsed, uint32_t* flags, em2_pair* pairs,
                       uint32_t* usedCount, cudaStream_t s, uint32_t* badFlags, int* scanSymmetric);
+// Rescoring of candidate lists with the exact path's similarities (exact.cu; capi.cu has the entry point).  Device pointers:
+// candidates [N][width] (ids only are read), candidateCount [N] (each <= width, checked by the caller), flags one word.
+// *badFlags (kRescore*) != 0: an id failed its checks, and pairs / usedCount hold nothing of use.
+int launchRescoreExact(em2_context* ctx, uint64_t N, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
+                       const double* sum1, const double* sum2, uint64_t width, const em2_pair* candidates,
+                       const uint32_t* candidateCount, uint64_t k, double similarityThreshold, uint32_t* flags, em2_pair* pairs,
+                       uint32_t* usedCount, cudaStream_t s, uint32_t* badFlags);
+// What the candidate ids of em2_rescore_similar_pairs got wrong, OR-ed over all rows.
+enum : uint32_t {
+    kRescoreBadId = 1,          // an id >= cellCount
+    kRescoreBadSelf = 2,        // a row lists its own cell
+    kRescoreBadDuplicate = 4,   // a row lists a cell twice
+};
 
 // Validation of old lists by the extension calls: what a stored entry got wrong, OR-ed over all entries.
 enum : uint32_t {

@@ -35,6 +35,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstring>
+#include <type_traits>
 #include <vector>
 
 namespace em2 {
@@ -555,13 +556,60 @@ __device__ __forceinline__ float storedCount(const uint64_t* __restrict__ toc, c
     return lo < end && counts[lo].gene == gene ? counts[lo].count : 0.f;
 }
 
-// One warp per old row a.  Every stored entry (a, b) is recomputed with the bits of the full job, the row cell on the dense
-// side as in both full-job kernels:
-//   integer path: the exact integer scalar product, the row's counts read from its digit planes;
+// Sum over b's stored entries x = lane, lane + 32, ... of term(counts[x]), in that order.  UNROLL: four loads in flight per
+// lane (off where term itself searches a CSR: the searches are the latency then, and the unrolled form spills); the terms are
+// added in the same order either way, so double sums keep their bits.
+template <class Acc, bool UNROLL, class Term>
+__device__ __forceinline__ Acc laneSum(uint64_t x, uint64_t end, const em2_count* __restrict__ counts, Term term)
+{
+    Acc acc = 0;
+    if constexpr (UNROLL) {
+        for (; x + 96 < end; x += 128) {
+            const em2_count q0 = counts[x], q1 = counts[x + 32], q2 = counts[x + 64], q3 = counts[x + 96];
+            acc += term(q0);
+            acc += term(q1);
+            acc += term(q2);
+            acc += term(q3);
+        }
+    }
+    for (; x < end; x += 32) acc += term(counts[x]);
+    return acc;
+}
+
+// r(a, b) with the bits the full job stores in row a, computed by one warp, the row cell a on the dense side as in both
+// full-job kernels.  rowCount(gene) is a's count of gene: uint32_t on the integer path, float on the general path; SEARCH:
+// it searches a's CSR (storedCount).
+//   integer path: the exact integer scalar product;
 //   general path: the general kernel's lane partition (b's entries strided over the lanes, float products, double sums) and
-//                 its shuffle tree, the row's counts found by search in its CSR.
-// Then r through pearsonNumerator / pearsonR.  Flags as em2_extend_similar_pairs (kExtend*).  outPairs / outUsed: the row as
-// em2_exact_similar_pairs writes it (unused slots zeroed) -- the result when nothing was appended.
+//                 its shuffle tree.
+// Then r through pearsonNumerator / pearsonR.  exactValidateKernel and exactRescoreKernel both call this, so their bits cannot
+// drift apart.  Every lane returns r.
+template <bool GENERAL, bool SEARCH, class RowCount>
+__device__ __forceinline__ double warpPairR(uint64_t b, const uint64_t* __restrict__ toc, const em2_count* __restrict__ counts,
+                                            RowCount rowCount, double n, double s1a, double va, const double* __restrict__ sum1,
+                                            const double* __restrict__ var, uint32_t lane)
+{
+    const uint64_t begin = toc[b] + lane, end = toc[b + 1];
+    double sp;
+    if constexpr (GENERAL) {
+        double acc = laneSum<double, !SEARCH>(begin, end, counts, [=](em2_count q) { return double(__fmul_rn(rowCount(q.gene), q.count)); });
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+        sp = acc;
+    } else {
+        unsigned long long acc = laneSum<unsigned long long, !SEARCH>(
+            begin, end, counts, [=](em2_count q) { return (unsigned long long)rowCount(q.gene) * uint32_t(q.count); });
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+        sp = double(acc);     // < 2^53: the host's s32 bounds keep the digit sums far below
+    }
+    return pearsonR(pearsonNumerator(n, sp, s1a, sum1[b]), va, var[b]);
+}
+
+// One warp per old row a.  Every stored entry (a, b) is recomputed with the bits of the full job (warpPairR), the row's
+// counts read from its digit planes (integer path) or found by search in its CSR (general path).  Flags as
+// em2_extend_similar_pairs (kExtend*).  outPairs / outUsed: the row as em2_exact_similar_pairs writes it (unused slots
+// zeroed) -- the result when nothing was appended.
 constexpr int kValWarps = 8;
 template <bool GENERAL>
 __global__ void __launch_bounds__(kValWarps * 32)
@@ -596,30 +644,17 @@ exactValidateKernel(uint64_t oldN, uint64_t geneCount, uint64_t gPad, const uint
             bad |= kExtendBadSelf;
             continue;
         }
-        const uint64_t b = e.cell, end = toc[b + 1];
-        double sp;
-        if (GENERAL) {
-            double acc = 0.;
-            for (uint64_t x = toc[b] + lane; x < end; x += 32) {
-                const em2_count q = counts[x];
-                acc += double(__fmul_rn(storedCount(toc, counts, a, q.gene), q.count));
-            }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-            sp = acc;
+        double r;
+        if constexpr (GENERAL) {
+            r = warpPairR<true, true>(e.cell, toc, counts, [=](uint32_t g) { return storedCount(toc, counts, a, g); }, n, s1a, va, sum1,
+                                var, lane);
         } else {
-            unsigned long long acc = 0;
-            for (uint64_t x = toc[b] + lane; x < end; x += 32) {
-                const em2_count q = counts[x];
-                uint32_t ca = lo[a * gPad + q.gene];
-                if (hi) ca |= uint32_t(hi[a * gPad + q.gene]) << 8;
-                acc += (unsigned long long)ca * uint32_t(q.count);
-            }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-            sp = double(acc);     // < 2^53: the host's s32 bounds keep the digit sums far below
+            r = warpPairR<false, false>(e.cell, toc, counts, [&](uint32_t g) {
+                uint32_t ca = lo[a * gPad + g];
+                if (hi) ca |= uint32_t(hi[a * gPad + g]) << 8;
+                return ca;
+            }, n, s1a, va, sum1, var, lane);
         }
-        const double r = pearsonR(pearsonNumerator(n, sp, s1a, sum1[b]), va, var[b]);
         if (!(r > threshold)) bad |= kExtendBadThreshold;
         else if (__float_as_uint(float(r)) != __float_as_uint(e.similarity)) bad |= kExtendBadSimilarity;
     }
@@ -685,6 +720,103 @@ exactMergeKernel(uint64_t oldN, uint32_t k, const em2_pair* __restrict__ oldPair
     if (lane == 0) usedCount[a] = total;
 }
 
+// ---- rescoring of candidate lists (launchRescoreExact) -------------------------------------------------------------------
+// A CTA of kRescoreWarps warps takes rows a = blockIdx.x, blockIdx.x + gridDim.x, ...  Row a's counts are scattered into a
+// dense shared-memory row (uint16 per gene on the integer path, where counts are <= 65535; float on the general path) and
+// cleared again afterwards, so a row costs nnz(a), not G.  DENSE == false (integer path, too many genes for that row): a's
+// counts are found by search in its CSR, with the same values.  One warp per candidate b computes r(a, b) with warpPairR, the
+// float em2_exact_similar_pairs stores in row a.  Keys (~orderable(r) << 32 | b), or (kRescoreReject << 32 | b) when r does
+// not pass the threshold, are sorted in shared memory (bitonic): the passing keys form a prefix, the row is its first k, and
+// a candidate listed twice gives two equal keys, adjacent after the sort.
+constexpr int kRescoreWarps = 8;
+constexpr uint32_t kRescoreReject = 0xffffffffu;     // above ~orderable(r) for every r in [-1, 1]
+
+template <bool GENERAL, bool DENSE>
+__global__ void __launch_bounds__(kRescoreWarps * 32)
+exactRescoreKernel(uint64_t cellCount, uint64_t geneCount, const uint64_t* __restrict__ toc, const em2_count* __restrict__ counts,
+                   const double* __restrict__ sum1, const double* __restrict__ var, double threshold, uint32_t width,
+                   uint32_t sortSize, const em2_pair* __restrict__ cand, const uint32_t* __restrict__ candUsed, uint32_t k,
+                   em2_pair* __restrict__ pairs, uint32_t* __restrict__ usedCount, uint32_t* __restrict__ flags)
+{
+    static_assert(DENSE || !GENERAL, "the general path always has its dense row (at most 25,600 genes)");
+    using Count = std::conditional_t<GENERAL, float, uint16_t>;
+    extern __shared__ __align__(16) uint64_t keys[];     // [sortSize] (a power of two >= width), then Count dense[geneCount]
+    Count* dense = reinterpret_cast<Count*>(keys + sortSize);
+    __shared__ uint32_t passed;
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const double n = double(geneCount);
+    uint32_t bad = 0;
+    if constexpr (DENSE) {
+        for (uint64_t g = threadIdx.x; g < geneCount; g += blockDim.x) dense[g] = Count(0);
+        __syncthreads();
+    }
+    for (uint64_t a = blockIdx.x; a < cellCount; a += gridDim.x) {
+        const uint32_t used = candUsed[a];                // <= width (checked on the host)
+        const uint64_t rowBegin = toc[a], rowEnd = toc[a + 1];
+        if constexpr (DENSE)
+            for (uint64_t e = rowBegin + threadIdx.x; e < rowEnd; e += blockDim.x) dense[counts[e].gene] = Count(counts[e].count);
+        for (uint32_t i = threadIdx.x; i < sortSize; i += blockDim.x) keys[i] = ~0ull;
+        if (threadIdx.x == 0) passed = 0;
+        __syncthreads();
+        const double s1a = sum1[a], va = var[a];
+        for (uint32_t i = warp; i < used; i += kRescoreWarps) {
+            const uint32_t b = cand[a * width + i].cell;
+            uint64_t key = (uint64_t(kRescoreReject) << 32) | b;
+            if (b >= cellCount) {
+                bad |= kRescoreBadId;
+            } else if (b == a) {
+                bad |= kRescoreBadSelf;
+            } else {
+                double r;
+                if constexpr (DENSE)
+                    r = warpPairR<GENERAL, false>(b, toc, counts, [&](uint32_t g) { return dense[g]; }, n, s1a, va, sum1, var, lane);
+                else
+                    r = warpPairR<false, true>(b, toc, counts, [=](uint32_t g) { return uint32_t(storedCount(toc, counts, a, g)); }, n, s1a,
+                                         va, sum1, var, lane);
+                if (r > threshold) key = (uint64_t(~orderable(float(r))) << 32) | b;
+            }
+            if (lane == 0) keys[i] = key;
+        }
+        __syncthreads();
+        for (uint32_t size = 2; size <= sortSize; size <<= 1) {
+            for (uint32_t stride = size >> 1; stride > 0; stride >>= 1) {
+                for (uint32_t t = threadIdx.x; t < sortSize / 2; t += blockDim.x) {
+                    const uint32_t i = ((t & ~(stride - 1)) << 1) | (t & (stride - 1)), j = i | stride;
+                    const uint64_t x = keys[i], y = keys[j];
+                    if ((x > y) == ((i & size) == 0)) {
+                        keys[i] = y;
+                        keys[j] = x;
+                    }
+                }
+                __syncthreads();
+            }
+        }
+        for (uint32_t i = threadIdx.x; i < used; i += blockDim.x) {
+            const uint64_t key = keys[i];
+            if (i && key == keys[i - 1]) bad |= kRescoreBadDuplicate;
+            if (uint32_t(key >> 32) != kRescoreReject && (i + 1 == used || uint32_t(keys[i + 1] >> 32) == kRescoreReject)) passed = i + 1;
+        }
+        __syncthreads();
+        const uint32_t kept = min(passed, k);
+        for (uint32_t e = threadIdx.x; e < k; e += blockDim.x) {
+            em2_pair out;
+            out.cell = 0;
+            out.similarity = 0.f;
+            if (e < kept) {
+                out.cell = uint32_t(keys[e]);
+                out.similarity = fromOrderable(~uint32_t(keys[e] >> 32));
+            }
+            pairs[a * k + e] = out;
+        }
+        if (threadIdx.x == 0) usedCount[a] = kept;
+        if constexpr (DENSE)
+            for (uint64_t e = rowBegin + threadIdx.x; e < rowEnd; e += blockDim.x) dense[counts[e].gene] = Count(0);
+        __syncthreads();
+    }
+    bad = __reduce_or_sync(0xffffffffu, bad);
+    if (lane == 0 && bad) atomicOr(flags, bad);
+}
+
 }  // namespace
 
 int checkExactArguments(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, uint64_t k, double similarityThreshold)
@@ -728,7 +860,7 @@ int exactArithmetic(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, co
     return EM2_OK;
 }
 
-// Per-cell operands of all cells for the chosen arithmetic.
+// Per-cell operands of all cells for the chosen arithmetic (planes == false: the variance term only, as the general path needs).
 struct ExactOperands {
     ExactArith arith;
     uint64_t cellCount, geneCount, gPad;
@@ -741,7 +873,7 @@ struct ExactOperands {
 };
 
 int exactPrepare(em2_context* ctx, const ExactArith& arith, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
-                 const em2_count* counts, const double* sum1, const double* sum2, cudaStream_t s, ExactOperands* o)
+                 const em2_count* counts, const double* sum1, const double* sum2, bool planes, cudaStream_t s, ExactOperands* o)
 {
     *o = ExactOperands{};
     o->arith = arith;
@@ -751,9 +883,9 @@ int exactPrepare(em2_context* ctx, const ExactArith& arith, uint64_t cellCount, 
     o->toc = toc;
     o->counts = counts;
     o->sum1 = sum1;
-    if (arith.general) {
-        if (2 * o->gPad * sizeof(float) > 200 * 1024)
-            return fail(ctx, EM2_ERR_INVALID, "em2_exact_similar_pairs: non-integer counts with more than 25,600 genes are not supported");
+    if (arith.general && 2 * o->gPad * sizeof(float) > 200 * 1024)
+        return fail(ctx, EM2_ERR_INVALID, "em2_exact_similar_pairs: non-integer counts with more than 25,600 genes are not supported");
+    if (arith.general || !planes) {
         void* varG = nullptr;
         EM2_TRY(reserve(ctx, em2_context::S_FLAGS, cellCount * sizeof(double), &varG));
         o->var = static_cast<double*>(varG);
@@ -937,7 +1069,7 @@ int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const 
     ExactArith arith;
     EM2_TRY(exactArithmetic(ctx, cellCount, geneCount, toc, counts, sum2, s, &arith));
     ExactOperands o;
-    EM2_TRY(exactPrepare(ctx, arith, cellCount, geneCount, toc, counts, sum1, sum2, s, &o));
+    EM2_TRY(exactPrepare(ctx, arith, cellCount, geneCount, toc, counts, sum1, sum2, true, s, &o));
     EM2_TRY(exactRect(ctx, o, 0, cellCount, 0, cellCount, k, similarityThreshold, true, pairs, usedCount, s));
     ctx->stats.variant_used = exactVariant(arith);
     return EM2_OK;
@@ -962,7 +1094,7 @@ int launchExtendExact(em2_context* ctx, uint64_t oldN, uint64_t N, uint64_t gene
         full = oldArith.general != arith.general;
     }
     ExactOperands o;
-    EM2_TRY(exactPrepare(ctx, arith, N, geneCount, toc, counts, sum1, sum2, s, &o));
+    EM2_TRY(exactPrepare(ctx, arith, N, geneCount, toc, counts, sum1, sum2, true, s, &o));
     ctx->stats.variant_used = exactVariant(arith);
     if (full) return exactRect(ctx, o, 0, N, 0, N, k, similarityThreshold, true, pairs, usedCount, s);
 
@@ -996,6 +1128,45 @@ int launchExtendExact(em2_context* ctx, uint64_t oldN, uint64_t N, uint64_t gene
     ctx->stats.kernel_launches++;
     EM2_CUDA(ctx, cudaGetLastError());
     *scanSymmetric = 1;
+    return EM2_OK;
+}
+
+int launchRescoreExact(em2_context* ctx, uint64_t N, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
+                       const double* sum1, const double* sum2, uint64_t width, const em2_pair* candidates,
+                       const uint32_t* candidateCount, uint64_t k, double similarityThreshold, uint32_t* flags, em2_pair* pairs,
+                       uint32_t* usedCount, cudaStream_t s, uint32_t* badFlags)
+{
+    *badFlags = 0;
+    EM2_TRY(checkExactArguments(ctx, N, geneCount, k, similarityThreshold));
+    // the arithmetic of the full job over all N cells; only the variance term is needed besides the sums
+    ExactArith arith;
+    EM2_TRY(exactArithmetic(ctx, N, geneCount, toc, counts, sum2, s, &arith));
+    ExactOperands o;
+    EM2_TRY(exactPrepare(ctx, arith, N, geneCount, toc, counts, sum1, sum2, false, s, &o));
+    ctx->stats.variant_used = exactVariant(arith);
+
+    uint32_t sortSize = 32;
+    while (sortSize < width) sortSize <<= 1;
+    const size_t keyBytes = size_t(sortSize) * sizeof(uint64_t);
+    const size_t denseBytes = geneCount * (arith.general ? sizeof(float) : sizeof(uint16_t));
+    const bool dense = keyBytes + denseBytes + 1024 <= size_t(ctx->prop.sharedMemPerBlockOptin);   // always on the general path
+    const size_t smem = keyBytes + (dense ? denseBytes : 0);
+    auto kernel = arith.general ? exactRescoreKernel<true, true> : dense ? exactRescoreKernel<false, true> : exactRescoreKernel<false, false>;
+    EM2_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    int perSm = 0;
+    EM2_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, kernel, kRescoreWarps * 32, smem));
+    if (perSm < 1) return fail(ctx, EM2_ERR_CUDA, "no CTA of the rescoring kernel fits on this device");
+    const unsigned grid = unsigned(std::min<uint64_t>(N, uint64_t(perSm) * ctx->smCount));
+    EM2_CUDA(ctx, cudaMemsetAsync(flags, 0, sizeof(uint32_t), s));
+    kernel<<<grid, kRescoreWarps * 32, smem, s>>>(N, geneCount, toc, counts, sum1, o.var, similarityThreshold, uint32_t(width), sortSize,
+                                                  candidates, candidateCount, uint32_t(k), pairs, usedCount, flags);
+    ctx->stats.kernel_launches++;
+    EM2_CUDA(ctx, cudaGetLastError());
+    void* pin = nullptr;
+    EM2_TRY(reservePinned(ctx, 2, 64, &pin));
+    EM2_CUDA(ctx, cudaMemcpyAsync(pin, flags, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    EM2_CUDA(ctx, cudaStreamSynchronize(s));
+    *badFlags = *static_cast<uint32_t*>(pin);
     return EM2_OK;
 }
 

@@ -369,3 +369,36 @@ void ExpressionMatrix::extendSimilarPairs0(const std::string& oldName, const std
     similarPairs.setUsedCounts(used);
     lastScanMs = gpu.stats().scan_ms;
 }
+
+void ExpressionMatrix::rescoreSimilarPairs(const std::string& name, const std::string& newName, size_t k, double similarityThreshold)
+{
+    if (newName == name)
+        throw std::runtime_error("rescoreSimilarPairs: the new SimilarPairs object needs a name other than " + name + ".");
+    if (k == 0 || k > 1024) throw std::runtime_error("rescoreSimilarPairs: k must be in [1, 1024] on the GPU path.");
+    if (similarityThreshold > 1.) throw std::runtime_error("similarityThreshold must not exceed 1.");
+    // the source object; throws if its gene set or cell set changed since it was created
+    const SimilarPairs source(directoryName, name, true);
+    const std::string geneSetName = source.geneSetName(), cellSetName = source.cellSetName();
+    const GeneSet& geneSet = findGeneSet(geneSetName);
+    const CellSet& cellSet = findCellSet(cellSetName);
+    const CellId n = source.cellCount();
+    Gpu& gpu = Gpu::instance();            // throws without a device: before anything is written to the data directory
+
+    // the counts of the source's gene set x cell set, as findSimilarPairs0 builds them (a temporary file unless in place)
+    ExpressionMatrixSubset subset(directoryName + "/tmp-ExpressionMatrixSubset-" + newName, geneSet, cellSet, cellExpressionCounts);
+    std::vector<uint32_t> candidateCount(n), used(n);
+    for (CellId c = 0; c < n; c++) candidateCount[c] = uint32_t(source.size(c));
+    SimilarPairs similarPairs(directoryName, newName, geneSetName, cellSetName, k);
+    try {
+        gpu.check(em2_rescore_similar_pairs(gpu.context(), n, subset.geneCount(), subset.toc(),
+                                            reinterpret_cast<const em2_count*>(subset.data()), source.k(),
+                                            reinterpret_cast<const em2_pair*>(source.begin(0)), candidateCount.data(), k,
+                                            similarityThreshold, reinterpret_cast<em2_pair*>(similarPairs.begin(0)), used.data()),
+                  "em2_rescore_similar_pairs");
+    } catch (...) {
+        similarPairs.remove();      // no valid-looking SimilarPairs-<new> set stays behind a failed call
+        throw;
+    }
+    similarPairs.setUsedCounts(used);
+    lastScanMs = gpu.stats().scan_ms;
+}

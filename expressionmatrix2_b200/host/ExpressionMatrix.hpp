@@ -76,6 +76,12 @@ public:
     // that do not belong to the counts, k or threshold are detected and throw, except lists made with a HIGHER threshold,
     // which give wrong lists.  The old object is not modified.
     void extendSimilarPairs0(const std::string& similarPairsName, const std::string& newSimilarPairsName, double similarityThreshold);
+    // The lists of SimilarPairs-<similarPairsName> (any findSimilarPairs* object) rescored with the exact similarities of
+    // findSimilarPairs0: SimilarPairs-<newSimilarPairsName>, on the same gene set and cell set, holds for each cell the k best
+    // of its listed cells by the similarity findSimilarPairs0 would store, among those above similarityThreshold.  Only the
+    // listed ids are read.  The source object is not modified.
+    void rescoreSimilarPairs(const std::string& similarPairsName, const std::string& newSimilarPairsName, size_t k,
+                             double similarityThreshold);
 
     // Scan variant for findSimilarPairs4 (em2_variant; 0 = automatic).
     int scanVariant = 0;

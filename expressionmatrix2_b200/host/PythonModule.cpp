@@ -105,6 +105,10 @@ PYBIND11_MODULE(ExpressionMatrix2, module)
              "Extends the lists of an existing findSimilarPairs0 object to the cells appended to its cell set since; "
              "the result is what findSimilarPairs0 would store on the grown cell set.  The old object is not modified.",
              arg("similarPairsName"), arg("newSimilarPairsName"), arg("similarityThreshold") = 0.2)
+        .def("rescoreSimilarPairs", &ExpressionMatrix::rescoreSimilarPairs,
+             "Rescores the lists of an existing SimilarPairs object with findSimilarPairs0's exact similarities: each cell keeps "
+             "the k best of its listed cells above similarityThreshold.  The source object is not modified.",
+             arg("similarPairsName"), arg("newSimilarPairsName"), arg("k") = 100, arg("similarityThreshold") = 0.2)
         .def("computeLshSignatures", &ExpressionMatrix::computeLshSignatures, arg("geneSetName") = "AllGenes",
              arg("cellSetName") = "AllCells", arg("lshName"), arg("lshCount") = 1024, arg("seed") = 231)
         .def_readwrite("scanVariant", &ExpressionMatrix::scanVariant)

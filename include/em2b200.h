@@ -306,6 +306,29 @@ int em2_extend_exact_similar_pairs(em2_context* ctx, uint64_t oldCellCount, uint
                                    const uint64_t* toc, const em2_count* counts, uint64_t k, double similarityThreshold,
                                    const em2_pair* oldPairs, const uint32_t* oldUsedCount, em2_pair* pairs, uint32_t* usedCount);
 
+/* Exact rescoring of candidate lists: for every cell a, the k best entries by (similarity desc, id asc) among its candidates
+ * b with r(a,b) > similarityThreshold, where r(a,b) is the float em2_exact_similar_pairs(cellCount, ...) stores for that pair
+ * in row a.  candidates/candidateCount: rows in the SimilarPairs payload layout, [cellCount][candidateWidth] with
+ * candidateCount[a] entries used -- any em2_*_similar_pairs or findSimilarPairs7 output; only the ids are read (the stored
+ * similarities are ignored) and their order within a row is free.  pairs [cellCount][k] / usedCount [cellCount] are written as
+ * em2_exact_similar_pairs writes its rows (unused slots zeroed); k > candidateWidth is allowed, rows then hold at most
+ * candidateWidth entries.  The arithmetic is decided as in em2_exact_similar_pairs from all cells' counts (option
+ * "exact_general" honoured): the exact integer scalar product, or the general kernel's lane partition and shuffle tree with
+ * row a on the dense side (in that path r(a,b) and r(b,a) can differ in the last bit); then r goes through the same double
+ * operations.  So with every other cell as a candidate the result equals em2_exact_similar_pairs bit for bit, and rescoring
+ * its own lists of width k' to k <= k' with the same threshold gives the first k entries of each row.  Only the counts, the
+ * candidates, the outputs and per-cell sums live on the device: no digit planes, no similarity matrix.
+ * Returns EM2_ERR_INVALID without writing any output if: an argument or limit of em2_exact_similar_pairs fails (including a
+ * stored gene id >= geneCount and the general path's 25,600-gene limit), candidateWidth is not in [1, 1024], a
+ * candidateCount exceeds candidateWidth, a candidate id is >= cellCount or equal to its row's cell, a row lists an id twice,
+ * or the output buffers overlap the candidates.
+ * Stats: h2d/d2h ms and bytes, sums_ms, scan_ms (the rescoring), total_ms, kernel_launches, variant_used as
+ * em2_exact_similar_pairs sets it. */
+int em2_rescore_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
+                              const em2_count* counts, uint64_t candidateWidth, const em2_pair* candidates,
+                              const uint32_t* candidateCount, uint64_t k, double similarityThreshold,
+                              em2_pair* pairs, uint32_t* usedCount);
+
 /* ------------------------------------------------------------------------------------------------
  * Device-resident calls: every pointer is a DEVICE pointer on the context's device, work is enqueued
  * on `stream` (a cudaStream_t passed as void*; NULL = legacy default stream) and the call returns
