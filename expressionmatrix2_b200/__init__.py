@@ -180,6 +180,18 @@ def _as_pairs(counts, gene_ids=None) -> np.ndarray:
     return counts
 
 
+def _old_lists(old_cell_count: int, old_ids, old_sims, old_used, k: int):
+    """The old lists of an extension call packed as SIMPAIR_DTYPE [old, k], and old_used as uint32 [old]."""
+    old = np.zeros((old_cell_count, k), SIMPAIR_DTYPE)
+    if old_cell_count:
+        old["cell"] = np.asarray(old_ids, np.uint32).reshape(old_cell_count, k)
+        old["similarity"] = np.asarray(old_sims, np.float32).reshape(old_cell_count, k)
+    old_used = np.ascontiguousarray(old_used, np.uint32)
+    if old_used.shape != (old_cell_count,):
+        raise ValueError("old_used must hold one count per old cell")
+    return old, old_used
+
+
 class Engine:
     """One context on one GPU (em2_context).  Not re-entrant."""
 
@@ -277,13 +289,7 @@ class Engine:
         are already exact."""
         sig = np.ascontiguousarray(signatures, np.uint64)
         n = sig.shape[0]
-        old = np.zeros((old_cell_count, k), SIMPAIR_DTYPE)
-        if old_cell_count:
-            old["cell"] = np.asarray(old_ids, np.uint32).reshape(old_cell_count, k)
-            old["similarity"] = np.asarray(old_sims, np.float32).reshape(old_cell_count, k)
-        old_used = np.ascontiguousarray(old_used, np.uint32)
-        if old_used.shape != (old_cell_count,):
-            raise ValueError("old_used must hold one count per old cell")
+        old, old_used = _old_lists(old_cell_count, old_ids, old_sims, old_used, k)
         out = np.zeros((n, k), SIMPAIR_DTYPE)
         used = np.zeros(n, np.uint32)
         self._check(self._L.em2_extend_similar_pairs(self._h, _ptr(sig), old_cell_count, n, lsh_count, k, similarity_threshold,
@@ -448,13 +454,7 @@ class Engine:
         toc = np.ascontiguousarray(toc, np.uint64)
         pairs = _as_pairs(counts, gene_ids)
         n = len(toc) - 1
-        old = np.zeros((old_cell_count, k), SIMPAIR_DTYPE)
-        if old_cell_count:
-            old["cell"] = np.asarray(old_ids, np.uint32).reshape(old_cell_count, k)
-            old["similarity"] = np.asarray(old_sims, np.float32).reshape(old_cell_count, k)
-        old_used = np.ascontiguousarray(old_used, np.uint32)
-        if old_used.shape != (old_cell_count,):
-            raise ValueError("old_used must hold one count per old cell")
+        old, old_used = _old_lists(old_cell_count, old_ids, old_sims, old_used, k)
         out = np.zeros((n, k), SIMPAIR_DTYPE)
         used = np.zeros(n, np.uint32)
         self._check(self._L.em2_extend_exact_similar_pairs(self._h, old_cell_count, n, gene_count, _ptr(toc), _ptr(pairs), k,

@@ -290,6 +290,46 @@ int checkScanArguments(em2_context* ctx, uint64_t cellCount, uint64_t lshCount, 
     return EM2_OK;
 }
 
+int readFlag(em2_context* ctx, const uint32_t* dFlag, cudaStream_t s, uint32_t* value)
+{
+    void* pin = nullptr;
+    EM2_TRY(reservePinned(ctx, 2, 64, &pin));
+    EM2_CUDA(ctx, cudaMemcpyAsync(pin, dFlag, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    EM2_CUDA(ctx, cudaStreamSynchronize(s));
+    *value = *static_cast<uint32_t*>(pin);
+    return EM2_OK;
+}
+
+static bool overlaps(const void* a, size_t aBytes, const void* b, size_t bBytes)
+{
+    const uintptr_t a0 = reinterpret_cast<uintptr_t>(a), b0 = reinterpret_cast<uintptr_t>(b);
+    return aBytes && bBytes && a0 < b0 + bBytes && b0 < a0 + aBytes;
+}
+
+bool outputsOverlap(const void* pairs, size_t pairBytes, const void* usedCount, size_t usedBytes, const void* in0, size_t in0Bytes,
+                    const void* in1, size_t in1Bytes)
+{
+    return overlaps(pairs, pairBytes, in0, in0Bytes) || overlaps(pairs, pairBytes, in1, in1Bytes) ||
+           overlaps(usedCount, usedBytes, in0, in0Bytes) || overlaps(usedCount, usedBytes, in1, in1Bytes);
+}
+
+std::string describeFlags(uint32_t f, const char* source)
+{
+    std::string r;
+    auto add = [&](uint32_t bit, const std::string& what) {
+        if (!(f & bit)) return;
+        if (!r.empty()) r += "; ";
+        r += what;
+    };
+    add(kExtendBadUsed, "a usedCount exceeds k");
+    add(kExtendBadId, "an id is not below oldCellCount");
+    add(kExtendBadSelf, "a row lists its own cell");
+    add(kExtendBadThreshold, "a stored pair does not pass the similarity threshold");
+    add(kExtendBadSimilarity, std::string("a stored similarity differs from the one ") + source + " give");
+    add(kExtendBadOrder, "a row is not sorted by decreasing similarity, then increasing id");
+    return r;
+}
+
 int uploadLut(em2_context* ctx, uint64_t lshCount, float** dLut)
 {
     std::vector<double> t(lshCount + 1);
@@ -998,124 +1038,6 @@ int em2_signature_graph(em2_context* ctx, const uint64_t* signatures, uint64_t c
         EM2_CUDA(ctx, cudaMemcpyAsync(edges, dEdges, *edgeCount * sizeof(em2_signature_edge), cudaMemcpyDeviceToHost, s));
     ctx->stats.d2h_bytes += kept * 4 + (*vertexCount + 1) * 8 + *edgeCount * sizeof(em2_signature_edge);
     EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
-}
-
-int em2_exact_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
-                            const em2_count* counts, uint64_t k, double similarityThreshold, em2_pair* pairs,
-                            uint32_t* usedCount)
-{
-    EM2_TRY(guardDevice(ctx));
-    if (!toc || !pairs || !usedCount || (!counts && cellCount && toc[cellCount]))
-        return fail(ctx, EM2_ERR_INVALID, "em2_exact_similar_pairs: null pointer");
-    resetStats(ctx);
-    const double t0 = nowMs();
-    if (cellCount == 0) return EM2_OK;
-    StageTimer T(ctx);
-    const uint64_t nnz = toc[cellCount];
-    void *dToc, *dCounts, *dSum1, *dSum2, *dPairs, *dUsed;
-    EM2_TRY(reserve(ctx, em2_context::S_TOC, (cellCount + 1) * sizeof(uint64_t), &dToc));
-    EM2_TRY(reserve(ctx, em2_context::S_COUNTS, nnz * sizeof(em2_count), &dCounts));
-    EM2_TRY(reserve(ctx, em2_context::S_SUM1, cellCount * sizeof(double), &dSum1));
-    EM2_TRY(reserve(ctx, em2_context::S_SUM2, cellCount * sizeof(double), &dSum2));
-    EM2_TRY(reserve(ctx, em2_context::S_PAIRS, cellCount * k * sizeof(em2_pair), &dPairs));
-    EM2_TRY(reserve(ctx, em2_context::S_USED, cellCount * sizeof(uint32_t), &dUsed));
-    cudaStream_t s = ctx->stream;
-    const int e0 = T.mark();
-    EM2_CUDA(ctx, cudaMemcpyAsync(dToc, toc, (cellCount + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    EM2_CUDA(ctx, cudaMemcpyAsync(dCounts, counts, nnz * sizeof(em2_count), cudaMemcpyHostToDevice, s));
-    ctx->stats.h2d_bytes += (cellCount + 1) * 8 + nnz * 8;
-    const int e1 = T.mark();
-    EM2_TRY(launchCellSums(ctx, cellCount, static_cast<uint64_t*>(dToc), static_cast<em2_count*>(dCounts),
-                           static_cast<double*>(dSum1), static_cast<double*>(dSum2), s));
-    const int e2 = T.mark();
-    EM2_TRY(launchExact(ctx, cellCount, geneCount, static_cast<uint64_t*>(dToc), static_cast<em2_count*>(dCounts),
-                        static_cast<double*>(dSum1), static_cast<double*>(dSum2), k, similarityThreshold,
-                        static_cast<em2_pair*>(dPairs), static_cast<uint32_t*>(dUsed), s));
-    const int e3 = T.mark();
-    EM2_CUDA(ctx, cudaMemcpyAsync(pairs, dPairs, cellCount * k * sizeof(em2_pair), cudaMemcpyDeviceToHost, s));
-    EM2_CUDA(ctx, cudaMemcpyAsync(usedCount, dUsed, cellCount * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    const int e4 = T.mark();
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    ctx->stats.h2d_ms = T.ms(e0, e1);
-    ctx->stats.sums_ms = T.ms(e1, e2);
-    ctx->stats.scan_ms = T.ms(e2, e3);
-    ctx->stats.d2h_ms = T.ms(e3, e4);
-    ctx->stats.d2h_bytes += cellCount * k * sizeof(em2_pair) + cellCount * 4;
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
-}
-
-int em2_rescore_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
-                              const em2_count* counts, uint64_t candidateWidth, const em2_pair* candidates,
-                              const uint32_t* candidateCount, uint64_t k, double similarityThreshold, em2_pair* pairs,
-                              uint32_t* usedCount)
-{
-    EM2_TRY(guardDevice(ctx));
-    const uint64_t N = cellCount, width = candidateWidth;
-    if (!toc || !pairs || !usedCount || !candidates || !candidateCount || (!counts && N && toc[N]))
-        return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: null pointer");
-    EM2_TRY(checkExactArguments(ctx, N, geneCount, k, similarityThreshold));
-    if (width == 0 || width > 1024) return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: candidateWidth must be in [1, 1024]");
-    const size_t pairBytes = N * k * sizeof(em2_pair), usedBytes = N * sizeof(uint32_t);
-    const size_t candBytes = N * width * sizeof(em2_pair), candUsedBytes = N * sizeof(uint32_t);
-    if (overlaps(pairs, pairBytes, candidates, candBytes) || overlaps(pairs, pairBytes, candidateCount, candUsedBytes) ||
-        overlaps(usedCount, usedBytes, candidates, candBytes) || overlaps(usedCount, usedBytes, candidateCount, candUsedBytes))
-        return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: the output buffers overlap the candidates");
-    for (uint64_t a = 0; a < N; a++)
-        if (candidateCount[a] > width)
-            return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: candidateCount[" + std::to_string(a) + "] exceeds candidateWidth");
-    resetStats(ctx);
-    const double t0 = nowMs();
-    if (N == 0) return EM2_OK;
-    cudaStream_t s = ctx->stream;
-    StageTimer T(ctx);
-    const uint64_t nnz = toc[N];
-    void *dToc, *dCounts, *dSum1, *dSum2, *dPairs, *dUsed, *dCand;
-    EM2_TRY(reserve(ctx, em2_context::S_TOC, (N + 1) * sizeof(uint64_t), &dToc));
-    EM2_TRY(reserve(ctx, em2_context::S_COUNTS, nnz * sizeof(em2_count), &dCounts));
-    EM2_TRY(reserve(ctx, em2_context::S_SUM1, N * sizeof(double), &dSum1));
-    EM2_TRY(reserve(ctx, em2_context::S_SUM2, N * sizeof(double), &dSum2));
-    EM2_TRY(reserve(ctx, em2_context::S_PAIRS, pairBytes, &dPairs));
-    EM2_TRY(reserve(ctx, em2_context::S_USED, usedBytes, &dUsed));
-    // [candidates N * width][candidateCount N][flags 4]
-    EM2_TRY(reserve(ctx, em2_context::S_RESCORE, candBytes + candUsedBytes + 16, &dCand));
-    auto* dCandUsed = reinterpret_cast<uint32_t*>(static_cast<em2_pair*>(dCand) + N * width);
-    uint32_t* dFlags = dCandUsed + N;
-
-    const int e0 = T.mark();
-    EM2_TRY(stageH2D(ctx, dToc, toc, (N + 1) * sizeof(uint64_t), s));
-    EM2_TRY(stageH2D(ctx, dCounts, counts, nnz * sizeof(em2_count), s));
-    EM2_TRY(stageH2D(ctx, dCand, candidates, candBytes, s));
-    EM2_TRY(stageH2D(ctx, dCandUsed, candidateCount, candUsedBytes, s));
-    ctx->stats.h2d_bytes += (N + 1) * 8 + nnz * 8 + candBytes + candUsedBytes;
-    const int e1 = T.mark();
-    EM2_TRY(launchCellSums(ctx, N, static_cast<uint64_t*>(dToc), static_cast<em2_count*>(dCounts), static_cast<double*>(dSum1),
-                           static_cast<double*>(dSum2), s));
-    const int e2 = T.mark();
-    uint32_t bad = 0;
-    EM2_TRY(launchRescoreExact(ctx, N, geneCount, static_cast<uint64_t*>(dToc), static_cast<em2_count*>(dCounts),
-                               static_cast<double*>(dSum1), static_cast<double*>(dSum2), width, static_cast<em2_pair*>(dCand),
-                               dCandUsed, k, similarityThreshold, dFlags, static_cast<em2_pair*>(dPairs), static_cast<uint32_t*>(dUsed),
-                               s, &bad));
-    if (bad) {
-        std::string what;
-        if (bad & kRescoreBadId) what += "; a candidate id is not below cellCount";
-        if (bad & kRescoreBadSelf) what += "; a row lists its own cell";
-        if (bad & kRescoreBadDuplicate) what += "; a row lists a candidate twice";
-        return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: invalid candidate lists: " + what.substr(2));
-    }
-    const int e3 = T.mark();
-    EM2_TRY(stageD2H(ctx, pairs, dPairs, pairBytes, s));
-    EM2_TRY(stageD2H(ctx, usedCount, dUsed, usedBytes, s));
-    const int e4 = T.mark();
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    ctx->stats.d2h_bytes += pairBytes + usedBytes;
-    ctx->stats.h2d_ms = T.ms(e0, e1);
-    ctx->stats.sums_ms = T.ms(e1, e2);
-    ctx->stats.scan_ms = T.ms(e2, e3);
-    ctx->stats.d2h_ms = T.ms(e3, e4);
     ctx->stats.total_ms = nowMs() - t0;
     return EM2_OK;
 }

@@ -64,8 +64,7 @@ struct em2_context {
         S_COLLOGFILL,    // symmetric scan: entries per log chunk + the chunk allocator
         S_DIST0, S_DIST1, S_DIST2, S_DIST3,   // multi-GPU exchange buffers (multi.cu)
         S_PERM,          // scan position -> cell id
-        S_EXTEND,        // em2_extend_similar_pairs: old lists, their keys, lengths and column bounds, the validation flags
-        S_RESCORE,       // em2_rescore_similar_pairs: candidate lists, their lengths, the check flags
+        S_EXTEND,        // the caller's input lists of the call in progress (old lists or candidates) and what the call keeps with them
         S_COUNT
     };
     int signatureMode = 0;   // 0 auto, 1 FP64 kernel only, 2 force the tensor-core filter path
@@ -86,7 +85,7 @@ struct em2_context {
     int denseWarpKernel = 0;           // 1: dense expansion of the filter path with the warp-per-cell kernel (tests / comparison)
     int filterCountsSigned = 0;   // 1: dense counts as s8 (<= 127) instead of u8 (<= 255) in the filter GEMM
     em2::DeviceBuffer scratch[S_COUNT];
-    em2::PinnedBuffer pinned[3];      // [2]: small read-back flags (symmetric scan)
+    em2::PinnedBuffer pinned[3];      // [2]: small read-back flags (readFlag)
     // pageable host buffers (mmap regions) are staged through two pinned bounce buffers (capi.cu, stageH2D / stageD2H)
     void* bounce[2] = {nullptr, nullptr};
     cudaEvent_t bounceFree[2] = {nullptr, nullptr};
@@ -155,6 +154,22 @@ int checkScanArguments(em2_context* ctx, uint64_t cellCount, uint64_t lshCount, 
 int stageH2D(em2_context* ctx, void* dst, const void* src, size_t bytes, cudaStream_t s);
 int stageD2H(em2_context* ctx, void* dst, const void* src, size_t bytes, cudaStream_t s);
 int fetchCounters(em2_context* ctx);
+// Reads one device flag word back through pinned[2] once everything before it on s is done.
+int readFlag(em2_context* ctx, const uint32_t* dFlag, cudaStream_t s, uint32_t* value);
+// Whether the output lists (pairs, usedCount) overlap either of a call's two input buffers.
+bool outputsOverlap(const void* pairs, size_t pairBytes, const void* usedCount, size_t usedBytes, const void* in0, size_t in0Bytes,
+                    const void* in1, size_t in1Bytes);
+// Validation of old lists by the extension calls: what a stored entry got wrong, OR-ed over all entries.
+enum : uint32_t {
+    kExtendBadUsed = 1,        // usedCount > k
+    kExtendBadId = 2,          // an id >= oldCellCount
+    kExtendBadSelf = 4,        // a row lists its own cell
+    kExtendBadThreshold = 8,   // the recomputed similarity does not pass the threshold
+    kExtendBadSimilarity = 16, // the stored similarity is not the recomputed one
+    kExtendBadOrder = 32,      // a row is not strictly increasing in (similarity desc, id asc)
+};
+// Text of those flags; `source` names what the similarities were recomputed from.
+std::string describeFlags(uint32_t flags, const char* source);
 int signaturesOnDevice(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
                        const double* U, uint64_t lshCount, uint64_t** dSigOut, double** dSum1Out, double** dSum2Out,
                        uint64_t sigTotalRows = 0, uint64_t sigRowOffset = 0, const double* dUready = nullptr);
@@ -245,46 +260,6 @@ int launchMismatchCounts(em2_context* ctx, const uint64_t* signatures, uint64_t 
                          const uint32_t* c0, const uint32_t* c1, uint32_t* out, cudaStream_t s);
 int launchMismatchBlock(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uint64_t lshCount,
                         uint64_t rowBegin, uint64_t rowEnd, int variant, uint16_t* out, cudaStream_t s);
-int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
-                const em2_count* counts, const double* sum1, const double* sum2, uint64_t k,
-                double similarityThreshold, em2_pair* pairs, uint32_t* usedCount, cudaStream_t s);
-// The exact path's argument checks: k in [1, 1024], the size limits, similarityThreshold <= 1.
-int checkExactArguments(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, uint64_t k, double similarityThreshold);
-// Extension of exact lists of cells [0, oldN) to cells [oldN, N) (exact.cu; extend.cu has the entry point).  Device pointers:
-// oldPairs / oldUsed the old lists, winPairs / winUsed scratch for oldN rows, flags one word.  *badFlags (kExtend*) != 0: the
-// old lists failed validation and nothing was computed.  *scanSymmetric: 1 = the rectangle ran, 0 = the full job or nothing
-// appended.
-int launchExtendExact(em2_context* ctx, uint64_t oldN, uint64_t N, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
-                      const double* sum1, const double* sum2, uint64_t k, double similarityThreshold, const em2_pair* oldPairs,
-                      const uint32_t* oldUsed, em2_pair* winPairs, uint32_t* winUsed, uint32_t* flags, em2_pair* pairs,
-                      uint32_t* usedCount, cudaStream_t s, uint32_t* badFlags, int* scanSymmetric);
-// Rescoring of candidate lists with the exact path's similarities (exact.cu; capi.cu has the entry point).  Device pointers:
-// candidates [N][width] (ids only are read), candidateCount [N] (each <= width, checked by the caller), flags one word.
-// *badFlags (kRescore*) != 0: an id failed its checks, and pairs / usedCount hold nothing of use.
-int launchRescoreExact(em2_context* ctx, uint64_t N, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
-                       const double* sum1, const double* sum2, uint64_t width, const em2_pair* candidates,
-                       const uint32_t* candidateCount, uint64_t k, double similarityThreshold, uint32_t* flags, em2_pair* pairs,
-                       uint32_t* usedCount, cudaStream_t s, uint32_t* badFlags);
-// What the candidate ids of em2_rescore_similar_pairs got wrong, OR-ed over all rows.
-enum : uint32_t {
-    kRescoreBadId = 1,          // an id >= cellCount
-    kRescoreBadSelf = 2,        // a row lists its own cell
-    kRescoreBadDuplicate = 4,   // a row lists a cell twice
-};
-
-// Validation of old lists by the extension calls: what a stored entry got wrong, OR-ed over all entries.
-enum : uint32_t {
-    kExtendBadUsed = 1,        // usedCount > k
-    kExtendBadId = 2,          // an id >= oldCellCount
-    kExtendBadSelf = 4,        // a row lists its own cell
-    kExtendBadThreshold = 8,   // the recomputed similarity does not pass the threshold
-    kExtendBadSimilarity = 16, // the stored similarity is not the recomputed one
-    kExtendBadOrder = 32,      // a row is not strictly increasing in (similarity desc, id asc)
-};
-// Text of those flags; `source` names what the similarities were recomputed from.
-std::string describeFlags(uint32_t flags, const char* source);
-// Whether two byte ranges overlap.
-bool overlaps(const void* a, size_t aBytes, const void* b, size_t bBytes);
 
 // ---- multi-GPU (multi.cu) -------------------------------------------------------------------------------------
 // Rank r owns the cells [r * shard, min(N, (r + 1) * shard)); shard is a multiple of 256 when there is more than one rank.

@@ -26,9 +26,9 @@
 // SAME dense planes (128B-swizzled TMA boxes).  Tiles are visited in 12 x 12 super-tiles so that the ~148
 // CTAs running at any moment share 24 row/column panels through L2 instead of streaming 148 distinct ones.
 //
-// launchExtendExact extends the lists of a job over the first N cells to cells appended after them with the same kernels:
-// the new rows against all columns, the old rows against a column window of the new cells (ExactParams.colBegin), and a
-// merge with the old lists after exactValidateKernel has recomputed every stored entry with the full job's bits.
+// The file ends with the exact path's three blocking calls, which share their host-side set-up (ExactCall):
+// em2_exact_similar_pairs (the full job), em2_extend_exact_similar_pairs (a job's lists extended to appended cells with the
+// same kernels) and em2_rescore_similar_pairs (candidate lists rescored with the full job's similarities).
 #include "common.cuh"
 #include "tc05.cuh"
 
@@ -473,6 +473,15 @@ __device__ __forceinline__ float fromOrderable(uint32_t o)
 {
     return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
 }
+__device__ __forceinline__ uint64_t sortKey(float similarity, uint32_t id) { return (uint64_t(~orderable(similarity)) << 32) | id; }
+__device__ __forceinline__ em2_pair keyPair(uint64_t key)
+{
+    em2_pair e;
+    e.cell = uint32_t(key);
+    e.similarity = fromOrderable(~uint32_t(key >> 32));
+    return e;
+}
+constexpr em2_pair kEmptyPair{0u, 0.f};     // an unused slot of a list
 
 constexpr int kSelWarps = 4;
 
@@ -515,7 +524,7 @@ exactSelectKernel(uint64_t rows, uint64_t cellCount, uint64_t ldOut, const float
         uint64_t key = ~0ull;
         if (id < cellCount) {
             const float f = __ldg(src + id);
-            if (f != kRejected) key = (uint64_t(~orderable(f)) << 32) | id;
+            if (f != kRejected) key = sortKey(f, uint32_t(id));
         }
         const bool pass = key < bound;
         const uint32_t mask = __ballot_sync(0xffffffffu, pass);
@@ -526,21 +535,11 @@ exactSelectKernel(uint64_t rows, uint64_t cellCount, uint64_t ldOut, const float
         }
     }
     prune();
-    for (uint32_t e = lane; e < k; e += 32) {
-        em2_pair out;
-        if (e < count) {
-            out.cell = uint32_t(buf[e]);
-            out.similarity = fromOrderable(~uint32_t(buf[e] >> 32));
-        } else {
-            out.cell = 0;
-            out.similarity = 0.f;
-        }
-        pairs[row * k + e] = out;
-    }
+    for (uint32_t e = lane; e < k; e += 32) pairs[row * k + e] = e < count ? keyPair(buf[e]) : kEmptyPair;
     if (lane == 0) usedCount[row] = count;
 }
 
-// ---- extension of old lists to appended cells (launchExtendExact) --------------------------------------------------
+// ---- extension of old lists to appended cells (em2_extend_exact_similar_pairs) -------------------------------------
 // The stored count of `gene` in cell c, 0 when there is none (genes ascend within a cell): the value the general kernel's
 // dense row holds for that gene.
 __device__ __forceinline__ float storedCount(const uint64_t* __restrict__ toc, const em2_count* __restrict__ counts, uint64_t c,
@@ -633,7 +632,7 @@ exactValidateKernel(uint64_t oldN, uint64_t geneCount, uint64_t gPad, const uint
     uint64_t prevKey = 0;
     for (uint32_t i = 0; i < used; i++) {
         const em2_pair e = row[i];
-        const uint64_t key = (uint64_t(~orderable(e.similarity)) << 32) | e.cell;
+        const uint64_t key = sortKey(e.similarity, e.cell);
         if (i && !(prevKey < key)) bad |= kExtendBadOrder;
         prevKey = key;
         if (e.cell >= oldN) {
@@ -659,13 +658,7 @@ exactValidateKernel(uint64_t oldN, uint64_t geneCount, uint64_t gPad, const uint
         else if (__float_as_uint(float(r)) != __float_as_uint(e.similarity)) bad |= kExtendBadSimilarity;
     }
     if (lane == 0 && bad) atomicOr(flags, bad);
-    for (uint32_t i = lane; i < k; i += 32) {
-        em2_pair out;
-        out.cell = 0;
-        out.similarity = 0.f;
-        if (i < used) out = row[i];
-        outPairs[a * k + i] = out;
-    }
+    for (uint32_t i = lane; i < k; i += 32) outPairs[a * k + i] = i < used ? row[i] : kEmptyPair;
     if (lane == 0) outUsed[a] = used;
 }
 
@@ -674,7 +667,7 @@ exactValidateKernel(uint64_t oldN, uint64_t geneCount, uint64_t gPad, const uint
 // place in the merged row is its own index plus the number of entries of the other list with a smaller key.
 __device__ __forceinline__ uint64_t pairKey(em2_pair e, uint32_t idOffset)
 {
-    return (uint64_t(~orderable(e.similarity)) << 32) | (e.cell + idOffset);
+    return sortKey(e.similarity, e.cell + idOffset);
 }
 __device__ __forceinline__ uint32_t countBelow(const em2_pair* list, uint32_t used, uint32_t idOffset, uint64_t key)
 {
@@ -711,16 +704,11 @@ exactMergeKernel(uint64_t oldN, uint32_t k, const em2_pair* __restrict__ oldPair
         if (pos < k) out[pos] = e;
     }
     const uint32_t total = min(k, uo + uw);
-    for (uint32_t i = total + lane; i < k; i += 32) {
-        em2_pair z;
-        z.cell = 0;
-        z.similarity = 0.f;
-        out[i] = z;
-    }
+    for (uint32_t i = total + lane; i < k; i += 32) out[i] = kEmptyPair;
     if (lane == 0) usedCount[a] = total;
 }
 
-// ---- rescoring of candidate lists (launchRescoreExact) -------------------------------------------------------------------
+// ---- rescoring of candidate lists (em2_rescore_similar_pairs) ------------------------------------------------------------
 // A CTA of kRescoreWarps warps takes rows a = blockIdx.x, blockIdx.x + gridDim.x, ...  Row a's counts are scattered into a
 // dense shared-memory row (uint16 per gene on the integer path, where counts are <= 65535; float on the general path) and
 // cleared again afterwards, so a row costs nnz(a), not G.  DENSE == false (integer path, too many genes for that row): a's
@@ -729,6 +717,12 @@ exactMergeKernel(uint64_t oldN, uint32_t k, const em2_pair* __restrict__ oldPair
 // not pass the threshold, are sorted in shared memory (bitonic): the passing keys form a prefix, the row is its first k, and
 // a candidate listed twice gives two equal keys, adjacent after the sort.
 constexpr int kRescoreWarps = 8;
+// What the candidate ids got wrong, OR-ed over all rows.
+enum : uint32_t {
+    kRescoreBadId = 1,          // an id >= cellCount
+    kRescoreBadSelf = 2,        // a row lists its own cell
+    kRescoreBadDuplicate = 4,   // a row lists a cell twice
+};
 constexpr uint32_t kRescoreReject = 0xffffffffu;     // above ~orderable(r) for every r in [-1, 1]
 
 template <bool GENERAL, bool DENSE>
@@ -773,7 +767,7 @@ exactRescoreKernel(uint64_t cellCount, uint64_t geneCount, const uint64_t* __res
                 else
                     r = warpPairR<false, true>(b, toc, counts, [=](uint32_t g) { return uint32_t(storedCount(toc, counts, a, g)); }, n, s1a,
                                          va, sum1, var, lane);
-                if (r > threshold) key = (uint64_t(~orderable(float(r))) << 32) | b;
+                if (r > threshold) key = sortKey(float(r), b);
             }
             if (lane == 0) keys[i] = key;
         }
@@ -798,16 +792,7 @@ exactRescoreKernel(uint64_t cellCount, uint64_t geneCount, const uint64_t* __res
         }
         __syncthreads();
         const uint32_t kept = min(passed, k);
-        for (uint32_t e = threadIdx.x; e < k; e += blockDim.x) {
-            em2_pair out;
-            out.cell = 0;
-            out.similarity = 0.f;
-            if (e < kept) {
-                out.cell = uint32_t(keys[e]);
-                out.similarity = fromOrderable(~uint32_t(keys[e] >> 32));
-            }
-            pairs[a * k + e] = out;
-        }
+        for (uint32_t e = threadIdx.x; e < k; e += blockDim.x) pairs[a * k + e] = e < kept ? keyPair(keys[e]) : kEmptyPair;
         if (threadIdx.x == 0) usedCount[a] = kept;
         if constexpr (DENSE)
             for (uint64_t e = rowBegin + threadIdx.x; e < rowEnd; e += blockDim.x) dense[counts[e].gene] = Count(0);
@@ -817,8 +802,7 @@ exactRescoreKernel(uint64_t cellCount, uint64_t geneCount, const uint64_t* __res
     if (lane == 0 && bad) atomicOr(flags, bad);
 }
 
-}  // namespace
-
+// The exact path's argument checks: k in [1, 1024], the size limits, similarityThreshold <= 1.
 int checkExactArguments(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, uint64_t k, double similarityThreshold)
 {
     if (k == 0 || k > 1024) return fail(ctx, EM2_ERR_INVALID, "k must be in [1, 1024]");
@@ -826,8 +810,6 @@ int checkExactArguments(em2_context* ctx, uint64_t cellCount, uint64_t geneCount
     if (!(similarityThreshold <= 1.)) return fail(ctx, EM2_ERR_INVALID, "similarityThreshold must be <= 1");   // CZI_ASSERT, FindSimilarPairs.cpp:27
     return EM2_OK;
 }
-
-namespace {
 
 // The arithmetic the exact path uses for a set of cells, decided from all of their counts: the general FP64 kernel, or the
 // integer tensor-core path with one or two digit planes.
@@ -1059,115 +1041,261 @@ int exactRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint6
 
 int exactVariant(const ExactArith& arith) { return arith.general ? EM2_VARIANT_POPC : EM2_VARIANT_MMA_I8; }   // POPC: "not the tensor-core path"
 
-}  // namespace
+// One blocking call on host buffers: toc and counts staged into the context's scratch, the cell sums, the lists copied back,
+// and the stage timings and byte counts of em2_stats.  The constructor resets the stats; the call's own input lists go
+// through input() between stage() and sums().
+struct ExactCall {
+    em2_context* ctx;
+    cudaStream_t s;
+    StageTimer T;
+    uint64_t N, geneCount, k = 0;
+    double t0;
+    int e0 = 0, e1 = 0, e2 = 0;
+    uint64_t* toc = nullptr;     // device copies of the caller's cells, their sums, and the device side of the lists
+    em2_count* counts = nullptr;
+    double *sum1 = nullptr, *sum2 = nullptr;
+    em2_pair* pairs = nullptr;
+    uint32_t* used = nullptr;
 
-int launchExact(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
-                const double* sum1, const double* sum2, uint64_t k, double similarityThreshold, em2_pair* pairs,
-                uint32_t* usedCount, cudaStream_t s)
+    ExactCall(em2_context* c, uint64_t cellCount, uint64_t genes) : ctx(c), s(c->stream), T(c), N(cellCount), geneCount(genes)
+    {
+        resetStats(ctx);
+        t0 = nowMs();
+    }
+
+    int stage(const uint64_t* hostToc, const em2_count* hostCounts, uint64_t listLength)
+    {
+        k = listLength;
+        const uint64_t nnz = hostToc[N];
+        void *dToc, *dCounts, *dSum1, *dSum2, *dPairs, *dUsed;
+        EM2_TRY(reserve(ctx, em2_context::S_TOC, (N + 1) * sizeof(uint64_t), &dToc));
+        EM2_TRY(reserve(ctx, em2_context::S_COUNTS, nnz * sizeof(em2_count), &dCounts));
+        EM2_TRY(reserve(ctx, em2_context::S_SUM1, N * sizeof(double), &dSum1));
+        EM2_TRY(reserve(ctx, em2_context::S_SUM2, N * sizeof(double), &dSum2));
+        EM2_TRY(reserve(ctx, em2_context::S_PAIRS, N * k * sizeof(em2_pair), &dPairs));
+        EM2_TRY(reserve(ctx, em2_context::S_USED, N * sizeof(uint32_t), &dUsed));
+        toc = static_cast<uint64_t*>(dToc);
+        counts = static_cast<em2_count*>(dCounts);
+        sum1 = static_cast<double*>(dSum1);
+        sum2 = static_cast<double*>(dSum2);
+        pairs = static_cast<em2_pair*>(dPairs);
+        used = static_cast<uint32_t*>(dUsed);
+        e0 = T.mark();
+        EM2_TRY(input(toc, hostToc, (N + 1) * sizeof(uint64_t)));
+        return input(counts, hostCounts, nnz * sizeof(em2_count));
+    }
+
+    int input(void* dst, const void* src, size_t bytes)
+    {
+        ctx->stats.h2d_bytes += bytes;
+        return stageH2D(ctx, dst, src, bytes, s);
+    }
+
+    int sums()
+    {
+        e1 = T.mark();
+        EM2_TRY(launchCellSums(ctx, N, toc, counts, sum1, sum2, s));
+        e2 = T.mark();
+        return EM2_OK;
+    }
+
+    // The arithmetic of the full job over all N cells and its per-cell operands (planes: see exactPrepare).
+    int operands(bool planes, ExactOperands* o)
+    {
+        ExactArith arith;
+        EM2_TRY(exactArithmetic(ctx, N, geneCount, toc, counts, sum2, s, &arith));
+        EM2_TRY(exactPrepare(ctx, arith, N, geneCount, toc, counts, sum1, sum2, planes, s, o));
+        ctx->stats.variant_used = exactVariant(arith);
+        return EM2_OK;
+    }
+
+    int finish(em2_pair* hostPairs, uint32_t* hostUsed)
+    {
+        const size_t pairBytes = N * k * sizeof(em2_pair), usedBytes = N * sizeof(uint32_t);
+        const int e3 = T.mark();
+        EM2_TRY(stageD2H(ctx, hostPairs, pairs, pairBytes, s));
+        EM2_TRY(stageD2H(ctx, hostUsed, used, usedBytes, s));
+        const int e4 = T.mark();
+        EM2_CUDA(ctx, cudaStreamSynchronize(s));
+        ctx->stats.d2h_bytes += pairBytes + usedBytes;
+        ctx->stats.h2d_ms = T.ms(e0, e1);
+        ctx->stats.sums_ms = T.ms(e1, e2);
+        ctx->stats.scan_ms = T.ms(e2, e3);
+        ctx->stats.d2h_ms = T.ms(e3, e4);
+        ctx->stats.total_ms = nowMs() - t0;
+        return EM2_OK;
+    }
+};
+
+}  // namespace
+}  // namespace em2
+
+using namespace em2;
+
+extern "C" {
+
+int em2_exact_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
+                            const em2_count* counts, uint64_t k, double similarityThreshold, em2_pair* pairs,
+                            uint32_t* usedCount)
 {
-    EM2_TRY(checkExactArguments(ctx, cellCount, geneCount, k, similarityThreshold));
-    ExactArith arith;
-    EM2_TRY(exactArithmetic(ctx, cellCount, geneCount, toc, counts, sum2, s, &arith));
+    EM2_TRY(guardDevice(ctx));
+    const uint64_t N = cellCount;
+    if (!toc || !pairs || !usedCount || (!counts && N && toc[N]))
+        return fail(ctx, EM2_ERR_INVALID, "em2_exact_similar_pairs: null pointer");
+    EM2_TRY(checkExactArguments(ctx, N, geneCount, k, similarityThreshold));
+    ExactCall c(ctx, N, geneCount);
+    if (N == 0) return EM2_OK;
+    EM2_TRY(c.stage(toc, counts, k));
+    EM2_TRY(c.sums());
     ExactOperands o;
-    EM2_TRY(exactPrepare(ctx, arith, cellCount, geneCount, toc, counts, sum1, sum2, true, s, &o));
-    EM2_TRY(exactRect(ctx, o, 0, cellCount, 0, cellCount, k, similarityThreshold, true, pairs, usedCount, s));
-    ctx->stats.variant_used = exactVariant(arith);
-    return EM2_OK;
+    EM2_TRY(c.operands(true, &o));
+    EM2_TRY(exactRect(ctx, o, 0, N, 0, N, k, similarityThreshold, true, c.pairs, c.used, c.s));
+    return c.finish(pairs, usedCount);
 }
 
-int launchExtendExact(em2_context* ctx, uint64_t oldN, uint64_t N, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
-                      const double* sum1, const double* sum2, uint64_t k, double similarityThreshold, const em2_pair* oldPairs,
-                      const uint32_t* oldUsed, em2_pair* winPairs, uint32_t* winUsed, uint32_t* flags, em2_pair* pairs,
-                      uint32_t* usedCount, cudaStream_t s, uint32_t* badFlags, int* scanSymmetric)
+// The lists of cells [0, oldCellCount) extended to the cells appended after them: the new rows against all columns, the old
+// rows against a column window of the new cells (ExactParams.colBegin), and a merge with the old lists after
+// exactValidateKernel has recomputed every stored entry with the full job's bits.
+int em2_extend_exact_similar_pairs(em2_context* ctx, uint64_t oldCellCount, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
+                                   const em2_count* counts, uint64_t k, double similarityThreshold, const em2_pair* oldPairs,
+                                   const uint32_t* oldUsedCount, em2_pair* pairs, uint32_t* usedCount)
 {
-    *badFlags = 0;
-    *scanSymmetric = 0;
+    EM2_TRY(guardDevice(ctx));
+    const uint64_t oldN = oldCellCount, N = cellCount;
+    if (!toc || !pairs || !usedCount || (!counts && N && toc[N]) || (oldN && (!oldPairs || !oldUsedCount)))
+        return fail(ctx, EM2_ERR_INVALID, "em2_extend_exact_similar_pairs: null pointer");
+    if (oldN > N) return fail(ctx, EM2_ERR_INVALID, "em2_extend_exact_similar_pairs: oldCellCount exceeds cellCount");
     EM2_TRY(checkExactArguments(ctx, N, geneCount, k, similarityThreshold));
-    // The arithmetic of the full job over all cells, and of the job the old lists came from.  If they differ, the old
-    // lists may hold other bits than a full run over all cells: compute the full job (exact by definition).
-    ExactArith arith;
-    EM2_TRY(exactArithmetic(ctx, N, geneCount, toc, counts, sum2, s, &arith));
+    const size_t oldPairBytes = oldN * k * sizeof(em2_pair), oldUsedBytes = oldN * sizeof(uint32_t);
+    if (outputsOverlap(pairs, N * k * sizeof(em2_pair), usedCount, N * sizeof(uint32_t), oldPairs, oldPairBytes, oldUsedCount,
+                       oldUsedBytes))
+        return fail(ctx, EM2_ERR_INVALID, "em2_extend_exact_similar_pairs: the output buffers overlap the old lists");
+    ExactCall c(ctx, N, geneCount);
+    if (N == 0) return EM2_OK;
+    cudaStream_t s = c.s;
+    // [oldPairs oldN * k][window pairs oldN * k][oldUsed oldN][window used oldN][flags 4]
+    void* ext = nullptr;
+    EM2_TRY(reserve(ctx, em2_context::S_EXTEND, 2 * (oldPairBytes + oldUsedBytes) + 16, &ext));
+    auto* dOldPairs = static_cast<em2_pair*>(ext);
+    em2_pair* dWinPairs = dOldPairs + oldN * k;
+    auto* dOldUsed = reinterpret_cast<uint32_t*>(dWinPairs + oldN * k);
+    uint32_t* dWinUsed = dOldUsed + oldN;
+    uint32_t* dFlags = dWinUsed + oldN;
+    EM2_TRY(c.stage(toc, counts, k));
+    EM2_TRY(c.input(dOldPairs, oldPairs, oldPairBytes));
+    EM2_TRY(c.input(dOldUsed, oldUsedCount, oldUsedBytes));
+    EM2_TRY(c.sums());
+    ExactOperands o;
+    EM2_TRY(c.operands(true, &o));
+    // The arithmetic of the job the old lists came from.  If it differs from the full job's, the old lists may hold other
+    // bits than a full run over all cells: compute the full job (exact by definition).
     bool full = oldN == 0;
     if (!full) {
         ExactArith oldArith;
-        EM2_TRY(exactArithmetic(ctx, oldN, geneCount, toc, counts, sum2, s, &oldArith));
-        full = oldArith.general != arith.general;
+        EM2_TRY(exactArithmetic(ctx, oldN, geneCount, c.toc, c.counts, c.sum2, s, &oldArith));
+        full = oldArith.general != o.arith.general;
     }
-    ExactOperands o;
-    EM2_TRY(exactPrepare(ctx, arith, N, geneCount, toc, counts, sum1, sum2, true, s, &o));
-    ctx->stats.variant_used = exactVariant(arith);
-    if (full) return exactRect(ctx, o, 0, N, 0, N, k, similarityThreshold, true, pairs, usedCount, s);
+    if (full) {
+        EM2_TRY(exactRect(ctx, o, 0, N, 0, N, k, similarityThreshold, true, c.pairs, c.used, s));
+        return c.finish(pairs, usedCount);
+    }
 
     // 1. the old lists against the counts; the caller's buffers are written only if all of them hold
-    EM2_CUDA(ctx, cudaMemsetAsync(flags, 0, sizeof(uint32_t), s));
+    EM2_CUDA(ctx, cudaMemsetAsync(dFlags, 0, sizeof(uint32_t), s));
     const unsigned valBlocks = unsigned((oldN + kValWarps - 1) / kValWarps);
-    if (arith.general)
-        exactValidateKernel<true><<<valBlocks, kValWarps * 32, 0, s>>>(oldN, geneCount, o.gPad, toc, counts, nullptr, nullptr, sum1,
-                                                                       o.var, similarityThreshold, uint32_t(k), oldPairs, oldUsed,
-                                                                       pairs, usedCount, flags);
+    if (o.arith.general)
+        exactValidateKernel<true><<<valBlocks, kValWarps * 32, 0, s>>>(oldN, geneCount, o.gPad, c.toc, c.counts, nullptr, nullptr, c.sum1,
+                                                                       o.var, similarityThreshold, uint32_t(k), dOldPairs, dOldUsed,
+                                                                       c.pairs, c.used, dFlags);
     else
-        exactValidateKernel<false><<<valBlocks, kValWarps * 32, 0, s>>>(oldN, geneCount, o.gPad, toc, counts, o.lo, o.hi, sum1,
-                                                                        o.var, similarityThreshold, uint32_t(k), oldPairs, oldUsed,
-                                                                        pairs, usedCount, flags);
+        exactValidateKernel<false><<<valBlocks, kValWarps * 32, 0, s>>>(oldN, geneCount, o.gPad, c.toc, c.counts, o.lo, o.hi, c.sum1,
+                                                                        o.var, similarityThreshold, uint32_t(k), dOldPairs, dOldUsed,
+                                                                        c.pairs, c.used, dFlags);
     ctx->stats.kernel_launches++;
     EM2_CUDA(ctx, cudaGetLastError());
-    void* pin = nullptr;
-    EM2_TRY(reservePinned(ctx, 2, 64, &pin));
-    EM2_CUDA(ctx, cudaMemcpyAsync(pin, flags, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    *badFlags = *static_cast<uint32_t*>(pin);
-    if (*badFlags || N == oldN) return EM2_OK;      // nothing appended: the validated old lists are the result
-
-    // 2. the appended rows against all columns: their final lists
-    EM2_TRY(exactRect(ctx, o, oldN, N, 0, N, k, similarityThreshold, false, pairs + oldN * k, usedCount + oldN, s));
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));        // the tile-list staging buffer is reused below
-    // 3. the old rows against the appended columns: each old row's k best new cells, merged with its old list
-    EM2_TRY(exactRect(ctx, o, 0, oldN, oldN, N, k, similarityThreshold, false, winPairs, winUsed, s));
-    exactMergeKernel<<<unsigned((oldN + kMergeWarps - 1) / kMergeWarps), kMergeWarps * 32, 0, s>>>(oldN, uint32_t(k), oldPairs, oldUsed,
-                                                                                                   winPairs, winUsed, pairs, usedCount);
-    ctx->stats.kernel_launches++;
-    EM2_CUDA(ctx, cudaGetLastError());
-    *scanSymmetric = 1;
-    return EM2_OK;
+    uint32_t bad = 0;
+    EM2_TRY(readFlag(ctx, dFlags, s, &bad));
+    if (bad)
+        return fail(ctx, EM2_ERR_INVALID,
+                    "em2_extend_exact_similar_pairs: the old lists do not belong to these counts or parameters (k, "
+                    "similarityThreshold): " + describeFlags(bad, "these counts"));
+    if (N > oldN) {       // nothing appended: the validated old lists are the result
+        // 2. the appended rows against all columns: their final lists
+        EM2_TRY(exactRect(ctx, o, oldN, N, 0, N, k, similarityThreshold, false, c.pairs + oldN * k, c.used + oldN, s));
+        EM2_CUDA(ctx, cudaStreamSynchronize(s));        // the tile-list staging buffer is reused below
+        // 3. the old rows against the appended columns: each old row's k best new cells, merged with its old list
+        EM2_TRY(exactRect(ctx, o, 0, oldN, oldN, N, k, similarityThreshold, false, dWinPairs, dWinUsed, s));
+        exactMergeKernel<<<unsigned((oldN + kMergeWarps - 1) / kMergeWarps), kMergeWarps * 32, 0, s>>>(
+            oldN, uint32_t(k), dOldPairs, dOldUsed, dWinPairs, dWinUsed, c.pairs, c.used);
+        ctx->stats.kernel_launches++;
+        EM2_CUDA(ctx, cudaGetLastError());
+        ctx->stats.scan_symmetric = 1;
+    }
+    return c.finish(pairs, usedCount);
 }
 
-int launchRescoreExact(em2_context* ctx, uint64_t N, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
-                       const double* sum1, const double* sum2, uint64_t width, const em2_pair* candidates,
-                       const uint32_t* candidateCount, uint64_t k, double similarityThreshold, uint32_t* flags, em2_pair* pairs,
-                       uint32_t* usedCount, cudaStream_t s, uint32_t* badFlags)
+// Each cell's k best candidates by the similarity em2_exact_similar_pairs stores (exactRescoreKernel).
+int em2_rescore_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
+                              const em2_count* counts, uint64_t candidateWidth, const em2_pair* candidates,
+                              const uint32_t* candidateCount, uint64_t k, double similarityThreshold, em2_pair* pairs,
+                              uint32_t* usedCount)
 {
-    *badFlags = 0;
+    EM2_TRY(guardDevice(ctx));
+    const uint64_t N = cellCount, width = candidateWidth;
+    if (!toc || !pairs || !usedCount || !candidates || !candidateCount || (!counts && N && toc[N]))
+        return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: null pointer");
     EM2_TRY(checkExactArguments(ctx, N, geneCount, k, similarityThreshold));
-    // the arithmetic of the full job over all N cells; only the variance term is needed besides the sums
-    ExactArith arith;
-    EM2_TRY(exactArithmetic(ctx, N, geneCount, toc, counts, sum2, s, &arith));
+    if (width == 0 || width > 1024) return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: candidateWidth must be in [1, 1024]");
+    const size_t candBytes = N * width * sizeof(em2_pair), candUsedBytes = N * sizeof(uint32_t);
+    if (outputsOverlap(pairs, N * k * sizeof(em2_pair), usedCount, N * sizeof(uint32_t), candidates, candBytes, candidateCount,
+                       candUsedBytes))
+        return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: the output buffers overlap the candidates");
+    for (uint64_t a = 0; a < N; a++)
+        if (candidateCount[a] > width)
+            return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: candidateCount[" + std::to_string(a) + "] exceeds candidateWidth");
+    ExactCall c(ctx, N, geneCount);
+    if (N == 0) return EM2_OK;
+    cudaStream_t s = c.s;
+    // [candidates N * width][candidateCount N][flags 4]
+    void* dCand = nullptr;
+    EM2_TRY(reserve(ctx, em2_context::S_EXTEND, candBytes + candUsedBytes + 16, &dCand));
+    auto* dCandUsed = reinterpret_cast<uint32_t*>(static_cast<em2_pair*>(dCand) + N * width);
+    uint32_t* dFlags = dCandUsed + N;
+    EM2_TRY(c.stage(toc, counts, k));
+    EM2_TRY(c.input(dCand, candidates, candBytes));
+    EM2_TRY(c.input(dCandUsed, candidateCount, candUsedBytes));
+    EM2_TRY(c.sums());
+    // only the variance term is needed besides the sums
     ExactOperands o;
-    EM2_TRY(exactPrepare(ctx, arith, N, geneCount, toc, counts, sum1, sum2, false, s, &o));
-    ctx->stats.variant_used = exactVariant(arith);
+    EM2_TRY(c.operands(false, &o));
 
     uint32_t sortSize = 32;
     while (sortSize < width) sortSize <<= 1;
     const size_t keyBytes = size_t(sortSize) * sizeof(uint64_t);
-    const size_t denseBytes = geneCount * (arith.general ? sizeof(float) : sizeof(uint16_t));
+    const size_t denseBytes = geneCount * (o.arith.general ? sizeof(float) : sizeof(uint16_t));
     const bool dense = keyBytes + denseBytes + 1024 <= size_t(ctx->prop.sharedMemPerBlockOptin);   // always on the general path
     const size_t smem = keyBytes + (dense ? denseBytes : 0);
-    auto kernel = arith.general ? exactRescoreKernel<true, true> : dense ? exactRescoreKernel<false, true> : exactRescoreKernel<false, false>;
+    auto kernel = o.arith.general ? exactRescoreKernel<true, true> : dense ? exactRescoreKernel<false, true> : exactRescoreKernel<false, false>;
     EM2_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     int perSm = 0;
     EM2_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, kernel, kRescoreWarps * 32, smem));
     if (perSm < 1) return fail(ctx, EM2_ERR_CUDA, "no CTA of the rescoring kernel fits on this device");
     const unsigned grid = unsigned(std::min<uint64_t>(N, uint64_t(perSm) * ctx->smCount));
-    EM2_CUDA(ctx, cudaMemsetAsync(flags, 0, sizeof(uint32_t), s));
-    kernel<<<grid, kRescoreWarps * 32, smem, s>>>(N, geneCount, toc, counts, sum1, o.var, similarityThreshold, uint32_t(width), sortSize,
-                                                  candidates, candidateCount, uint32_t(k), pairs, usedCount, flags);
+    EM2_CUDA(ctx, cudaMemsetAsync(dFlags, 0, sizeof(uint32_t), s));
+    kernel<<<grid, kRescoreWarps * 32, smem, s>>>(N, geneCount, c.toc, c.counts, c.sum1, o.var, similarityThreshold, uint32_t(width),
+                                                  sortSize, static_cast<em2_pair*>(dCand), dCandUsed, uint32_t(k), c.pairs, c.used, dFlags);
     ctx->stats.kernel_launches++;
     EM2_CUDA(ctx, cudaGetLastError());
-    void* pin = nullptr;
-    EM2_TRY(reservePinned(ctx, 2, 64, &pin));
-    EM2_CUDA(ctx, cudaMemcpyAsync(pin, flags, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    *badFlags = *static_cast<uint32_t*>(pin);
-    return EM2_OK;
+    uint32_t bad = 0;
+    EM2_TRY(readFlag(ctx, dFlags, s, &bad));
+    if (bad) {
+        std::string what;
+        if (bad & kRescoreBadId) what += "; a candidate id is not below cellCount";
+        if (bad & kRescoreBadSelf) what += "; a row lists its own cell";
+        if (bad & kRescoreBadDuplicate) what += "; a row lists a candidate twice";
+        return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: invalid candidate lists: " + what.substr(2));
+    }
+    return c.finish(pairs, usedCount);
 }
 
-}  // namespace em2
+}  // extern "C"

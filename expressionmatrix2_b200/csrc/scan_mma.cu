@@ -1637,7 +1637,7 @@ struct SymJob {
     uint64_t* outbox = nullptr;        // the filed log: every column cell's inbox, in position order
     void* cubTemp = nullptr;
     size_t cubBytes = 0, cubBytesShard = 0;   // exclusive scans of N + 1 and of shard + 1 counts
-    void* pinned = nullptr;    // the overflow flag's read-back; the multi-GPU size matrix (world x (world + 1) entries)
+    void* pinned = nullptr;    // pinned[2], also readFlag's: the multi-GPU size matrix (world x (world + 1) entries)
 
     SymJob(const em2_context* ctx, uint64_t k)
         : pair(ctx->symCtaPair != 1 && ctx->smCount >= 2), rowsPerItem(pair ? kPairRows : kRowsPerItem),
@@ -1785,10 +1785,9 @@ struct SymJob {
     // After the merge: the overflow flag decides whether the result stands
     int readOverflow(em2_context* ctx, cudaStream_t s, int* overflowed)
     {
-        uint32_t* host = static_cast<uint32_t*>(pinned);
-        EM2_CUDA(ctx, cudaMemcpyAsync(host, p.overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-        EM2_CUDA(ctx, cudaStreamSynchronize(s));
-        *overflowed = int(*host);
+        uint32_t flag = 0;
+        EM2_TRY(readFlag(ctx, p.overflow, s, &flag));
+        *overflowed = int(flag);
         return EM2_OK;
     }
 };

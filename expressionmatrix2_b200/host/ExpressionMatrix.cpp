@@ -47,6 +47,24 @@ std::ostream& timestamp(std::ostream& s)
     return s << out;
 }
 
+// Creates SimilarPairs-<name>, lets fill(payload, usedCounts) write its lists, then records the used counts.  On any exception
+// the object is removed again: no empty but valid-looking SimilarPairs-<name> set stays behind a failed call.
+template <class Fill>
+void createSimilarPairs(const std::string& directoryName, const std::string& name, const std::string& geneSetName,
+                        const std::string& cellSetName, size_t k, size_t cellCount, Fill fill)
+{
+    static_assert(sizeof(SimilarPairs::Pair) == sizeof(em2_pair), "pair<CellId,float> must be 8 bytes");
+    SimilarPairs similarPairs(directoryName, name, geneSetName, cellSetName, k);
+    std::vector<uint32_t> used(cellCount);
+    try {
+        fill(reinterpret_cast<em2_pair*>(similarPairs.begin(0)), used.data());
+    } catch (...) {
+        similarPairs.remove();
+        throw;
+    }
+    similarPairs.setUsedCounts(used);
+}
+
 bool startsWith(const std::string& s, const std::string& p) { return s.compare(0, p.size(), p) == 0; }
 bool endsWith(const std::string& s, const std::string& p)
 {
@@ -183,26 +201,17 @@ void ExpressionMatrix::findSimilarPairs4(std::ostream& out, const std::string& g
     GpuSet& gpu = GpuSet::instance();      // throws without a device: before anything is written to the data directory
 
     out << timestamp << "Initializing SimilarPairs object." << std::endl;
-    SimilarPairs similarPairs(directoryName, similarPairsName, geneSetName, cellSetName, k);
-
-    out << timestamp << "Expression matrix subset, LSH signatures and all cell pairs on " << gpu.name() << "." << std::endl;
     static_assert(sizeof(std::pair<GeneId, float>) == sizeof(em2_count), "pair<GeneId,float> must be 8 bytes");
-    static_assert(sizeof(SimilarPairs::Pair) == sizeof(em2_pair), "pair<CellId,float> must be 8 bytes");
-    std::vector<uint32_t> used(n);
-    try {
+    createSimilarPairs(directoryName, similarPairsName, geneSetName, cellSetName, k, n, [&](em2_pair* pairs, uint32_t* used) {
+        out << timestamp << "Expression matrix subset, LSH signatures and all cell pairs on " << gpu.name() << "." << std::endl;
         // every GPU copies its cells' rows out of the mapped CellExpressionCounts file and writes its rows of the result
         // straight into the mapped SimilarPairs-<name>-Pairs payload (both through the library's pinned bounce buffers)
         gpu.check(em2_multi_lsh_similar_pairs_subset(gpu.handle(), cellExpressionCounts.size(), cellExpressionCounts.tocBegin(),
                                                      reinterpret_cast<const em2_count*>(cellExpressionCounts.dataBegin()), geneCount(),
                                                      localIds.data(), geneSet.size(), n, cellSet.begin(), lshVectors.data(), lshCount, k,
-                                                     similarityThreshold, scanVariant,
-                                                     reinterpret_cast<em2_pair*>(similarPairs.begin(0)), used.data(), nullptr),
+                                                     similarityThreshold, scanVariant, pairs, used, nullptr),
                   "em2_multi_lsh_similar_pairs_subset");
-    } catch (...) {
-        similarPairs.remove();      // no empty but valid-looking SimilarPairs-<name> set stays behind a failed call
-        throw;
-    }
-    similarPairs.setUsedCounts(used);
+    });
     const em2_stats st = gpu.stats();
     lastSignatureMs = st.signatures_ms;
     lastScanMs = st.scan_ms;
@@ -239,20 +248,15 @@ void ExpressionMatrix::extendSimilarPairs4(const std::string& oldName, const std
     ExpressionMatrixSubset subset(directoryName + "/tmp-ExpressionMatrixSubset-" + newName, geneSet, cellSet, cellExpressionCounts);
     Lsh lsh(directoryName + "/tmp-Lsh-" + newName, subset, lshCount, seed);
     lastSignatureMs = gpu.stats().signatures_ms;
-    std::vector<uint32_t> oldUsed(oldCount), used(n);
+    std::vector<uint32_t> oldUsed(oldCount);
     for (CellId c = 0; c < oldCount; c++) oldUsed[c] = uint32_t(oldPairs.size(c));
     try {
-        SimilarPairs similarPairs(directoryName, newName, geneSetName, cellSetName, k);
-        try {
+        createSimilarPairs(directoryName, newName, geneSetName, cellSetName, k, n, [&](em2_pair* pairs, uint32_t* used) {
             gpu.check(em2_extend_similar_pairs(gpu.context(), lsh.getSignature(0).begin, oldCount, n, lshCount, k, similarityThreshold,
-                                               scanVariant, reinterpret_cast<const em2_pair*>(oldPairs.begin(0)), oldUsed.data(),
-                                               reinterpret_cast<em2_pair*>(similarPairs.begin(0)), used.data()),
+                                               scanVariant, reinterpret_cast<const em2_pair*>(oldPairs.begin(0)), oldUsed.data(), pairs,
+                                               used),
                       "em2_extend_similar_pairs");
-        } catch (...) {
-            similarPairs.remove();      // no valid-looking SimilarPairs-<new> set stays behind a failed call
-            throw;
-        }
-        similarPairs.setUsedCounts(used);
+        });
     } catch (...) {
         lsh.remove();
         throw;
@@ -309,22 +313,15 @@ void ExpressionMatrix::findSimilarPairs0(std::ostream& out, const std::string& g
     const GeneSet& geneSet = findGeneSet(geneSetName);
     const CellSet& cellSet = findCellSet(cellSetName);
     Gpu& gpu = Gpu::instance();            // throws without a device: before anything is written to the data directory
-    SimilarPairs similarPairs(directoryName, similarPairsName, geneSetName, cellSetName, k);
     ExpressionMatrixSubset subset(directoryName + "/tmp-ExpressionMatrixSubset-" + similarPairsName, geneSet, cellSet,
                                   cellExpressionCounts);
     out << timestamp << "Begin computing similarities for all cell pairs." << std::endl;
     const size_t n = subset.cellCount();
-    std::vector<uint32_t> used(n);
-    try {
+    createSimilarPairs(directoryName, similarPairsName, geneSetName, cellSetName, k, n, [&](em2_pair* pairs, uint32_t* used) {
         gpu.check(em2_exact_similar_pairs(gpu.context(), n, subset.geneCount(), subset.toc(),
-                                          reinterpret_cast<const em2_count*>(subset.data()), k, similarityThreshold,
-                                          reinterpret_cast<em2_pair*>(similarPairs.begin(0)), used.data()),
+                                          reinterpret_cast<const em2_count*>(subset.data()), k, similarityThreshold, pairs, used),
                   "em2_exact_similar_pairs");
-    } catch (...) {
-        similarPairs.remove();
-        throw;
-    }
-    similarPairs.setUsedCounts(used);
+    });
     lastScanMs = gpu.stats().scan_ms;
     out << "Time for all pairs: " << 1e-3 * lastScanMs << " s." << std::endl;
     if (n > 1) out << "Time per pair: " << 1e-3 * lastScanMs / (0.5 * double(n) * double(n - 1)) << " s." << std::endl;
@@ -353,20 +350,14 @@ void ExpressionMatrix::extendSimilarPairs0(const std::string& oldName, const std
     // the grown cell set's counts, as findSimilarPairs0 builds them (a temporary file, removed when `subset` goes away)
     ExpressionMatrixSubset subset(directoryName + "/tmp-ExpressionMatrixSubset-" + newName, geneSet, cellSet, cellExpressionCounts);
     const size_t n = subset.cellCount();
-    std::vector<uint32_t> oldUsed(oldCount), used(n);
+    std::vector<uint32_t> oldUsed(oldCount);
     for (CellId c = 0; c < oldCount; c++) oldUsed[c] = uint32_t(oldPairs.size(c));
-    SimilarPairs similarPairs(directoryName, newName, geneSetName, cellSetName, k);
-    try {
+    createSimilarPairs(directoryName, newName, geneSetName, cellSetName, k, n, [&](em2_pair* pairs, uint32_t* used) {
         gpu.check(em2_extend_exact_similar_pairs(gpu.context(), oldCount, n, subset.geneCount(), subset.toc(),
                                                  reinterpret_cast<const em2_count*>(subset.data()), k, similarityThreshold,
-                                                 reinterpret_cast<const em2_pair*>(oldPairs.begin(0)), oldUsed.data(),
-                                                 reinterpret_cast<em2_pair*>(similarPairs.begin(0)), used.data()),
+                                                 reinterpret_cast<const em2_pair*>(oldPairs.begin(0)), oldUsed.data(), pairs, used),
                   "em2_extend_exact_similar_pairs");
-    } catch (...) {
-        similarPairs.remove();      // no valid-looking SimilarPairs-<new> set stays behind a failed call
-        throw;
-    }
-    similarPairs.setUsedCounts(used);
+    });
     lastScanMs = gpu.stats().scan_ms;
 }
 
@@ -386,19 +377,14 @@ void ExpressionMatrix::rescoreSimilarPairs(const std::string& name, const std::s
 
     // the counts of the source's gene set x cell set, as findSimilarPairs0 builds them (a temporary file unless in place)
     ExpressionMatrixSubset subset(directoryName + "/tmp-ExpressionMatrixSubset-" + newName, geneSet, cellSet, cellExpressionCounts);
-    std::vector<uint32_t> candidateCount(n), used(n);
+    std::vector<uint32_t> candidateCount(n);
     for (CellId c = 0; c < n; c++) candidateCount[c] = uint32_t(source.size(c));
-    SimilarPairs similarPairs(directoryName, newName, geneSetName, cellSetName, k);
-    try {
+    createSimilarPairs(directoryName, newName, geneSetName, cellSetName, k, n, [&](em2_pair* pairs, uint32_t* used) {
         gpu.check(em2_rescore_similar_pairs(gpu.context(), n, subset.geneCount(), subset.toc(),
                                             reinterpret_cast<const em2_count*>(subset.data()), source.k(),
                                             reinterpret_cast<const em2_pair*>(source.begin(0)), candidateCount.data(), k,
-                                            similarityThreshold, reinterpret_cast<em2_pair*>(similarPairs.begin(0)), used.data()),
+                                            similarityThreshold, pairs, used),
                   "em2_rescore_similar_pairs");
-    } catch (...) {
-        similarPairs.remove();      // no valid-looking SimilarPairs-<new> set stays behind a failed call
-        throw;
-    }
-    similarPairs.setUsedCounts(used);
+    });
     lastScanMs = gpu.stats().scan_ms;
 }

@@ -106,6 +106,32 @@ def test_pageable_and_pinned_callers_agree(engine, oracle):
     _check_lists((np.ascontiguousarray(o["cell"]), np.ascontiguousarray(o["similarity"]), used.numpy().view(np.uint32)), base)
 
 
+def test_pageable_and_pinned_callers_agree_exact(engine):
+    """The same staging for em2_exact_similar_pairs: pageable buffers through the bounce buffers, pinned ones and
+    option "no_bounce" straight to the driver.  Same lists either way."""
+    import torch
+    N, G, k, thr = 2500, 700, 15, 0.2
+    toc, genes, counts, _ = _job(N, G, 64, seed=8)
+    pairs = em2.to_pairs(genes, counts)
+    base = engine.exact_similar_pairs(toc, pairs, G, k, thr)
+    assert engine.stats()["bounced_bytes"] >= pairs.nbytes
+    engine.set_option("no_bounce", 1)
+    try:
+        _check_lists(engine.exact_similar_pairs(toc, pairs, G, k, thr), base)
+        assert engine.stats()["bounced_bytes"] == 0
+    finally:
+        engine.set_option("no_bounce", 0)
+    p_toc = torch.from_numpy(toc.view(np.int64)).pin_memory()
+    p_pairs = torch.from_numpy(pairs.view(np.int64)).pin_memory()
+    out = torch.zeros((N, k, 2), dtype=torch.int32).pin_memory()
+    used = torch.zeros(N, dtype=torch.int32).pin_memory()
+    o = out.numpy().view(em2.SIMPAIR_DTYPE).reshape(N, k)
+    engine.exact_similar_pairs_into(p_toc.numpy().view(np.uint64), p_pairs.numpy().view(em2.PAIR_DTYPE), G, k, thr, o,
+                                    used.numpy().view(np.uint32))
+    assert engine.stats()["bounced_bytes"] == 0
+    _check_lists((np.ascontiguousarray(o["cell"]), np.ascontiguousarray(o["similarity"]), used.numpy().view(np.uint32)), base)
+
+
 @pytest.mark.parametrize("N,L,k,thr,clusters", [
     (5000, 1024, 50, 0.2, 12),      # symmetric-eligible whole-matrix job (tcgen05, K <= 1024)
     (2049, 1024, 20, -1.0, 0),      # ragged: rank 1 owns 1 + 1024 ... cells, no threshold

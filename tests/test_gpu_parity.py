@@ -376,6 +376,8 @@ def test_exact_path_general_counts(engine, oracle):
     bad = np.array([0, 2, 4], np.uint64), np.array([0, 1, 0, 9], np.uint32), np.array([1.5, 2, 3, 4], np.float32)
     with pytest.raises(em2.Em2Error):                                           # gene id 9 >= geneCount 2: malformed input
         engine.exact_similar_pairs(bad[0], bad[2], 2, 1, 0.0, gene_ids=bad[1])
+    with pytest.raises(em2.Em2Error, match="k must be"):                        # k is checked first, with no cells too
+        engine.exact_similar_pairs(np.zeros(1, np.uint64), np.zeros(0, np.float32), 2, 0, 0.0, gene_ids=np.zeros(0, np.uint32))
 
 
 # ---------------------------------------------------------------------------------------------------
