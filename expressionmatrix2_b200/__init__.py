@@ -433,6 +433,10 @@ class Engine:
                     "em2_exact_similar_pairs")
 
     def exact_similar_pairs(self, toc, counts, gene_count: int, k: int, similarity_threshold: float, gene_ids=None):
+        """findSimilarPairs0 (em2_exact_similar_pairs): each cell's k best others by Pearson r > similarity_threshold,
+        (similarity desc, id asc).  Integer counts in [0, 65535] use the integer tensor-core path; any other counts the general
+        arithmetic at any gene_count, through the tensor-core candidate filter when every count is non-negative (stats:
+        filter_cells, filter_uncertain, candidates_appended).  Returns (ids, sims, used)."""
         toc = np.ascontiguousarray(toc, np.uint64)
         pairs = _as_pairs(counts, gene_ids)
         n = len(toc) - 1
@@ -450,7 +454,7 @@ class Engine:
         Returns (ids, sims, used) for all rows, equal to exact_similar_pairs over all cells.  Raises Em2Error if the old lists
         do not belong to these counts, k and threshold.  Lists made with a HIGHER threshold than this call's cannot be
         detected (their rows lack the cells between the two thresholds) and give wrong lists; lists made with a lower
-        threshold are rejected or are already exact."""
+        threshold are rejected or are already exact.  Any gene_count, as exact_similar_pairs, with the same filter stats."""
         toc = np.ascontiguousarray(toc, np.uint64)
         pairs = _as_pairs(counts, gene_ids)
         n = len(toc) - 1
@@ -467,8 +471,8 @@ class Engine:
         """Exact rescoring of candidate lists (em2_rescore_similar_pairs): cand_ids [N, width] with cand_used [N] entries
         used per row, e.g. the ids of any *_similar_pairs result; their order within a row is free.  Returns (ids, sims, used)
         with each row's k best candidates by the similarity exact_similar_pairs stores for the pair (desc, then id asc) among
-        those above similarity_threshold.  Raises Em2Error on an id >= N, a row's own id, an id listed twice in a row, or
-        cand_used above the width."""
+        those above similarity_threshold, at any gene_count.  Raises Em2Error on an id >= N, a row's own id, an id listed twice
+        in a row, or cand_used above the width."""
         toc = np.ascontiguousarray(toc, np.uint64)
         pairs = _as_pairs(counts, gene_ids)
         n = len(toc) - 1

@@ -470,6 +470,8 @@ int em2_set_option(em2_context* ctx, const char* name, int64_t value)
     else if (n == "filter_counts_signed" && value >= 0 && value <= 1) ctx->filterCountsSigned = int(value);
     else if (n == "h2d_chunk_bytes" && value >= 0) ctx->h2dChunkBytes = uint64_t(value);
     else if (n == "exact_general" && value >= 0 && value <= 1) ctx->exactGeneral = int(value);
+    else if (n == "exact_filter" && value >= 0 && value <= 1) ctx->exactFilter = int(value);
+    else if (n == "exact_filter_cap" && value >= 0 && value <= 8192) ctx->exactFilterCap = uint32_t(value);
     else if (n == "exact_cta_pair" && value >= 0 && value <= 1) ctx->exactCtaPair = int(value);
     else if (n == "filter_parts" && value >= 0 && value <= 64) ctx->filterParts = int(value);
     else if (n == "filter_cta_pair" && value >= 0 && value <= 1) ctx->filterCtaPair = int(value);

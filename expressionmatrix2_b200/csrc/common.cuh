@@ -65,6 +65,8 @@ struct em2_context {
         S_DIST0, S_DIST1, S_DIST2, S_DIST3,   // multi-GPU exchange buffers (multi.cu)
         S_PERM,          // scan position -> cell id
         S_EXTEND,        // the caller's input lists of the call in progress (old lists or candidates) and what the call keeps with them
+        S_XCAND,         // exact path, general arithmetic: the filter's candidate lists of a row chunk, their counts, the overflow rows, counters
+        S_XROWS,         // exact path, general arithmetic: dense rows of the full evaluation when shared memory cannot hold them
         S_COUNT
     };
     int signatureMode = 0;   // 0 auto, 1 FP64 kernel only, 2 force the tensor-core filter path
@@ -73,6 +75,8 @@ struct em2_context {
     uint64_t exactMatrixBytes = 0;     // test knob: budget of the exact path's similarity matrix (0 = 8 GiB)
     uint64_t h2dChunkBytes = 0;        // test knob: CSR bytes per PCIe chunk of the blocking API (0 = 256 MiB)
     int exactGeneral = 0;              // 1: force the general FP64 kernel of the exact path (tests)
+    int exactFilter = 0;               // 1: general-arithmetic exact jobs evaluate every row in full instead of through the filter
+    uint32_t exactFilterCap = 0;       // candidate width per row of the exact path's filter (0 = max(1024, 2k))
     int exactCtaPair = 0;              // 1: the one-digit exact GEMM runs on CTA pairs (cta_group::2, M = 256)
     int filterParts = 0;               // test knob: chunks per filter call (0 = automatic)
     int filterCtaPair = 0;             // filter GEMM: 0 = CTA pairs (cta_group::2, M = 256), 1 = one CTA per tile

@@ -14,7 +14,8 @@
 // LL, HL+LH and HH in TMEM, and the epilogue recombines them as 65536 HH + 256 (HL+LH) + LL in double --
 // the same value the reference's merge loop produces while every product x_a*x_b is below 2^24 (counts <=
 // 4095; above that the reference rounds each product to float and agreement is to ~1e-7 relative; counts that
-// are not integers in [0, 65535] take exactGeneralKernel below).  The
+// are not integers in [0, 65535] take the general arithmetic below: the same GEMM on quantised counts as a candidate
+// filter, then exactRescoreKernel on each row's candidates).  The
 // epilogue then evaluates r with the reference's operation sequence (separate multiplies, subtract, sqrt,
 // divide, round-to-nearest doubles) and stores float(r) -- or a "rejected" marker when !(r > threshold) --
 // into a rows x N float matrix in HBM (the whole matrix when it fits: then only tiles on or above the diagonal are
@@ -25,6 +26,12 @@
 // warp 5 MMA issuer; tile 128 x 128 cells, K = genes in 128-byte chunks, both operands are row blocks of the
 // SAME dense planes (128B-swizzled TMA boxes).  Tiles are visited in 12 x 12 super-tiles so that the ~148
 // CTAs running at any moment share 24 row/column panels through L2 instead of streaming 148 distinct ones.
+//
+// General arithmetic (exactGeneralKernel's bits) on non-negative counts: each cell's counts as u16 fixed point with a per-cell
+// power-of-two scale (exactQuantizeKernel), the two-digit GEMM with an epilogue that stores r estimated from the exact integer
+// product and rejects only pairs whose rigorous upper bound cannot pass the threshold (filterHalfWidth), a per-row candidate
+// selection (exactFilterSelectKernel) and the exact decision on those candidates (exactRescoreKernel).  Rows with too many
+// candidates, and jobs the filter does not serve, are evaluated in full (exactFullRect).  DESIGN.md section 4.3d.
 //
 // The file ends with the exact path's three blocking calls, which share their host-side set-up (ExactCall):
 // em2_exact_similar_pairs (the full job), em2_extend_exact_similar_pairs (a job's lists extended to appended cells with the
@@ -66,7 +73,7 @@ __device__ __forceinline__ double pearsonR(double numerator, double va, double v
 // max count, integrality, max sum2, max nnz: decides the digit count on the host.
 __global__ void exactScanKernel(uint64_t cellCount, uint64_t geneCount, const uint64_t* __restrict__ toc,
                                 const em2_count* __restrict__ counts, const double* __restrict__ sum2,
-                                unsigned long long* __restrict__ out /* [0]=max count, [1]=bad flag, [2]=max sum2 bits, [3]=max nnz */)
+                                unsigned long long* __restrict__ out /* [0]=max count, [1]=bad flags, [2]=max sum2 bits, [3]=max nnz */)
 {
     const uint64_t nnz = toc[cellCount];
     uint32_t mx = 0, bad = 0;
@@ -74,7 +81,10 @@ __global__ void exactScanKernel(uint64_t cellCount, uint64_t geneCount, const ui
         const em2_count p = counts[e];
         const float c = p.count;
         if (p.gene >= geneCount) bad |= 2;                                         // malformed input
-        else if (!(c >= 0.f) || c > 65535.f || c != truncf(c)) bad |= 1;           // not a small integer: general path
+        else if (!(c >= 0.f) || c > 65535.f || c != truncf(c)) {                    // not a small integer: general path
+            bad |= 1;
+            if (!(c >= 0.f) || isinf(c)) bad |= 4;                                   // not a finite non-negative value: no filter
+        }
         else mx = max(mx, uint32_t(c));
     }
     double s2 = 0.;
@@ -132,6 +142,124 @@ exactDensifyKernel(uint64_t cellCount, uint64_t geneCount, uint64_t gPad, const 
     }
 }
 
+// ---- candidate filter of the general arithmetic (non-negative counts) --------------------------------------------------
+// Per cell a: x = 2^e (q + eta) with q = rint(x / 2^e) an integer in [0, 32767] and |eta| <= 1/2, e the smallest exponent that
+// keeps the largest q at or below 32767 (so hi digits are <= 127 and HH, HL + LH and LL each grow by at most 65025 per gene:
+// the s32 bound of the integer path, 65025 * maxNnz < 2^31, covers all three accumulators).  The GEMM gives P = sum q_a q_b
+// exactly, S^ = 2^(e_a + e_b) P, and r^ = (n S^ - s1a s1b) w_a w_b with w = 1 / sqrt(var).  With R = sqrt(sum x^2),
+// d = 2^(e-1) the largest |x - 2^e q|, and per-cell terms normalised by sqrt(n) w:
+//     rho = sqrt(n) R w,   mu = sqrt(n) w sqrt(nnz) (d + 2^-74),   sigma = s1 w,
+// |r_general(a,b) - r^(a,b)| <= filterHalfWidth(a, b) (DESIGN.md section 4.3d): quantisation (Cauchy-Schwarz:
+// rho_a mu_b + rho_b mu_a + mu_a mu_b, with 2^-74 covering float products that fall into the subnormal range), the general
+// arithmetic's float products and double sums (kSumErr rho_a rho_b while nnz < 33025), and the double operations of both
+// evaluations (kOpsErr (rho_a rho_b + sigma_a sigma_b)); the factor 1 + 2^-30 covers the rounding of the terms themselves.
+// Every product in it pairs an a-term with the same b-term, so the half-width and r^ are bitwise symmetric in (a, b).
+// The derivation takes every float product of the general arithmetic to be finite: with all counts of both cells below 2^64,
+// x_a x_b < 2^128 (1 - 2^-24) = FLT_MAX.  A cell with a larger count is kCellOdd.
+struct FilterCell {
+    double scale;     // 2^e
+    double w;         // 1 / sqrt(var)
+    double rho, mu, sigma;
+    uint32_t kind;    // kCell*
+};
+enum : uint32_t {
+    kCellNormal = 0,
+    kCellNever = 1,   // every stored count is 0: var = 0 and r = NaN against every cell, never stored
+    kCellOdd = 2,     // a non-zero count and no usable bound -- var <= 0 or not finite, or a count >= 2^64, whose float product with
+                      // a count of the same size overflows: its row is evaluated in full, as a column it is always a candidate
+};
+constexpr double kSumErr = 0x1p-24 + 0x1p-40;
+constexpr double kOpsErr = 0x1p-44;
+constexpr float kAlways = __builtin_huge_valf();   // stored instead of r^: no usable bound, the pair is always a candidate
+
+__device__ __forceinline__ double filterHalfWidth(const FilterCell& A, const FilterCell& B)
+{
+    const double rr = A.rho * B.rho;
+    const double e = (kSumErr + kOpsErr) * rr + (A.rho * B.mu + B.rho * A.mu) + A.mu * B.mu + kOpsErr * (A.sigma * B.sigma);
+    return e * (1. + 0x1p-30);
+}
+
+// The float the filter GEMM stores for (a, b): float(r^), kRejected when the upper bound r^ + E cannot pass the threshold,
+// kAlways when no bound applies.  P: the exact integer product of the quantised counts.
+__device__ __forceinline__ float filterEstimate(const FilterCell& A, const FilterCell& B, double P, double n, double s1a, double s1b,
+                                                double threshold)
+{
+    if (A.kind == kCellNever || B.kind == kCellNever) return kRejected;
+    if (A.kind != kCellNormal || B.kind != kCellNormal) return kAlways;
+    const double rHat = pearsonNumerator(n, P * (A.scale * B.scale), s1a, s1b) * (A.w * B.w);
+    const double e = filterHalfWidth(A, B);
+    if (!(rHat + e >= threshold)) return kRejected;     // r_general <= r^ + E <= threshold (NaN: rejected too)
+    const float f = float(rHat);
+    return f > kRejected && f < kAlways && e < 1e300 ? f : kAlways;
+}
+
+// [lo, hi] with lo <= r_general(a, b) <= hi, both as doubles, from the stored float f (its own rounding included).
+__device__ __forceinline__ void filterBounds(float f, const FilterCell& A, const FilterCell& B, double& lo, double& hi)
+{
+    if (f == kAlways) {
+        lo = -double(kAlways);
+        hi = double(kAlways);
+        return;
+    }
+    const double e = filterHalfWidth(A, B) + 0x1p-23 * fabs(double(f)) + 0x1p-50;
+    lo = double(f) - e;
+    hi = double(f) + e;
+}
+
+// One warp per cell: the quantised counts as two u8 digit planes (lo / hi, [cellCount][gPad], zero where nothing is stored)
+// and the cell's FilterCell.  var: exactDensifyKernel's variance term.
+__global__ void __launch_bounds__(256)
+exactQuantizeKernel(uint64_t cellCount, uint64_t geneCount, uint64_t gPad, const uint64_t* __restrict__ toc,
+                    const em2_count* __restrict__ counts, const double* __restrict__ sum1, const double* __restrict__ var,
+                    uint8_t* __restrict__ lo, uint8_t* __restrict__ hi, FilterCell* __restrict__ cells)
+{
+    const uint64_t cell = blockIdx.x * uint64_t(blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (cell >= cellCount) return;
+    const uint64_t begin = toc[cell], end = toc[cell + 1];
+    float mx = 0.f;
+    double sq = 0.;
+    for (uint64_t e = begin + lane; e < end; e += 32) {
+        const float x = counts[e].count;
+        mx = fmaxf(mx, x);
+        sq += double(x) * double(x);       // exact products, non-negative terms
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+        sq += __shfl_xor_sync(0xffffffffu, sq, o);
+    }
+    int ex = mx > 0.f ? ilogbf(mx) - 14 : 0;                  // mx / 2^ex in [16384, 32768)
+    if (mx > 0.f && rintf(scalbnf(mx, -ex)) > 32767.f) ex++;
+    const uint4 z = make_uint4(0, 0, 0, 0);
+    for (uint64_t o = uint64_t(lane) * 16; o < gPad; o += 512) {
+        *reinterpret_cast<uint4*>(lo + cell * gPad + o) = z;
+        *reinterpret_cast<uint4*>(hi + cell * gPad + o) = z;
+    }
+    __syncwarp();
+    for (uint64_t e = begin + lane; e < end; e += 32) {
+        const em2_count p = counts[e];
+        const uint32_t q = uint32_t(rintf(scalbnf(p.count, -ex)));     // exact scaling, round to nearest: |x - 2^ex q| <= 2^(ex-1)
+        lo[cell * gPad + p.gene] = uint8_t(q & 255u);
+        hi[cell * gPad + p.gene] = uint8_t(q >> 8);
+    }
+    if (lane == 0) {
+        FilterCell c;
+        const double n = double(geneCount), v = var[cell], rootN = sqrt(n);
+        c.scale = ldexp(1., ex);
+        c.w = 1. / sqrt(v);
+        c.rho = rootN * sqrt(sq) * c.w;
+        c.mu = rootN * c.w * sqrt(double(end - begin)) * (ldexp(1., ex - 1) + 0x1p-74);
+        c.sigma = sum1[cell] * c.w;
+        if (!(mx > 0.f)) c.kind = kCellNever;
+        else if (!(mx < 0x1p64f) || !(v > 0.) || !(v < 1e300) || !(c.w > 0.) || !(c.rho < 1e150) || !(c.mu < 1e150) ||
+                 !(c.sigma < 1e150))
+            c.kind = kCellOdd;
+        else c.kind = kCellNormal;
+        cells[cell] = c;
+    }
+}
+
 struct ExactParams {
     uint64_t cellCount;          // end of the column window (N for whole-matrix calls)
     uint64_t colBegin;           // first column of the window: column j of the output is cell colBegin + j
@@ -151,6 +279,7 @@ struct ExactParams {
     const float* rinv;
     float thresholdLow;          // float(threshold) - 1e-4: below this the float estimate of r rejects outright
     float* out;
+    const FilterCell* cells;     // filter epilogue (general arithmetic): per-cell scale and bound terms
 };
 
 // The work list is built on the host: only the tiles that are needed (symmetric mode drops those below the diagonal),
@@ -167,7 +296,9 @@ __device__ __forceinline__ bool itemToTile(const ExactParams& p, uint32_t item, 
     return true;
 }
 
-template <int DIGITS, bool PAIR>
+// FILTER (two digits): the epilogue stores filterEstimate instead of r (general arithmetic's candidate filter); the main loop
+// is the same.
+template <int DIGITS, bool PAIR, bool FILTER = false>
 __global__ void __launch_bounds__(kXThreads, 1)
 exactGemmKernel(const __grid_constant__ CUtensorMap mapLo, const __grid_constant__ CUtensorMap mapHi, const ExactParams p)
 {
@@ -181,6 +312,7 @@ exactGemmKernel(const __grid_constant__ CUtensorMap mapLo, const __grid_constant
     // is short of operand bandwidth, not of tensor throughput (a third of its loads miss L2 and, with ~200 KB in
     // flight per SM, DRAM latency caps a 128 x 256 tile at ~50 % of the tensor peak).
     static_assert(!PAIR || DIGITS == 1, "the CTA-pair form exists for one digit plane");
+    static_assert(!FILTER || (DIGITS == 2 && !PAIR), "the filter epilogue runs on two digit planes");
     constexpr uint32_t kBLoadBytes = PAIR ? kBPlaneBytes / 2 : kBPlaneBytes;
     constexpr int kStages = PAIR ? 6 : DIGITS == 1 ? 4 : 3;
     constexpr uint32_t kStageBytes = DIGITS * (kXPlaneBytes + kBLoadBytes);       // A planes then B planes
@@ -323,7 +455,9 @@ exactGemmKernel(const __grid_constant__ CUtensorMap mapLo, const __grid_constant
             const bool valid = localRow < p.rows;
             const uint64_t a = p.rowBegin + (valid ? localRow : 0);
             const double s1a = p.sum1[a], va = p.var[a];
-            const float rinvA = p.rinv[a];
+            const float rinvA = FILTER ? 0.f : p.rinv[a];
+            FilterCell cellA;
+            if constexpr (FILTER) cellA = p.cells[a];
             const uint32_t buf = tileIter % kAccBufs;
             const uint32_t use = tileIter / kAccBufs;
             mbarWait(accFull + buf, use & 1);
@@ -358,13 +492,17 @@ exactGemmKernel(const __grid_constant__ CUtensorMap mapLo, const __grid_constant
                         if (b < p.cellCount && b != a) {
                             double sp = double(ll[j]);                                        // u8 x u8 sums are non-negative
                             if (DIGITS == 2) sp = fma(fma(double(hh[j]), 256., double(xx[j])), 256., sp);   // exact
-                            const double num = pearsonNumerator(n, sp, s1a, __ldg(p.sum1 + b));
-                            // float estimate of r (relative error < 1e-6, |r| <= 1): only candidates within
-                            // 1e-4 of the threshold or above it pay for the exact double sqrt and divide
-                            const float estimate = float(num) * rinvA * __ldg(p.rinv + b);
-                            if (!(estimate < p.thresholdLow)) {
-                                const double r = pearsonR(num, va, __ldg(p.var + b));
-                                if (r > p.threshold) res = float(r);
+                            if constexpr (FILTER) {
+                                res = filterEstimate(cellA, p.cells[b], sp, n, s1a, __ldg(p.sum1 + b), p.threshold);
+                            } else {
+                                const double num = pearsonNumerator(n, sp, s1a, __ldg(p.sum1 + b));
+                                // float estimate of r (relative error < 1e-6, |r| <= 1): only candidates within
+                                // 1e-4 of the threshold or above it pay for the exact double sqrt and divide
+                                const float estimate = float(num) * rinvA * __ldg(p.rinv + b);
+                                if (!(estimate < p.thresholdLow)) {
+                                    const double r = pearsonR(num, va, __ldg(p.var + b));
+                                    if (r > p.threshold) res = float(r);
+                                }
                             }
                         }
                         r4[jj] = res;
@@ -404,36 +542,41 @@ exactGemmKernel(const __grid_constant__ CUtensorMap mapLo, const __grid_constant
     }
 }
 
-// ---- general counts (non-integer, negative, or too large for the digit planes) ------------------------------
+// ---- general counts (non-integer, negative, or too large for the digit planes): full evaluation -----------------------
 // The reference's arithmetic directly: scalar product = sum over shared genes of float(x_a * x_b) accumulated in
 // double (src/ExpressionMatrixSubset.cpp:95-112), here with the partial sums of 32 lanes combined in double, so the
 // result can differ from the sequential sum in the last bits of the double (never more than ~1e-15 relative;
-// tests allow 1e-6 on the stored float).  A CTA keeps TWO query rows as dense float vectors in shared memory;
-// each of its 8 warps walks other cells' stored counts 32 at a time.  Every CTA streams the whole CSR through L2, so
-// the kernel is L2-bandwidth bound: 7.2 s at 50k cells x 20k genes (the tensor-core path: 35 ms; the reference: 8437 s)
-// -- the fallback for normalised data, not the fast path.
+// tests allow 1e-6 on the stored float).  A CTA keeps TWO query rows as dense float vectors -- in shared memory
+// (SHARED, up to 25,600 genes) or in its own slice of denseG [gridDim.x][2][gPad] -- and each of its 8 warps walks
+// other cells' stored counts 32 at a time.  Every CTA streams the whole CSR through L2, so the kernel is L2-bandwidth
+// bound: 12.2 s at 50k cells x 20k genes of log1p counts when it evaluates every row (the reference: 8437 s); exactRect's
+// filter path uses it (through exactFullRect) only for the rows it cannot decide and for jobs it does not serve.
+// Output row i (of `rows`) is cell rowBegin + rowList[i], or rowBegin + i without a list.
 constexpr int kGenWarps = 8;
 
+template <bool SHARED>
 __global__ void __launch_bounds__(kGenWarps * 32)
 exactGeneralKernel(uint64_t colBegin, uint64_t colEnd, uint64_t geneCount, uint64_t gPad, uint64_t rowBegin, uint64_t rows,
-                   const uint64_t* __restrict__ toc, const em2_count* __restrict__ counts, const double* __restrict__ sum1,
-                   const double* __restrict__ var, double threshold, uint64_t ldOut, float* __restrict__ out)
+                   const uint32_t* __restrict__ rowList, float* __restrict__ denseG, const uint64_t* __restrict__ toc,
+                   const em2_count* __restrict__ counts, const double* __restrict__ sum1, const double* __restrict__ var,
+                   double threshold, uint64_t ldOut, float* __restrict__ out)
 {
-    extern __shared__ __align__(16) float dense[];      // [2][gPad]
+    extern __shared__ __align__(16) float denseS[];      // [2][gPad] (SHARED)
+    float* dense = SHARED ? denseS : denseG + uint64_t(blockIdx.x) * 2 * gPad;
     const uint64_t local0 = uint64_t(blockIdx.x) * 2;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (uint64_t i = threadIdx.x; i < 2 * gPad; i += blockDim.x) dense[i] = 0.f;
     __syncthreads();
+    const bool has1 = local0 + 1 < rows;
+    const uint64_t a0 = rowBegin + (rowList ? rowList[local0] : local0);
+    const uint64_t a1 = has1 ? rowBegin + (rowList ? rowList[local0 + 1] : local0 + 1) : a0;
     for (int r = 0; r < 2; r++) {
-        const uint64_t lr = local0 + r;
-        if (lr >= rows) continue;
-        const uint64_t a = rowBegin + lr;
+        if (r == 1 && !has1) continue;
+        const uint64_t a = r == 0 ? a0 : a1;
         for (uint64_t e = toc[a] + threadIdx.x; e < toc[a + 1]; e += blockDim.x) dense[r * gPad + counts[e].gene] = counts[e].count;
     }
     __syncthreads();
     const double n = double(geneCount);
-    const uint64_t a0 = rowBegin + local0, a1 = a0 + 1;
-    const bool has1 = local0 + 1 < rows;
     const double s1a0 = sum1[a0], va0 = var[a0];
     const double s1a1 = has1 ? sum1[a1] : 0., va1 = has1 ? var[a1] : 0.;
     for (uint64_t b = colBegin + warp; b < colEnd; b += kGenWarps) {
@@ -486,10 +629,11 @@ constexpr em2_pair kEmptyPair{0u, 0.f};     // an unused slot of a list
 constexpr int kSelWarps = 4;
 
 // One warp per row: stream the row, keep keys below the running bound in a shared-memory buffer, prune the
-// buffer to its k smallest keys (rank by counting; keys are unique) whenever it is nearly full.
+// buffer to its k smallest keys (rank by counting; keys are unique) whenever it is nearly full.  Row i of sim goes to list
+// rowList[i] of pairs / usedCount, or to list i without a row list.
 __global__ void __launch_bounds__(kSelWarps * 32)
 exactSelectKernel(uint64_t rows, uint64_t cellCount, uint64_t ldOut, const float* __restrict__ sim, uint32_t k,
-                  uint32_t cap, em2_pair* __restrict__ pairs, uint32_t* __restrict__ usedCount)
+                  uint32_t cap, const uint32_t* __restrict__ rowList, em2_pair* __restrict__ pairs, uint32_t* __restrict__ usedCount)
 {
     extern __shared__ __align__(16) uint64_t sbuf[];        // kSelWarps x 2 x cap
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -535,8 +679,100 @@ exactSelectKernel(uint64_t rows, uint64_t cellCount, uint64_t ldOut, const float
         }
     }
     prune();
-    for (uint32_t e = lane; e < k; e += 32) pairs[row * k + e] = e < count ? keyPair(buf[e]) : kEmptyPair;
-    if (lane == 0) usedCount[row] = count;
+    const uint64_t dst = rowList ? rowList[row] : row;
+    for (uint32_t e = lane; e < k; e += 32) pairs[dst * k + e] = e < count ? keyPair(buf[e]) : kEmptyPair;
+    if (lane == 0) usedCount[dst] = count;
+}
+
+// Candidate selection of the filter path: one warp per row of a chunk of filterEstimate values (row i is cell rowBegin + i,
+// column j cell colBegin + j).  Pass 1: T = the k-th largest float(lo) among the columns with lo > threshold (those surely
+// pass), keys as exactSelectKernel's; -inf when fewer than k columns surely pass.  Pass 2: the columns with hi >= threshold
+// and float(hi) >= T go to the row's candidate list (ids relative to colBegin).  float() is monotone, so every column of the
+// row's true top-k -- final float F >= T, ties broken by id -- has float(hi) >= F >= T.  A row with more than `width`
+// candidates, or whose own cell has no bound (kCellOdd), gets no list: its index (listBase + i) goes to overflowRows for
+// full evaluation.  counters: [0] overflow rows, [1] candidates listed.
+__global__ void __launch_bounds__(kSelWarps * 32)
+exactFilterSelectKernel(uint64_t rows, uint64_t rowBegin, uint64_t cols, uint64_t colBegin, uint64_t ldOut,
+                        const float* __restrict__ sim, const FilterCell* __restrict__ cells, double threshold, uint32_t k,
+                        uint32_t cap, uint32_t width, em2_pair* __restrict__ cand, uint32_t* __restrict__ candUsed,
+                        uint64_t listBase, uint32_t* __restrict__ overflowRows, unsigned long long* __restrict__ counters)
+{
+    extern __shared__ __align__(16) uint64_t sbuf[];        // kSelWarps x 2 x cap
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint64_t row = uint64_t(blockIdx.x) * kSelWarps + warp;
+    if (row >= rows) return;
+    uint64_t* buf = sbuf + size_t(warp) * 2 * cap;
+    uint64_t* tmp = buf + cap;
+    uint32_t count = 0;
+    uint64_t bound = ~0ull;
+    const float* src = sim + row * ldOut;
+    const uint32_t lt = (1u << lane) - 1u;
+    const FilterCell A = cells[rowBegin + row];
+
+    auto prune = [&]() {
+        __syncwarp();
+        for (uint32_t e = lane; e < count; e += 32) {
+            const uint64_t key = buf[e];
+            uint32_t rank = 0;
+            for (uint32_t f = 0; f < count; f++) rank += (buf[f] < key);
+            if (rank < k) tmp[rank] = key;
+        }
+        __syncwarp();
+        const uint32_t kept = count < k ? count : k;
+        for (uint32_t e = lane; e < kept; e += 32) buf[e] = tmp[e];
+        __syncwarp();
+        count = kept;
+        if (kept == k) bound = buf[k - 1];
+    };
+
+    for (uint64_t base = 0; base < cols; base += 32) {
+        const uint64_t id = base + lane;
+        uint64_t key = ~0ull;
+        if (id < cols) {
+            const float f = __ldg(src + id);
+            if (f != kRejected) {
+                double lo, hi;
+                filterBounds(f, A, cells[colBegin + id], lo, hi);
+                if (lo > threshold) key = sortKey(float(lo), uint32_t(id));
+            }
+        }
+        const bool pass = key < bound;
+        const uint32_t mask = __ballot_sync(0xffffffffu, pass);
+        if (mask) {
+            if (pass) buf[count + __popc(mask & lt)] = key;
+            count += __popc(mask);
+            if (count + 32 > cap) prune();
+        }
+    }
+    prune();
+    const float T = count == k ? fromOrderable(~uint32_t(buf[k - 1] >> 32)) : -kAlways;
+    const bool odd = A.kind == kCellOdd;
+    uint32_t listed = 0;
+    for (uint64_t base = 0; base < cols && !odd && listed <= width; base += 32) {
+        const uint64_t id = base + lane;
+        bool take = false;
+        if (id < cols) {
+            const float f = __ldg(src + id);
+            if (f != kRejected) {
+                double lo, hi;
+                filterBounds(f, A, cells[colBegin + id], lo, hi);
+                take = hi >= threshold && float(hi) >= T;
+            }
+        }
+        const uint32_t mask = __ballot_sync(0xffffffffu, take);
+        const uint32_t at = listed + __popc(mask & lt);
+        if (take && at < width) cand[row * width + at] = em2_pair{uint32_t(id), 0.f};
+        listed += __popc(mask);
+    }
+    if (lane == 0) {
+        if (odd || listed > width) {
+            candUsed[row] = 0;
+            overflowRows[atomicAdd(counters, 1ull)] = uint32_t(listBase + row);
+        } else {
+            candUsed[row] = listed;
+            atomicAdd(counters + 1, (unsigned long long)listed);
+        }
+    }
 }
 
 // ---- extension of old lists to appended cells (em2_extend_exact_similar_pairs) -------------------------------------
@@ -709,10 +945,11 @@ exactMergeKernel(uint64_t oldN, uint32_t k, const em2_pair* __restrict__ oldPair
 }
 
 // ---- rescoring of candidate lists (em2_rescore_similar_pairs) ------------------------------------------------------------
-// A CTA of kRescoreWarps warps takes rows a = blockIdx.x, blockIdx.x + gridDim.x, ...  Row a's counts are scattered into a
-// dense shared-memory row (uint16 per gene on the integer path, where counts are <= 65535; float on the general path) and
-// cleared again afterwards, so a row costs nnz(a), not G.  DENSE == false (integer path, too many genes for that row): a's
-// counts are found by search in its CSR, with the same values.  One warp per candidate b computes r(a, b) with warpPairR, the
+// A CTA of kRescoreWarps warps takes rows i = blockIdx.x, blockIdx.x + gridDim.x, ... of `rows`: cell a = rowBegin + i, whose
+// candidate ids are relative to colBegin (column cells colBegin .. colBegin + cols - 1; the rescoring call has both offsets 0,
+// the filter path passes its rectangle's).  Row a's counts are scattered into a dense shared-memory row (uint16 per gene on
+// the integer path, where counts are <= 65535; float on the general path) and cleared again afterwards, so a row costs nnz(a),
+// not G.  DENSE == false (too many genes for that row): a's counts are found by search in its CSR, with the same values.  One warp per candidate b computes r(a, b) with warpPairR, the
 // float em2_exact_similar_pairs stores in row a.  Keys (~orderable(r) << 32 | b), or (kRescoreReject << 32 | b) when r does
 // not pass the threshold, are sorted in shared memory (bitonic): the passing keys form a prefix, the row is its first k, and
 // a candidate listed twice gives two equal keys, adjacent after the sort.
@@ -725,14 +962,17 @@ enum : uint32_t {
 };
 constexpr uint32_t kRescoreReject = 0xffffffffu;     // above ~orderable(r) for every r in [-1, 1]
 
+// The row and column offsets apply to the general forms only (the filter path's rectangles); the integer forms serve the
+// rescoring call, whose offsets are 0, and compile as without them.  Register caps of the general forms (40 with a dense
+// row, 48 without): no spills.
 template <bool GENERAL, bool DENSE>
-__global__ void __launch_bounds__(kRescoreWarps * 32)
-exactRescoreKernel(uint64_t cellCount, uint64_t geneCount, const uint64_t* __restrict__ toc, const em2_count* __restrict__ counts,
-                   const double* __restrict__ sum1, const double* __restrict__ var, double threshold, uint32_t width,
-                   uint32_t sortSize, const em2_pair* __restrict__ cand, const uint32_t* __restrict__ candUsed, uint32_t k,
-                   em2_pair* __restrict__ pairs, uint32_t* __restrict__ usedCount, uint32_t* __restrict__ flags)
+__global__ void __launch_bounds__(kRescoreWarps * 32, GENERAL ? (DENSE ? 6 : 5) : 0)
+exactRescoreKernel(uint64_t rows, uint64_t rowBegin, uint64_t cols, uint64_t colBegin, uint64_t geneCount,
+                   const uint64_t* __restrict__ toc, const em2_count* __restrict__ counts, const double* __restrict__ sum1,
+                   const double* __restrict__ var, double threshold, uint32_t width, uint32_t sortSize,
+                   const em2_pair* __restrict__ cand, const uint32_t* __restrict__ candUsed, uint32_t k, em2_pair* __restrict__ pairs,
+                   uint32_t* __restrict__ usedCount, uint32_t* __restrict__ flags)
 {
-    static_assert(DENSE || !GENERAL, "the general path always has its dense row (at most 25,600 genes)");
     using Count = std::conditional_t<GENERAL, float, uint16_t>;
     extern __shared__ __align__(16) uint64_t keys[];     // [sortSize] (a power of two >= width), then Count dense[geneCount]
     Count* dense = reinterpret_cast<Count*>(keys + sortSize);
@@ -744,19 +984,21 @@ exactRescoreKernel(uint64_t cellCount, uint64_t geneCount, const uint64_t* __res
         for (uint64_t g = threadIdx.x; g < geneCount; g += blockDim.x) dense[g] = Count(0);
         __syncthreads();
     }
-    for (uint64_t a = blockIdx.x; a < cellCount; a += gridDim.x) {
-        const uint32_t used = candUsed[a];                // <= width (checked on the host)
-        const uint64_t rowBegin = toc[a], rowEnd = toc[a + 1];
+    for (uint64_t row = blockIdx.x; row < rows; row += gridDim.x) {
+        const uint64_t a = GENERAL ? rowBegin + row : row;
+        const uint32_t used = candUsed[row];              // <= width (checked on the host)
+        const uint64_t csrBegin = toc[a], csrEnd = toc[a + 1];
         if constexpr (DENSE)
-            for (uint64_t e = rowBegin + threadIdx.x; e < rowEnd; e += blockDim.x) dense[counts[e].gene] = Count(counts[e].count);
+            for (uint64_t e = csrBegin + threadIdx.x; e < csrEnd; e += blockDim.x) dense[counts[e].gene] = Count(counts[e].count);
         for (uint32_t i = threadIdx.x; i < sortSize; i += blockDim.x) keys[i] = ~0ull;
         if (threadIdx.x == 0) passed = 0;
         __syncthreads();
         const double s1a = sum1[a], va = var[a];
         for (uint32_t i = warp; i < used; i += kRescoreWarps) {
-            const uint32_t b = cand[a * width + i].cell;
-            uint64_t key = (uint64_t(kRescoreReject) << 32) | b;
-            if (b >= cellCount) {
+            const uint32_t id = cand[row * width + i].cell;
+            const uint64_t b = GENERAL ? colBegin + id : id;
+            uint64_t key = (uint64_t(kRescoreReject) << 32) | id;
+            if (id >= cols) {
                 bad |= kRescoreBadId;
             } else if (b == a) {
                 bad |= kRescoreBadSelf;
@@ -764,10 +1006,13 @@ exactRescoreKernel(uint64_t cellCount, uint64_t geneCount, const uint64_t* __res
                 double r;
                 if constexpr (DENSE)
                     r = warpPairR<GENERAL, false>(b, toc, counts, [&](uint32_t g) { return dense[g]; }, n, s1a, va, sum1, var, lane);
+                else if constexpr (GENERAL)
+                    r = warpPairR<true, true>(b, toc, counts, [=](uint32_t g) { return storedCount(toc, counts, a, g); }, n, s1a, va, sum1,
+                                              var, lane);
                 else
                     r = warpPairR<false, true>(b, toc, counts, [=](uint32_t g) { return uint32_t(storedCount(toc, counts, a, g)); }, n, s1a,
                                          va, sum1, var, lane);
-                if (r > threshold) key = sortKey(float(r), b);
+                if (r > threshold) key = sortKey(float(r), id);
             }
             if (lane == 0) keys[i] = key;
         }
@@ -792,10 +1037,10 @@ exactRescoreKernel(uint64_t cellCount, uint64_t geneCount, const uint64_t* __res
         }
         __syncthreads();
         const uint32_t kept = min(passed, k);
-        for (uint32_t e = threadIdx.x; e < k; e += blockDim.x) pairs[a * k + e] = e < kept ? keyPair(keys[e]) : kEmptyPair;
-        if (threadIdx.x == 0) usedCount[a] = kept;
+        for (uint32_t e = threadIdx.x; e < k; e += blockDim.x) pairs[row * k + e] = e < kept ? keyPair(keys[e]) : kEmptyPair;
+        if (threadIdx.x == 0) usedCount[row] = kept;
         if constexpr (DENSE)
-            for (uint64_t e = rowBegin + threadIdx.x; e < rowEnd; e += blockDim.x) dense[counts[e].gene] = Count(0);
+            for (uint64_t e = csrBegin + threadIdx.x; e < csrEnd; e += blockDim.x) dense[counts[e].gene] = Count(0);
         __syncthreads();
     }
     bad = __reduce_or_sync(0xffffffffu, bad);
@@ -811,11 +1056,13 @@ int checkExactArguments(em2_context* ctx, uint64_t cellCount, uint64_t geneCount
     return EM2_OK;
 }
 
-// The arithmetic the exact path uses for a set of cells, decided from all of their counts: the general FP64 kernel, or the
-// integer tensor-core path with one or two digit planes.
+// The arithmetic the exact path uses for a set of cells, decided from all of their counts: the general FP64 arithmetic, or
+// the integer tensor-core path with one or two digit planes.  filter: a general-arithmetic job the candidate filter serves
+// (every count finite and non-negative, the s32 accumulators safe for the longest cell, option "exact_filter" not 1).
 struct ExactArith {
     bool general;
     int digits;
+    bool filter;
 };
 
 int exactArithmetic(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
@@ -839,10 +1086,12 @@ int exactArithmetic(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, co
     // FP64 kernel (exactGeneralKernel); "exact_general" = 1 forces it (tests).
     arith->general = (h[1] & 1) || llBound >= 2147483648. || maxSum2 / 128. >= 2147483648. || ctx->exactGeneral != 0;
     arith->digits = digits;
+    // the filter's quantised counts are <= 32767: each of HH, HL + LH and LL grows by at most 65025 per stored gene
+    arith->filter = arith->general && !(h[1] & 4) && 65025. * double(h[3]) < 2147483648. && ctx->exactFilter != 1;
     return EM2_OK;
 }
 
-// Per-cell operands of all cells for the chosen arithmetic (planes == false: the variance term only, as the general path needs).
+// Per-cell operands of all cells for the chosen arithmetic (planes == false: the variance term only, as the rescoring needs).
 struct ExactOperands {
     ExactArith arith;
     uint64_t cellCount, geneCount, gPad;
@@ -851,7 +1100,8 @@ struct ExactOperands {
     const double* sum1;
     double* var;                 // n * sum2 - sum1^2
     float* rinv;                 // integer path: float reciprocal roots of var (the epilogue's pre-filter)
-    uint8_t *lo, *hi;            // integer path: digit planes [cellCount][gPad] (hi: two digits only)
+    uint8_t *lo, *hi;            // digit planes [cellCount][gPad] (hi: two digits only); the filter's quantised counts
+    FilterCell* cells;           // filter path: per-cell scale and bound terms (null: general rows are evaluated in full)
 };
 
 int exactPrepare(em2_context* ctx, const ExactArith& arith, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
@@ -865,15 +1115,25 @@ int exactPrepare(em2_context* ctx, const ExactArith& arith, uint64_t cellCount, 
     o->toc = toc;
     o->counts = counts;
     o->sum1 = sum1;
-    if (arith.general && 2 * o->gPad * sizeof(float) > 200 * 1024)
-        return fail(ctx, EM2_ERR_INVALID, "em2_exact_similar_pairs: non-integer counts with more than 25,600 genes are not supported");
     if (arith.general || !planes) {
+        const bool filter = planes && arith.filter;
         void* varG = nullptr;
-        EM2_TRY(reserve(ctx, em2_context::S_FLAGS, cellCount * sizeof(double), &varG));
+        EM2_TRY(reserve(ctx, em2_context::S_FLAGS, cellCount * (sizeof(double) + (filter ? sizeof(FilterCell) : 0)), &varG));
         o->var = static_cast<double*>(varG);
         // per-cell variance term (the densify kernel's by-product in the tensor-core path)
         exactDensifyKernel<<<unsigned((cellCount + 7) / 8), 256, 0, s>>>(cellCount, geneCount, 0, toc, counts, sum1, sum2, nullptr,
                                                                         nullptr, o->var, nullptr);
+        ctx->stats.kernel_launches++;
+        EM2_CUDA(ctx, cudaGetLastError());
+        if (!filter) return EM2_OK;
+        // the filter's quantised counts as two digit planes, and the bound's per-cell terms
+        void* lo = nullptr;
+        EM2_TRY(reserve(ctx, em2_context::S_DENSE, cellCount * o->gPad * 2, &lo));
+        o->lo = static_cast<uint8_t*>(lo);
+        o->hi = o->lo + cellCount * o->gPad;
+        o->cells = reinterpret_cast<FilterCell*>(o->var + cellCount);
+        exactQuantizeKernel<<<unsigned((cellCount + 7) / 8), 256, 0, s>>>(cellCount, geneCount, o->gPad, toc, counts, sum1, o->var, o->lo,
+                                                                         o->hi, o->cells);
         ctx->stats.kernel_launches++;
         EM2_CUDA(ctx, cudaGetLastError());
         return EM2_OK;
@@ -893,45 +1153,75 @@ int exactPrepare(em2_context* ctx, const ExactArith& arith, uint64_t cellCount, 
     return EM2_OK;
 }
 
+// Full evaluation with the general arithmetic: rows rowBegin + rowList[i] (i < rowCount), or rowBegin + i without a list, against
+// the column window [colBegin, colEnd), each row's k best into list rowList[i] (or i) of pairs / usedCount, ids relative to colBegin.
+// Rows go in chunks under the similarity-matrix budget; when two dense float rows do not fit in shared memory (more than 25,600
+// genes) they live in global scratch, at most 4 GiB of it per chunk.
+int exactFullRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint64_t rowCount, const uint32_t* rowList,
+                  uint64_t colBegin, uint64_t colEnd, uint64_t k, double similarityThreshold, em2_pair* pairs, uint32_t* usedCount,
+                  cudaStream_t s)
+{
+    const uint64_t cols = colEnd - colBegin, gPad = o.gPad;
+    if (rowCount == 0 || cols == 0) return EM2_OK;
+    const uint64_t budget = ctx->exactMatrixBytes ? ctx->exactMatrixBytes : (48ull << 30);
+    const uint64_t ldG = roundUp(cols, 256);
+    uint64_t chunkG = std::max<uint64_t>(2, budget / (ldG * sizeof(float)) / 2 * 2);
+    const size_t smemG = 2 * gPad * sizeof(float);
+    const bool shared = smemG <= 200 * 1024;
+    if (!shared) chunkG = std::min<uint64_t>(chunkG, std::max<uint64_t>(2, (4ull << 30) / smemG * 2));
+    chunkG = std::min<uint64_t>(chunkG, roundUp(rowCount, 2));
+    void *simG = nullptr, *denseG = nullptr;
+    EM2_TRY(reserve(ctx, em2_context::S_CAND, chunkG * ldG * sizeof(float), &simG));
+    if (!shared) EM2_TRY(reserve(ctx, em2_context::S_XROWS, chunkG / 2 * smemG, &denseG));
+    if (shared) EM2_CUDA(ctx, cudaFuncSetAttribute(exactGeneralKernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemG)));
+    const uint32_t capG = uint32_t(2 * k + 64);
+    const size_t smemSelG = size_t(kSelWarps) * 2 * capG * sizeof(uint64_t);
+    EM2_CUDA(ctx, cudaFuncSetAttribute(exactSelectKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemSelG)));
+    for (uint64_t begin = 0; begin < rowCount; begin += chunkG) {
+        const uint64_t rows = std::min(chunkG, rowCount - begin);
+        const uint64_t first = rowList ? rowBegin : rowBegin + begin;
+        const uint32_t* list = rowList ? rowList + begin : nullptr;
+        const unsigned grid = unsigned((rows + 1) / 2);
+        if (shared)
+            exactGeneralKernel<true><<<grid, kGenWarps * 32, smemG, s>>>(colBegin, colEnd, o.geneCount, gPad, first, rows, list, nullptr,
+                                                                         o.toc, o.counts, o.sum1, o.var, similarityThreshold, ldG,
+                                                                         static_cast<float*>(simG));
+        else
+            exactGeneralKernel<false><<<grid, kGenWarps * 32, 0, s>>>(colBegin, colEnd, o.geneCount, gPad, first, rows, list,
+                                                                      static_cast<float*>(denseG), o.toc, o.counts, o.sum1, o.var,
+                                                                      similarityThreshold, ldG, static_cast<float*>(simG));
+        ctx->stats.kernel_launches++;
+        EM2_CUDA(ctx, cudaGetLastError());
+        exactSelectKernel<<<unsigned((rows + kSelWarps - 1) / kSelWarps), kSelWarps * 32, smemSelG, s>>>(
+            rows, cols, ldG, static_cast<const float*>(simG), uint32_t(k), capG, list, rowList ? pairs : pairs + begin * k,
+            rowList ? usedCount : usedCount + begin);
+        ctx->stats.kernel_launches++;
+        EM2_CUDA(ctx, cudaGetLastError());
+    }
+    ctx->stats.filter_uncertain += rowCount;
+    return EM2_OK;
+}
+
 // Rows [rowBegin, rowEnd) against the column window [colBegin, colEnd): each row's k best (similarity desc, column asc)
 // among the window's cells other than itself with r > threshold, into pairs / usedCount from the list of row rowBegin on,
 // with ids RELATIVE TO colBegin.  Rows go in chunks under the similarity-matrix budget.  wholeMatrix (all rows against all
 // columns): when the whole N x N matrix fits the budget, only the tiles on or above the diagonal are computed (half the
-// MMAs) and mirrored.
+// MMAs) and mirrored.  General arithmetic: through the candidate filter when the operands have its terms (o.cells), the
+// rows it cannot decide and every row otherwise evaluated in full (exactFullRect).  Stats (added up over the calls of one
+// job): filter_cells = rows decided through the filter, filter_uncertain = rows evaluated in full, candidates_appended =
+// pairs the filter's rows recomputed exactly.
 int exactRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint64_t rowEnd, uint64_t colBegin, uint64_t colEnd,
               uint64_t k, double similarityThreshold, bool wholeMatrix, em2_pair* pairs, uint32_t* usedCount, cudaStream_t s)
 {
     const uint64_t rowCount = rowEnd - rowBegin, cols = colEnd - colBegin, gPad = o.gPad;
     if (rowCount == 0 || cols == 0) return EM2_OK;
     const uint64_t budget = ctx->exactMatrixBytes ? ctx->exactMatrixBytes : (48ull << 30);
-    if (o.arith.general) {
-        const uint64_t ldG = roundUp(cols, 256);
-        uint64_t chunkG = std::max<uint64_t>(2, budget / (ldG * sizeof(float)) / 2 * 2);
-        chunkG = std::min<uint64_t>(chunkG, roundUp(rowCount, 2));
-        void* simG = nullptr;
-        EM2_TRY(reserve(ctx, em2_context::S_CAND, chunkG * ldG * sizeof(float), &simG));
-        const size_t smemG = 2 * gPad * sizeof(float);
-        EM2_CUDA(ctx, cudaFuncSetAttribute(exactGeneralKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemG)));
-        const uint32_t capG = uint32_t(2 * k + 64);
-        const size_t smemSelG = size_t(kSelWarps) * 2 * capG * sizeof(uint64_t);
-        EM2_CUDA(ctx, cudaFuncSetAttribute(exactSelectKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemSelG)));
-        for (uint64_t begin = 0; begin < rowCount; begin += chunkG) {
-            const uint64_t rows = std::min(chunkG, rowCount - begin);
-            exactGeneralKernel<<<unsigned((rows + 1) / 2), kGenWarps * 32, smemG, s>>>(
-                colBegin, colEnd, o.geneCount, gPad, rowBegin + begin, rows, o.toc, o.counts, o.sum1, o.var, similarityThreshold,
-                ldG, static_cast<float*>(simG));
-            ctx->stats.kernel_launches++;
-            EM2_CUDA(ctx, cudaGetLastError());
-            exactSelectKernel<<<unsigned((rows + kSelWarps - 1) / kSelWarps), kSelWarps * 32, smemSelG, s>>>(
-                rows, cols, ldG, static_cast<const float*>(simG), uint32_t(k), capG, pairs + begin * k, usedCount + begin);
-            ctx->stats.kernel_launches++;
-            EM2_CUDA(ctx, cudaGetLastError());
-        }
-        return EM2_OK;
-    }
+    if (o.arith.general && !o.cells)
+        return exactFullRect(ctx, o, rowBegin, rowCount, nullptr, colBegin, colEnd, k, similarityThreshold, pairs, usedCount, s);
+    const bool filter = o.arith.general;
 
     // ---- row chunks: GEMM + epilogue into the similarity matrix, then selection --------------------------
-    const int digits = o.arith.digits;
+    const int digits = filter ? 2 : o.arith.digits;
     const uint64_t cellCount = o.cellCount;
     const uint64_t ldOut = roundUp(cols, 256);
     uint64_t chunkRows = std::max<uint64_t>(kXTile, budget / (ldOut * sizeof(float)) / kXTile * kXTile);
@@ -949,7 +1239,40 @@ int exactRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint6
     const size_t smemGemm = 1024 + size_t(stages) * digits * (kXPlaneBytes + size_t(colsPerTile) * kXChunk) + 256;
     const uint32_t cap = uint32_t(2 * k + 64);
     const size_t smemSel = size_t(kSelWarps) * 2 * cap * sizeof(uint64_t);
-    EM2_CUDA(ctx, cudaFuncSetAttribute(exactSelectKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemSel)));
+    EM2_CUDA(ctx, cudaFuncSetAttribute(filter ? (const void*)exactFilterSelectKernel : (const void*)exactSelectKernel,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemSel)));
+
+    // filter: [counters 64 B: overflow rows, candidates, rescoring flags][candidate lists chunkRows x width][their counts]
+    // [overflow rows rowCount]; the candidates are rescored with a dense shared-memory row when it fits (about 41k genes at
+    // the default width), else by search in the row's CSR
+    uint32_t width = 0, sortSize = 32;
+    unsigned long long* counters = nullptr;
+    em2_pair* cand = nullptr;
+    uint32_t *candUsed = nullptr, *overflow = nullptr;
+    size_t smemR = 0;
+    unsigned gridR = 0;
+    auto rescore = exactRescoreKernel<true, true>;
+    if (filter) {
+        width = ctx->exactFilterCap ? ctx->exactFilterCap : uint32_t(std::max<uint64_t>(1024, 2 * k));
+        while (sortSize < width) sortSize <<= 1;
+        void* x = nullptr;
+        EM2_TRY(reserve(ctx, em2_context::S_XCAND, 64 + chunkRows * (width * sizeof(em2_pair) + sizeof(uint32_t)) + rowCount * sizeof(uint32_t),
+                        &x));
+        counters = static_cast<unsigned long long*>(x);
+        cand = reinterpret_cast<em2_pair*>(counters + 8);
+        candUsed = reinterpret_cast<uint32_t*>(cand + chunkRows * width);
+        overflow = candUsed + chunkRows;
+        EM2_CUDA(ctx, cudaMemsetAsync(counters, 0, 64, s));
+        const size_t keyBytes = size_t(sortSize) * sizeof(uint64_t), denseBytes = o.geneCount * sizeof(float);
+        const bool dense = keyBytes + denseBytes + 1024 <= size_t(ctx->prop.sharedMemPerBlockOptin);
+        smemR = keyBytes + (dense ? denseBytes : 0);
+        if (!dense) rescore = exactRescoreKernel<true, false>;
+        EM2_CUDA(ctx, cudaFuncSetAttribute(rescore, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemR)));
+        int perSm = 0;
+        EM2_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, rescore, kRescoreWarps * 32, smemR));
+        if (perSm < 1) return fail(ctx, EM2_ERR_CUDA, "no CTA of the rescoring kernel fits on this device");
+        gridR = unsigned(std::min<uint64_t>(chunkRows, uint64_t(perSm) * ctx->smCount));
+    }
 
     for (uint64_t begin = 0; begin < rowCount; begin += chunkRows) {
         const uint64_t rows = std::min(chunkRows, rowCount - begin);
@@ -999,6 +1322,7 @@ int exactRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint6
         p.rinv = o.rinv;
         p.thresholdLow = float(similarityThreshold) - 1e-4f;
         p.out = static_cast<float*>(simMatrix);
+        p.cells = o.cells;
         if (pair) {
             const size_t smemPair = 1024 + 6 * (kXPlaneBytes + size_t(colsPerTile / 2) * kXChunk) + 256;
             EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemPair)));
@@ -1021,7 +1345,11 @@ int exactRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint6
             EM2_CUDA(ctx, cudaLaunchKernelEx(&cfg, exactGemmKernel<1, true>, mapLo, mapHi, p));
         } else {
             const unsigned grid = unsigned(std::min<uint32_t>(p.items, uint32_t(ctx->smCount)));
-            if (digits == 1) {
+            if (filter) {
+                EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<2, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                   int(smemGemm)));
+                exactGemmKernel<2, false, true><<<grid, kXThreads, smemGemm, s>>>(mapLo, mapHi, p);
+            } else if (digits == 1) {
                 EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemGemm)));
                 exactGemmKernel<1, false><<<grid, kXThreads, smemGemm, s>>>(mapLo, mapHi, p);
             } else {
@@ -1031,12 +1359,31 @@ int exactRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint6
         }
         ctx->stats.kernel_launches++;
         EM2_CUDA(ctx, cudaGetLastError());
-        exactSelectKernel<<<unsigned((rows + kSelWarps - 1) / kSelWarps), kSelWarps * 32, smemSel, s>>>(
-            rows, cols, ldOut, static_cast<const float*>(simMatrix), uint32_t(k), cap, pairs + begin * k, usedCount + begin);
+        const unsigned gridSel = unsigned((rows + kSelWarps - 1) / kSelWarps);
+        if (filter) {
+            exactFilterSelectKernel<<<gridSel, kSelWarps * 32, smemSel, s>>>(
+                rows, rowBegin + begin, cols, colBegin, ldOut, static_cast<const float*>(simMatrix), o.cells, similarityThreshold,
+                uint32_t(k), cap, width, cand, candUsed, begin, overflow, counters);
+            ctx->stats.kernel_launches++;
+            EM2_CUDA(ctx, cudaGetLastError());
+            rescore<<<std::min<unsigned>(gridR, unsigned(rows)), kRescoreWarps * 32, smemR, s>>>(
+                rows, rowBegin + begin, cols, colBegin, o.geneCount, o.toc, o.counts, o.sum1, o.var, similarityThreshold, width, sortSize,
+                cand, candUsed, uint32_t(k), pairs + begin * k, usedCount + begin, reinterpret_cast<uint32_t*>(counters + 2));
+        } else {
+            exactSelectKernel<<<gridSel, kSelWarps * 32, smemSel, s>>>(rows, cols, ldOut, static_cast<const float*>(simMatrix), uint32_t(k),
+                                                                       cap, nullptr, pairs + begin * k, usedCount + begin);
+        }
         ctx->stats.kernel_launches++;
         EM2_CUDA(ctx, cudaGetLastError());
     }
-    return EM2_OK;
+    if (!filter) return EM2_OK;
+    // the rows the filter could not decide (their lists above are empty placeholders): full evaluation
+    unsigned long long h[2];
+    EM2_CUDA(ctx, cudaMemcpyAsync(h, counters, sizeof(h), cudaMemcpyDeviceToHost, s));
+    EM2_CUDA(ctx, cudaStreamSynchronize(s));
+    ctx->stats.filter_cells += rowCount - h[0];
+    ctx->stats.candidates_appended += h[1];
+    return exactFullRect(ctx, o, rowBegin, h[0], overflow, colBegin, colEnd, k, similarityThreshold, pairs, usedCount, s);
 }
 
 int exactVariant(const ExactArith& arith) { return arith.general ? EM2_VARIANT_POPC : EM2_VARIANT_MMA_I8; }   // POPC: "not the tensor-core path"
@@ -1273,17 +1620,19 @@ int em2_rescore_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t gen
     while (sortSize < width) sortSize <<= 1;
     const size_t keyBytes = size_t(sortSize) * sizeof(uint64_t);
     const size_t denseBytes = geneCount * (o.arith.general ? sizeof(float) : sizeof(uint16_t));
-    const bool dense = keyBytes + denseBytes + 1024 <= size_t(ctx->prop.sharedMemPerBlockOptin);   // always on the general path
+    const bool dense = keyBytes + denseBytes + 1024 <= size_t(ctx->prop.sharedMemPerBlockOptin);
     const size_t smem = keyBytes + (dense ? denseBytes : 0);
-    auto kernel = o.arith.general ? exactRescoreKernel<true, true> : dense ? exactRescoreKernel<false, true> : exactRescoreKernel<false, false>;
+    auto kernel = o.arith.general ? (dense ? exactRescoreKernel<true, true> : exactRescoreKernel<true, false>)
+                                  : dense ? exactRescoreKernel<false, true> : exactRescoreKernel<false, false>;
     EM2_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     int perSm = 0;
     EM2_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, kernel, kRescoreWarps * 32, smem));
     if (perSm < 1) return fail(ctx, EM2_ERR_CUDA, "no CTA of the rescoring kernel fits on this device");
     const unsigned grid = unsigned(std::min<uint64_t>(N, uint64_t(perSm) * ctx->smCount));
     EM2_CUDA(ctx, cudaMemsetAsync(dFlags, 0, sizeof(uint32_t), s));
-    kernel<<<grid, kRescoreWarps * 32, smem, s>>>(N, geneCount, c.toc, c.counts, c.sum1, o.var, similarityThreshold, uint32_t(width),
-                                                  sortSize, static_cast<em2_pair*>(dCand), dCandUsed, uint32_t(k), c.pairs, c.used, dFlags);
+    kernel<<<grid, kRescoreWarps * 32, smem, s>>>(N, 0, N, 0, geneCount, c.toc, c.counts, c.sum1, o.var, similarityThreshold,
+                                                  uint32_t(width), sortSize, static_cast<em2_pair*>(dCand), dCandUsed, uint32_t(k), c.pairs,
+                                                  c.used, dFlags);
     ctx->stats.kernel_launches++;
     EM2_CUDA(ctx, cudaGetLastError());
     uint32_t bad = 0;

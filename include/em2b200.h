@@ -134,7 +134,9 @@ int em2_get_stats(const em2_context* ctx, em2_stats* stats);
  *                      most pairs and on large jobs, 5-15 % slower on ~100k densely clustered cells)
  *   "cand_cap_extra"   candidate regions hold (2 + n) k + 32 keys;  "popc_csa" carry-save levels of the POPC scan (0..2)
  *   "exact_matrix_bytes" budget of the exact path's similarity matrix (default 48 GiB);  "exact_cta_pair" 1 = CTA-pair GEMM
- *   "exact_general"    1 = force the exact path's general FP64 kernel
+ *   "exact_general"    1 = force the exact path's general FP64 arithmetic
+ *   "exact_filter"     1 = general-arithmetic exact jobs evaluate every row in full instead of through the candidate filter
+ *   "exact_filter_cap" candidate width per row of that filter (default max(1024, 2k)); rows with more go to full evaluation
  *   "sym_cta_pair"     1 = the symmetric scan runs on single CTAs instead of CTA pairs (cta_group::2, M = 256)
  *   "sym_near_half_width" symmetric scan: super blocks (256 cells) on each side of a row's own that the near window covers
  *                      (0 = automatic: max(16, N / 32 columns in total))
@@ -278,7 +280,14 @@ int em2_find_similar_pairs7(em2_context* ctx, const uint64_t* signatures, uint64
 /* Exact path (findSimilarPairs0, src/ExpressionMatrixFindSimilarPairs.cpp:16-88 with
  * ExpressionMatrixSubset::computeCellSimilarity, src/ExpressionMatrixSubset.cpp:83-133):
  * Pearson correlation over all genes, deterministic top-k by (similarity desc, cellId asc) among
- * pairs with similarity > threshold. */
+ * pairs with similarity > threshold.
+ * Counts that are integers in [0, 65535] take the integer tensor-core path.  All other counts take the general arithmetic
+ * (float products, double sums over 32 lanes and a shuffle tree, then the reference's double operations), at any geneCount.
+ * When every count is finite and non-negative and 65025 * (largest number of stored entries of a cell) < 2^31, a tensor-core
+ * candidate filter serves it: quantised counts, a rigorous bound on r, and each row's candidates recomputed in the general
+ * arithmetic.  Rows with more candidates than option "exact_filter_cap", rows of cells without a usable bound (zero variance,
+ * a count >= 2^64), and every row of other jobs are evaluated in full.  The bits are the same either way.  Stats (general arithmetic): filter_cells = rows decided through the filter, filter_uncertain = rows
+ * evaluated in full, candidates_appended = pairs recomputed exactly; variant_used = EM2_VARIANT_POPC. */
 int em2_exact_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
                             const em2_count* counts, uint64_t k, double similarityThreshold, em2_pair* pairs,
                             uint32_t* usedCount);
@@ -301,7 +310,8 @@ int em2_exact_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneC
  * k best of its old list and its new candidates: about M*(2N+M) pair evaluations instead of (N+M)^2/2 or, once the N x N
  * similarity matrix exceeds option "exact_matrix_bytes", (N+M)^2 (N = oldCellCount, M = cellCount - oldCellCount).
  * Stats: scan_symmetric 1 = that rectangle ran; 0 = the full job (oldCellCount = 0, or the arithmetic differs) or nothing
- * was appended; variant_used as em2_exact_similar_pairs sets it. */
+ * was appended; variant_used, filter_cells, filter_uncertain and candidates_appended as em2_exact_similar_pairs sets them
+ * (added up over the rectangle's two parts).  No gene limit on either arithmetic. */
 int em2_extend_exact_similar_pairs(em2_context* ctx, uint64_t oldCellCount, uint64_t cellCount, uint64_t geneCount,
                                    const uint64_t* toc, const em2_count* counts, uint64_t k, double similarityThreshold,
                                    const em2_pair* oldPairs, const uint32_t* oldUsedCount, em2_pair* pairs, uint32_t* usedCount);
@@ -318,8 +328,10 @@ int em2_extend_exact_similar_pairs(em2_context* ctx, uint64_t oldCellCount, uint
  * operations.  So with every other cell as a candidate the result equals em2_exact_similar_pairs bit for bit, and rescoring
  * its own lists of width k' to k <= k' with the same threshold gives the first k entries of each row.  Only the counts, the
  * candidates, the outputs and per-cell sums live on the device: no digit planes, no similarity matrix.
+ * Any geneCount up to the exact path's limit: a's counts sit in a shared-memory row when it fits, else they are found by
+ * search in a's CSR, with the same values.
  * Returns EM2_ERR_INVALID without writing any output if: an argument or limit of em2_exact_similar_pairs fails (including a
- * stored gene id >= geneCount and the general path's 25,600-gene limit), candidateWidth is not in [1, 1024], a
+ * stored gene id >= geneCount), candidateWidth is not in [1, 1024], a
  * candidateCount exceeds candidateWidth, a candidate id is >= cellCount or equal to its row's cell, a row lists an id twice,
  * or the output buffers overlap the candidates.
  * Stats: h2d/d2h ms and bytes, sums_ms, scan_ms (the rescoring), total_ms, kernel_launches, variant_used as
