@@ -81,6 +81,7 @@ def lib():
     L.em2_exact_similar_pairs.argtypes = [vp, u64, u64, vp, vp, u64, dbl, vp, vp]
     L.em2_extend_exact_similar_pairs.argtypes = [vp, u64, u64, u64, vp, vp, u64, dbl, vp, vp, vp, vp]
     L.em2_rescore_similar_pairs.argtypes = [vp, u64, u64, vp, vp, u64, vp, vp, u64, dbl, vp, vp]
+    L.em2_analyze_lsh.argtypes = [vp, u64, u64, vp, vp, vp, u64, u64, vp, vp, vp, vp, vp]
     L.em2_cell_graph_edges.argtypes = [vp, u64, u64, vp, vp, vp, dbl, u64, vp, u64, vp]
     L.em2_signature_graph.argtypes = [vp, vp, u64, u64, u64, vp, vp, u64, vp, vp, u64, vp]
     L.em2_find_similar_pairs7.argtypes = [vp, vp, u64, u64, u64, dbl, vp, u64, C.c_uint32, u64, vp, vp]
@@ -490,6 +491,30 @@ class Engine:
                                                       _ptr(cand_used), k, similarity_threshold, _ptr(out), _ptr(used)),
                     "em2_rescore_similar_pairs")
         return np.ascontiguousarray(out["cell"]), np.ascontiguousarray(out["similarity"]), used
+
+    def analyze_lsh(self, toc, counts, gene_count: int, signatures, lsh_count: int, bin_count: int = 20, gene_ids=None) -> dict:
+        """LSH accuracy on these cells (em2_analyze_lsh): every pair a < b, its exact similarity r (the float exact_similar_pairs
+        stores for b in row a, no threshold) against its LSH similarity s = float(cos(pi m / L)) from the signatures (uint64
+        [N, W], e.g. compute_signatures), in bin_count equal bins of r over [-1, 1].  Returns a dict of numpy arrays:
+        pair_count uint64 [B], sum_error / sum_squared_error float64 [B] (sums of e = s - r and e^2 per bin), joint uint64 [B, B]
+        (pairs by bin of r, bin of s) and undefined_pairs (pairs with r = NaN, in no bin).  It answers what the reference's
+        analyzeLsh diagnostic answers (RMS error of the LSH estimate per similarity bin against the theoretical sigma), but the
+        reference's output format is not reproduced: its source is not part of this project."""
+        toc = np.ascontiguousarray(toc, np.uint64)
+        pairs = _as_pairs(counts, gene_ids)
+        n = len(toc) - 1
+        sig = np.ascontiguousarray(signatures, np.uint64)
+        if sig.size != n * word_count(lsh_count):
+            raise ValueError("signatures must hold word_count(lsh_count) words per cell")
+        B = int(bin_count)
+        out = {"pair_count": np.zeros(B, np.uint64), "sum_error": np.zeros(B, np.float64),
+               "sum_squared_error": np.zeros(B, np.float64), "joint": np.zeros((B, B), np.uint64)}
+        undefined = C.c_uint64(0)
+        self._check(self._L.em2_analyze_lsh(self._h, n, gene_count, _ptr(toc), _ptr(pairs), _ptr(sig), lsh_count, B,
+                                            _ptr(out["pair_count"]), _ptr(out["sum_error"]), _ptr(out["sum_squared_error"]),
+                                            _ptr(out["joint"]), C.byref(undefined)), "em2_analyze_lsh")
+        out["undefined_pairs"] = np.uint64(undefined.value)
+        return out
 
     # ---- device-resident calls (torch CUDA tensors or raw device pointers) ------------------------
     def cell_sums_device(self, n, d_toc, d_counts, d_sum1, d_sum2=None, stream=None):

@@ -33,9 +33,10 @@
 // selection (exactFilterSelectKernel) and the exact decision on those candidates (exactRescoreKernel).  Rows with too many
 // candidates, and jobs the filter does not serve, are evaluated in full (exactFullRect).  DESIGN.md section 4.3d.
 //
-// The file ends with the exact path's three blocking calls, which share their host-side set-up (ExactCall):
+// The file ends with the exact path's four blocking calls, which share their host-side set-up (ExactCall):
 // em2_exact_similar_pairs (the full job), em2_extend_exact_similar_pairs (a job's lists extended to appended cells with the
-// same kernels) and em2_rescore_similar_pairs (candidate lists rescored with the full job's similarities).
+// same kernels), em2_rescore_similar_pairs (candidate lists rescored with the full job's similarities) and em2_analyze_lsh
+// (every pair's similarity against its LSH estimate, binned: lshAnalysisKernel on the chunks of the similarity matrix).
 #include "common.cuh"
 #include "tc05.cuh"
 
@@ -1047,11 +1048,143 @@ exactRescoreKernel(uint64_t rows, uint64_t rowBegin, uint64_t cols, uint64_t col
     if (lane == 0 && bad) atomicOr(flags, bad);
 }
 
+// ---- LSH accuracy analysis (em2_analyze_lsh) ----------------------------------------------------------------------------
+// Every pair (a, b), b > a, of a similarity-matrix chunk (kRejected: r is NaN) against its LSH similarity s = float(table[m]),
+// m the Hamming distance of the two signatures.  Bins: bin(x) = min(B - 1, max(0, floor((x + 1) * B / 2))) in double, the same
+// operations on the host (the LUT's bin(s)) and in the tests.
+__device__ __forceinline__ uint32_t analysisBin(double x, double halfBins, uint32_t binCount)
+{
+    const double t = floor(__dmul_rn(__dadd_rn(x, 1.), halfBins));
+    return t <= 0. ? 0u : t >= double(binCount - 1) ? binCount - 1 : uint32_t(t);
+}
+
+constexpr int kBinWarps = 8;
+constexpr uint32_t kSigTile = 16;     // signature words per column-tile step
+// One warp per row (rows blockIdx.x * 8 + warp, then + gridDim.x * 8, ...), lanes over its columns b > a, coalesced.  The 32
+// columns' signatures are contiguous: the warp copies them kSigTile words at a time into its shared tile (coalesced; one
+// lane per column would touch 32 cache lines per load) and each lane XORs its column's words with the row's.  A CTA keeps the
+// joint histogram as u32 counts in shared memory (hardware-aggregated increments) and flushes it to the u64 outputs every
+// roundsPerFlush rounds of 8 rows, before a count can overflow.  The sums of e = s - r and e^2 per bin(r) are kept per warp in
+// shared memory without atomics (shared-memory double atomics are compare-and-swap loops): in each step the lanes with the
+// same bin(r) are added up by the lowest of them (__match_any_sync).  lut[m] = {bits of float(table[m]), bin(s)}, copied to
+// shared memory when lutShared.  out: [joint B * B][undefined], sums: [Σe B][Σe² B].
+__global__ void __launch_bounds__(kBinWarps * 32)
+lshAnalysisKernel(uint64_t rows, uint64_t rowBegin, uint64_t colBegin, uint64_t colEnd, uint64_t ldOut, const float* __restrict__ sim,
+                  const uint64_t* __restrict__ sig, uint32_t words, const uint2* __restrict__ lut, uint32_t lutEntries, bool lutShared,
+                  uint32_t binCount, uint32_t roundsPerFlush, unsigned long long* __restrict__ out, double* __restrict__ sums)
+{
+    // [kBinWarps][2][B] sums, [kBinWarps][32] scratch, [kBinWarps][32][kSigTile + 1] column tiles, [B][B] histogram, LUT
+    extern __shared__ __align__(16) double binSums[];
+    double* scratch = binSums + kBinWarps * 2 * binCount;
+    uint64_t* tiles = reinterpret_cast<uint64_t*>(scratch + kBinWarps * 32);
+    uint32_t* hist = reinterpret_cast<uint32_t*>(tiles + kBinWarps * 32 * (kSigTile + 1));
+    uint2* lutS = reinterpret_cast<uint2*>(hist + ((binCount * binCount + 1) & ~1u));
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5, B = binCount;
+    for (uint32_t i = threadIdx.x; i < kBinWarps * 2 * B; i += blockDim.x) binSums[i] = 0.;
+    for (uint32_t i = threadIdx.x; i < B * B; i += blockDim.x) hist[i] = 0u;
+    if (lutShared)
+        for (uint32_t i = threadIdx.x; i < lutEntries; i += blockDim.x) lutS[i] = lut[i];
+    __syncthreads();
+    const uint2* table = lutShared ? lutS : lut;
+    double* mySums = binSums + warp * 2 * B;
+    double* myScratch = scratch + warp * 32;
+    uint64_t* myTile = tiles + warp * 32 * (kSigTile + 1);
+    const double halfBins = 0.5 * double(B);
+    const uint64_t cols = colEnd - colBegin;
+    unsigned long long undefined = 0;
+
+    auto flush = [&]() {
+        __syncthreads();
+        for (uint32_t i = threadIdx.x; i < B * B; i += blockDim.x)
+            if (hist[i]) {
+                atomicAdd(out + i, (unsigned long long)hist[i]);
+                hist[i] = 0u;
+            }
+        for (uint32_t i = threadIdx.x; i < 2 * B; i += blockDim.x) {
+            const uint32_t part = i / B, bin = i % B;
+            double t = 0.;
+            for (int w = 0; w < kBinWarps; w++) {
+                t += binSums[(w * 2 + part) * B + bin];
+                binSums[(w * 2 + part) * B + bin] = 0.;
+            }
+            if (t != 0.) atomicAdd(sums + i, t);
+        }
+        __syncthreads();
+    };
+
+    uint32_t rounds = 0;
+    for (uint64_t r0 = uint64_t(blockIdx.x) * kBinWarps; r0 < rows; r0 += uint64_t(gridDim.x) * kBinWarps) {
+        const uint64_t i = r0 + warp;
+        if (i < rows) {
+            const uint64_t a = rowBegin + i;
+            const uint64_t* sa = sig + a * words;
+            const float* src = sim + i * ldOut;
+            const uint64_t first = a + 1 - colBegin;                  // column of cell a + 1
+            for (uint64_t j0 = first & ~uint64_t(31); j0 < cols; j0 += 32) {
+                const uint64_t j = j0 + lane;
+                const bool has = j >= first && j < cols;
+                const float r = has ? __ldg(src + j) : kRejected;
+                const bool pair = has && r != kRejected;
+                if (has && !pair) undefined++;
+                uint32_t m = 0;
+                const uint64_t* tileSrc = sig + (colBegin + j0) * words;     // the signatures of columns j0 .. j0 + 31
+                for (uint32_t w0 = 0; w0 < words; w0 += kSigTile) {
+                    __syncwarp();
+                    for (uint32_t t = lane; t < 32 * kSigTile; t += 32) {
+                        const uint32_t c = t / kSigTile, w = t % kSigTile;
+                        if (w0 + w < words && j0 + c < cols) myTile[c * (kSigTile + 1) + w] = __ldg(tileSrc + c * words + w0 + w);
+                    }
+                    __syncwarp();
+                    if (pair) {
+                        const uint32_t n = min(kSigTile, words - w0);
+                        for (uint32_t w = 0; w < n; w++) m += __popcll(__ldg(sa + w0 + w) ^ myTile[lane * (kSigTile + 1) + w]);
+                    }
+                }
+                uint32_t key = B;                                     // bin(r), or B: no pair in this lane
+                double e = 0.;
+                if (pair) {
+                    const uint2 t = table[m];
+                    key = analysisBin(double(r), halfBins, B);
+                    atomicAdd(hist + key * B + t.y, 1u);
+                    e = double(__uint_as_float(t.x)) - double(r);
+                }
+                const uint32_t same = __match_any_sync(0xffffffffu, key);
+                myScratch[lane] = e;
+                __syncwarp();
+                if (key < B && lane == uint32_t(__ffs(same) - 1)) {
+                    double se = 0., sq = 0.;
+                    for (uint32_t left = same; left; left &= left - 1) {
+                        const double x = myScratch[__ffs(left) - 1];
+                        se += x;
+                        sq += x * x;
+                    }
+                    mySums[key] += se;
+                    mySums[B + key] += sq;
+                }
+                __syncwarp();
+            }
+        }
+        if (++rounds == roundsPerFlush) {       // the same count in every warp of the CTA
+            flush();
+            rounds = 0;
+        }
+    }
+    flush();
+    if (undefined) atomicAdd(out + B * B, undefined);
+}
+
+// The exact path's size limits.
+int checkExactSize(em2_context* ctx, uint64_t cellCount, uint64_t geneCount)
+{
+    if (cellCount > 0x7fffff00ull || geneCount > 0x7fffff00ull) return fail(ctx, EM2_ERR_INVALID, "matrix too large for the exact path");
+    return EM2_OK;
+}
+
 // The exact path's argument checks: k in [1, 1024], the size limits, similarityThreshold <= 1.
 int checkExactArguments(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, uint64_t k, double similarityThreshold)
 {
     if (k == 0 || k > 1024) return fail(ctx, EM2_ERR_INVALID, "k must be in [1, 1024]");
-    if (cellCount > 0x7fffff00ull || geneCount > 0x7fffff00ull) return fail(ctx, EM2_ERR_INVALID, "matrix too large for the exact path");
+    EM2_TRY(checkExactSize(ctx, cellCount, geneCount));
     if (!(similarityThreshold <= 1.)) return fail(ctx, EM2_ERR_INVALID, "similarityThreshold must be <= 1");   // CZI_ASSERT, FindSimilarPairs.cpp:27
     return EM2_OK;
 }
@@ -1153,27 +1286,189 @@ int exactPrepare(em2_context* ctx, const ExactArith& arith, uint64_t cellCount, 
     return EM2_OK;
 }
 
+// ---- chunks of the similarity matrix -----------------------------------------------------------------------------------
+// A chunk is rows [rowBegin, rowBegin + rows) (or rowBegin + rowList[i]) against the column window [colBegin, colEnd): row i,
+// column j holds the float for cells (row i's cell, colBegin + j), ldOut floats per row, kRejected where r does not pass the
+// threshold (NaN never does) and on the diagonal.  Two producers write chunks: exactGeneralKernel (general arithmetic, every
+// pair in full) and exactGemmKernel (digit planes; with the filter epilogue on the general arithmetic's quantised planes).
+// exactSelectKernel, exactFilterSelectKernel and lshAnalysisKernel consume them.
+uint64_t exactMatrixBudget(const em2_context* ctx) { return ctx->exactMatrixBytes ? ctx->exactMatrixBytes : (48ull << 30); }
+
+// exactGeneralKernel's set-up: two dense float rows per CTA, in shared memory up to 25,600 genes, else in global scratch (at
+// most 4 GiB of it, which caps the rows of a chunk).
+struct GeneralMatrix {
+    bool shared;
+    size_t rowBytes;        // the two dense rows of one CTA
+    uint64_t maxRows;       // rows per chunk (even)
+    float* denseG;
+};
+
+int generalMatrix(em2_context* ctx, const ExactOperands& o, uint64_t chunkRows, GeneralMatrix* g)
+{
+    g->rowBytes = 2 * o.gPad * sizeof(float);
+    g->shared = g->rowBytes <= 200 * 1024;
+    g->maxRows = g->shared ? chunkRows : std::min<uint64_t>(chunkRows, std::max<uint64_t>(2, (4ull << 30) / g->rowBytes * 2));
+    g->denseG = nullptr;
+    if (g->shared) {
+        EM2_CUDA(ctx, cudaFuncSetAttribute(exactGeneralKernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(g->rowBytes)));
+    } else {
+        void* d = nullptr;
+        EM2_TRY(reserve(ctx, em2_context::S_XROWS, g->maxRows / 2 * g->rowBytes, &d));
+        g->denseG = static_cast<float*>(d);
+    }
+    return EM2_OK;
+}
+
+int generalChunk(em2_context* ctx, const ExactOperands& o, const GeneralMatrix& g, uint64_t rowBegin, uint64_t rows,
+                 const uint32_t* rowList, uint64_t colBegin, uint64_t colEnd, double threshold, uint64_t ldOut, float* out, cudaStream_t s)
+{
+    const unsigned grid = unsigned((rows + 1) / 2);
+    if (g.shared)
+        exactGeneralKernel<true><<<grid, kGenWarps * 32, g.rowBytes, s>>>(colBegin, colEnd, o.geneCount, o.gPad, rowBegin, rows, rowList,
+                                                                          nullptr, o.toc, o.counts, o.sum1, o.var, threshold, ldOut, out);
+    else
+        exactGeneralKernel<false><<<grid, kGenWarps * 32, 0, s>>>(colBegin, colEnd, o.geneCount, o.gPad, rowBegin, rows, rowList, g.denseG,
+                                                                  o.toc, o.counts, o.sum1, o.var, threshold, ldOut, out);
+    ctx->stats.kernel_launches++;
+    EM2_CUDA(ctx, cudaGetLastError());
+    return EM2_OK;
+}
+
+// exactGemmKernel's set-up for the operands' arithmetic: two digit planes with the filter epilogue on the general arithmetic,
+// else the integer path's one or two planes.
+struct GemmMatrix {
+    CUtensorMap mapLo, mapHi;
+    int digits;
+    bool filter;
+    uint32_t colsPerTile;
+    size_t smem;
+    uint32_t chunks;        // chunks launched so far: each one's tile list goes through the same pinned staging buffer
+};
+
+int gemmMatrix(em2_context* ctx, const ExactOperands& o, GemmMatrix* g)
+{
+    g->filter = o.arith.general;
+    g->digits = g->filter ? 2 : o.arith.digits;
+    EM2_TRY(makeTensorMapU8(ctx, &g->mapLo, o.lo, o.cellCount, o.gPad, o.gPad, kXTile));
+    // one digit: the second map is the same plane with a 256-row box (the B operand of the N = 256 tiles)
+    EM2_TRY(makeTensorMapU8(ctx, &g->mapHi, g->digits == 2 ? o.hi : o.lo, o.cellCount, o.gPad, o.gPad, g->digits == 2 ? kXTile : 256));
+    g->colsPerTile = g->digits == 1 ? 256 : kXTile;
+    const int stages = g->digits == 1 ? 4 : 3;
+    g->smem = 1024 + size_t(stages) * g->digits * (kXPlaneBytes + size_t(g->colsPerTile) * kXChunk) + 256;
+    g->chunks = 0;
+    return EM2_OK;
+}
+
+// symmetric (rows and columns both all cells): only the tiles on or above the diagonal are computed, and mirrored.
+int gemmChunk(em2_context* ctx, const ExactOperands& o, GemmMatrix& g, uint64_t rowBegin, uint64_t rows, uint64_t colBegin,
+              uint64_t colEnd, uint64_t ldOut, bool symmetric, double threshold, float* out, cudaStream_t s)
+{
+    const uint32_t colsPerTile = g.colsPerTile;
+    ExactParams p{};
+    p.cellCount = colEnd;
+    p.colBegin = colBegin;
+    p.rowBegin = rowBegin;
+    p.rows = rows;
+    p.geneCount = o.geneCount;
+    p.kChunks = uint32_t(o.gPad / kXChunk);
+    const bool pair = g.digits == 1 && ctx->exactCtaPair != 0;
+    p.rowsPerItem = pair ? 2 * kXTile : kXTile;
+    p.rowBlocks = uint32_t((rows + p.rowsPerItem - 1) / p.rowsPerItem);
+    p.colsPerTile = colsPerTile;
+    p.colTiles = uint32_t(ldOut / colsPerTile);
+    const uint32_t superRows = (p.rowBlocks + kXSuper - 1) / kXSuper;
+    p.superCols = (p.colTiles + kXSuper - 1) / kXSuper;
+    p.symmetric = symmetric ? 1 : 0;
+    {
+        // needed tiles in super-tile order (see itemToTile)
+        std::vector<uint2> list;
+        list.reserve(size_t(p.rowBlocks) * p.colTiles / (symmetric ? 2 : 1) + 1024);
+        const uint32_t colBlocksPerTile = colsPerTile / kXTile, rowBlocksPerItem = p.rowsPerItem / kXTile;
+        for (uint32_t sr = 0; sr < superRows; sr++)
+            for (uint32_t sc = 0; sc < p.superCols; sc++)
+                for (uint32_t r = sr * kXSuper; r < std::min<uint32_t>((sr + 1) * kXSuper, p.rowBlocks); r++)
+                    for (uint32_t c = sc * kXSuper; c < std::min<uint32_t>((sc + 1) * kXSuper, p.colTiles); c++) {
+                        // symmetric: needed iff the tile's LAST 128-column block is on or above the FIRST 128-row block
+                        if (symmetric && (c + 1) * colBlocksPerTile - 1 < r * rowBlocksPerItem) continue;
+                        list.push_back(make_uint2(r, c));
+                    }
+        p.items = uint32_t(list.size());
+        void* dList = nullptr;
+        EM2_TRY(reserve(ctx, em2_context::S_ROWPERM, list.size() * sizeof(uint2) + 16, &dList));
+        void* pin = nullptr;
+        if (g.chunks++ > 0) EM2_CUDA(ctx, cudaStreamSynchronize(s));      // the previous chunk's list copy used the same staging
+        EM2_TRY(reservePinned(ctx, 0, list.size() * sizeof(uint2) + 16, &pin));
+        std::memcpy(pin, list.data(), list.size() * sizeof(uint2));
+        EM2_CUDA(ctx, cudaMemcpyAsync(dList, pin, list.size() * sizeof(uint2), cudaMemcpyHostToDevice, s));
+        p.tiles = static_cast<const uint2*>(dList);
+    }
+    p.idesc = instrDescI8(false, false, p.rowsPerItem, colsPerTile);
+    p.ldOut = ldOut;
+    p.threshold = threshold;
+    p.sum1 = o.sum1;
+    p.var = o.var;
+    p.rinv = o.rinv;
+    p.thresholdLow = float(threshold) - 1e-4f;
+    p.out = out;
+    p.cells = o.cells;
+    const size_t smemGemm = g.smem;
+    const CUtensorMap &mapLo = g.mapLo, &mapHi = g.mapHi;
+    if (pair) {
+        const size_t smemPair = 1024 + 6 * (kXPlaneBytes + size_t(colsPerTile / 2) * kXChunk) + 256;
+        EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemPair)));
+        cudaLaunchConfig_t cfg = {};
+        cfg.blockDim = dim3(kXThreads);
+        cfg.dynamicSmemBytes = smemPair;
+        cfg.stream = s;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeClusterDimension;
+        attr[0].val.clusterDim.x = 2;
+        attr[0].val.clusterDim.y = 1;
+        attr[0].val.clusterDim.z = 1;
+        cfg.attrs = attr;
+        cfg.numAttrs = 1;
+        cfg.gridDim = dim3(2 * unsigned(ctx->smCount / 2));
+        int clusters = 0;
+        EM2_CUDA(ctx, cudaOccupancyMaxActiveClusters(&clusters, exactGemmKernel<1, true>, &cfg));
+        if (clusters < 1) return fail(ctx, EM2_ERR_CUDA, "no CTA pair of the exact kernel fits on this device");
+        cfg.gridDim = dim3(2 * std::min<unsigned>(unsigned(clusters), unsigned(ctx->smCount / 2)));
+        EM2_CUDA(ctx, cudaLaunchKernelEx(&cfg, exactGemmKernel<1, true>, mapLo, mapHi, p));
+    } else {
+        const unsigned grid = unsigned(std::min<uint32_t>(p.items, uint32_t(ctx->smCount)));
+        if (g.filter) {
+            EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<2, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               int(smemGemm)));
+            exactGemmKernel<2, false, true><<<grid, kXThreads, smemGemm, s>>>(mapLo, mapHi, p);
+        } else if (g.digits == 1) {
+            EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemGemm)));
+            exactGemmKernel<1, false><<<grid, kXThreads, smemGemm, s>>>(mapLo, mapHi, p);
+        } else {
+            EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemGemm)));
+            exactGemmKernel<2, false><<<grid, kXThreads, smemGemm, s>>>(mapLo, mapHi, p);
+        }
+    }
+    ctx->stats.kernel_launches++;
+    EM2_CUDA(ctx, cudaGetLastError());
+    return EM2_OK;
+}
+
 // Full evaluation with the general arithmetic: rows rowBegin + rowList[i] (i < rowCount), or rowBegin + i without a list, against
 // the column window [colBegin, colEnd), each row's k best into list rowList[i] (or i) of pairs / usedCount, ids relative to colBegin.
-// Rows go in chunks under the similarity-matrix budget; when two dense float rows do not fit in shared memory (more than 25,600
-// genes) they live in global scratch, at most 4 GiB of it per chunk.
+// Rows go in chunks under the similarity-matrix budget.
 int exactFullRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint64_t rowCount, const uint32_t* rowList,
                   uint64_t colBegin, uint64_t colEnd, uint64_t k, double similarityThreshold, em2_pair* pairs, uint32_t* usedCount,
                   cudaStream_t s)
 {
-    const uint64_t cols = colEnd - colBegin, gPad = o.gPad;
+    const uint64_t cols = colEnd - colBegin;
     if (rowCount == 0 || cols == 0) return EM2_OK;
-    const uint64_t budget = ctx->exactMatrixBytes ? ctx->exactMatrixBytes : (48ull << 30);
     const uint64_t ldG = roundUp(cols, 256);
-    uint64_t chunkG = std::max<uint64_t>(2, budget / (ldG * sizeof(float)) / 2 * 2);
-    const size_t smemG = 2 * gPad * sizeof(float);
-    const bool shared = smemG <= 200 * 1024;
-    if (!shared) chunkG = std::min<uint64_t>(chunkG, std::max<uint64_t>(2, (4ull << 30) / smemG * 2));
-    chunkG = std::min<uint64_t>(chunkG, roundUp(rowCount, 2));
-    void *simG = nullptr, *denseG = nullptr;
+    GeneralMatrix g;
+    EM2_TRY(generalMatrix(ctx, o, std::min<uint64_t>(std::max<uint64_t>(2, exactMatrixBudget(ctx) / (ldG * sizeof(float)) / 2 * 2),
+                                                     roundUp(rowCount, 2)),
+                          &g));
+    const uint64_t chunkG = g.maxRows;
+    void* simG = nullptr;
     EM2_TRY(reserve(ctx, em2_context::S_CAND, chunkG * ldG * sizeof(float), &simG));
-    if (!shared) EM2_TRY(reserve(ctx, em2_context::S_XROWS, chunkG / 2 * smemG, &denseG));
-    if (shared) EM2_CUDA(ctx, cudaFuncSetAttribute(exactGeneralKernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemG)));
     const uint32_t capG = uint32_t(2 * k + 64);
     const size_t smemSelG = size_t(kSelWarps) * 2 * capG * sizeof(uint64_t);
     EM2_CUDA(ctx, cudaFuncSetAttribute(exactSelectKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemSelG)));
@@ -1181,17 +1476,7 @@ int exactFullRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, u
         const uint64_t rows = std::min(chunkG, rowCount - begin);
         const uint64_t first = rowList ? rowBegin : rowBegin + begin;
         const uint32_t* list = rowList ? rowList + begin : nullptr;
-        const unsigned grid = unsigned((rows + 1) / 2);
-        if (shared)
-            exactGeneralKernel<true><<<grid, kGenWarps * 32, smemG, s>>>(colBegin, colEnd, o.geneCount, gPad, first, rows, list, nullptr,
-                                                                         o.toc, o.counts, o.sum1, o.var, similarityThreshold, ldG,
-                                                                         static_cast<float*>(simG));
-        else
-            exactGeneralKernel<false><<<grid, kGenWarps * 32, 0, s>>>(colBegin, colEnd, o.geneCount, gPad, first, rows, list,
-                                                                      static_cast<float*>(denseG), o.toc, o.counts, o.sum1, o.var,
-                                                                      similarityThreshold, ldG, static_cast<float*>(simG));
-        ctx->stats.kernel_launches++;
-        EM2_CUDA(ctx, cudaGetLastError());
+        EM2_TRY(generalChunk(ctx, o, g, first, rows, list, colBegin, colEnd, similarityThreshold, ldG, static_cast<float*>(simG), s));
         exactSelectKernel<<<unsigned((rows + kSelWarps - 1) / kSelWarps), kSelWarps * 32, smemSelG, s>>>(
             rows, cols, ldG, static_cast<const float*>(simG), uint32_t(k), capG, list, rowList ? pairs : pairs + begin * k,
             rowList ? usedCount : usedCount + begin);
@@ -1213,30 +1498,21 @@ int exactFullRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, u
 int exactRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint64_t rowEnd, uint64_t colBegin, uint64_t colEnd,
               uint64_t k, double similarityThreshold, bool wholeMatrix, em2_pair* pairs, uint32_t* usedCount, cudaStream_t s)
 {
-    const uint64_t rowCount = rowEnd - rowBegin, cols = colEnd - colBegin, gPad = o.gPad;
+    const uint64_t rowCount = rowEnd - rowBegin, cols = colEnd - colBegin;
     if (rowCount == 0 || cols == 0) return EM2_OK;
-    const uint64_t budget = ctx->exactMatrixBytes ? ctx->exactMatrixBytes : (48ull << 30);
     if (o.arith.general && !o.cells)
         return exactFullRect(ctx, o, rowBegin, rowCount, nullptr, colBegin, colEnd, k, similarityThreshold, pairs, usedCount, s);
     const bool filter = o.arith.general;
 
     // ---- row chunks: GEMM + epilogue into the similarity matrix, then selection --------------------------
-    const int digits = filter ? 2 : o.arith.digits;
-    const uint64_t cellCount = o.cellCount;
     const uint64_t ldOut = roundUp(cols, 256);
-    uint64_t chunkRows = std::max<uint64_t>(kXTile, budget / (ldOut * sizeof(float)) / kXTile * kXTile);
+    uint64_t chunkRows = std::max<uint64_t>(kXTile, exactMatrixBudget(ctx) / (ldOut * sizeof(float)) / kXTile * kXTile);
     chunkRows = std::min<uint64_t>(chunkRows, roundUp(rowCount, kXTile));
-    const bool symmetric = wholeMatrix && chunkRows >= cellCount;
+    const bool symmetric = wholeMatrix && chunkRows >= o.cellCount;
     void* simMatrix = nullptr;
     EM2_TRY(reserve(ctx, em2_context::S_CAND, chunkRows * ldOut * sizeof(float), &simMatrix));
-
-    CUtensorMap mapLo, mapHi;
-    EM2_TRY(makeTensorMapU8(ctx, &mapLo, o.lo, cellCount, gPad, gPad, kXTile));
-    // one digit: the second map is the same plane with a 256-row box (the B operand of the N = 256 tiles)
-    EM2_TRY(makeTensorMapU8(ctx, &mapHi, digits == 2 ? o.hi : o.lo, cellCount, gPad, gPad, digits == 2 ? kXTile : 256));
-    const uint32_t colsPerTile = digits == 1 ? 256 : kXTile;
-    const int stages = digits == 1 ? 4 : 3;
-    const size_t smemGemm = 1024 + size_t(stages) * digits * (kXPlaneBytes + size_t(colsPerTile) * kXChunk) + 256;
+    GemmMatrix gemm;
+    EM2_TRY(gemmMatrix(ctx, o, &gemm));
     const uint32_t cap = uint32_t(2 * k + 64);
     const size_t smemSel = size_t(kSelWarps) * 2 * cap * sizeof(uint64_t);
     EM2_CUDA(ctx, cudaFuncSetAttribute(filter ? (const void*)exactFilterSelectKernel : (const void*)exactSelectKernel,
@@ -1276,89 +1552,8 @@ int exactRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint6
 
     for (uint64_t begin = 0; begin < rowCount; begin += chunkRows) {
         const uint64_t rows = std::min(chunkRows, rowCount - begin);
-        ExactParams p{};
-        p.cellCount = colEnd;
-        p.colBegin = colBegin;
-        p.rowBegin = rowBegin + begin;
-        p.rows = rows;
-        p.geneCount = o.geneCount;
-        p.kChunks = uint32_t(gPad / kXChunk);
-        const bool pair = digits == 1 && ctx->exactCtaPair != 0;
-        p.rowsPerItem = pair ? 2 * kXTile : kXTile;
-        p.rowBlocks = uint32_t((rows + p.rowsPerItem - 1) / p.rowsPerItem);
-        p.colsPerTile = colsPerTile;
-        p.colTiles = uint32_t(ldOut / colsPerTile);
-        const uint32_t superRows = (p.rowBlocks + kXSuper - 1) / kXSuper;
-        p.superCols = (p.colTiles + kXSuper - 1) / kXSuper;
-        p.symmetric = symmetric ? 1 : 0;
-        {
-            // needed tiles in super-tile order (see itemToTile)
-            std::vector<uint2> list;
-            list.reserve(size_t(p.rowBlocks) * p.colTiles / (symmetric ? 2 : 1) + 1024);
-            const uint32_t colBlocksPerTile = colsPerTile / kXTile, rowBlocksPerItem = p.rowsPerItem / kXTile;
-            for (uint32_t sr = 0; sr < superRows; sr++)
-                for (uint32_t sc = 0; sc < p.superCols; sc++)
-                    for (uint32_t r = sr * kXSuper; r < std::min<uint32_t>((sr + 1) * kXSuper, p.rowBlocks); r++)
-                        for (uint32_t c = sc * kXSuper; c < std::min<uint32_t>((sc + 1) * kXSuper, p.colTiles); c++) {
-                            // symmetric: needed iff the tile's LAST 128-column block is on or above the FIRST 128-row block
-                            if (symmetric && (c + 1) * colBlocksPerTile - 1 < r * rowBlocksPerItem) continue;
-                            list.push_back(make_uint2(r, c));
-                        }
-            p.items = uint32_t(list.size());
-            void* dList = nullptr;
-            EM2_TRY(reserve(ctx, em2_context::S_ROWPERM, list.size() * sizeof(uint2) + 16, &dList));
-            void* pin = nullptr;
-            if (begin > 0) EM2_CUDA(ctx, cudaStreamSynchronize(s));      // the previous chunk's list copy used the same staging
-            EM2_TRY(reservePinned(ctx, 0, list.size() * sizeof(uint2) + 16, &pin));
-            std::memcpy(pin, list.data(), list.size() * sizeof(uint2));
-            EM2_CUDA(ctx, cudaMemcpyAsync(dList, pin, list.size() * sizeof(uint2), cudaMemcpyHostToDevice, s));
-            p.tiles = static_cast<const uint2*>(dList);
-        }
-        p.idesc = instrDescI8(false, false, p.rowsPerItem, colsPerTile);
-        p.ldOut = ldOut;
-        p.threshold = similarityThreshold;
-        p.sum1 = o.sum1;
-        p.var = o.var;
-        p.rinv = o.rinv;
-        p.thresholdLow = float(similarityThreshold) - 1e-4f;
-        p.out = static_cast<float*>(simMatrix);
-        p.cells = o.cells;
-        if (pair) {
-            const size_t smemPair = 1024 + 6 * (kXPlaneBytes + size_t(colsPerTile / 2) * kXChunk) + 256;
-            EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemPair)));
-            cudaLaunchConfig_t cfg = {};
-            cfg.blockDim = dim3(kXThreads);
-            cfg.dynamicSmemBytes = smemPair;
-            cfg.stream = s;
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeClusterDimension;
-            attr[0].val.clusterDim.x = 2;
-            attr[0].val.clusterDim.y = 1;
-            attr[0].val.clusterDim.z = 1;
-            cfg.attrs = attr;
-            cfg.numAttrs = 1;
-            cfg.gridDim = dim3(2 * unsigned(ctx->smCount / 2));
-            int clusters = 0;
-            EM2_CUDA(ctx, cudaOccupancyMaxActiveClusters(&clusters, exactGemmKernel<1, true>, &cfg));
-            if (clusters < 1) return fail(ctx, EM2_ERR_CUDA, "no CTA pair of the exact kernel fits on this device");
-            cfg.gridDim = dim3(2 * std::min<unsigned>(unsigned(clusters), unsigned(ctx->smCount / 2)));
-            EM2_CUDA(ctx, cudaLaunchKernelEx(&cfg, exactGemmKernel<1, true>, mapLo, mapHi, p));
-        } else {
-            const unsigned grid = unsigned(std::min<uint32_t>(p.items, uint32_t(ctx->smCount)));
-            if (filter) {
-                EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<2, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   int(smemGemm)));
-                exactGemmKernel<2, false, true><<<grid, kXThreads, smemGemm, s>>>(mapLo, mapHi, p);
-            } else if (digits == 1) {
-                EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemGemm)));
-                exactGemmKernel<1, false><<<grid, kXThreads, smemGemm, s>>>(mapLo, mapHi, p);
-            } else {
-                EM2_CUDA(ctx, cudaFuncSetAttribute(exactGemmKernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemGemm)));
-                exactGemmKernel<2, false><<<grid, kXThreads, smemGemm, s>>>(mapLo, mapHi, p);
-            }
-        }
-        ctx->stats.kernel_launches++;
-        EM2_CUDA(ctx, cudaGetLastError());
+        EM2_TRY(gemmChunk(ctx, o, gemm, rowBegin + begin, rows, colBegin, colEnd, ldOut, symmetric, similarityThreshold,
+                          static_cast<float*>(simMatrix), s));
         const unsigned gridSel = unsigned((rows + kSelWarps - 1) / kSelWarps);
         if (filter) {
             exactFilterSelectKernel<<<gridSel, kSelWarps * 32, smemSel, s>>>(
@@ -1446,30 +1641,43 @@ struct ExactCall {
         return EM2_OK;
     }
 
-    // The arithmetic of the full job over all N cells and its per-cell operands (planes: see exactPrepare).
-    int operands(bool planes, ExactOperands* o)
+    // The arithmetic of the full job over all N cells and its per-cell operands (planes: see exactPrepare; filter == false:
+    // general-arithmetic rows are evaluated in full, so the filter's operands are not made).
+    int operands(bool planes, ExactOperands* o, bool filter = true)
     {
         ExactArith arith;
         EM2_TRY(exactArithmetic(ctx, N, geneCount, toc, counts, sum2, s, &arith));
+        arith.filter = arith.filter && filter;
         EM2_TRY(exactPrepare(ctx, arith, N, geneCount, toc, counts, sum1, sum2, planes, s, o));
         ctx->stats.variant_used = exactVariant(arith);
         return EM2_OK;
     }
 
-    int finish(em2_pair* hostPairs, uint32_t* hostUsed)
+    int output(void* dst, const void* src, size_t bytes)
     {
-        const size_t pairBytes = N * k * sizeof(em2_pair), usedBytes = N * sizeof(uint32_t);
-        const int e3 = T.mark();
-        EM2_TRY(stageD2H(ctx, hostPairs, pairs, pairBytes, s));
-        EM2_TRY(stageD2H(ctx, hostUsed, used, usedBytes, s));
+        ctx->stats.d2h_bytes += bytes;
+        return stageD2H(ctx, dst, src, bytes, s);
+    }
+
+    // The end of a call whose outputs were queued with output() after event e3.
+    int close(int e3)
+    {
         const int e4 = T.mark();
         EM2_CUDA(ctx, cudaStreamSynchronize(s));
-        ctx->stats.d2h_bytes += pairBytes + usedBytes;
         ctx->stats.h2d_ms = T.ms(e0, e1);
         ctx->stats.sums_ms = T.ms(e1, e2);
-        ctx->stats.scan_ms = T.ms(e2, e3);
         ctx->stats.d2h_ms = T.ms(e3, e4);
         ctx->stats.total_ms = nowMs() - t0;
+        return EM2_OK;
+    }
+
+    int finish(em2_pair* hostPairs, uint32_t* hostUsed)
+    {
+        const int e3 = T.mark();
+        EM2_TRY(output(hostPairs, pairs, N * k * sizeof(em2_pair)));
+        EM2_TRY(output(hostUsed, used, N * sizeof(uint32_t)));
+        EM2_TRY(close(e3));
+        ctx->stats.scan_ms = T.ms(e2, e3);
         return EM2_OK;
     }
 };
@@ -1645,6 +1853,138 @@ int em2_rescore_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t gen
         return fail(ctx, EM2_ERR_INVALID, "em2_rescore_similar_pairs: invalid candidate lists: " + what.substr(2));
     }
     return c.finish(pairs, usedCount);
+}
+
+// Every pair's r (the full job's float, no threshold) against its LSH similarity, binned by lshAnalysisKernel chunk by chunk.
+// The similarity stage computes the upper triangle only: the symmetric whole-matrix GEMM when the N x N matrix fits the budget,
+// else row chunks [r0, r1) against the column window [r0, N) (GEMM or general kernel), so the diagonal blocks are the only pairs
+// computed twice.
+int em2_analyze_lsh(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
+                    const uint64_t* signatures, uint64_t lshCount, uint64_t binCount, uint64_t* pairCount, double* sumError,
+                    double* sumSquaredError, uint64_t* joint, uint64_t* undefinedPairs)
+{
+    EM2_TRY(guardDevice(ctx));
+    const uint64_t N = cellCount, B = binCount;
+    if (!toc || !pairCount || !sumError || !sumSquaredError || !joint || !undefinedPairs || (!signatures && N) || (!counts && N && toc[N]))
+        return fail(ctx, EM2_ERR_INVALID, "em2_analyze_lsh: null pointer");
+    EM2_TRY(checkExactSize(ctx, N, geneCount));
+    if (B == 0 || B > 128) return fail(ctx, EM2_ERR_INVALID, "em2_analyze_lsh: binCount must be in [1, 128]");
+    if (lshCount == 0 || lshCount > 65535) return fail(ctx, EM2_ERR_INVALID, "em2_analyze_lsh: lshCount must be in [1, 65535]");
+    // a CTA's u32 histogram takes one round of kBinWarps rows of up to N pairs each between two flushes
+    if (uint64_t(kBinWarps) * N > 0xffffffffull) return fail(ctx, EM2_ERR_INVALID, "em2_analyze_lsh: cellCount must be below 2^29");
+    const uint64_t W = wordCount(lshCount);
+    const uint64_t pad = lshCount % 64 ? ~0ull >> (lshCount % 64) : 0;     // bits beyond lshCount in the last word
+    for (uint64_t c = 0; c < N; c++)
+        if (signatures[c * W + W - 1] & pad)
+            return fail(ctx, EM2_ERR_INVALID, "em2_analyze_lsh: signature of cell " + std::to_string(c) + " has bits set beyond lshCount");
+
+    ExactCall c(ctx, N, geneCount);
+    const size_t histBytes = (B * B + 1) * sizeof(uint64_t), sumBytes = 2 * B * sizeof(double);
+    if (N == 0) {
+        std::memset(joint, 0, B * B * sizeof(uint64_t));
+        std::memset(pairCount, 0, B * sizeof(uint64_t));
+        std::memset(sumError, 0, B * sizeof(double));
+        std::memset(sumSquaredError, 0, B * sizeof(double));
+        *undefinedPairs = 0;
+        return EM2_OK;
+    }
+    cudaStream_t s = c.s;
+    // [joint B * B][undefined][Σe B][Σe² B], then the LUT and the signatures
+    std::vector<uint2> lut(lshCount + 1);
+    {
+        std::vector<double> table(lshCount + 1);
+        em2_similarity_table(lshCount, table.data());
+        for (uint64_t m = 0; m <= lshCount; m++) {
+            const float f = float(table[m]);
+            uint32_t bits;
+            std::memcpy(&bits, &f, 4);
+            const double t = std::floor((double(f) + 1.) * (0.5 * double(B)));
+            lut[m] = make_uint2(bits, t <= 0. ? 0u : t >= double(B - 1) ? uint32_t(B - 1) : uint32_t(t));
+        }
+    }
+    const size_t lutBytes = lut.size() * sizeof(uint2), sigBytes = N * W * sizeof(uint64_t);
+    void* x = nullptr;
+    EM2_TRY(reserve(ctx, em2_context::S_EXTEND, histBytes + sumBytes + lutBytes + sigBytes, &x));
+    auto* dHist = static_cast<unsigned long long*>(x);
+    auto* dSums = reinterpret_cast<double*>(dHist + B * B + 1);
+    auto* dLut = reinterpret_cast<uint2*>(dSums + 2 * B);
+    auto* dSig = reinterpret_cast<uint64_t*>(dLut + lut.size());
+    EM2_TRY(c.stage(toc, counts, 0));
+    EM2_TRY(c.input(dLut, lut.data(), lutBytes));
+    EM2_TRY(c.input(dSig, signatures, sigBytes));
+    EM2_CUDA(ctx, cudaMemsetAsync(dHist, 0, histBytes + sumBytes, s));
+    EM2_TRY(c.sums());
+    ExactOperands o;
+    EM2_TRY(c.operands(true, &o, false));       // no threshold: the candidate filter would reject nothing
+
+    // rows per chunk: under the budget for the widest window, and at most max(N / 8, 4096) -- the diagonal blocks are computed
+    // twice, about N * rows / 2 extra pairs
+    const double threshold = -HUGE_VAL;         // nothing passes it but NaN
+    const uint64_t ldFull = roundUp(N, 256), budget = exactMatrixBudget(ctx);
+    const uint64_t step = o.arith.general ? 2 : kXTile;
+    const uint64_t budgetRows = std::max<uint64_t>(step, budget / (ldFull * sizeof(float)) / step * step);
+    const bool symmetric = !o.arith.general && budgetRows >= N;
+    uint64_t chunkRows = symmetric ? N : std::min<uint64_t>(budgetRows, std::min(roundUp(N, step), std::max<uint64_t>(4096, roundUp((N + 7) / 8, step))));
+    GeneralMatrix gen{};
+    GemmMatrix gemm{};
+    if (o.arith.general) {
+        EM2_TRY(generalMatrix(ctx, o, chunkRows, &gen));
+        chunkRows = gen.maxRows;
+    } else {
+        EM2_TRY(gemmMatrix(ctx, o, &gemm));
+    }
+    const uint64_t capacity = chunkRows * ldFull;              // floats of the chunk buffer
+    void* simMatrix = nullptr;
+    EM2_TRY(reserve(ctx, em2_context::S_CAND, capacity * sizeof(float), &simMatrix));
+    float* sim = static_cast<float*>(simMatrix);
+
+    const bool lutShared = lutBytes <= 16384;
+    const size_t smemBin = size_t(kBinWarps) * (2 * B + 32) * sizeof(double) + size_t(kBinWarps) * 32 * (kSigTile + 1) * sizeof(uint64_t) +
+                           roundUp(B * B, 2) * sizeof(uint32_t) + (lutShared ? lutBytes : 0);
+    EM2_CUDA(ctx, cudaFuncSetAttribute(lshAnalysisKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smemBin)));
+    int perSm = 0;
+    EM2_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, lshAnalysisKernel, kBinWarps * 32, smemBin));
+    if (perSm < 1) return fail(ctx, EM2_ERR_CUDA, "no CTA of the LSH analysis kernel fits on this device");
+    double simMs = 0., binMs = 0.;
+    for (uint64_t r0 = 0; r0 < N;) {
+        const uint64_t colBegin = symmetric ? 0 : r0, ldOut = roundUp(N - colBegin, 256);
+        // a narrower window leaves room for more rows in the same buffer
+        const uint64_t fit = std::max<uint64_t>(step, capacity / ldOut / step * step);
+        const uint64_t rows = symmetric ? N : std::min(N - r0, o.arith.general ? std::min(fit, gen.maxRows) : fit);
+        const int m0 = c.T.mark();
+        if (o.arith.general)
+            EM2_TRY(generalChunk(ctx, o, gen, r0, rows, nullptr, colBegin, N, threshold, ldOut, sim, s));
+        else
+            EM2_TRY(gemmChunk(ctx, o, gemm, r0, rows, colBegin, N, ldOut, symmetric, threshold, sim, s));
+        const int m1 = c.T.mark();
+        const uint32_t roundsPerFlush = uint32_t(std::max<uint64_t>(1, 0xffffffffull / (uint64_t(kBinWarps) * (N - colBegin))));
+        const unsigned grid = unsigned(std::min<uint64_t>((rows + kBinWarps - 1) / kBinWarps, uint64_t(perSm) * ctx->smCount));
+        lshAnalysisKernel<<<grid, kBinWarps * 32, smemBin, s>>>(rows, r0, colBegin, N, ldOut, sim, dSig, uint32_t(W), dLut, uint32_t(lut.size()),
+                                                                lutShared, uint32_t(B), roundsPerFlush, dHist, dSums);
+        ctx->stats.kernel_launches++;
+        EM2_CUDA(ctx, cudaGetLastError());
+        const int m2 = c.T.mark();
+        EM2_CUDA(ctx, cudaStreamSynchronize(s));
+        simMs += c.T.ms(m0, m1);
+        binMs += c.T.ms(m1, m2);
+        c.T.next = m0;                          // the three events serve every chunk
+        r0 += rows;
+    }
+
+    const int e3 = c.T.mark();
+    EM2_TRY(c.output(joint, dHist, B * B * sizeof(uint64_t)));
+    EM2_TRY(c.output(undefinedPairs, dHist + B * B, sizeof(uint64_t)));
+    EM2_TRY(c.output(sumError, dSums, B * sizeof(double)));
+    EM2_TRY(c.output(sumSquaredError, dSums + B, B * sizeof(double)));
+    EM2_TRY(c.close(e3));
+    for (uint64_t b = 0; b < B; b++) {
+        uint64_t t = 0;
+        for (uint64_t j = 0; j < B; j++) t += joint[b * B + j];
+        pairCount[b] = t;
+    }
+    ctx->stats.scan_ms = simMs;
+    ctx->stats.finalize_ms = binMs;
+    return EM2_OK;
 }
 
 }  // extern "C"

@@ -5,7 +5,9 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <ctime>
+#include <fstream>
 #include <iostream>
 
 #include "Gpu.hpp"
@@ -387,4 +389,67 @@ void ExpressionMatrix::rescoreSimilarPairs(const std::string& name, const std::s
                   "em2_rescore_similar_pairs");
     });
     lastScanMs = gpu.stats().scan_ms;
+}
+
+ExpressionMatrix::LshAnalysis ExpressionMatrix::analyzeLsh(const std::string& geneSetName, const std::string& cellSetName, size_t lshCount,
+                                                        unsigned int seed, size_t binCount, const std::string& csvFileName)
+{
+    if (lshCount == 0 || lshCount > 65535) throw std::runtime_error("analyzeLsh: lshCount must be in [1, 65535] on the GPU path.");
+    if (binCount == 0 || binCount > 128) throw std::runtime_error("analyzeLsh: binCount must be in [1, 128].");
+    const GeneSet& geneSet = findGeneSet(geneSetName);
+    const CellSet& cellSet = findCellSet(cellSetName);
+    Gpu& gpu = Gpu::instance();            // throws without a device: before anything is written to the data directory
+
+    // the counts as findSimilarPairs0 builds them and the signatures as computeLshSignatures makes them, both temporary
+    ExpressionMatrixSubset subset(directoryName + "/tmp-ExpressionMatrixSubset-analyzeLsh", geneSet, cellSet, cellExpressionCounts);
+    Lsh lsh(directoryName + "/tmp-Lsh-analyzeLsh", subset, lshCount, seed);
+    lastSignatureMs = gpu.stats().signatures_ms;
+    LshAnalysis a;
+    a.binCount = binCount;
+    a.lshCount = lshCount;
+    a.pairCount.resize(binCount);
+    a.sumError.resize(binCount);
+    a.sumSquaredError.resize(binCount);
+    a.joint.resize(binCount * binCount);
+    try {
+        gpu.check(em2_analyze_lsh(gpu.context(), subset.cellCount(), subset.geneCount(), subset.toc(),
+                                  reinterpret_cast<const em2_count*>(subset.data()), lsh.getSignature(0).begin, lshCount, binCount,
+                                  a.pairCount.data(), a.sumError.data(), a.sumSquaredError.data(), a.joint.data(), &a.undefinedPairs),
+                  "em2_analyze_lsh");
+    } catch (...) {
+        lsh.remove();
+        throw;
+    }
+    lsh.remove();
+    lastScanMs = gpu.stats().scan_ms;
+    if (csvFileName.empty()) return a;
+
+    std::ofstream csv(csvFileName);
+    if (!csv) throw std::runtime_error("analyzeLsh: could not open " + csvFileName);
+    csv.precision(17);
+    const double B = double(binCount), L = double(lshCount), pi = std::acos(-1.);
+    const auto edge = [&](size_t b) { return -1. + 2. * double(b) / B; };
+    csv << "BinBegin,BinEnd,PairCount,MeanError,RmsError,TheoreticalSigma\n";
+    for (size_t b = 0; b < binCount; b++) {
+        const double s = -1. + (2. * double(b) + 1.) / B;          // the bin centre
+        const double p = 1. - std::acos(s) / pi;
+        const double sigma = pi * std::sqrt(1. - s * s) * std::sqrt(p * (1. - p) / L);
+        csv << edge(b) << ',' << edge(b + 1) << ',' << a.pairCount[b] << ',';
+        if (a.pairCount[b])
+            csv << a.sumError[b] / double(a.pairCount[b]) << ',' << std::sqrt(a.sumSquaredError[b] / double(a.pairCount[b]));
+        else
+            csv << "nan,nan";
+        csv << ',' << sigma << '\n';
+    }
+    // the joint histogram: one row per bin of r, one column per bin of s
+    csv << "\nBinBegin,BinEnd";
+    for (size_t j = 0; j < binCount; j++) csv << ",LshBin" << j;
+    csv << '\n';
+    for (size_t b = 0; b < binCount; b++) {
+        csv << edge(b) << ',' << edge(b + 1);
+        for (size_t j = 0; j < binCount; j++) csv << ',' << a.joint[b * binCount + j];
+        csv << '\n';
+    }
+    if (!csv) throw std::runtime_error("analyzeLsh: error writing " + csvFileName);
+    return a;
 }

@@ -83,6 +83,22 @@ public:
     void rescoreSimilarPairs(const std::string& similarPairsName, const std::string& newSimilarPairsName, size_t k,
                              double similarityThreshold);
 
+    // LSH accuracy on this gene set and cell set (what the reference's analyzeLsh diagnostic answers, not its output format):
+    // every cell pair a < b binned by its findSimilarPairs0 similarity r (no threshold) over binCount equal bins of [-1, 1],
+    // against the findSimilarPairs4 similarity s of the same pair with signatures of lshCount bits from `seed` (a temporary Lsh
+    // object, removed on every path).  Returns the bins (em2_analyze_lsh); with a csvFileName, also writes
+    // BinBegin,BinEnd,PairCount,MeanError,RmsError,TheoreticalSigma per bin (error = s - r, sigma = the reference's
+    // pi sin(theta) sqrt(p (1 - p) / L) at the bin centre, nan for bins without pairs) and then the joint histogram.
+    struct LshAnalysis {
+        size_t binCount = 0, lshCount = 0;
+        std::vector<uint64_t> pairCount;          // [binCount]
+        std::vector<double> sumError, sumSquaredError;
+        std::vector<uint64_t> joint;              // [binCount][binCount]: bin of r, bin of s
+        uint64_t undefinedPairs = 0;              // pairs with a cell of zero variance (r is NaN)
+    };
+    LshAnalysis analyzeLsh(const std::string& geneSetName, const std::string& cellSetName, size_t lshCount, unsigned int seed,
+                           size_t binCount, const std::string& csvFileName);
+
     // Scan variant for findSimilarPairs4 (em2_variant; 0 = automatic).
     int scanVariant = 0;
     // Device timings of the last hot-path call (milliseconds): signatures, scan.

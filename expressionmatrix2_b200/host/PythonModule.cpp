@@ -109,6 +109,24 @@ PYBIND11_MODULE(ExpressionMatrix2, module)
              "Rescores the lists of an existing SimilarPairs object with findSimilarPairs0's exact similarities: each cell keeps "
              "the k best of its listed cells above similarityThreshold.  The source object is not modified.",
              arg("similarPairsName"), arg("newSimilarPairsName"), arg("k") = 100, arg("similarityThreshold") = 0.2)
+        .def("analyzeLsh",
+             [](ExpressionMatrix& e, const std::string& geneSetName, const std::string& cellSetName, size_t lshCount, unsigned int seed,
+                size_t binCount, const std::string& csvFileName) {
+                 const ExpressionMatrix::LshAnalysis a = e.analyzeLsh(geneSetName, cellSetName, lshCount, seed, binCount, csvFileName);
+                 const size_t B = a.binCount;
+                 py::dict d;
+                 d["pair_count"] = py::array_t<uint64_t>(B, a.pairCount.data());
+                 d["sum_error"] = py::array_t<double>(B, a.sumError.data());
+                 d["sum_squared_error"] = py::array_t<double>(B, a.sumSquaredError.data());
+                 d["joint"] = py::array_t<uint64_t>({B, B}, a.joint.data());
+                 d["undefined_pairs"] = py::int_(a.undefinedPairs);
+                 return d;
+             },
+             "LSH accuracy: every cell pair binned by its findSimilarPairs0 similarity against its findSimilarPairs4 similarity "
+             "(pair counts, sums of the error and its square per bin, the joint histogram, pairs with an undefined similarity); "
+             "optionally written to a csv file.",
+             arg("geneSetName") = "AllGenes", arg("cellSetName") = "AllCells", arg("lshCount") = 1024, arg("seed") = 231,
+             arg("binCount") = 20, arg("csvFileName") = "")
         .def("computeLshSignatures", &ExpressionMatrix::computeLshSignatures, arg("geneSetName") = "AllGenes",
              arg("cellSetName") = "AllCells", arg("lshName"), arg("lshCount") = 1024, arg("seed") = 231)
         .def_readwrite("scanVariant", &ExpressionMatrix::scanVariant)

@@ -341,6 +341,29 @@ int em2_rescore_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t gen
                               const uint32_t* candidateCount, uint64_t k, double similarityThreshold,
                               em2_pair* pairs, uint32_t* usedCount);
 
+/* LSH accuracy on the caller's own data (the question behind every choice of lshCount and similarityThreshold, which the
+ * reference's analyzeLsh diagnostic answers): every unordered pair {a, b}, a < b, of the cellCount cells with
+ *   r = the float em2_exact_similar_pairs stores for b in row a, without a threshold (its arithmetic, decided from all cells'
+ *       counts with option "exact_general" honoured: symmetric on the integer path, row a's value on the general path), and
+ *   s = float(table[m]), m the Hamming distance of the two signatures, table = em2_similarity_table(lshCount): the float
+ *       em2_find_similar_pairs stores for the pair,
+ * binned by bin(x) = min(B - 1, max(0, floor((double(x) + 1) * (0.5 * B)))) in double, B = binCount equal bins over [-1, 1].
+ * Outputs (host buffers, all overwritten): pairCount[B] the pairs with bin(r) = b; sumError[B] / sumSquaredError[B] the sums of
+ * e and e^2 over them, e = double(s) - double(r), added in no particular order; joint[B][B] the pairs by (bin(r), bin(s));
+ * *undefinedPairs the pairs whose r is NaN (a cell of zero variance), which are in no bin.  All but the two sums are exact.
+ * signatures: uint64[cellCount*W] in the layout above (bits beyond lshCount zero), e.g. from em2_compute_signatures or an
+ * Lsh-<name> object.  Returns EM2_ERR_INVALID without writing any output if: a pointer is null, a size limit of
+ * em2_exact_similar_pairs fails (including a stored gene id >= geneCount), binCount is not in [1, 128], lshCount is not in
+ * [1, 65535], cellCount >= 2^29, or a signature has a bit set beyond lshCount.
+ * The similarity stage computes the upper triangle with the exact path's kernels: the whole-matrix symmetric GEMM when the
+ * N x N float matrix fits option "exact_matrix_bytes", else row chunks against the column window from their first row on; the
+ * general arithmetic evaluates every pair in full (no threshold, so no candidate filter: about as long as option
+ * "exact_filter" = 1, 12.2 s at 50k cells x 20k genes on a B200 at 1000 W).  Stats: h2d/d2h ms and bytes, sums_ms, scan_ms (the
+ * similarity stage), finalize_ms (the binning), total_ms, kernel_launches, variant_used as em2_exact_similar_pairs sets it. */
+int em2_analyze_lsh(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
+                    const uint64_t* signatures, uint64_t lshCount, uint64_t binCount, uint64_t* pairCount, double* sumError,
+                    double* sumSquaredError, uint64_t* joint, uint64_t* undefinedPairs);
+
 /* ------------------------------------------------------------------------------------------------
  * Device-resident calls: every pointer is a DEVICE pointer on the context's device, work is enqueued
  * on `stream` (a cudaStream_t passed as void*; NULL = legacy default stream) and the call returns
