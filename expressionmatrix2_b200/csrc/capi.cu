@@ -195,9 +195,39 @@ int guardDevice(em2_context* ctx)
     return EM2_OK;
 }
 
-void resetStats(em2_context* ctx)
+HostCall::HostCall(em2_context* c) : ctx(c), s(c->stream)
 {
     std::memset(&ctx->stats, 0, sizeof(ctx->stats));
+    t0 = nowMs();
+}
+
+int HostCall::mark()
+{
+    cudaEventRecord(ctx->ev[next], s);
+    return next++;
+}
+
+double HostCall::ms(int a, int b)
+{
+    float t = 0.f;
+    cudaEventElapsedTime(&t, ctx->ev[a], ctx->ev[b]);
+    return double(t);
+}
+
+int HostCall::close()
+{
+    EM2_CUDA(ctx, cudaStreamSynchronize(s));
+    ctx->stats.total_ms = nowMs() - t0;
+    return EM2_OK;
+}
+
+// anything the driver knows (pinned / registered host memory, managed or device memory) needs no staging
+static bool isPinned(const void* p)
+{
+    cudaPointerAttributes attr{};
+    const cudaError_t e = cudaPointerGetAttributes(&attr, p);
+    if (e != cudaSuccess) cudaGetLastError();
+    return e == cudaSuccess && attr.type != cudaMemoryTypeUnregistered;
 }
 
 // Host -> device copy of a caller's buffer.  Pinned (or registered) memory goes straight to the copy engine.  Pageable
@@ -217,13 +247,9 @@ static int ensureBounceBuffers(em2_context* ctx)
 int stageH2D(em2_context* ctx, void* dst, const void* src, size_t bytes, cudaStream_t s)
 {
     if (bytes == 0) return EM2_OK;
-    cudaPointerAttributes attr{};
-    const cudaError_t pe = cudaPointerGetAttributes(&attr, src);
-    if (pe != cudaSuccess) cudaGetLastError();
-    // anything the driver knows (pinned / registered host memory, managed or device memory) needs no staging
-    const bool pinned = pe == cudaSuccess && attr.type != cudaMemoryTypeUnregistered;
-    if (pinned || ctx->noBounce) {
+    if (isPinned(src) || ctx->noBounce) {
         EM2_CUDA(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDefault, s));
+        ctx->stats.h2d_bytes += bytes;
         return EM2_OK;
     }
     constexpr size_t kPiece = kBouncePiece;
@@ -234,6 +260,7 @@ int stageH2D(em2_context* ctx, void* dst, const void* src, size_t bytes, cudaStr
         copierOf(ctx)->copy(ctx->bounce[i], static_cast<const char*>(src) + off, n);
         EM2_CUDA(ctx, cudaMemcpyAsync(static_cast<char*>(dst) + off, ctx->bounce[i], n, cudaMemcpyHostToDevice, s));
         EM2_CUDA(ctx, cudaEventRecord(ctx->bounceFree[i], s));
+        ctx->stats.h2d_bytes += n;
         ctx->stats.bounced_bytes += n;
     }
     return EM2_OK;
@@ -243,13 +270,9 @@ int stageH2D(em2_context* ctx, void* dst, const void* src, size_t bytes, cudaStr
 int stageD2H(em2_context* ctx, void* dst, const void* src, size_t bytes, cudaStream_t s)
 {
     if (bytes == 0) return EM2_OK;
-    cudaPointerAttributes attr{};
-    const cudaError_t pe = cudaPointerGetAttributes(&attr, dst);
-    if (pe != cudaSuccess) cudaGetLastError();
-    // anything the driver knows (pinned / registered host memory, managed or device memory) needs no staging
-    const bool pinned = pe == cudaSuccess && attr.type != cudaMemoryTypeUnregistered;
-    if (pinned || ctx->noBounce) {
+    if (isPinned(dst) || ctx->noBounce) {
         EM2_CUDA(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDefault, s));
+        ctx->stats.d2h_bytes += bytes;
         return EM2_OK;
     }
     constexpr size_t kPiece = kBouncePiece;
@@ -269,6 +292,7 @@ int stageD2H(em2_context* ctx, void* dst, const void* src, size_t bytes, cudaStr
         EM2_CUDA(ctx, cudaEventRecord(ctx->bounceFree[i], s));
         pendingOff[i] = off;
         pendingBytes[i] = n;
+        ctx->stats.d2h_bytes += n;
         ctx->stats.bounced_bytes += n;
     }
     for (int j = 0; j < 2; j++, i ^= 1)
@@ -282,12 +306,18 @@ int stageD2H(em2_context* ctx, void* dst, const void* src, size_t bytes, cudaStr
 
 // Argument limits of every blocking entry point, checked BEFORE the first allocation or copy (sizes below are
 // computed from lshCount: 0 would underflow the word count).
+const char* scanArgumentError(uint64_t cellCount, uint64_t lshCount, uint64_t k)
+{
+    if (lshCount == 0 || lshCount > 65535) return "lshCount must be in [1, 65535]";
+    if (k == 0 || k > 1024) return "k must be in [1, 1024]";
+    if (cellCount > 0xfffffff0ull) return "cellCount exceeds the 32-bit CellId range";
+    return nullptr;
+}
+
 int checkScanArguments(em2_context* ctx, uint64_t cellCount, uint64_t lshCount, uint64_t k)
 {
-    if (lshCount == 0 || lshCount > 65535) return fail(ctx, EM2_ERR_INVALID, "lshCount must be in [1, 65535]");
-    if (k == 0 || k > 1024) return fail(ctx, EM2_ERR_INVALID, "k must be in [1, 1024]");
-    if (cellCount > 0xfffffff0ull) return fail(ctx, EM2_ERR_INVALID, "cellCount exceeds the 32-bit CellId range");
-    return EM2_OK;
+    const char* m = scanArgumentError(cellCount, lshCount, k);
+    return m ? fail(ctx, EM2_ERR_INVALID, m) : EM2_OK;
 }
 
 int readFlag(em2_context* ctx, const uint32_t* dFlag, cudaStream_t s, uint32_t* value)
@@ -340,8 +370,7 @@ int uploadLut(em2_context* ctx, uint64_t lshCount, float** dLut)
     for (uint64_t m = 0; m <= lshCount; m++) f[m] = float(t[m]);   // SimilarPairs stores float(similarity)
     void* d = nullptr;
     EM2_TRY(reserve(ctx, em2_context::S_LUT, (lshCount + 1) * sizeof(float), &d));
-    EM2_CUDA(ctx, cudaMemcpyAsync(d, f, (lshCount + 1) * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-    ctx->stats.h2d_bytes += (lshCount + 1) * sizeof(float);
+    EM2_TRY(stageH2D(ctx, d, f, (lshCount + 1) * sizeof(float), ctx->stream));
     *dLut = static_cast<float*>(d);
     return EM2_OK;
 }
@@ -601,10 +630,8 @@ int em2::signaturesOnDevice(em2_context* ctx, uint64_t cellCount, uint64_t geneC
         dU = const_cast<double*>(dUready);      // the hyperplanes are on the device already (multi-GPU: sharded copy + all-gather)
     } else {
         EM2_TRY(stageH2D(ctx, dU, U, geneCount * lshCount * sizeof(double), c));
-        ctx->stats.h2d_bytes += geneCount * lshCount * 8;
     }
     EM2_CUDA(ctx, cudaEventRecord(ev[1], c));
-    ctx->stats.h2d_bytes += (cellCount + 1) * 8 + nnz * 8;
 
     EM2_CUDA(ctx, cudaStreamWaitEvent(s, ev[1], 0));
     SignaturePlan plan;
@@ -648,10 +675,6 @@ int em2::signaturesOnDevice(em2_context* ctx, uint64_t cellCount, uint64_t geneC
     return EM2_OK;
 }
 
-extern "C" {
-
-}  // extern "C"
-
 int em2::fetchCounters(em2_context* ctx)
 {
     uint64_t h[8] = {};
@@ -664,33 +687,26 @@ int em2::fetchCounters(em2_context* ctx)
     return EM2_OK;
 }
 
-extern "C" {
-
-}  // extern "C"
-
-int em2::scanToHost(em2_context* ctx, StageTimer& T, const uint64_t* dSig, uint64_t cellCount, uint64_t lshCount,
-                      uint64_t rowBegin, uint64_t rowEnd, uint64_t k, double similarityThreshold, int variant,
-                      em2_pair* pairs, uint32_t* usedCount)
+int em2::HostCall::scan(const uint64_t* dSig, uint64_t cellCount, uint64_t lshCount, uint64_t rowBegin, uint64_t rowEnd, uint64_t k,
+                        double similarityThreshold, int variant, em2_pair* pairs, uint32_t* usedCount)
 {
     const uint64_t rows = rowEnd - rowBegin;
-    cudaStream_t s = ctx->stream;
     float* dLut = nullptr;
     EM2_TRY(uploadLut(ctx, lshCount, &dLut));
     const int64_t mismatchMax = em2_mismatch_max(lshCount, similarityThreshold);
     void *dPairs, *dUsed;
     EM2_TRY(reserve(ctx, em2_context::S_PAIRS, rows * k * sizeof(em2_pair), &dPairs));
     EM2_TRY(reserve(ctx, em2_context::S_USED, rows * sizeof(uint32_t), &dUsed));
-    const int e0 = T.mark();
+    const int e0 = mark();
     EM2_TRY(launchScanTopK(ctx, dSig, cellCount, lshCount, rowBegin, rowEnd, k, mismatchMax, dLut, variant,
                            static_cast<em2_pair*>(dPairs), static_cast<uint32_t*>(dUsed), s));
-    const int e1 = T.mark();
-    EM2_TRY(stageD2H(ctx, pairs, dPairs, rows * k * sizeof(em2_pair), s));
-    EM2_TRY(stageD2H(ctx, usedCount, dUsed, rows * sizeof(uint32_t), s));
-    const int e2 = T.mark();
+    const int e1 = mark();
+    EM2_TRY(output(pairs, dPairs, rows * k * sizeof(em2_pair)));
+    EM2_TRY(output(usedCount, dUsed, rows * sizeof(uint32_t)));
+    const int e2 = mark();
     EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    ctx->stats.d2h_bytes += rows * k * sizeof(em2_pair) + rows * sizeof(uint32_t);
-    ctx->stats.scan_ms += T.ms(e0, e1);
-    ctx->stats.d2h_ms += T.ms(e1, e2);
+    ctx->stats.scan_ms += ms(e0, e1);
+    ctx->stats.d2h_ms += ms(e1, e2);
     return EM2_OK;
 }
 
@@ -704,25 +720,19 @@ int em2_compute_signatures(em2_context* ctx, uint64_t cellCount, uint64_t geneCo
     if (!toc || !lshVectors || !signatures || (!counts && cellCount && toc[cellCount]))
         return fail(ctx, EM2_ERR_INVALID, "em2_compute_signatures: null pointer");
     EM2_TRY(checkScanArguments(ctx, cellCount, lshCount, 1));
-    resetStats(ctx);
-    const double t0 = nowMs();
+    HostCall c(ctx);
     if (cellCount == 0) return EM2_OK;
-    StageTimer T(ctx);
     uint64_t* dSig;
     double *dSum1, *dSum2;
     EM2_TRY(signaturesOnDevice(ctx, cellCount, geneCount, toc, counts, lshVectors, lshCount, &dSig, &dSum1, &dSum2));
-    const uint64_t W = wordCount(lshCount);
-    const int e0 = T.mark();
-    EM2_CUDA(ctx, cudaMemcpyAsync(signatures, dSig, cellCount * W * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    if (sum1) EM2_CUDA(ctx, cudaMemcpyAsync(sum1, dSum1, cellCount * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    if (sum2) EM2_CUDA(ctx, cudaMemcpyAsync(sum2, dSum2, cellCount * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    const int e1 = T.mark();
-    EM2_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    ctx->stats.d2h_ms += T.ms(e0, e1);
-    ctx->stats.d2h_bytes += cellCount * W * 8 + (sum1 ? cellCount * 8 : 0) + (sum2 ? cellCount * 8 : 0);
+    const int e0 = c.mark();
+    EM2_TRY(c.output(signatures, dSig, cellCount * wordCount(lshCount) * sizeof(uint64_t)));
+    if (sum1) EM2_TRY(c.output(sum1, dSum1, cellCount * sizeof(double)));
+    if (sum2) EM2_TRY(c.output(sum2, dSum2, cellCount * sizeof(double)));
+    const int e1 = c.mark();
     EM2_TRY(fetchCounters(ctx));
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
+    ctx->stats.d2h_ms += c.ms(e0, e1);
+    return c.close();
 }
 
 int em2_find_similar_pairs(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uint64_t lshCount,
@@ -733,25 +743,21 @@ int em2_find_similar_pairs(em2_context* ctx, const uint64_t* signatures, uint64_
     if (!signatures || !pairs || !usedCount) return fail(ctx, EM2_ERR_INVALID, "em2_find_similar_pairs: null pointer");
     if (rowEnd > cellCount || rowBegin > rowEnd) return fail(ctx, EM2_ERR_INVALID, "row range outside [0, cellCount]");
     EM2_TRY(checkScanArguments(ctx, cellCount, lshCount, k));
-    resetStats(ctx);
-    const double t0 = nowMs();
+    HostCall c(ctx);
     if (rowEnd == rowBegin) return EM2_OK;
-    StageTimer T(ctx);
     const uint64_t W = wordCount(lshCount);
     void *dSig, *dCounters;
     EM2_TRY(reserve(ctx, em2_context::S_SIG, cellCount * W * sizeof(uint64_t), &dSig));
     EM2_TRY(reserve(ctx, em2_context::S_COUNTERS, 64, &dCounters));
-    const int e0 = T.mark();
-    EM2_CUDA(ctx, cudaMemsetAsync(dCounters, 0, 64, ctx->stream));
-    EM2_CUDA(ctx, cudaMemcpyAsync(dSig, signatures, cellCount * W * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
-    const int e1 = T.mark();
-    ctx->stats.h2d_bytes += cellCount * W * 8;
-    EM2_TRY(scanToHost(ctx, T, static_cast<uint64_t*>(dSig), cellCount, lshCount, rowBegin, rowEnd, k,
-                       similarityThreshold, variant, pairs, usedCount));
-    ctx->stats.h2d_ms += T.ms(e0, e1);
+    const int e0 = c.mark();
+    EM2_CUDA(ctx, cudaMemsetAsync(dCounters, 0, 64, c.s));
+    EM2_TRY(c.input(dSig, signatures, cellCount * W * sizeof(uint64_t)));
+    const int e1 = c.mark();
+    EM2_TRY(c.scan(static_cast<uint64_t*>(dSig), cellCount, lshCount, rowBegin, rowEnd, k, similarityThreshold, variant, pairs,
+                   usedCount));
+    ctx->stats.h2d_ms += c.ms(e0, e1);
     EM2_TRY(fetchCounters(ctx));
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
+    return c.close();
 }
 
 int em2_lsh_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc,
@@ -763,31 +769,25 @@ int em2_lsh_similar_pairs(em2_context* ctx, uint64_t cellCount, uint64_t geneCou
     if (!toc || !lshVectors || !pairs || !usedCount || (!counts && cellCount && toc[cellCount]))
         return fail(ctx, EM2_ERR_INVALID, "em2_lsh_similar_pairs: null pointer");
     EM2_TRY(checkScanArguments(ctx, cellCount, lshCount, k));
-    resetStats(ctx);
-    const double t0 = nowMs();
+    HostCall c(ctx);
     if (cellCount == 0) return EM2_OK;
-    StageTimer T(ctx);
     uint64_t* dSig;
     double *dSum1, *dSum2;
     EM2_TRY(signaturesOnDevice(ctx, cellCount, geneCount, toc, counts, lshVectors, lshCount, &dSig, &dSum1, &dSum2));
-    if (signaturesOut) {
-        const uint64_t W = wordCount(lshCount);
-        EM2_CUDA(ctx, cudaMemcpyAsync(signaturesOut, dSig, cellCount * W * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-        ctx->stats.d2h_bytes += cellCount * W * 8;
-    }
-    EM2_TRY(scanToHost(ctx, T, dSig, cellCount, lshCount, 0, cellCount, k, similarityThreshold, variant, pairs, usedCount));
+    if (signaturesOut) EM2_TRY(c.output(signaturesOut, dSig, cellCount * wordCount(lshCount) * sizeof(uint64_t)));
+    EM2_TRY(c.scan(dSig, cellCount, lshCount, 0, cellCount, k, similarityThreshold, variant, pairs, usedCount));
     EM2_TRY(fetchCounters(ctx));
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
+    return c.close();
 }
 
 }  // extern "C"
 
-// Selected cells' rows -> device, then the subset kernels.  Leaves the local CSR in S_TOC / S_COUNTS.
-int em2::subsetOnDevice(em2_context* ctx, uint64_t globalCellCount, const uint64_t* globalToc, const em2_count* globalCounts,
-                          uint64_t globalGeneCount, const uint32_t* geneLocalId, uint64_t cellCount, const uint32_t* cellSet,
-                          uint64_t** dTocOut, em2_count** dCountsOut, uint64_t* nnzLocal)
+// Selected cells' rows -> device, then the subset kernels (h2d_ms).  Leaves the local CSR in S_TOC / S_COUNTS.
+int em2::subsetOnDevice(HostCall& c, uint64_t globalCellCount, const uint64_t* globalToc, const em2_count* globalCounts,
+                        uint64_t globalGeneCount, const uint32_t* geneLocalId, uint64_t cellCount, const uint32_t* cellSet,
+                        uint64_t** dTocOut, em2_count** dCountsOut, uint64_t* nnzLocal)
 {
+    em2_context* ctx = c.ctx;
     for (uint64_t i = 0; i < cellCount; i++) {
         if (cellSet[i] >= globalCellCount) return fail(ctx, EM2_ERR_INVALID, "cell set entry outside the expression matrix");
         if (i && cellSet[i] <= cellSet[i - 1]) return fail(ctx, EM2_ERR_INVALID, "Cell set is not sorted.");   // CZI_ASSERT, Subset.cpp:18
@@ -804,28 +804,24 @@ int em2::subsetOnDevice(em2_context* ctx, uint64_t globalCellCount, const uint64
     EM2_TRY(reserve(ctx, em2_context::S_GENEMAP, globalGeneCount * sizeof(uint32_t), &dMap));
     EM2_TRY(reserve(ctx, em2_context::S_TOC, (cellCount + 1) * sizeof(uint64_t), &dToc));
     EM2_TRY(reserve(ctx, em2_context::S_COUNTS, srcNnz * sizeof(em2_count), &dCounts));
-    cudaStream_t s = ctx->stream;
-    EM2_CUDA(ctx, cudaEventRecord(ctx->ev[14], s));
-    EM2_CUDA(ctx, cudaMemcpyAsync(dSrcToc, srcToc, (cellCount + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    EM2_TRY(stageH2D(ctx, dMap, geneLocalId, globalGeneCount * sizeof(uint32_t), s));
+    const int e0 = c.mark();
+    EM2_TRY(c.input(dSrcToc, srcToc, (cellCount + 1) * sizeof(uint64_t)));
+    EM2_TRY(c.input(dMap, geneLocalId, globalGeneCount * sizeof(uint32_t)));
     // runs of consecutive cells are contiguous in the global file: one copy per run
     for (uint64_t i = 0; i < cellCount;) {
         uint64_t j = i;
         while (j + 1 < cellCount && cellSet[j + 1] == cellSet[j] + 1) j++;
         const uint64_t b = globalToc[cellSet[i]], e = globalToc[cellSet[j] + 1];
-        if (e > b) EM2_TRY(stageH2D(ctx, static_cast<em2_count*>(dSrc) + srcToc[i], globalCounts + b, (e - b) * sizeof(em2_count), s));
+        if (e > b) EM2_TRY(c.input(static_cast<em2_count*>(dSrc) + srcToc[i], globalCounts + b, (e - b) * sizeof(em2_count)));
         i = j + 1;
     }
-    EM2_CUDA(ctx, cudaEventRecord(ctx->ev[15], s));
-    ctx->stats.h2d_bytes += (cellCount + 1) * 8 + globalGeneCount * 4 + srcNnz * 8;
+    const int e1 = c.mark();
     EM2_TRY(launchSubset(ctx, cellCount, static_cast<uint64_t*>(dSrcToc), static_cast<em2_count*>(dSrc),
                          static_cast<uint32_t*>(dMap), globalGeneCount, static_cast<uint64_t*>(dToc),
-                         static_cast<em2_count*>(dCounts), s));
-    EM2_CUDA(ctx, cudaMemcpyAsync(nnzLocal, static_cast<uint64_t*>(dToc) + cellCount, sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    float t = 0.f;
-    cudaEventElapsedTime(&t, ctx->ev[14], ctx->ev[15]);
-    ctx->stats.h2d_ms += double(t);
+                         static_cast<em2_count*>(dCounts), c.s));
+    EM2_CUDA(ctx, cudaMemcpyAsync(nnzLocal, static_cast<uint64_t*>(dToc) + cellCount, sizeof(uint64_t), cudaMemcpyDeviceToHost, c.s));
+    EM2_CUDA(ctx, cudaStreamSynchronize(c.s));
+    ctx->stats.h2d_ms += c.ms(e0, e1);
     *dTocOut = static_cast<uint64_t*>(dToc);
     *dCountsOut = static_cast<em2_count*>(dCounts);
     return EM2_OK;
@@ -841,30 +837,25 @@ int em2_subset(em2_context* ctx, uint64_t globalCellCount, const uint64_t* globa
     EM2_TRY(guardDevice(ctx));
     if (!globalToc || !geneLocalId || !localToc || !localNnz || (cellCount && !cellSet) || (!globalCounts && globalToc[globalCellCount]))
         return fail(ctx, EM2_ERR_INVALID, "em2_subset: null pointer");
-    resetStats(ctx);
-    const double t0 = nowMs();
+    HostCall c(ctx);
     uint64_t* dToc = nullptr;
     em2_count* dCounts = nullptr;
     uint64_t nnz = 0;
-    EM2_TRY(subsetOnDevice(ctx, globalCellCount, globalToc, globalCounts, globalGeneCount, geneLocalId, cellCount, cellSet,
-                           &dToc, &dCounts, &nnz));
+    EM2_TRY(subsetOnDevice(c, globalCellCount, globalToc, globalCounts, globalGeneCount, geneLocalId, cellCount, cellSet, &dToc,
+                           &dCounts, &nnz));
     *localNnz = nnz;
     if (nnz > localCapacity) return fail(ctx, EM2_ERR_INVALID, "em2_subset: localCounts capacity is smaller than the subset");
-    cudaStream_t s = ctx->stream;
-    EM2_CUDA(ctx, cudaMemcpyAsync(localToc, dToc, (cellCount + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
-    if (nnz && localCounts) EM2_CUDA(ctx, cudaMemcpyAsync(localCounts, dCounts, nnz * sizeof(em2_count), cudaMemcpyDeviceToHost, s));
-    ctx->stats.d2h_bytes += (cellCount + 1) * 8 + nnz * 8;
+    EM2_TRY(c.output(localToc, dToc, (cellCount + 1) * sizeof(uint64_t)));
+    if (localCounts) EM2_TRY(c.output(localCounts, dCounts, nnz * sizeof(em2_count)));
     if (sum1 && cellCount) {
         void *dSum1, *dSum2;
         EM2_TRY(reserve(ctx, em2_context::S_SUM1, cellCount * sizeof(double), &dSum1));
         EM2_TRY(reserve(ctx, em2_context::S_SUM2, cellCount * sizeof(double), &dSum2));
-        EM2_TRY(launchCellSums(ctx, cellCount, dToc, dCounts, static_cast<double*>(dSum1), static_cast<double*>(dSum2), s));
-        EM2_CUDA(ctx, cudaMemcpyAsync(sum1, dSum1, cellCount * sizeof(double), cudaMemcpyDeviceToHost, s));
-        if (sum2) EM2_CUDA(ctx, cudaMemcpyAsync(sum2, dSum2, cellCount * sizeof(double), cudaMemcpyDeviceToHost, s));
+        EM2_TRY(launchCellSums(ctx, cellCount, dToc, dCounts, static_cast<double*>(dSum1), static_cast<double*>(dSum2), c.s));
+        EM2_TRY(c.output(sum1, dSum1, cellCount * sizeof(double)));
+        if (sum2) EM2_TRY(c.output(sum2, dSum2, cellCount * sizeof(double)));
     }
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
+    return c.close();
 }
 
 int em2_lsh_similar_pairs_subset(em2_context* ctx, uint64_t globalCellCount, const uint64_t* globalToc,
@@ -877,11 +868,9 @@ int em2_lsh_similar_pairs_subset(em2_context* ctx, uint64_t globalCellCount, con
     if (!globalToc || !geneLocalId || !lshVectors || !pairs || !usedCount || (cellCount && !cellSet))
         return fail(ctx, EM2_ERR_INVALID, "em2_lsh_similar_pairs_subset: null pointer");
     EM2_TRY(checkScanArguments(ctx, cellCount, lshCount, k));
-    resetStats(ctx);
-    const double t0 = nowMs();
+    HostCall c(ctx);
     if (cellCount == 0) return EM2_OK;
-    StageTimer T(ctx);
-    cudaStream_t s = ctx->stream;
+    cudaStream_t s = c.s;
     const uint64_t W = wordCount(lshCount);
     void *dU, *dSum1, *dSum2, *dSig, *dCounters;
     EM2_TRY(reserve(ctx, em2_context::S_U, geneCount * lshCount * sizeof(double), &dU));
@@ -891,33 +880,27 @@ int em2_lsh_similar_pairs_subset(em2_context* ctx, uint64_t globalCellCount, con
     EM2_TRY(reserve(ctx, em2_context::S_COUNTERS, 64, &dCounters));
     EM2_CUDA(ctx, cudaMemsetAsync(dCounters, 0, 64, s));
     // hyperplanes ride on the copy stream while the subset is built
-    EM2_CUDA(ctx, cudaMemcpyAsync(dU, lshVectors, geneCount * lshCount * sizeof(double), cudaMemcpyHostToDevice, ctx->copyStream));
+    EM2_TRY(stageH2D(ctx, dU, lshVectors, geneCount * lshCount * sizeof(double), ctx->copyStream));
     EM2_CUDA(ctx, cudaEventRecord(ctx->ev[13], ctx->copyStream));
-    ctx->stats.h2d_bytes += geneCount * lshCount * 8;
     uint64_t* dToc = nullptr;
     em2_count* dCounts = nullptr;
     uint64_t nnz = 0;
-    EM2_TRY(subsetOnDevice(ctx, globalCellCount, globalToc, globalCounts, globalGeneCount, geneLocalId, cellCount, cellSet,
-                           &dToc, &dCounts, &nnz));
+    EM2_TRY(subsetOnDevice(c, globalCellCount, globalToc, globalCounts, globalGeneCount, geneLocalId, cellCount, cellSet, &dToc,
+                           &dCounts, &nnz));
     EM2_CUDA(ctx, cudaStreamWaitEvent(s, ctx->ev[13], 0));
-    const int e0 = T.mark();
+    const int e0 = c.mark();
     EM2_TRY(launchCellSums(ctx, cellCount, dToc, dCounts, static_cast<double*>(dSum1), static_cast<double*>(dSum2), s));
-    const int e1 = T.mark();
+    const int e1 = c.mark();
     EM2_TRY(launchSignatures(ctx, cellCount, geneCount, dToc, dCounts, static_cast<double*>(dSum1), static_cast<double*>(dSum2),
                              static_cast<double*>(dU), lshCount, lshCount, nnz, static_cast<uint64_t*>(dSig),
                              static_cast<uint64_t*>(dCounters), s));
-    const int e2 = T.mark();
-    if (signaturesOut) {
-        EM2_CUDA(ctx, cudaMemcpyAsync(signaturesOut, dSig, cellCount * W * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
-        ctx->stats.d2h_bytes += cellCount * W * 8;
-    }
-    EM2_TRY(scanToHost(ctx, T, static_cast<uint64_t*>(dSig), cellCount, lshCount, 0, cellCount, k, similarityThreshold, variant,
-                       pairs, usedCount));
-    ctx->stats.sums_ms += T.ms(e0, e1);
-    ctx->stats.signatures_ms += T.ms(e1, e2);
+    const int e2 = c.mark();
+    if (signaturesOut) EM2_TRY(c.output(signaturesOut, dSig, cellCount * W * sizeof(uint64_t)));
+    EM2_TRY(c.scan(static_cast<uint64_t*>(dSig), cellCount, lshCount, 0, cellCount, k, similarityThreshold, variant, pairs, usedCount));
+    ctx->stats.sums_ms += c.ms(e0, e1);
+    ctx->stats.signatures_ms += c.ms(e1, e2);
     EM2_TRY(fetchCounters(ctx));
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
+    return c.close();
 }
 
 int em2_cell_graph_edges(em2_context* ctx, uint64_t cellCount, uint64_t k, const em2_pair* pairs, const uint32_t* usedCount,
@@ -928,30 +911,22 @@ int em2_cell_graph_edges(em2_context* ctx, uint64_t cellCount, uint64_t k, const
     if (!edgeCount || (cellCount && (!pairs || !usedCount || !vertexOf)) || (capacity && !edges))
         return fail(ctx, EM2_ERR_INVALID, "em2_cell_graph_edges: null pointer");
     if (k == 0) return fail(ctx, EM2_ERR_INVALID, "em2_cell_graph_edges: k must be positive");
-    resetStats(ctx);
-    const double t0 = nowMs();
+    HostCall c(ctx);
     *edgeCount = 0;
     if (cellCount == 0) return EM2_OK;
-    cudaStream_t s = ctx->stream;
     void *dPairs, *dUsed, *dVertex, *dEdges;
     EM2_TRY(reserve(ctx, em2_context::S_PAIRS, cellCount * k * sizeof(em2_pair), &dPairs));
     EM2_TRY(reserve(ctx, em2_context::S_USED, cellCount * sizeof(uint32_t), &dUsed));
     EM2_TRY(reserve(ctx, em2_context::S_GENEMAP, cellCount * sizeof(uint32_t), &dVertex));
     EM2_TRY(reserve(ctx, em2_context::S_SRCCOUNTS, std::max<uint64_t>(capacity, 1) * sizeof(em2_edge), &dEdges));
-    EM2_CUDA(ctx, cudaMemcpyAsync(dPairs, pairs, cellCount * k * sizeof(em2_pair), cudaMemcpyHostToDevice, s));
-    EM2_CUDA(ctx, cudaMemcpyAsync(dUsed, usedCount, cellCount * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-    EM2_CUDA(ctx, cudaMemcpyAsync(dVertex, vertexOf, cellCount * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-    ctx->stats.h2d_bytes += cellCount * (k * 8 + 8);
+    EM2_TRY(c.input(dPairs, pairs, cellCount * k * sizeof(em2_pair)));
+    EM2_TRY(c.input(dUsed, usedCount, cellCount * sizeof(uint32_t)));
+    EM2_TRY(c.input(dVertex, vertexOf, cellCount * sizeof(uint32_t)));
     EM2_TRY(launchCellGraphEdges(ctx, cellCount, k, static_cast<em2_pair*>(dPairs), static_cast<uint32_t*>(dUsed),
                                  static_cast<uint32_t*>(dVertex), similarityThreshold, maxConnectivity,
-                                 static_cast<em2_edge*>(dEdges), capacity, edgeCount, s));
-    if (*edgeCount) {
-        EM2_CUDA(ctx, cudaMemcpyAsync(edges, dEdges, *edgeCount * sizeof(em2_edge), cudaMemcpyDeviceToHost, s));
-        ctx->stats.d2h_bytes += *edgeCount * sizeof(em2_edge);
-    }
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
+                                 static_cast<em2_edge*>(dEdges), capacity, edgeCount, c.s));
+    EM2_TRY(c.output(edges, dEdges, *edgeCount * sizeof(em2_edge)));
+    return c.close();
 }
 
 int em2_find_similar_pairs7(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uint64_t lshCount, uint64_t k,
@@ -961,18 +936,15 @@ int em2_find_similar_pairs7(em2_context* ctx, const uint64_t* signatures, uint64
     EM2_TRY(guardDevice(ctx));
     if (!lshSliceLengths || (cellCount && (!signatures || !pairs || !usedCount)))
         return fail(ctx, EM2_ERR_INVALID, "em2_find_similar_pairs7: null pointer");
-    if (lshCount == 0 || lshCount > 65535) return fail(ctx, EM2_ERR_INVALID, "lshCount must be in [1, 65535]");
-    if (k == 0 || k > 1024) return fail(ctx, EM2_ERR_INVALID, "k must be in [1, 1024]");
+    EM2_TRY(checkScanArguments(ctx, cellCount, lshCount, k));
     if (log2BucketCount == 0 || log2BucketCount > 32) return fail(ctx, EM2_ERR_INVALID, "log2BucketCount must be in [1, 32]");
-    if (cellCount > 0xfffffff0ull) return fail(ctx, EM2_ERR_INVALID, "cellCount exceeds the 32-bit CellId range");
     for (uint64_t i = 0; i < sliceLengthCount; i++) {
         // the reference's own checks (src/ExpressionMatrixLsh.cpp:552-564)
         if (i && lshSliceLengths[i] >= lshSliceLengths[i - 1]) return fail(ctx, EM2_ERR_INVALID, "The slice lengths are not in decreasing order.");
         if (lshSliceLengths[i] > 64) return fail(ctx, EM2_ERR_INVALID, "Each slice length can be at most 64 bits.");
         if (lshSliceLengths[i] < 1) return fail(ctx, EM2_ERR_INVALID, "Each slice length must be positive.");
     }
-    resetStats(ctx);
-    const double t0 = nowMs();
+    HostCall c(ctx);
     if (cellCount == 0) return EM2_OK;
     // Lsh::computeMismatchCountThresholdFromSimilarityThreshold (src/Lsh.hpp:86-95): (first m with table[m] < threshold) - 1
     std::vector<double> table(lshCount + 1);
@@ -985,7 +957,6 @@ int em2_find_similar_pairs7(em2_context* ctx, const uint64_t* signatures, uint64
         }
     if (first > lshCount) return fail(ctx, EM2_ERR_INVALID, "similarityThreshold is below every similarity (the reference asserts here)");
     const uint32_t mismatchThreshold = first == 0 ? 0xffffffffu : uint32_t(first - 1);
-    cudaStream_t s = ctx->stream;
     const uint64_t W = wordCount(lshCount);
     void *dSig, *dPairs, *dUsed;
     EM2_TRY(reserve(ctx, em2_context::S_SIG, cellCount * W * sizeof(uint64_t), &dSig));
@@ -993,17 +964,13 @@ int em2_find_similar_pairs7(em2_context* ctx, const uint64_t* signatures, uint64
     EM2_TRY(reserve(ctx, em2_context::S_USED, cellCount * sizeof(uint32_t), &dUsed));
     float* dLut = nullptr;
     EM2_TRY(uploadLut(ctx, lshCount, &dLut));
-    EM2_CUDA(ctx, cudaMemcpyAsync(dSig, signatures, cellCount * W * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    ctx->stats.h2d_bytes += cellCount * W * sizeof(uint64_t);
+    EM2_TRY(c.input(dSig, signatures, cellCount * W * sizeof(uint64_t)));
     EM2_TRY(launchBucketedSearch(ctx, static_cast<uint64_t*>(dSig), cellCount, lshCount, k, mismatchThreshold, dLut, lshSliceLengths,
                                  sliceLengthCount, maxCheck, uint32_t(log2BucketCount), static_cast<em2_pair*>(dPairs),
-                                 static_cast<uint32_t*>(dUsed), s));
-    EM2_CUDA(ctx, cudaMemcpyAsync(pairs, dPairs, cellCount * k * sizeof(em2_pair), cudaMemcpyDeviceToHost, s));
-    EM2_CUDA(ctx, cudaMemcpyAsync(usedCount, dUsed, cellCount * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    ctx->stats.d2h_bytes += cellCount * k * sizeof(em2_pair) + cellCount * sizeof(uint32_t);
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
+                                 static_cast<uint32_t*>(dUsed), c.s));
+    EM2_TRY(c.output(pairs, dPairs, cellCount * k * sizeof(em2_pair)));
+    EM2_TRY(c.output(usedCount, dUsed, cellCount * sizeof(uint32_t)));
+    return c.close();
 }
 
 int em2_signature_graph(em2_context* ctx, const uint64_t* signatures, uint64_t cellCount, uint64_t lshCount,
@@ -1013,14 +980,12 @@ int em2_signature_graph(em2_context* ctx, const uint64_t* signatures, uint64_t c
     EM2_TRY(guardDevice(ctx));
     if (!vertexCount || !edgeCount || !vertexOffsets || (cellCount && (!signatures || !cellOrder)) || (edgeCapacity && !edges))
         return fail(ctx, EM2_ERR_INVALID, "em2_signature_graph: null pointer");
-    if (lshCount == 0 || lshCount > 65535) return fail(ctx, EM2_ERR_INVALID, "em2_signature_graph: lshCount must be in [1, 65535]");
-    resetStats(ctx);
-    const double t0 = nowMs();
+    if (const char* m = scanArgumentError(0, lshCount, 1)) return fail(ctx, EM2_ERR_INVALID, std::string("em2_signature_graph: ") + m);
+    HostCall c(ctx);
     *vertexCount = 0;
     *edgeCount = 0;
     vertexOffsets[0] = 0;
     if (cellCount == 0) return EM2_OK;
-    cudaStream_t s = ctx->stream;
     const uint64_t W = wordCount(lshCount);
     const uint64_t vCap = std::min<uint64_t>(vertexCapacity, cellCount);
     void *dSig, *dOrder, *dOffsets, *dEdges;
@@ -1028,20 +993,15 @@ int em2_signature_graph(em2_context* ctx, const uint64_t* signatures, uint64_t c
     EM2_TRY(reserve(ctx, em2_context::S_USED, cellCount * sizeof(uint32_t), &dOrder));
     EM2_TRY(reserve(ctx, em2_context::S_SUM1, (cellCount + 1) * sizeof(uint64_t), &dOffsets));
     EM2_TRY(reserve(ctx, em2_context::S_SRCCOUNTS, std::max<uint64_t>(edgeCapacity, 1) * sizeof(em2_signature_edge), &dEdges));
-    EM2_CUDA(ctx, cudaMemcpyAsync(dSig, signatures, cellCount * W * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    ctx->stats.h2d_bytes += cellCount * W * sizeof(uint64_t);
+    EM2_TRY(c.input(dSig, signatures, cellCount * W * sizeof(uint64_t)));
     uint64_t kept = 0;
     EM2_TRY(launchSignatureGraph(ctx, static_cast<uint64_t*>(dSig), cellCount, lshCount, minCellCount, static_cast<uint32_t*>(dOrder),
                                  static_cast<uint64_t*>(dOffsets), vCap, vertexCount, &kept, static_cast<em2_signature_edge*>(dEdges),
-                                 edgeCapacity, edgeCount, s));
-    if (kept) EM2_CUDA(ctx, cudaMemcpyAsync(cellOrder, dOrder, kept * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    EM2_CUDA(ctx, cudaMemcpyAsync(vertexOffsets, dOffsets, (*vertexCount + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
-    if (*edgeCount)
-        EM2_CUDA(ctx, cudaMemcpyAsync(edges, dEdges, *edgeCount * sizeof(em2_signature_edge), cudaMemcpyDeviceToHost, s));
-    ctx->stats.d2h_bytes += kept * 4 + (*vertexCount + 1) * 8 + *edgeCount * sizeof(em2_signature_edge);
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
+                                 edgeCapacity, edgeCount, c.s));
+    EM2_TRY(c.output(cellOrder, dOrder, kept * sizeof(uint32_t)));
+    EM2_TRY(c.output(vertexOffsets, dOffsets, (*vertexCount + 1) * sizeof(uint64_t)));
+    EM2_TRY(c.output(edges, dEdges, *edgeCount * sizeof(em2_signature_edge)));
+    return c.close();
 }
 
 }  // extern "C"

@@ -131,32 +131,36 @@ int reservePinned(em2_context* ctx, int which, size_t bytes, void** out);
         if (rc__ != EM2_OK) return rc__; \
     } while (0)
 
-// events on the context stream, for the per-stage timings of em2_stats
-struct StageTimer {
-    em2_context* ctx;
-    int next = 0;
-    explicit StageTimer(em2_context* c) : ctx(c) {}
-    int mark()   // records an event on the context stream, returns its index
-    {
-        cudaEventRecord(ctx->ev[next], ctx->stream);
-        return next++;
-    }
-    double ms(int a, int b)
-    {
-        float t = 0.f;
-        cudaEventElapsedTime(&t, ctx->ev[a], ctx->ev[b]);
-        return double(t);
-    }
-};
-
 // ---- helpers of the blocking host-buffer calls (capi.cu), shared with the multi-GPU driver (multi.cu) ----------
 double nowMs();
 int guardDevice(em2_context* ctx);
-void resetStats(em2_context* ctx);
 int uploadLut(em2_context* ctx, uint64_t lshCount, float** dLut);
+// The limits of lshCount, k and cellCount of the LSH calls: the message of the first one violated, or null.
+const char* scanArgumentError(uint64_t cellCount, uint64_t lshCount, uint64_t k);
 int checkScanArguments(em2_context* ctx, uint64_t cellCount, uint64_t lshCount, uint64_t k);
+// Copies between a caller's host buffer and the device: pageable memory through the context's pinned bounce buffers, anything
+// else straight to the copy engine.  Each adds the bytes it queued to em2_stats (h2d_bytes / d2h_bytes, bounced_bytes).
 int stageH2D(em2_context* ctx, void* dst, const void* src, size_t bytes, cudaStream_t s);
 int stageD2H(em2_context* ctx, void* dst, const void* src, size_t bytes, cudaStream_t s);
+
+// One blocking call on the caller's host buffers (or one rank of an em2_multi call): the constructor resets em2_stats and
+// starts the clock of total_ms, input() / output() move a caller's buffer on the context stream, mark() / ms() time the
+// stages with the context's events, and close() waits for the stream and sets total_ms.
+struct HostCall {
+    em2_context* ctx;
+    cudaStream_t s;
+    double t0;
+    int next = 0;        // the event of ctx->ev that mark() records next
+    explicit HostCall(em2_context* c);
+    int mark();          // records an event on the context stream, returns its index
+    double ms(int a, int b);
+    int input(void* dst, const void* src, size_t bytes) { return stageH2D(ctx, dst, src, bytes, s); }
+    int output(void* dst, const void* src, size_t bytes) { return stageD2H(ctx, dst, src, bytes, s); }
+    // Lists of rows [rowBegin, rowEnd) of the signatures dSig on the device into the caller's pairs / usedCount (scan_ms, d2h_ms).
+    int scan(const uint64_t* dSig, uint64_t cellCount, uint64_t lshCount, uint64_t rowBegin, uint64_t rowEnd, uint64_t k,
+             double similarityThreshold, int variant, em2_pair* pairs, uint32_t* usedCount);
+    int close();
+};
 int fetchCounters(em2_context* ctx);
 // Reads one device flag word back through pinned[2] once everything before it on s is done.
 int readFlag(em2_context* ctx, const uint32_t* dFlag, cudaStream_t s, uint32_t* value);
@@ -177,12 +181,9 @@ std::string describeFlags(uint32_t flags, const char* source);
 int signaturesOnDevice(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, const uint64_t* toc, const em2_count* counts,
                        const double* U, uint64_t lshCount, uint64_t** dSigOut, double** dSum1Out, double** dSum2Out,
                        uint64_t sigTotalRows = 0, uint64_t sigRowOffset = 0, const double* dUready = nullptr);
-int subsetOnDevice(em2_context* ctx, uint64_t globalCellCount, const uint64_t* globalToc, const em2_count* globalCounts,
+int subsetOnDevice(HostCall& c, uint64_t globalCellCount, const uint64_t* globalToc, const em2_count* globalCounts,
                    uint64_t globalGeneCount, const uint32_t* geneLocalId, uint64_t cellCount, const uint32_t* cellSet,
                    uint64_t** dTocOut, em2_count** dCountsOut, uint64_t* nnzLocal);
-int scanToHost(em2_context* ctx, StageTimer& T, const uint64_t* dSig, uint64_t cellCount, uint64_t lshCount,
-               uint64_t rowBegin, uint64_t rowEnd, uint64_t k, double similarityThreshold, int variant,
-               em2_pair* pairs, uint32_t* usedCount);
 
 inline uint64_t wordCount(uint64_t lshCount) { return (lshCount - 1) / 64 + 1; }
 inline uint64_t roundUp(uint64_t x, uint64_t m) { return (x + m - 1) / m * m; }

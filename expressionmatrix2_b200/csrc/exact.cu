@@ -33,7 +33,7 @@
 // selection (exactFilterSelectKernel) and the exact decision on those candidates (exactRescoreKernel).  Rows with too many
 // candidates, and jobs the filter does not serve, are evaluated in full (exactFullRect).  DESIGN.md section 4.3d.
 //
-// The file ends with the exact path's four blocking calls, which share their host-side set-up (ExactCall):
+// The file ends with the exact path's four blocking calls, which share their host-side set-up (ExactCall, a HostCall):
 // em2_exact_similar_pairs (the full job), em2_extend_exact_similar_pairs (a job's lists extended to appended cells with the
 // same kernels), em2_rescore_similar_pairs (candidate lists rescored with the full job's similarities) and em2_analyze_lsh
 // (every pair's similarity against its LSH estimate, binned: lshAnalysisKernel on the chunks of the similarity matrix).
@@ -1583,15 +1583,10 @@ int exactRect(em2_context* ctx, const ExactOperands& o, uint64_t rowBegin, uint6
 
 int exactVariant(const ExactArith& arith) { return arith.general ? EM2_VARIANT_POPC : EM2_VARIANT_MMA_I8; }   // POPC: "not the tensor-core path"
 
-// One blocking call on host buffers: toc and counts staged into the context's scratch, the cell sums, the lists copied back,
-// and the stage timings and byte counts of em2_stats.  The constructor resets the stats; the call's own input lists go
-// through input() between stage() and sums().
-struct ExactCall {
-    em2_context* ctx;
-    cudaStream_t s;
-    StageTimer T;
+// One blocking call of the exact path: toc and counts staged into the context's scratch, the cell sums, the lists copied back,
+// and the stage timings of em2_stats.  The call's own input lists go through input() between stage() and sums().
+struct ExactCall : HostCall {
     uint64_t N, geneCount, k = 0;
-    double t0;
     int e0 = 0, e1 = 0, e2 = 0;
     uint64_t* toc = nullptr;     // device copies of the caller's cells, their sums, and the device side of the lists
     em2_count* counts = nullptr;
@@ -1599,11 +1594,7 @@ struct ExactCall {
     em2_pair* pairs = nullptr;
     uint32_t* used = nullptr;
 
-    ExactCall(em2_context* c, uint64_t cellCount, uint64_t genes) : ctx(c), s(c->stream), T(c), N(cellCount), geneCount(genes)
-    {
-        resetStats(ctx);
-        t0 = nowMs();
-    }
+    ExactCall(em2_context* c, uint64_t cellCount, uint64_t genes) : HostCall(c), N(cellCount), geneCount(genes) {}
 
     int stage(const uint64_t* hostToc, const em2_count* hostCounts, uint64_t listLength)
     {
@@ -1622,22 +1613,16 @@ struct ExactCall {
         sum2 = static_cast<double*>(dSum2);
         pairs = static_cast<em2_pair*>(dPairs);
         used = static_cast<uint32_t*>(dUsed);
-        e0 = T.mark();
+        e0 = mark();
         EM2_TRY(input(toc, hostToc, (N + 1) * sizeof(uint64_t)));
         return input(counts, hostCounts, nnz * sizeof(em2_count));
     }
 
-    int input(void* dst, const void* src, size_t bytes)
-    {
-        ctx->stats.h2d_bytes += bytes;
-        return stageH2D(ctx, dst, src, bytes, s);
-    }
-
     int sums()
     {
-        e1 = T.mark();
+        e1 = mark();
         EM2_TRY(launchCellSums(ctx, N, toc, counts, sum1, sum2, s));
-        e2 = T.mark();
+        e2 = mark();
         return EM2_OK;
     }
 
@@ -1653,31 +1638,24 @@ struct ExactCall {
         return EM2_OK;
     }
 
-    int output(void* dst, const void* src, size_t bytes)
-    {
-        ctx->stats.d2h_bytes += bytes;
-        return stageD2H(ctx, dst, src, bytes, s);
-    }
-
     // The end of a call whose outputs were queued with output() after event e3.
     int close(int e3)
     {
-        const int e4 = T.mark();
-        EM2_CUDA(ctx, cudaStreamSynchronize(s));
-        ctx->stats.h2d_ms = T.ms(e0, e1);
-        ctx->stats.sums_ms = T.ms(e1, e2);
-        ctx->stats.d2h_ms = T.ms(e3, e4);
-        ctx->stats.total_ms = nowMs() - t0;
+        const int e4 = mark();
+        EM2_TRY(HostCall::close());
+        ctx->stats.h2d_ms = ms(e0, e1);
+        ctx->stats.sums_ms = ms(e1, e2);
+        ctx->stats.d2h_ms = ms(e3, e4);
         return EM2_OK;
     }
 
     int finish(em2_pair* hostPairs, uint32_t* hostUsed)
     {
-        const int e3 = T.mark();
+        const int e3 = mark();
         EM2_TRY(output(hostPairs, pairs, N * k * sizeof(em2_pair)));
         EM2_TRY(output(hostUsed, used, N * sizeof(uint32_t)));
         EM2_TRY(close(e3));
-        ctx->stats.scan_ms = T.ms(e2, e3);
+        ctx->stats.scan_ms = ms(e2, e3);
         return EM2_OK;
     }
 };
@@ -1869,7 +1847,7 @@ int em2_analyze_lsh(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, co
         return fail(ctx, EM2_ERR_INVALID, "em2_analyze_lsh: null pointer");
     EM2_TRY(checkExactSize(ctx, N, geneCount));
     if (B == 0 || B > 128) return fail(ctx, EM2_ERR_INVALID, "em2_analyze_lsh: binCount must be in [1, 128]");
-    if (lshCount == 0 || lshCount > 65535) return fail(ctx, EM2_ERR_INVALID, "em2_analyze_lsh: lshCount must be in [1, 65535]");
+    if (const char* m = scanArgumentError(0, lshCount, 1)) return fail(ctx, EM2_ERR_INVALID, std::string("em2_analyze_lsh: ") + m);
     // a CTA's u32 histogram takes one round of kBinWarps rows of up to N pairs each between two flushes
     if (uint64_t(kBinWarps) * N > 0xffffffffull) return fail(ctx, EM2_ERR_INVALID, "em2_analyze_lsh: cellCount must be below 2^29");
     const uint64_t W = wordCount(lshCount);
@@ -1951,27 +1929,27 @@ int em2_analyze_lsh(em2_context* ctx, uint64_t cellCount, uint64_t geneCount, co
         // a narrower window leaves room for more rows in the same buffer
         const uint64_t fit = std::max<uint64_t>(step, capacity / ldOut / step * step);
         const uint64_t rows = symmetric ? N : std::min(N - r0, o.arith.general ? std::min(fit, gen.maxRows) : fit);
-        const int m0 = c.T.mark();
+        const int m0 = c.mark();
         if (o.arith.general)
             EM2_TRY(generalChunk(ctx, o, gen, r0, rows, nullptr, colBegin, N, threshold, ldOut, sim, s));
         else
             EM2_TRY(gemmChunk(ctx, o, gemm, r0, rows, colBegin, N, ldOut, symmetric, threshold, sim, s));
-        const int m1 = c.T.mark();
+        const int m1 = c.mark();
         const uint32_t roundsPerFlush = uint32_t(std::max<uint64_t>(1, 0xffffffffull / (uint64_t(kBinWarps) * (N - colBegin))));
         const unsigned grid = unsigned(std::min<uint64_t>((rows + kBinWarps - 1) / kBinWarps, uint64_t(perSm) * ctx->smCount));
         lshAnalysisKernel<<<grid, kBinWarps * 32, smemBin, s>>>(rows, r0, colBegin, N, ldOut, sim, dSig, uint32_t(W), dLut, uint32_t(lut.size()),
                                                                 lutShared, uint32_t(B), roundsPerFlush, dHist, dSums);
         ctx->stats.kernel_launches++;
         EM2_CUDA(ctx, cudaGetLastError());
-        const int m2 = c.T.mark();
+        const int m2 = c.mark();
         EM2_CUDA(ctx, cudaStreamSynchronize(s));
-        simMs += c.T.ms(m0, m1);
-        binMs += c.T.ms(m1, m2);
-        c.T.next = m0;                          // the three events serve every chunk
+        simMs += c.ms(m0, m1);
+        binMs += c.ms(m1, m2);
+        c.next = m0;                            // the three events serve every chunk
         r0 += rows;
     }
 
-    const int e3 = c.T.mark();
+    const int e3 = c.mark();
     EM2_TRY(c.output(joint, dHist, B * B * sizeof(uint64_t)));
     EM2_TRY(c.output(undefinedPairs, dHist + B * B, sizeof(uint64_t)));
     EM2_TRY(c.output(sumError, dSums, B * sizeof(double)));

@@ -88,11 +88,9 @@ int em2_extend_similar_pairs(em2_context* ctx, const uint64_t* signatures, uint6
     const size_t oldPairBytes = oldN * k * sizeof(em2_pair), oldUsedBytes = oldN * sizeof(uint32_t);
     if (outputsOverlap(pairs, pairBytes, usedCount, usedBytes, oldPairs, oldPairBytes, oldUsedCount, oldUsedBytes))
         return fail(ctx, EM2_ERR_INVALID, "em2_extend_similar_pairs: the output buffers overlap the old lists");
-    resetStats(ctx);
-    const double t0 = nowMs();
+    HostCall c(ctx);
     if (N == 0) return EM2_OK;
-    cudaStream_t s = ctx->stream;
-    StageTimer T(ctx);
+    cudaStream_t s = c.s;
     const uint64_t W = wordCount(lshCount);
     void *dSig, *dCounters, *dPairs, *dUsed;
     EM2_TRY(reserve(ctx, em2_context::S_SIG, N * W * sizeof(uint64_t), &dSig));
@@ -110,21 +108,20 @@ int em2_extend_similar_pairs(em2_context* ctx, const uint64_t* signatures, uint6
     auto* outPairs = static_cast<em2_pair*>(dPairs);
     auto* outUsed = static_cast<uint32_t*>(dUsed);
 
-    const int e0 = T.mark();
+    const int e0 = c.mark();
     EM2_CUDA(ctx, cudaMemsetAsync(dCounters, 0, 64, s));
     EM2_CUDA(ctx, cudaMemsetAsync(dFlags, 0, 16, s));
-    EM2_CUDA(ctx, cudaMemcpyAsync(dSig, signatures, N * W * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    EM2_TRY(stageH2D(ctx, dOldPairs, oldPairs, oldPairBytes, s));
-    EM2_TRY(stageH2D(ctx, dOldUsed, oldUsedCount, oldUsedBytes, s));
-    const int e1 = T.mark();
-    ctx->stats.h2d_bytes += N * W * 8 + oldPairBytes + oldUsedBytes;
+    EM2_TRY(c.input(dSig, signatures, N * W * sizeof(uint64_t)));
+    EM2_TRY(c.input(dOldPairs, oldPairs, oldPairBytes));
+    EM2_TRY(c.input(dOldUsed, oldUsedCount, oldUsedBytes));
+    const int e1 = c.mark();
     float* dLut = nullptr;
     EM2_TRY(uploadLut(ctx, lshCount, &dLut));
     const int64_t mismatchMax = em2_mismatch_max(lshCount, similarityThreshold);
     const uint32_t tau0 = scanTau0(mismatchMax, lshCount);
 
     // 1. the old lists against the signatures; nothing is written to the caller's buffers unless all of them hold
-    const int e2 = T.mark();
+    const int e2 = c.mark();
     if (oldN) {
         validateOldListsKernel<<<unsigned((oldN + kValidateWarps - 1) / kValidateWarps), kValidateWarps * 32, 0, s>>>(
             static_cast<const uint64_t*>(dSig), uint32_t(W), oldN, uint32_t(k), mismatchMax, tau0, dLut, dOldPairs, dOldUsed, dKeys,
@@ -157,19 +154,16 @@ int em2_extend_similar_pairs(em2_context* ctx, const uint64_t* signatures, uint6
                                    outUsed, s));
         }
     }
-    const int e3 = T.mark();
-    EM2_TRY(stageD2H(ctx, pairs, outPairs, pairBytes, s));
-    EM2_TRY(stageD2H(ctx, usedCount, outUsed, usedBytes, s));
-    const int e4 = T.mark();
-    EM2_CUDA(ctx, cudaStreamSynchronize(s));
-    ctx->stats.scan_symmetric = scanSymmetric;
-    ctx->stats.d2h_bytes += pairBytes + usedBytes;
-    ctx->stats.h2d_ms += T.ms(e0, e1);
-    ctx->stats.scan_ms += T.ms(e2, e3);
-    ctx->stats.d2h_ms += T.ms(e3, e4);
+    const int e3 = c.mark();
+    EM2_TRY(c.output(pairs, outPairs, pairBytes));
+    EM2_TRY(c.output(usedCount, outUsed, usedBytes));
+    const int e4 = c.mark();
     EM2_TRY(fetchCounters(ctx));
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
+    ctx->stats.scan_symmetric = scanSymmetric;
+    ctx->stats.h2d_ms += c.ms(e0, e1);
+    ctx->stats.scan_ms += c.ms(e2, e3);
+    ctx->stats.d2h_ms += c.ms(e3, e4);
+    return c.close();
 }
 
 }  // extern "C"

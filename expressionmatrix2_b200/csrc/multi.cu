@@ -249,7 +249,7 @@ int em2_scan_topk_dist_device(em2_context* ctx, const uint64_t* localSignatures,
 {
     EM2_TRY(guardDevice(ctx));
     if (!similarityTable || !pairs || !usedCount) return fail(ctx, EM2_ERR_INVALID, "em2_scan_topk_dist_device: null pointer");
-    if (lshCount == 0 || lshCount > 65535) return fail(ctx, EM2_ERR_INVALID, "lshCount must be in [1, 65535]");
+    if (const char* m = scanArgumentError(0, lshCount, 1)) return fail(ctx, EM2_ERR_INVALID, m);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const DistPartition part = distPartition(cellCount, ctx->world, ctx->rank);
     const uint64_t W = wordCount(lshCount);
@@ -404,10 +404,8 @@ int hyperplanesSharded(em2_context* ctx, const double* U, uint64_t geneCount, ui
     int rc = statusSoFar;
     if (rc == EM2_OK) rc = reserve(ctx, em2_context::S_U, rowsPer * P * lshCount * sizeof(double), &dU);
     const uint64_t b = std::min(geneCount, uint64_t(ctx->rank) * rowsPer), e = std::min(geneCount, b + rowsPer);
-    if (rc == EM2_OK && e > b) {
+    if (rc == EM2_OK && e > b)
         rc = stageH2D(ctx, static_cast<double*>(dU) + b * lshCount, U + b * lshCount, (e - b) * lshCount * sizeof(double), ctx->copyStream);
-        ctx->stats.h2d_bytes += (e - b) * lshCount * 8;
-    }
     EM2_TRY(distAgree(ctx, rc));
     EM2_TRY(distAllGather(ctx, dU, rowsPer * lshCount, sizeof(double), ctx->copyStream));
     *dUOut = static_cast<double*>(dU);
@@ -508,21 +506,20 @@ int em2_multi_get_stats(const em2_multi* mg, int index, em2_stats* stats)
 //
 // Every rank passes through the same agreement steps (distAgree) whatever its own status: signaturesFn takes the status
 // so far and must run its collectives' agreements even when it is a failure; distScanTopK holds the last one.
-using SignaturesFn = std::function<int(em2_context*, const DistPartition&, uint64_t**, int)>;
+using SignaturesFn = std::function<int(HostCall&, const DistPartition&, uint64_t**, int)>;
 
 static int multiRank(em2_multi* mg, int i, uint64_t cellCount, uint64_t lshCount, uint64_t k, double similarityThreshold,
                      int variant, em2_pair* pairs, uint32_t* usedCount, uint64_t* signaturesOut, const SignaturesFn& signaturesFn)
 {
     em2_context* ctx = mg->ctx[size_t(i)];
     const int rc0 = guardDevice(ctx);
-    resetStats(ctx);
-    const double t0 = nowMs();
+    HostCall c(ctx);
     const DistPartition part = distPartition(cellCount, ctx->world, ctx->rank);
     const uint64_t rows = part.rowEnd - part.rowBegin;
     const uint64_t W = wordCount(lshCount);
-    cudaStream_t s = ctx->stream;
+    cudaStream_t s = c.s;
     uint64_t* allSig = nullptr;
-    int rc = signaturesFn(ctx, part, &allSig, rc0);
+    int rc = signaturesFn(c, part, &allSig, rc0);
     float* dLut = nullptr;
     void *dPairs = nullptr, *dUsed = nullptr, *dCounters = nullptr;
     if (rc == EM2_OK) rc = uploadLut(ctx, lshCount, &dLut);
@@ -530,42 +527,29 @@ static int multiRank(em2_multi* mg, int i, uint64_t cellCount, uint64_t lshCount
     if (rc == EM2_OK) rc = reserve(ctx, em2_context::S_USED, std::max<uint64_t>(rows, 1) * sizeof(uint32_t), &dUsed);
     if (rc == EM2_OK) rc = reserve(ctx, em2_context::S_COUNTERS, 64, &dCounters);
     const int64_t mismatchMax = em2_mismatch_max(lshCount, similarityThreshold);
-    StageTimer T(ctx);
-    const int e0 = T.mark();
+    const int e0 = c.mark();
     EM2_TRY(distScanTopK(ctx, allSig, cellCount, lshCount, k, mismatchMax, dLut, variant, static_cast<em2_pair*>(dPairs),
                          static_cast<uint32_t*>(dUsed), s, rc));
-    const int e1 = T.mark();
-    if (rows) {
-        EM2_TRY(stageD2H(ctx, pairs + part.rowBegin * k, dPairs, rows * k * sizeof(em2_pair), s));
-        EM2_TRY(stageD2H(ctx, usedCount + part.rowBegin, dUsed, rows * sizeof(uint32_t), s));
-        ctx->stats.d2h_bytes += rows * k * sizeof(em2_pair) + rows * sizeof(uint32_t);
-        if (signaturesOut) {
-            EM2_TRY(stageD2H(ctx, signaturesOut + part.rowBegin * W, allSig + part.rowBegin * W, rows * W * sizeof(uint64_t), s));
-            ctx->stats.d2h_bytes += rows * W * 8;
-        }
-    }
-    const int e2 = T.mark();
+    const int e1 = c.mark();
+    EM2_TRY(c.output(pairs + part.rowBegin * k, dPairs, rows * k * sizeof(em2_pair)));
+    EM2_TRY(c.output(usedCount + part.rowBegin, dUsed, rows * sizeof(uint32_t)));
+    if (signaturesOut) EM2_TRY(c.output(signaturesOut + part.rowBegin * W, allSig + part.rowBegin * W, rows * W * sizeof(uint64_t)));
+    const int e2 = c.mark();
     EM2_CUDA(ctx, cudaStreamSynchronize(s));
     distCollectTimes(ctx);
-    ctx->stats.scan_ms += T.ms(e0, e1) - ctx->stats.allgather_ms;
-    ctx->stats.d2h_ms += T.ms(e1, e2);
+    ctx->stats.scan_ms += c.ms(e0, e1) - ctx->stats.allgather_ms;
+    ctx->stats.d2h_ms += c.ms(e1, e2);
     EM2_TRY(fetchCounters(ctx));
-    ctx->stats.total_ms = nowMs() - t0;
-    return EM2_OK;
+    return c.close();
 }
 
 static int multiCheck(em2_multi* mg, uint64_t cellCount, uint64_t lshCount, uint64_t k, const void* pairs, const void* usedCount)
 {
     if (!mg) return EM2_ERR_INVALID;
-    auto bad = [&](const char* m) {
-        mg->error = m;
-        return EM2_ERR_INVALID;
-    };
-    if (cellCount && (!pairs || !usedCount)) return bad("null output pointer");
-    if (lshCount == 0 || lshCount > 65535) return bad("lshCount must be in [1, 65535]");
-    if (k == 0 || k > 1024) return bad("k must be in [1, 1024]");
-    if (cellCount > 0xfffffff0ull) return bad("cellCount exceeds the 32-bit CellId range");
-    return EM2_OK;
+    const char* m = cellCount && (!pairs || !usedCount) ? "null output pointer" : scanArgumentError(cellCount, lshCount, k);
+    if (!m) return EM2_OK;
+    mg->error = m;
+    return EM2_ERR_INVALID;
 }
 
 int em2_multi_find_similar_pairs(em2_multi* mg, const uint64_t* signatures, uint64_t cellCount, uint64_t lshCount, uint64_t k,
@@ -578,7 +562,8 @@ int em2_multi_find_similar_pairs(em2_multi* mg, const uint64_t* signatures, uint
         return EM2_ERR_INVALID;
     }
     const uint64_t W = wordCount(lshCount);
-    auto sigFn = [&](em2_context* ctx, const DistPartition& part, uint64_t** allSig, int status) -> int {
+    auto sigFn = [&](HostCall& c, const DistPartition& part, uint64_t** allSig, int status) -> int {
+        em2_context* ctx = c.ctx;
         EM2_TRY(status);
         void* all = nullptr;
         EM2_TRY(reserve(ctx, em2_context::S_SIG, part.shard * uint64_t(ctx->world) * W * sizeof(uint64_t), &all));
@@ -587,11 +572,7 @@ int em2_multi_find_similar_pairs(em2_multi* mg, const uint64_t* signatures, uint
         EM2_TRY(reserve(ctx, em2_context::S_COUNTERS, 64, &dCounters));
         EM2_CUDA(ctx, cudaMemsetAsync(dCounters, 0, 64, ctx->stream));
         const uint64_t rows = part.rowEnd - part.rowBegin;
-        if (rows) {
-            EM2_TRY(stageH2D(ctx, *allSig + part.rowBegin * W, signatures + part.rowBegin * W, rows * W * sizeof(uint64_t), ctx->stream));
-            ctx->stats.h2d_bytes += rows * W * 8;
-        }
-        return EM2_OK;
+        return c.input(*allSig + part.rowBegin * W, signatures + part.rowBegin * W, rows * W * sizeof(uint64_t));
     };
     const int rc = runOnAll(mg, [&](int i) {
         return multiRank(mg, i, cellCount, lshCount, k, similarityThreshold, variant, pairs, usedCount, nullptr, sigFn);
@@ -612,7 +593,8 @@ int em2_multi_lsh_similar_pairs(em2_multi* mg, uint64_t cellCount, uint64_t gene
         return EM2_ERR_INVALID;
     }
     const uint64_t W = wordCount(lshCount);
-    auto sigFn = [&](em2_context* ctx, const DistPartition& part, uint64_t** allSig, int status) -> int {
+    auto sigFn = [&](HostCall& c, const DistPartition& part, uint64_t** allSig, int status) -> int {
+        em2_context* ctx = c.ctx;
         const uint64_t rows = part.rowEnd - part.rowBegin;
         double* dU = nullptr;
         // signaturesOnDevice orders its compute stream behind the copy stream's events, which follow the all-gather
@@ -654,9 +636,10 @@ int em2_multi_lsh_similar_pairs_subset(em2_multi* mg, uint64_t globalCellCount, 
         return EM2_ERR_INVALID;
     }
     const uint64_t W = wordCount(lshCount);
-    auto sigFn = [&](em2_context* ctx, const DistPartition& part, uint64_t** allSig, int status) -> int {
+    auto sigFn = [&](HostCall& c, const DistPartition& part, uint64_t** allSig, int status) -> int {
+        em2_context* ctx = c.ctx;
         const uint64_t rows = part.rowEnd - part.rowBegin;
-        cudaStream_t s = ctx->stream;
+        cudaStream_t s = c.s;
         double* dU = nullptr;
         if (ctx->world > 1) {
             EM2_TRY(hyperplanesSharded(ctx, lshVectors, geneCount, lshCount, &dU, status));
@@ -666,7 +649,6 @@ int em2_multi_lsh_similar_pairs_subset(em2_multi* mg, uint64_t globalCellCount, 
             EM2_TRY(reserve(ctx, em2_context::S_U, geneCount * lshCount * sizeof(double), &p));
             dU = static_cast<double*>(p);
             EM2_TRY(stageH2D(ctx, dU, lshVectors, geneCount * lshCount * sizeof(double), ctx->copyStream));
-            ctx->stats.h2d_bytes += geneCount * lshCount * 8;
         }
         EM2_CUDA(ctx, cudaEventRecord(ctx->ev[11], ctx->copyStream));
         void *all = nullptr, *dSum1 = nullptr, *dSum2 = nullptr, *dCounters = nullptr;
@@ -680,20 +662,18 @@ int em2_multi_lsh_similar_pairs_subset(em2_multi* mg, uint64_t globalCellCount, 
             uint64_t* dToc = nullptr;
             em2_count* dCounts = nullptr;
             uint64_t nnz = 0;
-            EM2_TRY(subsetOnDevice(ctx, globalCellCount, globalToc, globalCounts, globalGeneCount, geneLocalId, rows,
+            EM2_TRY(subsetOnDevice(c, globalCellCount, globalToc, globalCounts, globalGeneCount, geneLocalId, rows,
                                    cellSet + part.rowBegin, &dToc, &dCounts, &nnz));
             EM2_CUDA(ctx, cudaStreamWaitEvent(s, ctx->ev[11], 0));
-            StageTimer T(ctx);
-            T.next = 8;
-            const int a = T.mark();
+            const int a = c.mark();
             EM2_TRY(launchCellSums(ctx, rows, dToc, dCounts, static_cast<double*>(dSum1), static_cast<double*>(dSum2), s));
-            const int b = T.mark();
+            const int b = c.mark();
             EM2_TRY(launchSignatures(ctx, rows, geneCount, dToc, dCounts, static_cast<double*>(dSum1), static_cast<double*>(dSum2),
                                      dU, lshCount, lshCount, nnz, *allSig + part.rowBegin * W, static_cast<uint64_t*>(dCounters), s));
-            const int c = T.mark();
+            const int e = c.mark();
             EM2_CUDA(ctx, cudaStreamSynchronize(s));
-            ctx->stats.sums_ms += T.ms(a, b);
-            ctx->stats.signatures_ms += T.ms(b, c);
+            ctx->stats.sums_ms += c.ms(a, b);
+            ctx->stats.signatures_ms += c.ms(b, e);
         } else {
             EM2_CUDA(ctx, cudaStreamWaitEvent(s, ctx->ev[11], 0));
         }
